@@ -22,6 +22,8 @@ bench ray generators (qbvh.rs:949-986): uniform and axis-aligned sets, plus the 
 traversal orders, Mrays/s against the fetch roofline.
 
 All timing is on the device (CUDA events on the launching stream), max over ranks.  Rank 0 prints ONE JSON line.
+`--dump-outputs DIR` makes rank 0 write, after the timed steps, what the timed path computed in its last step as
+DIR/<name>.npy (see OutputDump), so that two builds run with the same arguments can be compared output for output.
 `--impl reference` times the CPU oracle -- our C++ restatement of the reference's renderer (the Rust original cannot
 be built here) -- on all host cores on bounded samples of the same workload.
 """
@@ -202,6 +204,40 @@ def load_pkg():
     pkg = importlib.import_module("yet-another-raytracer_b200")
     pkg.load_library()
     return pkg
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SWEEP_SAMPLE = 1 << 16  # rays per sweep row whose hits are written (a fixed, seeded sample of the 16 Mi)
+
+
+class OutputDump:
+    """--dump-outputs DIR: float32 / float64 arrays as DIR/<name>.npy, at most DUMP_MAX_BYTES in all.
+
+    render: `film` -- the (H, W, 3) f64 XYZ film the timed steps accumulated into, as the caller holds it after the last
+            step (with --total-spp: `rgba`, the (H, W, 4) finalised frame the last step read back); `last_step_counts` --
+            [rays, paths] of that step.
+    sweep:  `<mesh>_<rays>_<order>_hits` per row -- columns t, u, v, prim_id, obj_id, front_face of the hits the last
+            timed step wrote for the rays at `sweep_sample_index`; `david_uniform_near_f32_hits` -- t, u, v, prim_id of
+            yart_closest_hit_f32 on the same sample.  A miss is stored as the library returns it: t = +inf, ids MISS."""
+
+    def __init__(self, path):
+        self.dir = Path(path)
+        self.dir.mkdir(parents=True, exist_ok=True)
+        self.nbytes = 0
+
+    def write(self, name, array):
+        a = np.ascontiguousarray(array)
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError("%s: dumps are float32 or float64, not %s" % (name, a.dtype))
+        self.nbytes += a.nbytes
+        if self.nbytes > DUMP_MAX_BYTES:
+            raise RuntimeError("--dump-outputs: %s takes the dump past %d bytes" % (name, DUMP_MAX_BYTES))
+        np.save(self.dir / (name + ".npy"), a)
+
+
+def hit_columns(hits, fields=("t", "u", "v", "prim_id", "obj_id", "front_face")):
+    """Hit records -> (n, len(fields)) f64 (the u32 ids are exact in f64)."""
+    return np.stack([hits[f].astype(np.float64) for f in fields], axis=1)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -525,6 +561,14 @@ def run_render(args):
     rig.barrier()
     clocks = sampler.stop() if sampler else None
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:  # before the legs below reuse the film
+        dump = OutputDump(args.dump_outputs)
+        if strong_only:
+            dump.write("rgba", rgba_host.numpy().astype(np.float32))
+        else:
+            dump.write("film", film.cpu().numpy())
+        last = (r, p) if strong_only else (st.rays, st.paths)
+        dump.write("last_step_counts", np.array(last, dtype=np.float64))
 
     # ---- timed region 2: end to end through the C ABI with HOST buffers (`e2e`) ----
     K2 = min(K, 8)
@@ -676,6 +720,11 @@ def run_sweep(args):
     lo, hi = importlib.import_module("yet-another-raytracer_b200.sharding").shard_range(0, n, rank, N)
     table, headline = [], None
     d_hits = torch.empty((hi - lo) * 40, dtype=torch.uint8, device="cuda")
+    dump = OutputDump(args.dump_outputs) if args.dump_outputs and rank == 0 else None
+    if dump is not None:
+        sample = np.sort(np.random.default_rng(SEED).choice(hi - lo, min(DUMP_SWEEP_SAMPLE, hi - lo), replace=False))
+        dump.write("sweep_sample_index", sample.astype(np.float64))
+        d_sample = torch.from_numpy(sample).cuda()
     sampler = ClockSampler(rig.local) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -700,6 +749,9 @@ def run_sweep(args):
                     launches += st.kernel_launches
                 e1.record(rig.stream)
                 rig.barrier()
+                if dump is not None:
+                    got = d_hits.view(-1, 40)[d_sample].cpu().numpy().reshape(-1).view(pkg.HIT_DTYPE)
+                    dump.write("%s_%s_%s_hits" % (mesh_name, kind, oname), hit_columns(got))
                 (nodes, tris), (ms, kms) = rig.reduce_max_sum([stc.node_visits, stc.tri_tests], [e0.elapsed_time(e1), kernel_ms])
                 bpr = (NODE_BYTES * nodes + TRI_BYTES * tris) / n + SWEEP_STREAM_BYTES_PER_RAY
                 row = {"mesh": mesh_name, "rays": kind, "order": oname, "mrays_per_s": n * K / ms / 1e3,
@@ -721,6 +773,9 @@ def run_sweep(args):
                         ctx.closest_hit_f32_device(d_r32.data_ptr(), hi - lo, d_hits.data_ptr(), 0, 0.0, float("inf"), order)
                     f1.record(rig.stream)
                     rig.barrier()
+                    if dump is not None:
+                        got = d_hits[:(hi - lo) * 16].view(-1, 16)[d_sample].cpu().numpy().reshape(-1).view(pkg.abi.HIT_F32_DTYPE)
+                        dump.write("david_uniform_near_f32_hits", hit_columns(got, ("t", "u", "v", "prim_id")))
                     _, (fms,) = rig.reduce_max_sum([0.0], [f0.elapsed_time(f1)])
                     headline["f32_records_mrays_per_s"] = n * K / fms / 1e3
                     del d_r32
@@ -836,12 +891,17 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-time-to-image", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = (3 if args.total_spp else TOTAL_SPP // SPP_PER_STEP) if args.workload == "render" else 5
     if args.steps < 1:
         raise SystemExit("--steps must be >= 1")
     args.warmup = max(args.warmup, 0)
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("--dump-outputs: the reference arm sizes its steps from a timing probe, so its outputs differ "
+                         "from run to run")
     if args.impl == "reference":
         return run_reference(args)
     return run_sweep(args) if args.workload == "sweep" else run_render(args)

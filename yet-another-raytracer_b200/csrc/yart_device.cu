@@ -533,9 +533,6 @@ int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
       T.root = m.root;
       T.n_nodes = m.n_nodes;
       T.n_tris = m.n_tris;
-#ifdef YART_BOUNDS_CHECK
-      if (getenv("YART_FAULT_INJECT")) T.n_nodes = 1; // prove the checks are live (tests/test_gpu_bounds.py)
-#endif
       T.obj_index = i;
       T.wrap = o.wrap & (YART_WRAP_ROTATE_Y | YART_WRAP_TRANSLATE);
       T.refill_threshold = (uint32_t)std::max(1, std::min(32, rt));
