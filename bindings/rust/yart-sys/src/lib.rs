@@ -8,7 +8,7 @@
 #![allow(non_camel_case_types)]
 use std::os::raw::{c_char, c_int, c_void};
 
-pub const YART_ABI_VERSION: u32 = 1;
+pub const YART_ABI_VERSION: u32 = 2;
 pub const YART_OK: c_int = 0;
 pub const YART_ERR_INVALID: c_int = -1;
 pub const YART_ERR_CUDA: c_int = -2;
@@ -179,6 +179,10 @@ extern "C" {
                             order: u32, flags: u32, hits: *mut yart_hit, stats: *mut yart_stats) -> c_int;
     pub fn yart_closest_hit_f32(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray_f32, n: u64, t_min: f32, t_max: f32,
                                 order: u32, flags: u32, hits: *mut yart_hit_f32, stats: *mut yart_stats) -> c_int;
+    pub fn yart_occluded(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray, n: u64, t_min: f64, t_max: f64,
+                         flags: u32, occluded: *mut u8, stats: *mut yart_stats) -> c_int;
+    pub fn yart_occluded_f32(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray_f32, n: u64, t_min: f32, t_max: f32,
+                             flags: u32, occluded: *mut u8, stats: *mut yart_stats) -> c_int;
     pub fn yart_render(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts, film_xyz: *mut f64,
                        stats: *mut yart_stats) -> c_int;
     pub fn yart_film_finalize(ctx: *mut yart_ctx, film_xyz: *const f64, width: u32, height: u32, spp: u32, flags: u32,

@@ -64,6 +64,20 @@ impl GpuScene {
         }).collect())
     }
 
+    /// Batched occlusion query (`yart_occluded`): `true` where the ray hits anything of the world in (t_min, t_max) --
+    /// exactly where `hit_many` would return `Some` -- found with a traversal that stops at the first hit.  Shadow rays
+    /// toward a point q from p: direction q - p and a t_max just below 1.
+    pub fn occluded_many(&self, rays: &[Ray], t_min: f64, t_max: f64) -> Result<Vec<bool>> {
+        let raw: Vec<sys::yart_ray> = rays.iter().map(|r| sys::yart_ray { origin: r.origin, direction: r.direction }).collect();
+        let mut flags = vec![0u8; rays.len()];
+        let rc = unsafe {
+            sys::yart_occluded(self.ctx, sys::YART_TARGET_WORLD, raw.as_ptr(), raw.len() as u64, t_min, t_max, 0,
+                               flags.as_mut_ptr(), ptr::null_mut())
+        };
+        if rc != 0 { return Err(self.ctx_err(rc)); }
+        Ok(flags.iter().map(|&f| f != 0).collect())
+    }
+
     /// `Hittable::hit` for a single ray (hittable.rs:24) -- for drop-in tests; use `hit_many` for work.
     pub fn hit(&self, ray: &Ray, t_min: f64, t_max: f64) -> Option<Hit> {
         self.hit_many(std::slice::from_ref(ray), t_min, t_max).ok().and_then(|mut v| v.pop().flatten())

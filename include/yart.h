@@ -391,6 +391,23 @@ int yart_closest_hit_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* ray
                          float t_min, float t_max, uint32_t order, uint32_t flags,
                          yart_hit_f32* hits, yart_stats* stats /* may be NULL */);
 
+/* Batched occlusion query (Embree's rtcOccluded, an OptiX any-hit that terminates on the first hit): occluded[i] = 1
+ * if ray i hits anything of `target` (a mesh index or YART_TARGET_WORLD) that yart_closest_hit(..., YART_ORDER_REFERENCE,
+ * ...) would report with the same t_min / t_max, else 0 -- exactly, for every ray, with all the reference's quirks
+ * (flat leaves never entered, NaN slabs, the strict `t_max > t`, constant media drawing the same Philox numbers).
+ * The traversal stops at the first hit it finds; nothing but the flag is computed.  There is no order argument: the
+ * answer does not depend on the order the tree is walked in.  For shadow rays toward a point q from p, use the
+ * direction q - p and a t_max just below 1.
+ * flags: YART_FLAG_DEVICE_PTRS only (rays and occluded are then device arrays; rays aligned as for
+ * yart_closest_hit); any other bit is YART_ERR_INVALID.  Host arrays go through the same chunk pipeline as
+ * yart_closest_hit.  stats (may be NULL): rays, gpu_ms = trace_ms, kernel_launches = trace_launches; the visit
+ * counters stay 0. */
+int yart_occluded(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint64_t n, double t_min, double t_max,
+                  uint32_t flags, uint8_t* occluded, yart_stats* stats /* may be NULL */);
+/* The same on single-precision ray records, widened exactly as in yart_closest_hit_f32. */
+int yart_occluded_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* rays, uint64_t n, float t_min,
+                      float t_max, uint32_t flags, uint8_t* occluded, yart_stats* stats /* may be NULL */);
+
 /* Batched `render(config)` sample loop (main.rs:650-708) for samples
  * [sample_begin, sample_end): adds, per pixel and in sample order, the sanitised XYZ of each
  * sample (sanitize_sample_xyz main.rs:448-459) into film_xyz[height][width][3] (f64; host

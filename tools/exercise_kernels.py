@@ -22,6 +22,7 @@ for scene, w, h, spp in (("david", 48, 32, 2), ("cornell-box-smoke", 32, 32, 2),
     rays, _, _ = ctx.camera_rays(cam, w, h, 0, 1)
     for order in (0, 1):
         ctx.closest_hit(rays, y.TARGET_WORLD, 0.001, float("inf"), order, count_visits=True)
+    ctx.occluded(rays, y.TARGET_WORLD, 0.001, float("inf"))  # k_occlude + k_analytic_occluded
     print(scene, st.rays, int(rgba.sum()))
 p = y.ScenePreset("david"); ctx.set_scene(p)
 o, d = raysets.uniform(20000, [-60, 0, -90], [70, 200, 60])
@@ -30,12 +31,14 @@ weird = y.make_rays([(0, 0, 0), (0, 0, 5), (np.nan, 0, 0), (0, 0, 5)], [(0, 0, 0
 for r in (rays, weird, rays[:1], rays[:33]):
     for order in (0, 1):
         ctx.closest_hit(r, 0, 0.0, float("inf"), order)
+    ctx.occluded(r, 0, 0.0, float("inf"))
 # round-2 entry points: f32 records, sampling flags, path-ray dump, device films + a one-rank communicator
 r32 = np.empty(len(rays), dtype=y.abi.RAY_F32_DTYPE)
 r32["origin"], r32["direction"] = rays["origin"], rays["direction"]
 for order in (0, 1):
     ctx.closest_hit_f32(r32, 0, 0.0, float("inf"), order)
     ctx.closest_hit_f32(r32[:33], y.TARGET_WORLD, 0.001, float("inf"), order)
+ctx.occluded_f32(r32, 0, 0.0, float("inf"))
 cam = p.camera(48, 32)
 flags = y.FLAG_UNBIASED_LIGHT_PICK | y.FLAG_RUSSIAN_ROULETTE | y.FLAG_DEPTH_ZERO_BLACK
 ctx.render(cam, 48, 32, 0, 3, 50, 1, flags=flags)

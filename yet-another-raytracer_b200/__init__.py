@@ -88,6 +88,8 @@ def load_library():
         "yart_ctx_set_scene": (i32, [vp, P(abi.SceneDesc)]),
         "yart_closest_hit": (i32, [vp, u32, vp, u64, f64, f64, u32, u32, vp, P(abi.Stats)]),
         "yart_closest_hit_f32": (i32, [vp, u32, vp, u64, C.c_float, C.c_float, u32, u32, vp, P(abi.Stats)]),
+        "yart_occluded": (i32, [vp, u32, vp, u64, f64, f64, u32, vp, P(abi.Stats)]),
+        "yart_occluded_f32": (i32, [vp, u32, vp, u64, C.c_float, C.c_float, u32, vp, P(abi.Stats)]),
         "yart_render": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, P(abi.Stats)]),
         "yart_film_finalize": (i32, [vp, vp, u32, u32, u32, u32, vp]),
         "yart_generate_camera_rays": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, vp, vp]),
@@ -122,7 +124,7 @@ EXPORTED_SYMBOLS = [
     "yart_ctx_set_builder", "yart_measure_fetch_peak", "yart_comm_unique_id", "yart_comm_init_rank", "yart_comm_init",
     "yart_comm_destroy", "yart_comm_info", "yart_comm_last_error", "yart_film_reduce", "yart_film_create",
     "yart_film_clear", "yart_film_read", "yart_film_destroy", "yart_preset_note", "yart_closest_hit_f32",
-    "yart_dump_path_rays", "yart_host_register", "yart_host_unregister",
+    "yart_dump_path_rays", "yart_host_register", "yart_host_unregister", "yart_occluded", "yart_occluded_f32",
 ]
 
 
@@ -374,6 +376,47 @@ class Context:
         flags = FLAG_DEVICE_PTRS | (FLAG_COUNT_VISITS if count_visits else 0)
         self._check(_lib.yart_closest_hit(self._h, target, C.c_void_p(rays_ptr), n, t_min, t_max, order, flags,
                                           C.c_void_p(hits_ptr), C.byref(st)))
+        return st
+
+    def occluded(self, rays, target=TARGET_WORLD, t_min=0.001, t_max=float("inf"), out=None):
+        """Batched occlusion query (yart_occluded) with host buffers: (bool array, stats); True where the ray hits
+        anything in (t_min, t_max) -- exactly where closest_hit(..., ORDER_REFERENCE) reports a hit.  `out`: an
+        optional preallocated (e.g. pinned) uint8 array as long as rays."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        out = self._occluded_out(out, rays.shape[0])
+        st = abi.Stats()
+        self._check(_lib.yart_occluded(self._h, target, rays.ctypes.data, rays.shape[0], t_min, t_max, 0,
+                                       out.ctypes.data, C.byref(st)))
+        return out.view(np.bool_), st
+
+    def occluded_f32(self, rays, target=TARGET_WORLD, t_min=0.001, t_max=float("inf"), out=None):
+        """yart_occluded_f32 with host buffers: rays is an array of abi.RAY_F32_DTYPE."""
+        rays = np.ascontiguousarray(rays, dtype=abi.RAY_F32_DTYPE)
+        out = self._occluded_out(out, rays.shape[0])
+        st = abi.Stats()
+        self._check(_lib.yart_occluded_f32(self._h, target, rays.ctypes.data, rays.shape[0], t_min, t_max, 0,
+                                           out.ctypes.data, C.byref(st)))
+        return out.view(np.bool_), st
+
+    @staticmethod
+    def _occluded_out(out, n):
+        if out is None:
+            return np.empty(n, dtype=np.uint8)
+        if out.dtype != np.uint8 or out.shape != (n,) or not out.flags.c_contiguous:
+            raise ValueError("out must be a contiguous uint8 array as long as rays")
+        return out
+
+    def occluded_device(self, rays_ptr, n, out_ptr, target=TARGET_WORLD, t_min=0.001, t_max=float("inf")):
+        """Same with device pointers: rays (yart_ray records) and out (n bytes) on this context's GPU."""
+        st = abi.Stats()
+        self._check(_lib.yart_occluded(self._h, target, C.c_void_p(rays_ptr), n, t_min, t_max, FLAG_DEVICE_PTRS,
+                                       C.c_void_p(out_ptr), C.byref(st)))
+        return st
+
+    def occluded_f32_device(self, rays_ptr, n, out_ptr, target=TARGET_WORLD, t_min=0.001, t_max=float("inf")):
+        st = abi.Stats()
+        self._check(_lib.yart_occluded_f32(self._h, target, C.c_void_p(rays_ptr), n, t_min, t_max, FLAG_DEVICE_PTRS,
+                                           C.c_void_p(out_ptr), C.byref(st)))
         return st
 
     def _opts(self, width, height, sample_begin, sample_end, max_depth, seed, order, batch_spp, flags):

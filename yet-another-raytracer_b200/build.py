@@ -34,8 +34,8 @@ HOST_EXE = PKG / "yart"  # the native command-line host (host/yart_main.cpp): th
 OBJ_DIR = PKG / "build"
 
 SOURCES = ["host_obj.cpp", "host_qbvh.cpp", "host_presets.cpp", "host_api.cpp", "yart_device.cu", "device_trace_lean.cu",
-           "device_build.cu", "device_comm.cu"]
-HEADERS = ["host_common.h", "device_common.cuh", "device_trace.cuh", "device_shade.cuh", "device_build.h"]
+           "device_build.cu", "device_comm.cu", "device_occlude.cu"]
+HEADERS = ["host_common.h", "device_common.cuh", "device_trace.cuh", "device_shade.cuh", "device_build.h", "device_occlude.h"]
 INCLUDES = ["yart.h", "yart_rng.h", "yart_spectral_tables.h"]
 
 COMPILE_FLAGS = [

@@ -1,5 +1,5 @@
 // yart_device.cu -- the device half of the C ABI (include/yart.h): context, scene upload,
-// yart_closest_hit, yart_render, yart_film_finalize, yart_generate_camera_rays.
+// yart_closest_hit, yart_occluded, yart_render, yart_film_finalize, yart_generate_camera_rays.
 //
 // There is no CPU fallback anywhere in this file: every entry point launches the sm_100a
 // kernels of device_trace.cuh / device_shade.cuh or fails with YART_ERR_CUDA.
@@ -16,6 +16,7 @@
 
 #include "../../include/yart_spectral_tables.h"
 #include "device_build.h"
+#include "device_occlude.h"
 #include "device_shade.cuh"
 #include "host_common.h"
 
@@ -387,6 +388,7 @@ struct yart_ctx {
 
   // work buffers
   DevBuf rays, hits_export, time, wavelength, throughput, hits, queue_a, queue_b, counts, work, counters, film, rgba;
+  DevBuf occluded; // staging of yart_occluded's flags for host arrays
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> ev_pool;
   // host-buffer closest-hit queries: copy streams + events of the chunk pipeline (made on first use)
@@ -596,6 +598,173 @@ int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
   return YART_OK;
 }
 
+// What is the same for every pass of one occlusion query.
+struct OcclusionArgs {
+  OccludeCommon c;
+  const yart_object* d_objects;
+  const yart_object* h_objects;
+  uint32_t n_objects;
+  uint32_t pixel_base;
+  uint32_t* work_counters; // one zeroed u32 per mesh pass (at least n_objects)
+};
+
+// yart_occluded as passes over the rays in list order, like run_passes: one k_occlude per mesh instance, one
+// k_analytic_occluded per run of consecutive analytic objects.  c.occluded must be zeroed: a pass only ever writes 1,
+// and the passes after the first skip the rays already marked.  An empty world launches nothing.
+int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launches) {
+  static const int rt = tune_env("YART_TUNE_RT", 8), nt = tune_env("YART_TUNE_NT", 12);
+  static const int carve = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
+  // A closest-hit pass starts a ray that nothing has hit yet from t_max if it is the first mesh pass, and from
+  // fmin(+inf, t_max) otherwise (the recorded miss is +inf).  The two differ only for a NaN t_max.
+  const double t_max_later = std::fmin(INFINITY, q.c.t_max);
+  bool first = true;
+  uint32_t i = 0, n_trav = 0;
+  auto is_mesh = [&](uint32_t k) {
+    return q.h_objects[k].kind == YART_OBJ_MESH && !(q.h_objects[k].wrap & YART_WRAP_MEDIUM);
+  };
+  while (i < q.n_objects) {
+    if (is_mesh(i)) {
+      const yart_object& o = q.h_objects[i];
+      const DevMesh& m = ctx->h_meshes[o.index];
+      OccludeParams T;
+      memset(&T, 0, sizeof(T));
+      T.c = q.c;
+      T.c.first_pass = first ? 1u : 0u;
+      T.c.t_max = first ? q.c.t_max : t_max_later;
+      T.nodes = m.nodes;
+      T.tris = m.tris;
+      T.leafgeo = m.leafgeo;
+      T.root = m.root;
+      T.n_nodes = m.n_nodes;
+      T.n_tris = m.n_tris;
+      T.wrap = o.wrap & (YART_WRAP_ROTATE_Y | YART_WRAP_TRANSLATE);
+      T.refill_threshold = (uint32_t)std::max(1, std::min(32, rt));
+      T.node_threshold = (uint32_t)std::max(1, std::min(32, nt));
+      T.sin_theta = o.sin_theta;
+      T.cos_theta = o.cos_theta;
+      for (int k = 0; k < 3; ++k) T.offset[k] = o.offset[k];
+      for (int k = 0; k < 3; ++k) T.bound[k] = m.bound[k];
+      T.work_counter = q.work_counters + n_trav++;
+      const OccludeKernel k = yart::occlude_kernel(ctx->max_stack);
+      int& per_sm = ctx->traverse_blocks[(const void*)k]; // (occupancy query + carveout once per variant, as above)
+      if (per_sm == 0) {
+        cudaFuncSetAttribute(reinterpret_cast<const void*>(k), cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+        CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(k), kTraceThreads, 0));
+        per_sm = std::max(per_sm, 1);
+      }
+      k<<<per_sm * ctx->sm_count, kTraceThreads, 0, ctx->stream>>>(T); // persistent: one resident wave
+      i++;
+    } else {
+      uint32_t j = i;
+      while (j < q.n_objects && !is_mesh(j)) ++j;
+      AnalyticOccludedParams A;
+      memset(&A, 0, sizeof(A));
+      A.c = q.c;
+      A.c.first_pass = first ? 1u : 0u;
+      A.c.t_max = t_max_later;
+      A.scene = ctx->scene;
+      A.objects = q.d_objects;
+      A.obj_begin = i;
+      A.obj_end = j;
+      A.pixel_base = q.pixel_base;
+      A.media = ctx->has_media ? 1u : 0u;
+      yart::analytic_occluded_kernel()<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(A);
+      i = j;
+    }
+    first = false;
+    if (launches) (*launches)++;
+  }
+  CUDA_TRY(ctx, cudaGetLastError());
+  return YART_OK;
+}
+
+// One batched query over n rays.  Device arrays: run(0, n) once, between ctx->ev0 and ctx->ev1.  Host arrays: the
+// rays are uploaded into d_in and the results downloaded from d_out (staging buffers of at least n records) in chunks,
+// the upload of chunk i+1 and the download of chunk i-1 overlapping the kernels of chunk i on two copy streams (PCIe is
+// full duplex; the transfers, not the traversal, bound such a call: 88 B per closest hit against ~1.5 ns of kernel
+// time).  With pageable host memory the copies block the calling thread, so the kernels of a chunk are queued BEFORE
+// the next upload is issued; with pinned memory everything is asynchronous.
+// run(off, len) enqueues on ctx->stream the kernels that read the ray records at d_in + off * in_bytes and leave
+// out_bytes per ray at d_out + off * out_bytes.  Everything is enqueued on return; after a synchronisation of
+// ctx->stream, chunked_kernel_ms gives the kernels' time.
+template <class Run>
+int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* out, size_t out_bytes, uint64_t n,
+                const char* d_in, char* d_out, Run&& run, uint64_t* n_chunks_out) {
+  const int chunk_env = tune_env("YART_TUNE_HOST_CHUNK", 1 << 19); // (rays per chunk, read per call; 2^19 measured best: tools/host_chunk_probe.py)
+  const uint64_t chunk = dev ? n : (uint64_t)std::max(chunk_env, 1024);
+  const uint64_t n_chunks = (n + chunk - 1) / chunk;
+  *n_chunks_out = n_chunks;
+  char* stage_in = const_cast<char*>(d_in); // (host arrays: d_in is the context's staging buffer)
+  if (dev || n_chunks == 1) {
+    if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(stage_in, in, n * in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream)); // (stats->gpu_ms: the kernels, not the copies)
+    const int rc = run(0, n);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, n * out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  } else {
+    if (!ctx->copy_in) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking));
+    if (!ctx->copy_out) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking));
+    while (ctx->chunk_events.size() < 3 * n_chunks + 1) {
+      cudaEvent_t e;
+      CUDA_TRY(ctx, cudaEventCreate(&e));
+      ctx->chunk_events.push_back(e);
+    }
+    cudaEvent_t* up = ctx->chunk_events.data();                   // up[i]: chunk i is on the device
+    cudaEvent_t* done = ctx->chunk_events.data() + n_chunks;      // done[i]: chunk i's results are in d_out
+    cudaEvent_t* begun = ctx->chunk_events.data() + 2 * n_chunks; // begun[i]: chunk i's kernels start (its upload is in)
+    cudaEvent_t start = ctx->chunk_events[3 * n_chunks];
+    // (the device buffers may still be read by earlier work on the context's stream)
+    CUDA_TRY(ctx, cudaEventRecord(start, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_in, start, 0));
+    auto upload_chunk = [&](uint64_t i) -> int {
+      const uint64_t off = i * chunk, len = std::min(chunk, n - off);
+      CUDA_TRY(ctx, cudaMemcpyAsync(stage_in + off * in_bytes, static_cast<const char*>(in) + off * in_bytes,
+                                    len * in_bytes, cudaMemcpyHostToDevice, ctx->copy_in));
+      CUDA_TRY(ctx, cudaEventRecord(up[i], ctx->copy_in));
+      return YART_OK;
+    };
+    int rc = upload_chunk(0);
+    if (rc) return rc;
+    for (uint64_t i = 0; i < n_chunks; ++i) {
+      const uint64_t off = i * chunk, len = std::min(chunk, n - off);
+      CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, up[i], 0));
+      CUDA_TRY(ctx, cudaEventRecord(begun[i], ctx->stream));
+      if ((rc = run(off, len)) != YART_OK) break;
+      CUDA_TRY(ctx, cudaEventRecord(done[i], ctx->stream));
+      if (i + 1 < n_chunks && (rc = upload_chunk(i + 1)) != YART_OK) break;
+      CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_out, done[i], 0));
+      CUDA_TRY(ctx, cudaMemcpyAsync(static_cast<char*>(out) + off * out_bytes, d_out + off * out_bytes, len * out_bytes,
+                                    cudaMemcpyDeviceToHost, ctx->copy_out));
+    }
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    // nothing of this call may outlive it, error or not
+    cudaStreamSynchronize(ctx->copy_in);
+    cudaError_t ce = cudaStreamSynchronize(ctx->copy_out);
+    if (rc) {
+      cudaStreamSynchronize(ctx->stream);
+      return rc;
+    }
+    CUDA_TRY(ctx, ce);
+  }
+  return YART_OK;
+}
+
+// the kernels of a finished run_chunked call: ev0 -> ev1, or the chunks without the waits for their uploads in between
+int chunked_kernel_ms(yart_ctx* ctx, uint64_t n_chunks, bool dev, float* ms) {
+  *ms = 0.f;
+  if (dev || n_chunks == 1) {
+    CUDA_TRY(ctx, cudaEventElapsedTime(ms, ctx->ev0, ctx->ev1));
+  } else {
+    for (uint64_t i = 0; i < n_chunks; ++i) {
+      float part = 0.f;
+      CUDA_TRY(ctx, cudaEventElapsedTime(&part, ctx->chunk_events[2 * n_chunks + i], ctx->chunk_events[n_chunks + i]));
+      *ms += part;
+    }
+  }
+  return YART_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -661,7 +830,8 @@ void yart_ctx_destroy(yart_ctx* ctx) {
   cudaDeviceSynchronize();
   ctx->free_scene();
   DevBuf* bufs[] = {&ctx->rays, &ctx->hits_export, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits,
-                    &ctx->queue_a, &ctx->queue_b, &ctx->counts, &ctx->work, &ctx->counters, &ctx->film, &ctx->rgba};
+                    &ctx->queue_a, &ctx->queue_b, &ctx->counts, &ctx->work, &ctx->counters, &ctx->film, &ctx->rgba,
+                    &ctx->occluded};
   for (DevBuf* b : bufs) b->release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->chunk_events) cudaEventDestroy(e);
@@ -1178,79 +1348,16 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bo
     CUDA_TRY(ctx, cudaGetLastError());
     return YART_OK;
   };
-  // Host buffers: the arrays go through in chunks, the upload of chunk i+1 and the download of chunk i-1 overlapping the
-  // kernels of chunk i on two copy streams (PCIe is full duplex; the transfers, not the traversal, bound this call:
-  // 88 B per ray against ~1.5 ns of kernel time).  With pageable host memory the copies block the calling thread, so
-  // the kernels of a chunk are queued BEFORE the next upload is issued; with pinned memory everything is asynchronous.
-  const int chunk_env = tune_env("YART_TUNE_HOST_CHUNK", 1 << 19); // (rays per chunk, read per call; 2^19 measured best: tools/host_chunk_probe.py)
-  const uint64_t chunk = dev ? n : (uint64_t)std::max(chunk_env, 1024);
-  const uint64_t n_chunks = (n + chunk - 1) / chunk;
-  if (dev || n_chunks == 1) {
-    if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rays.p, rays, n * ray_bytes, cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream)); // (stats->gpu_ms: the kernels, not the copies)
-    const int rc = run_range(0, n);
-    if (rc) return rc;
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(hits, d_hits, n * hit_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  } else {
-    if (!ctx->copy_in) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking));
-    if (!ctx->copy_out) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking));
-    while (ctx->chunk_events.size() < 3 * n_chunks + 1) {
-      cudaEvent_t e;
-      CUDA_TRY(ctx, cudaEventCreate(&e));
-      ctx->chunk_events.push_back(e);
-    }
-    cudaEvent_t* up = ctx->chunk_events.data();                   // up[i]: chunk i is on the device
-    cudaEvent_t* done = ctx->chunk_events.data() + n_chunks;      // done[i]: chunk i's hits are exported
-    cudaEvent_t* begun = ctx->chunk_events.data() + 2 * n_chunks; // begun[i]: chunk i's kernels start (its upload is in)
-    cudaEvent_t start = ctx->chunk_events[3 * n_chunks];
-    // (the device buffers may still be read by earlier work on the context's stream)
-    CUDA_TRY(ctx, cudaEventRecord(start, ctx->stream));
-    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_in, start, 0));
-    auto upload_chunk = [&](uint64_t i) -> int {
-      const uint64_t off = i * chunk, len = std::min(chunk, n - off);
-      CUDA_TRY(ctx, cudaMemcpyAsync(ctx->rays.as<char>() + off * ray_bytes, static_cast<const char*>(rays) + off * ray_bytes,
-                                    len * ray_bytes, cudaMemcpyHostToDevice, ctx->copy_in));
-      CUDA_TRY(ctx, cudaEventRecord(up[i], ctx->copy_in));
-      return YART_OK;
-    };
-    int rc = upload_chunk(0);
-    if (rc) return rc;
-    for (uint64_t i = 0; i < n_chunks; ++i) {
-      const uint64_t off = i * chunk, len = std::min(chunk, n - off);
-      CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, up[i], 0));
-      CUDA_TRY(ctx, cudaEventRecord(begun[i], ctx->stream));
-      if ((rc = run_range(off, len)) != YART_OK) break;
-      CUDA_TRY(ctx, cudaEventRecord(done[i], ctx->stream));
-      if (i + 1 < n_chunks && (rc = upload_chunk(i + 1)) != YART_OK) break;
-      CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_out, done[i], 0));
-      CUDA_TRY(ctx, cudaMemcpyAsync(static_cast<char*>(hits) + off * hit_bytes, d_hits + off * hit_bytes, len * hit_bytes,
-                                    cudaMemcpyDeviceToHost, ctx->copy_out));
-    }
-    CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-    // nothing of this call may outlive it, error or not
-    cudaStreamSynchronize(ctx->copy_in);
-    cudaError_t ce = cudaStreamSynchronize(ctx->copy_out);
-    if (rc) {
-      cudaStreamSynchronize(ctx->stream);
-      return rc;
-    }
-    CUDA_TRY(ctx, ce);
-  }
+  uint64_t n_chunks = 0;
+  const int rc = run_chunked(ctx, dev, rays, ray_bytes, hits, hit_bytes, n, d_rays, d_hits, run_range, &n_chunks);
+  if (rc) return rc;
   unsigned long long c[2] = {0, 0};
   if (count) CUDA_TRY(ctx, cudaMemcpyAsync(c, ctx->counters.p, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   if (stats) {
     float ms = 0.f;
-    if (dev || n_chunks == 1) {
-      CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    } else { // the kernels of the chunks, without the waits for their uploads in between
-      for (uint64_t i = 0; i < n_chunks; ++i) {
-        float part = 0.f;
-        CUDA_TRY(ctx, cudaEventElapsedTime(&part, ctx->chunk_events[2 * n_chunks + i], ctx->chunk_events[n_chunks + i]));
-        ms += part;
-      }
-    }
+    const int erc = chunked_kernel_ms(ctx, n_chunks, dev, &ms);
+    if (erc) return erc;
     stats->rays = n;
     stats->node_visits = c[0];
     stats->tri_tests = c[1];
@@ -1276,6 +1383,111 @@ int yart_closest_hit_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* ray
   YART_ABI_GUARD_BEGIN
   return closest_hit_impl(ctx, target, rays, true, n, (double)t_min, (double)t_max, order, flags, hits, stats);
   YART_ABI_GUARD_END(ctx, "yart_closest_hit_f32")
+}
+
+static int occluded_impl(yart_ctx* ctx, uint32_t target, const void* rays, bool f32, uint64_t n, double t_min, double t_max,
+                         uint32_t flags, uint8_t* occluded, yart_stats* stats) {
+  const char* fn = f32 ? "yart_occluded_f32" : "yart_occluded";
+  if (!ctx->have_scene) {
+    ctx->err = std::string(fn) + ": no scene (call yart_ctx_set_scene first)";
+    return YART_ERR_INVALID;
+  }
+  if ((n && (!rays || !occluded)) || n > 0xFFFFFFF0ull) {
+    ctx->err = std::string(fn) + ": bad argument";
+    return YART_ERR_INVALID;
+  }
+  if (flags & ~(uint32_t)YART_FLAG_DEVICE_PTRS) {
+    ctx->err = std::string(fn) + ": the only flag it takes is YART_FLAG_DEVICE_PTRS";
+    return YART_ERR_INVALID;
+  }
+  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
+  if (dev && (reinterpret_cast<uintptr_t>(rays) & (f32 ? 7u : 15u))) {
+    ctx->err = std::string(fn) + (f32 ? ": device ray arrays must be 8-byte aligned" : ": device ray arrays must be 16-byte aligned");
+    return YART_ERR_INVALID;
+  }
+  if (target != YART_TARGET_WORLD && target >= ctx->n_meshes) {
+    ctx->err = std::string(fn) + ": target is neither a mesh index nor YART_TARGET_WORLD";
+    return YART_ERR_INVALID;
+  }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (stats) memset(stats, 0, sizeof(*stats));
+  if (n == 0) return YART_OK;
+  const size_t ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray);
+  const char* d_rays = static_cast<const char*>(rays);
+  char* d_out = reinterpret_cast<char*>(occluded);
+  if (!dev) { // (no export pass: the kernels write the flags straight into the staging buffer that is downloaded)
+    CUDA_TRY(ctx, ctx->rays.reserve(n * ray_bytes));
+    CUDA_TRY(ctx, ctx->occluded.reserve(n));
+    d_rays = ctx->rays.as<char>();
+    d_out = ctx->occluded.as<char>();
+  }
+  const uint32_t n_list = (target == YART_TARGET_WORLD) ? ctx->scene.n_objects : 1u;
+  const size_t work_bytes = ((size_t)n_list + 2) * sizeof(uint32_t);
+  CUDA_TRY(ctx, ctx->work.reserve(work_bytes));
+
+  yart_object solo;
+  memset(&solo, 0, sizeof(solo));
+  solo.kind = YART_OBJ_MESH;
+  solo.cos_theta = 1.0;
+  OcclusionArgs q;
+  memset(&q, 0, sizeof(q));
+  q.c.t_min = t_min;
+  q.c.t_max = t_max;
+  if (target == YART_TARGET_WORLD) {
+    q.d_objects = ctx->scene.objects;
+    q.h_objects = ctx->h_objects.data();
+    q.n_objects = ctx->scene.n_objects;
+  } else {
+    solo.index = target;
+    q.d_objects = ctx->d_solo + target;
+    q.h_objects = &solo;
+    q.n_objects = 1;
+  }
+  q.work_counters = ctx->work.as<uint32_t>();
+  uint64_t launches = 0;
+  // the passes over rays [off, off + len), on the context's stream
+  auto run_range = [&](uint64_t off, uint64_t len) -> int {
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, work_bytes, ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(d_out + off, 0, len, ctx->stream));
+    const char* r = d_rays + off * ray_bytes;
+    q.c.rays = f32 ? nullptr : reinterpret_cast<const yart_ray*>(r);
+    q.c.rays32 = f32 ? reinterpret_cast<const yart_ray_f32*>(r) : nullptr;
+    q.c.occluded = reinterpret_cast<uint8_t*>(d_out + off);
+    q.c.n_rays = (uint32_t)len;
+    q.pixel_base = (uint32_t)off; // (keeps a ray's Philox stream = its index in the caller's array)
+    return run_occlusion_passes(ctx, q, &launches);
+  };
+  uint64_t n_chunks = 0;
+  const int rc = run_chunked(ctx, dev, rays, ray_bytes, occluded, 1, n, d_rays, d_out, run_range, &n_chunks);
+  if (rc) return rc;
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (stats) {
+    float ms = 0.f;
+    const int erc = chunked_kernel_ms(ctx, n_chunks, dev, &ms);
+    if (erc) return erc;
+    stats->rays = n;
+    stats->kernel_launches = launches;
+    stats->trace_launches = (uint32_t)launches;
+    stats->gpu_ms = ms;
+    stats->trace_ms = ms;
+  }
+  return YART_OK;
+}
+
+int yart_occluded(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint64_t n, double t_min, double t_max,
+                  uint32_t flags, uint8_t* occluded, yart_stats* stats) {
+  if (!ctx) return YART_ERR_INVALID;
+  YART_ABI_GUARD_BEGIN
+  return occluded_impl(ctx, target, rays, false, n, t_min, t_max, flags, occluded, stats);
+  YART_ABI_GUARD_END(ctx, "yart_occluded")
+}
+
+int yart_occluded_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* rays, uint64_t n, float t_min, float t_max,
+                      uint32_t flags, uint8_t* occluded, yart_stats* stats) {
+  if (!ctx) return YART_ERR_INVALID;
+  YART_ABI_GUARD_BEGIN
+  return occluded_impl(ctx, target, rays, true, n, (double)t_min, (double)t_max, flags, occluded, stats);
+  YART_ABI_GUARD_END(ctx, "yart_occluded_f32")
 }
 
 static int fill_render_params(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, RenderParams& R) {
