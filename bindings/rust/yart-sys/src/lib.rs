@@ -48,6 +48,7 @@ pub const YART_FLAG_COUNT_VISITS: u32 = 2;
 pub const YART_FLAG_UNBIASED_LIGHT_PICK: u32 = 4;
 pub const YART_FLAG_RUSSIAN_ROULETTE: u32 = 8;
 pub const YART_FLAG_DEPTH_ZERO_BLACK: u32 = 16;
+pub const YART_FLAG_NEXT_EVENT: u32 = 32;
 pub const YART_COMM_ID_BYTES: usize = 128;
 pub const YART_BUILDER_HOST: u32 = 0;
 pub const YART_BUILDER_DEVICE: u32 = 1;

@@ -151,15 +151,17 @@ impl<'a, T> Drop for Pinned<'a, T> {
 }
 
 /// Better sampling switches of `yart_render_opts.flags` -- all off is the reference's estimator bit for bit
-/// (hittable.rs:113-122 light pick over len-1, main.rs:544-546 depth exhaustion = 1.0, no roulette).
+/// (hittable.rs:113-122 light pick over len-1, main.rs:544-546 depth exhaustion = 1.0, no roulette, no light sampling).
+/// `next_event` (next-event estimation with MIS) implies `unbiased_light_pick`.
 #[derive(Clone, Copy, Debug, Default)]
-pub struct Sampling { pub unbiased_light_pick: bool, pub russian_roulette: bool, pub depth_zero_black: bool }
+pub struct Sampling { pub unbiased_light_pick: bool, pub russian_roulette: bool, pub depth_zero_black: bool, pub next_event: bool }
 
 impl Sampling {
     fn bits(self) -> u32 {
         (if self.unbiased_light_pick { sys::YART_FLAG_UNBIASED_LIGHT_PICK } else { 0 })
             | (if self.russian_roulette { sys::YART_FLAG_RUSSIAN_ROULETTE } else { 0 })
             | (if self.depth_zero_black { sys::YART_FLAG_DEPTH_ZERO_BLACK } else { 0 })
+            | (if self.next_event { sys::YART_FLAG_NEXT_EVENT } else { 0 })
     }
 }
 

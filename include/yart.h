@@ -242,14 +242,26 @@ enum {
                                          averages over all of them (hittable.rs:113-122 vs :103-111)            */
   YART_FLAG_RUSSIAN_ROULETTE = 8u,    /* from bounce 4 on a path survives with probability clamp(throughput, 0.05, 1)
                                          and is reweighted by 1/q (unbiased; the reference has no roulette)      */
-  YART_FLAG_DEPTH_ZERO_BLACK = 16u    /* a path cut at max_depth contributes 0; the reference's ray_reflectance
+  YART_FLAG_DEPTH_ZERO_BLACK = 16u,   /* a path cut at max_depth contributes 0; the reference's ray_reflectance
                                          returns 1.0 at depth 0 (main.rs:544-546)                                */
+  YART_FLAG_NEXT_EVENT = 32u          /* next-event estimation with MIS (yart_render / yart_dump_path_rays only):
+                                         at every Lambertian hit before max_depth one extra direction is drawn
+                                         from the lights (uniform pick, YART_SLOT_NEE_*) and traced as a
+                                         closest-hit shadow ray; a front-facing DiffuseLight it hits adds its
+                                         emission with the power-heuristic weight p_l^2 / (p_l^2 + p_mix^2).
+                                         Emission that the mixture-sampled continuation reaches is weighted
+                                         p_mix^2 / (p_mix^2 + p_l^2) to match.  The path rays, and so
+                                         yart_dump_path_rays and stats.rays, are those of the flag-off render.
+                                         Implies YART_FLAG_UNBIASED_LIGHT_PICK (MIS needs the mixture's true
+                                         density).  Costs 76 more bytes of device state per path in flight. */
 };
 
 #define YART_TARGET_WORLD 0xFFFFFFFFu
 
 typedef struct yart_stats {
-  uint64_t rays;            /* closest-hit queries executed (1 ray = 1 world.hit, main.rs:548) */
+  uint64_t rays;            /* closest-hit queries executed (1 ray = 1 world.hit, main.rs:548); yart_render counts
+                               path rays only, not the shadow rays of YART_FLAG_NEXT_EVENT, whose passes are
+                               included in trace_ms, kernel_launches and trace_launches */
   uint64_t paths;           /* camera samples started                                           */
   uint64_t node_visits;     /* only with YART_FLAG_COUNT_VISITS                                 */
   uint64_t tri_tests;       /* only with YART_FLAG_COUNT_VISITS                                 */

@@ -33,6 +33,12 @@
 #define YART_SLOT_DIELECTRIC 2u    /* u0 = reflect-vs-refract draw (material.rs:274)                */
 #define YART_SLOT_RR 3u            /* u0 = Russian-roulette survival draw (only with YART_FLAG_RUSSIAN_ROULETTE;
                                       the reference has none)                                      */
+#define YART_SLOT_NEE_PICK 4u      /* u0 = which light the next-event sample aims at, floor(u0*len)
+                                      (only with YART_FLAG_NEXT_EVENT; the reference has none)      */
+#define YART_SLOT_NEE_DIR 5u       /* u0 = r1, u1 = r2 of that light's random() for the sample      */
+#define YART_NEE_BOUNCE_BASE 0x10000u /* the shadow ray of bounce k is a world.hit of its own: it draws
+                                      its ConstantMedium free paths at bounce YART_NEE_BOUNCE_BASE + k,
+                                      so they do not reuse (and correlate with) the path's draws at k */
 #define YART_RR_FIRST_BOUNCE 4u    /* roulette is played from this bounce on ...                    */
 #define YART_RR_MIN_SURVIVAL 0.05  /* ... with survival probability clamp(throughput, this, 1)      */
 #define YART_SLOT_SPHERE 0x100u    /* + 2*i, +2*i+1: i-th rejection iteration of

@@ -18,6 +18,7 @@ for scene, w, h, spp in (("david", 48, 32, 2), ("cornell-box-smoke", 32, 32, 2),
     ctx.set_scene(p)
     cam = p.camera(w, h)
     film, st = ctx.render(cam, w, h, 0, spp, 50, 1)
+    ctx.render(cam, w, h, 0, spp, 50, 1, flags=y.FLAG_NEXT_EVENT)
     rgba = ctx.film_finalize(film, spp)
     rays, _, _ = ctx.camera_rays(cam, w, h, 0, 1)
     for order in (0, 1):
@@ -42,6 +43,7 @@ ctx.occluded_f32(r32, 0, 0.0, float("inf"))
 cam = p.camera(48, 32)
 flags = y.FLAG_UNBIASED_LIGHT_PICK | y.FLAG_RUSSIAN_ROULETTE | y.FLAG_DEPTH_ZERO_BLACK
 ctx.render(cam, 48, 32, 0, 3, 50, 1, flags=flags)
+ctx.render(cam, 48, 32, 0, 3, 50, 1, flags=flags | y.FLAG_NEXT_EVENT)  # k_shade<true>, shadow passes, k_nee_resolve
 ctx.render(cam, 48, 32, 0, 3, 5, 1, batch_spp=2)
 dumped, n = ctx.dump_path_rays(cam, 48, 32, 0, 2, 1 << 16)
 assert n == len(dumped) > 48 * 32 * 2
@@ -77,6 +79,7 @@ for seed in range(6):
     for order in (0, 1):
         ctx.closest_hit(y.make_rays(o, d), y.TARGET_WORLD, 0.001, float("inf"), order, count_visits=bool(order))
     ctx.render(sc.camera(32, 24), 32, 24, 0, 3, 12, 1, flags=flags if seed % 2 else 0)
+    ctx.render(sc.camera(32, 24), 32, 24, 0, 3, 12, 1, flags=y.FLAG_NEXT_EVENT)
 for seed, n_tris in ((1, 6), (2, 33), (3, 1000)):
     pos, nrm, uv = fuzz_soup(seed, n_tris)
     desc, keep = soup_scene(pos, nrm, uv)

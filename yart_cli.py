@@ -5,7 +5,7 @@
                        [--max-depth D] [--vfov F] [--aperture A]            (reference flags)
                        [--seed S] [--order near|reference] [--device D] [--gpus N]   (additions)
                        [--preview-every N] [--checkpoint FILE] [--resume]    (additions)
-                       [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black]   (better sampling, off by default)
+                       [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event]   (better sampling, off by default)
 
 `--workers` is accepted for compatibility and ignored (the render runs on the GPU).  Option resolution
 follows resolve_render_options / resolve_dimensions (main.rs:166-209); the image is finalised exactly like
@@ -64,6 +64,9 @@ def build_parser(scene_names):
     ap.add_argument("--russian-roulette", action="store_true", dest="russian_roulette")
     ap.add_argument("--depth-zero-black", action="store_true", dest="depth_zero_black",
                     help="paths cut at --max-depth contribute 0 (the reference returns 1.0, main.rs:544-546)")
+    ap.add_argument("--next-event", action="store_true", dest="next_event",
+                    help="next-event estimation with MIS: one shadow ray toward a light per diffuse hit "
+                         "(implies --unbiased-light-pick)")
     ap.add_argument("--preview-every", type=positive_int, default=None, dest="preview_every",
                     help="write the image after every N samples per pixel")
     ap.add_argument("--checkpoint", default=None, help=".npz file holding the film and the samples done so far")
@@ -82,7 +85,7 @@ def _identity(args, o):
 def _flags(args):
     y = importlib.import_module("yet-another-raytracer_b200")
     return ((y.FLAG_UNBIASED_LIGHT_PICK if args.unbiased_light_pick else 0) | (y.FLAG_RUSSIAN_ROULETTE if args.russian_roulette else 0) |
-            (y.FLAG_DEPTH_ZERO_BLACK if args.depth_zero_black else 0))
+            (y.FLAG_DEPTH_ZERO_BLACK if args.depth_zero_black else 0) | (y.FLAG_NEXT_EVENT if args.next_event else 0))
 
 
 def save_checkpoint(path, film, done, ident):

@@ -18,7 +18,7 @@ from pathlib import Path
 import numpy as np
 
 from . import _abi as abi
-from ._abi import (FLAG_COUNT_VISITS, FLAG_DEPTH_ZERO_BLACK, FLAG_DEVICE_PTRS, FLAG_RUSSIAN_ROULETTE,
+from ._abi import (FLAG_COUNT_VISITS, FLAG_DEPTH_ZERO_BLACK, FLAG_DEVICE_PTRS, FLAG_NEXT_EVENT, FLAG_RUSSIAN_ROULETTE,
                    FLAG_UNBIASED_LIGHT_PICK, HIT_DTYPE, MISS, ORDER_NEAR, ORDER_REFERENCE, RAY_DTYPE, TARGET_WORLD,
                    make_rays)
 
@@ -472,16 +472,16 @@ class Context:
         return rays, wl, tm
 
     def dump_path_rays(self, camera, width, height, sample_begin, sample_end, cap, max_depth=50, seed=1, batch_spp=0,
-                       out_ptr=None):
+                       out_ptr=None, flags=0):
         """Every ray the renderer traces for these samples, in wavefront order (yart_dump_path_rays).  Returns
         (rays[:min(n, cap)], n) with host output, or n alone when out_ptr (a device pointer with room for cap) is given."""
         n = C.c_uint64()
         if out_ptr is not None:
-            o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, ORDER_NEAR, batch_spp, FLAG_DEVICE_PTRS)
+            o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, ORDER_NEAR, batch_spp, FLAG_DEVICE_PTRS | flags)
             self._check(_lib.yart_dump_path_rays(self._h, C.byref(camera), C.byref(o), C.c_void_p(out_ptr), cap, C.byref(n)))
             return int(n.value)
         rays = np.empty(cap, dtype=RAY_DTYPE)
-        o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, ORDER_NEAR, batch_spp, 0)
+        o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, ORDER_NEAR, batch_spp, flags)
         self._check(_lib.yart_dump_path_rays(self._h, C.byref(camera), C.byref(o), rays.ctypes.data, cap, C.byref(n)))
         return rays[:min(int(n.value), cap)], int(n.value)
 

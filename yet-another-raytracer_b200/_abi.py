@@ -19,6 +19,7 @@ NOISE_SQUARE, NOISE_TRILINEAR, NOISE_SMOOTH, NOISE_MARBLE, NOISE_NET = range(5)
 ORDER_REFERENCE, ORDER_NEAR = 0, 1
 FLAG_DEVICE_PTRS, FLAG_COUNT_VISITS = 1, 2
 FLAG_UNBIASED_LIGHT_PICK, FLAG_RUSSIAN_ROULETTE, FLAG_DEPTH_ZERO_BLACK = 4, 8, 16
+FLAG_NEXT_EVENT = 32
 TARGET_WORLD = 0xFFFFFFFF
 MISS = 0xFFFFFFFF
 

@@ -6,6 +6,8 @@
 // values that can differ from the CPU oracle are the last bits of libm-style functions
 // (sin, cos, log, acos, atan2, pow), whose CUDA implementations are not glibc's.
 #pragma once
+#include <type_traits>
+
 #include "device_trace.cuh"
 
 namespace yart {
@@ -432,6 +434,17 @@ struct PathState { // SoA over the paths of one batch, indexed by path id = pixe
   // path's own -- by then dead -- ray record: k_film_accumulate reads it from there.
 };
 
+// YART_FLAG_NEXT_EVENT only, indexed by path id like PathState.  The stage kernels take it as their LAST parameter
+// (null in the flag-off instances), so that the parameters before it keep their offsets there.
+struct NeeState {
+  yart_ray* rays;       // the shadow ray a Lambertian bounce aims at a light
+  double* pending;      // what that ray adds per unit of emission it finds: thr_in * atten * spdf / p_l * MIS weight
+  double* sum;          // light-sample contributions collected so far (added to the sample by k_film_accumulate)
+  double* w_emit;       // MIS weight of emission the path's current ray reaches (1 unless it left a Lambertian hit)
+  uint32_t* queue;      // the paths with a shadow ray this bounce
+  uint32_t* counts;     // counts[bounce]: length of that queue
+};
+
 struct RenderParams {
   DevScene scene;
   DevCamera cam;
@@ -443,7 +456,7 @@ struct RenderParams {
   // objects [tail_begin, tail_end) of the world list -- a trailing run of plain spheres -- are intersected by
   // k_shade itself (it has the ray and the hit in hand) instead of costing a pass over the queue
   uint32_t tail_begin, tail_end;
-  uint32_t flags; // YART_FLAG_UNBIASED_LIGHT_PICK | RUSSIAN_ROULETTE | DEPTH_ZERO_BLACK (all off = the reference)
+  uint32_t flags; // YART_FLAG_UNBIASED_LIGHT_PICK | RUSSIAN_ROULETTE | DEPTH_ZERO_BLACK | NEXT_EVENT (all off = the reference)
   uint64_t seed;
 };
 
@@ -487,7 +500,8 @@ YART_DEV void camera_sample(const DevCamera& c, const Rng& rng, uint32_t px, uin
   time = c.time0 + (c.time1 - c.time0) * ut;
 }
 
-__global__ void __launch_bounds__(256) k_raygen(const RenderParams R, uint32_t* queue, uint32_t* queue_count) {
+template <bool NEE>
+__global__ void __launch_bounds__(256) k_raygen(const RenderParams R, uint32_t* queue, uint32_t* queue_count, const NeeState N) {
   const uint64_t n = (uint64_t)R.n_pixels * R.spp_batch;
   const uint32_t lane = threadIdx.x & 31;
   for (uint64_t base = blockIdx.x * (uint64_t)blockDim.x; base < n; base += (uint64_t)gridDim.x * blockDim.x) {
@@ -506,10 +520,13 @@ __global__ void __launch_bounds__(256) k_raygen(const RenderParams R, uint32_t* 
         R.st.time[id] = time;
         R.st.wavelength[id] = wl;
         R.st.throughput[id] = 1.0;
+        if constexpr (NEE) N.w_emit[id] = 1.0;
         alive = true;
       } else { // outside the reference's 8x8 tiles (main.rs:643-646): never sampled
         store_sample(R.st.rays + id, 0.0, 0.0, 0.0);
+        if constexpr (NEE) R.st.wavelength[id] = 0.0; // (k_film_accumulate<true> reads it: outside the CIE table, weight 0)
       }
+      if constexpr (NEE) N.sum[id] = 0.0;
     }
     const uint32_t ballot = __ballot_sync(0xffffffffu, alive);
     if (ballot) {
@@ -548,7 +565,13 @@ __global__ void __launch_bounds__(256) k_camera_rays(const RenderParams R, yart_
 // One bounce of one path: everything k_shade does for path `id` except the compaction of the survivors.
 // Returns true when the path goes on (its next ray and throughput are stored), false when it ended (its sample
 // value is stored).
-YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
+// NEE (YART_FLAG_NEXT_EVENT): a Lambertian bounce before max_depth may also store a shadow ray and its pending weight;
+// the emission the path reaches is MIS-weighted, and an ended path stores the scalar thr * terminal instead of its
+// XYZ (k_film_accumulate<true> adds the light samples and applies the CIE weights).  Returns bit 0 = goes on,
+// bit 1 = has a shadow ray.  (No out-parameter: that perturbs the register allocation of the flag-off instance.)
+template <bool NEE>
+YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& R, const NeeState& N, uint32_t id, uint32_t bounce) {
+  bool shadow = false;
   const DevScene& S = R.scene;
   bool alive = false;
   const uint32_t pixel = R.pixel_base + id / R.spp_batch;
@@ -563,6 +586,7 @@ YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
   double terminal = 0.0;
   bool done = true;
   D3 next_d = d3(0, 0, 0), next_o = d3(0, 0, 0);
+  double w_next = 1.0; // (NEE) the MIS weight of emission next_d reaches: 1 unless this is a Lambertian bounce
   if (h.obj == YART_MISS) {
     terminal = rgb_reflect(S, S.background, wl); // main.rs:587
   } else {
@@ -573,6 +597,9 @@ YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
     if (mat.kind == YART_MAT_DIFFUSE_LIGHT) emitted = rec.front_face ? texture_value(S, mat.texture, wl, rec) : 0.0;
     if (mat.kind == YART_MAT_NONE || mat.kind == YART_MAT_DIFFUSE_LIGHT) {
       terminal = emitted;
+      if constexpr (NEE) {
+        if (emitted != 0.0) terminal = emitted * N.w_emit[id];
+      }
     } else if (mat.kind == YART_MAT_METAL) {
       D3 reflected = reflect(unit_vector(wd), rec.normal);
       next_d = reflected + mat.fuzz * random_in_unit_sphere(rng, bounce);
@@ -630,11 +657,34 @@ YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
       const double cos_pdf = cosv <= 0.0 ? 0.0 : cosv / kPi;
       const double p0 = have_lights ? lights_pdf_value(S, rec.p, dir) : cos_pdf;
       const double pdf_val = 0.5 * p0 + 0.5 * cos_pdf;
+      // the light sample pairs with the emission bounce+1 would collect: none at max_depth, whose next hit is never traced.
+      // (thr is still the throughput carried into this bounce here)
+      if constexpr (NEE) {
+        if (have_lights && bounce < R.max_depth) {
+          double u_light, unused, s1, s2;
+          rng_draw(rng, bounce, YART_SLOT_NEE_PICK, u_light, unused);
+          rng_draw(rng, bounce, YART_SLOT_NEE_DIR, s1, s2);
+          uint32_t k = (uint32_t)(u_light * (double)S.n_lights);
+          if (k > S.n_lights - 1) k = S.n_lights - 1;
+          const D3 dl = light_random(S.lights[k], rec.p, s1, s2);
+          const double p_l = lights_pdf_value(S, rec.p, dl);
+          const double cl = dot(unit_vector(dl), uvw.w);
+          const double p_m = 0.5 * p_l + 0.5 * (cl <= 0.0 ? 0.0 : cl / kPi);
+          const double csl = dot(rec.normal, unit_vector(dl));
+          const double spdf_l = csl < 0.0 ? 0.0 : csl / kPi;
+          if (isfinite(p_l) && p_l > 0.0 && spdf_l > 0.0) {
+            store_ray(N.rays + id, rec.p, dl);
+            N.pending[id] = thr * atten * spdf_l / p_l * (p_l * p_l / (p_l * p_l + p_m * p_m));
+            shadow = true;
+          }
+        }
+      }
       if (!isfinite(pdf_val) || pdf_val <= 0.0) {
         terminal = emitted;
       } else {
         const double cs = dot(rec.normal, unit_vector(dir));
         const double spdf = cs < 0.0 ? 0.0 : cs / kPi;
+        if constexpr (NEE) w_next = have_lights ? pdf_val * pdf_val / (pdf_val * pdf_val + p0 * p0) : 1.0;
         thr = thr * atten * spdf / pdf_val;
         next_o = rec.p;
         next_d = dir;
@@ -660,15 +710,21 @@ YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
   }
   if (done) {
     const double refl = thr * terminal;
-    double cie[3];
-    xyz_from_wavelength(S, wl, cie);
-    store_sample(R.st.rays + id, cie[0] * refl, cie[1] * refl, cie[2] * refl);
+    if constexpr (NEE) {
+      store_sample(R.st.rays + id, refl, 0.0, 0.0);
+    } else {
+      double cie[3];
+      xyz_from_wavelength(S, wl, cie);
+      store_sample(R.st.rays + id, cie[0] * refl, cie[1] * refl, cie[2] * refl);
+    }
   } else {
     store_ray(R.st.rays + id, next_o, next_d);
     R.st.throughput[id] = thr;
+    if constexpr (NEE) N.w_emit[id] = w_next;
     alive = true;
   }
-  return alive;
+  if constexpr (NEE) return (alive ? 1u : 0u) | (shadow ? 2u : 0u);
+  else return alive;
 }
 
 #ifndef YART_SHADE_THREADS
@@ -678,8 +734,24 @@ YART_DEV bool shade_path(const RenderParams& R, uint32_t id, uint32_t bounce) {
 #define YART_SHADE_MIN_BLOCKS (1024 / YART_SHADE_THREADS)
 #endif
 constexpr int kShadeThreads = YART_SHADE_THREADS;
+
+// append `id` to a queue when `take`: one atomic per warp
+YART_DEV void warp_append(bool take, uint32_t id, uint32_t* queue, uint32_t* count, uint32_t cap) {
+  const uint32_t lane = threadIdx.x & 31;
+  const uint32_t ballot = __ballot_sync(0xffffffffu, take);
+  if (ballot) {
+    uint32_t pos = 0;
+    const int leader = __ffs(ballot) - 1;
+    if ((int)lane == leader) pos = atomicAdd(count, (uint32_t)__popc(ballot));
+    pos = __shfl_sync(0xffffffffu, pos, leader);
+    YART_CHECK(pos + __popc(ballot) <= cap);
+    if (take) queue[pos + __popc(ballot & ((1u << lane) - 1u))] = id;
+  }
+}
+
+template <bool NEE>
 __global__ void __launch_bounds__(kShadeThreads, YART_SHADE_MIN_BLOCKS) k_shade(const RenderParams R, const uint32_t* queue, const uint32_t* queue_count,
-                                                uint32_t* next_queue, uint32_t* next_count, uint32_t bounce) {
+                                                uint32_t* next_queue, uint32_t* next_count, uint32_t bounce, const NeeState N) {
   const DevScene& S = R.scene;
   const uint32_t n = *queue_count;
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -745,12 +817,19 @@ __global__ void __launch_bounds__(kShadeThreads, YART_SHADE_MIN_BLOCKS) k_shade(
       __syncthreads();
     }
     const uint32_t item = base + threadIdx.x;
-    bool alive = false;
+    bool alive = false, shadow = false;
     uint32_t id = 0;
     if (item < n) {
       id = s_ids[threadIdx.x];
-      alive = shade_path(R, id, bounce);
+      if constexpr (NEE) {
+        const uint32_t r = shade_path<true>(R, N, id, bounce);
+        alive = (r & 1u) != 0;
+        shadow = (r & 2u) != 0;
+      } else {
+        alive = shade_path<false>(R, N, id, bounce);
+      }
     }
+    if constexpr (NEE) warp_append(shadow, id, N.queue, N.counts + bounce, R.n_pixels * R.spp_batch);
     // stream compaction: one atomic per warp
     const uint32_t ballot = __ballot_sync(0xffffffffu, alive);
     if (ballot) {
@@ -765,8 +844,39 @@ __global__ void __launch_bounds__(kShadeThreads, YART_SHADE_MIN_BLOCKS) k_shade(
   }
 }
 
+// YART_FLAG_NEXT_EVENT: the shadow rays of one bounce have been traced (closest hit in R.st.hits, as far as the passes
+// go); finish their world.hit with the trailing spheres k_shade folds in, and collect the emission of a front-facing
+// DiffuseLight.  A path may have ended in the same bounce: its light sample still counts.
+__global__ void __launch_bounds__(256) k_nee_resolve(const RenderParams R, uint32_t bounce, const NeeState N) {
+  const DevScene& S = R.scene;
+  const uint32_t n = N.counts[bounce];
+  for (uint32_t item = blockIdx.x * blockDim.x + threadIdx.x; item < n; item += gridDim.x * blockDim.x) {
+    const uint32_t id = N.queue[item];
+    YART_CHECK(id < R.n_pixels * R.spp_batch);
+    D3 wo, wd;
+    load_ray(N.rays + id, wo, wd);
+    DevHit h = R.st.hits[id];
+    for (uint32_t oi = R.tail_begin; oi < R.tail_end; ++oi) { // the same calls as k_shade's tail
+      const yart_object& so = S.objects[oi];
+      double t;
+      if (sphere_t(d3(so.p[0], so.p[1], so.p[2]), so.p[3], wo, wd, 0.001, h.t, t)) {
+        h.t = t; h.bu = 0.0; h.bv = 0.0; h.obj = oi; h.prim = 0;
+      }
+    }
+    if (h.obj == YART_MISS) continue;
+    YART_CHECK(h.obj < S.n_objects);
+    HitRec rec;
+    world_record(S, h, wo, wd, R.st.time[id], rec);
+    const yart_material& mat = S.materials[rec.material];
+    if (mat.kind != YART_MAT_DIFFUSE_LIGHT || !rec.front_face) continue;
+    N.sum[id] += N.pending[id] * texture_value(S, mat.texture, R.st.wavelength[id], rec);
+  }
+}
+
 // sanitize_sample_xyz (main.rs:448-459) + `pixel_color_xyz += sample` in sample order (main.rs:707)
-__global__ void __launch_bounds__(256) k_film_accumulate(const RenderParams R, double* film) {
+// NEE: the stored value is the scalar thr * terminal; the sample is cie(wl) * (that + the light samples' sum).
+template <bool NEE>
+__global__ void __launch_bounds__(256) k_film_accumulate(const RenderParams R, double* film, const NeeState N) {
   for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < R.n_pixels; p += gridDim.x * blockDim.x) {
     double* px = film + (size_t)(R.pixel_base + p) * 3;
     double ax = px[0], ay = px[1], az = px[2];
@@ -774,6 +884,13 @@ __global__ void __launch_bounds__(256) k_film_accumulate(const RenderParams R, d
     for (uint32_t s = 0; s < R.spp_batch; ++s) {
       double x, y, z;
       load_sample(c + s, x, y, z);
+      if constexpr (NEE) {
+        const size_t id = (size_t)p * R.spp_batch + s;
+        const double refl = x + N.sum[id];
+        double cie[3];
+        xyz_from_wavelength(R.scene, R.st.wavelength[id], cie);
+        x = cie[0] * refl; y = cie[1] * refl; z = cie[2] * refl;
+      }
       if (!isfinite(x) || !isfinite(y) || !isfinite(z)) {
         x = y = z = 0.0;
       } else if (!(y <= 0.0 || y <= 20.0)) {

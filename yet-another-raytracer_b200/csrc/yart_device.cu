@@ -388,6 +388,7 @@ struct yart_ctx {
 
   // work buffers
   DevBuf rays, hits_export, time, wavelength, throughput, hits, queue_a, queue_b, counts, work, counters, film, rgba;
+  DevBuf nee_rays, nee_pending, nee_sum, nee_w, queue_s; // YART_FLAG_NEXT_EVENT's per-path state (NeeState)
   DevBuf occluded; // staging of yart_occluded's flags for host arrays
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> ev_pool;
@@ -1503,7 +1504,8 @@ static int fill_render_params(yart_ctx* ctx, const yart_camera* cam, const yart_
   R.height = o->height;
   R.max_depth = o->max_depth;
   R.seed = o->seed;
-  R.flags = o->flags & (YART_FLAG_UNBIASED_LIGHT_PICK | YART_FLAG_RUSSIAN_ROULETTE | YART_FLAG_DEPTH_ZERO_BLACK);
+  R.flags = o->flags & (YART_FLAG_UNBIASED_LIGHT_PICK | YART_FLAG_RUSSIAN_ROULETTE | YART_FLAG_DEPTH_ZERO_BLACK | YART_FLAG_NEXT_EVENT);
+  if (R.flags & YART_FLAG_NEXT_EVENT) R.flags |= YART_FLAG_UNBIASED_LIGHT_PICK; // MIS needs the mixture's true density
   {
     // A trailing run of plain spheres that directly follows a mesh pass is intersected inside k_shade (which
     // reads the ray and the hit anyway) -- saves one read-modify-write pass over the queue per bounce.
@@ -1603,11 +1605,19 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
     // (minus a margin), so that a busy GPU gets smaller batches instead of a failed cudaMalloc.
     static const int max_paths_log2 = std::max(10, std::min(30, tune_env("YART_TUNE_MAX_PATHS_LOG2", 28)));
     uint64_t kMaxPaths = 1ull << max_paths_log2;
+    const bool nee = (R.flags & YART_FLAG_NEXT_EVENT) != 0;
     {
-      const uint64_t kStateBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(DevHit) + 2 * sizeof(uint32_t);
+      // YART_FLAG_NEXT_EVENT adds 76 B: 48 shadow ray + 8 pending + 8 light-sample sum + 8 emission weight + 4 shadow queue
+      // (the shadow passes write their hits into the path hits, which are dead from k_shade to the next bounce's passes)
+      const uint64_t kNeeBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(uint32_t);
+      const uint64_t kStateBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(DevHit) + 2 * sizeof(uint32_t) +
+                                          (nee ? kNeeBytesPerPath : 0);
+      if (!nee) // a flag-off render does not keep an earlier NEE render's state alive (no-op when there is none)
+        for (DevBuf* b : {&ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s}) b->release();
       size_t free_b = 0, total_b = 0;
       CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
-      const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b};
+      const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b,
+                              &ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s};
       uint64_t avail = free_b; // what the state buffers may grow into: free memory + what they already hold
       for (const DevBuf* b : held) avail += b->cap;
       const uint64_t margin = (256ull << 20) + (dev ? 0 : film_bytes);
@@ -1617,7 +1627,8 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
       if (mem_cap_mb > 0) kMaxPaths = std::min<uint64_t>(kMaxPaths, ((uint64_t)mem_cap_mb << 20) / kStateBytesPerPath);
       if (kMaxPaths < 1024) {
         ctx->err = "yart_render: not enough free device memory for the path state (" + std::to_string(free_b >> 20) +
-                   " MiB free of " + std::to_string(total_b >> 20) + " MiB; 112 bytes per path in flight)";
+                   " MiB free of " + std::to_string(total_b >> 20) + " MiB; " + std::to_string(kStateBytesPerPath) +
+                   " bytes per path in flight)";
         return YART_ERR_NOMEM;
       }
     }
@@ -1634,12 +1645,30 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
     CUDA_TRY(ctx, ctx->queue_a.reserve(cap * sizeof(uint32_t)));
     CUDA_TRY(ctx, ctx->queue_b.reserve(cap * sizeof(uint32_t)));
     const uint32_t D = o->max_depth;
-    const size_t n_counts = (size_t)D + 2;
+    // with NEE: path counts [0, D+2), then the shadow queue's count of bounce b at D+2+b; path work counters, then the
+    // shadow passes' ones
+    const size_t n_counts = (size_t)D + 2 + (nee ? (size_t)D + 1 : 0);
     const size_t n_obj_slots = (size_t)ctx->scene.n_objects + 1;
-    const size_t n_work = n_obj_slots * D;
+    const size_t n_work = n_obj_slots * D * (nee ? 2 : 1);
     CUDA_TRY(ctx, ctx->counts.reserve(n_counts * sizeof(uint32_t)));
     CUDA_TRY(ctx, ctx->work.reserve(n_work * sizeof(uint32_t)));
-    while (ctx->ev_pool.size() < 2 * (size_t)D) {
+    NeeState N;
+    memset(&N, 0, sizeof(N));
+    if (nee) {
+      CUDA_TRY(ctx, ctx->nee_rays.reserve(cap * sizeof(yart_ray)));
+      CUDA_TRY(ctx, ctx->nee_pending.reserve(cap * sizeof(double)));
+      CUDA_TRY(ctx, ctx->nee_sum.reserve(cap * sizeof(double)));
+      CUDA_TRY(ctx, ctx->nee_w.reserve(cap * sizeof(double)));
+      CUDA_TRY(ctx, ctx->queue_s.reserve(cap * sizeof(uint32_t)));
+      N.rays = ctx->nee_rays.as<yart_ray>();
+      N.pending = ctx->nee_pending.as<double>();
+      N.sum = ctx->nee_sum.as<double>();
+      N.w_emit = ctx->nee_w.as<double>();
+      N.queue = ctx->queue_s.as<uint32_t>();
+      N.counts = ctx->counts.as<uint32_t>() + D + 2;
+    }
+    // events: [0, 2D) closest-hit passes per bounce, [2D, 4D) YART_DEBUG_BOUNCES's shade timing, [4D, 6D) shadow passes
+    while (ctx->ev_pool.size() < (nee ? 6 : 2) * (size_t)D) {
       cudaEvent_t e;
       CUDA_TRY(ctx, cudaEventCreate(&e));
       ctx->ev_pool.push_back(e);
@@ -1669,7 +1698,8 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
         CUDA_TRY(ctx, cudaMemsetAsync(work, 0, n_work * sizeof(uint32_t), ctx->stream));
         uint32_t* qa = ctx->queue_a.as<uint32_t>();
         uint32_t* qb = ctx->queue_b.as<uint32_t>();
-        k_raygen<<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1);
+        if (nee) k_raygen<true><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
+        else k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
         launches++;
         uint32_t b_done = 0;
         for (uint32_t b = 1; b <= D; ++b) {
@@ -1712,9 +1742,25 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
             }
             CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->stream));
           }
-          k_shade<<<std::max(1, stream_grid * 256 / kShadeThreads), kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b);
+          const int shade_grid = std::max(1, stream_grid * 256 / kShadeThreads);
+          if (nee) k_shade<true><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
+          else k_shade<false><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
           launches += 1;
           if (dbg_shade_ev) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1) + 1], ctx->stream));
+          if (nee && b < D) { // the shadow rays k_shade queued: the same world query, on their own queue and Philox stream
+            QueryArgs sq = q;
+            sq.c.rays = N.rays;
+            sq.c.queue = N.queue;
+            sq.c.n_items_dev = N.counts + b;
+            sq.bounce = YART_NEE_BOUNCE_BASE + b;
+            sq.work_counters = work + (size_t)(D + b - 1) * n_obj_slots;
+            CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->stream));
+            rc = run_passes(ctx, sq, &trace_launches);
+            if (rc) return rc;
+            CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1) + 1], ctx->stream));
+            k_nee_resolve<<<stream_grid, 256, 0, ctx->stream>>>(R, b, N);
+            launches += 1;
+          }
           std::swap(qa, qb);
           b_done = b;
           // the tail of the bounce loop is nearly empty: look at the live count now and then
@@ -1725,7 +1771,8 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
             if (live == 0) break;
           }
         }
-        k_film_accumulate<<<stream_grid, 256, 0, ctx->stream>>>(R, d_film);
+        if (nee) k_film_accumulate<true><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
+        else k_film_accumulate<false><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
         launches++;
         CUDA_TRY(ctx, cudaGetLastError());
         CUDA_TRY(ctx, cudaMemcpyAsync(h_counts.data(), counts, n_counts * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1738,12 +1785,19 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
           float ms = 0.f;
           CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[2 * (b - 1)], ctx->ev_pool[2 * (b - 1) + 1]));
           trace_ms += ms;
+          if (nee && b < D) {
+            float shadow_ms = 0.f;
+            CUDA_TRY(ctx, cudaEventElapsedTime(&shadow_ms, ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->ev_pool[4 * D + 2 * (b - 1) + 1]));
+            trace_ms += shadow_ms;
+          }
           if (debug_bounces) {
             float gap = 0.f; // from the end of this bounce's closest-hit stage to the start of the next one
             if (b < b_done) cudaEventElapsedTime(&gap, ctx->ev_pool[2 * (b - 1) + 1], ctx->ev_pool[2 * b]);
             float shade = 0.f;
             cudaEventElapsedTime(&shade, ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->ev_pool[2 * D + 2 * (b - 1) + 1]);
-            fprintf(stderr, "bounce %2u: rays %9u  closest-hit %8.3f ms  shade %8.3f ms  shade+gap %8.3f ms\n", b, h_counts[b], ms, shade, gap);
+            fprintf(stderr, "bounce %2u: rays %9u  closest-hit %8.3f ms  shade %8.3f ms  shade+gap %8.3f ms", b, h_counts[b], ms, shade, gap);
+            if (nee) fprintf(stderr, "  shadow rays %9u", b < D ? h_counts[D + 2 + b] : 0u);
+            fprintf(stderr, "\n");
           }
         }
       }

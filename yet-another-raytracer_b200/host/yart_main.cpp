@@ -9,7 +9,7 @@
 //
 // Additions: --seed S (the reference is OS-seeded), --device D, --gpus N (N GPUs of this box: one host thread per
 // context, yart_comm_init + yart_film_reduce = one in-place ncclReduce of the f64 film), --order near|reference,
-// --unbiased-light-pick / --russian-roulette / --depth-zero-black (better sampling, OFF by default), --assets DIR,
+// --unbiased-light-pick / --russian-roulette / --depth-zero-black / --next-event (better sampling, OFF by default), --assets DIR,
 // --dry-run (print the resolved options as one JSON line and exit: what the reference's unit tests check,
 // main.rs:868-915), --list-scenes.  `--workers` is accepted and ignored.  There is no CPU mode.
 //
@@ -117,7 +117,7 @@ struct Cli {
   fprintf(stderr, "error: %s\n\nUsage: yart --scene <SCENE> [--output <OUTPUT>] [--width <WIDTH>] [--height <HEIGHT>] "
                   "[--samples <SAMPLES>] [--max-depth <MAX_DEPTH>] [--workers <WORKERS>] [--vfov <VFOV>] [--aperture <APERTURE>]\n"
                   "            [--seed S] [--device D] [--gpus N] [--order near|reference] [--assets DIR] [--dry-run] [--list-scenes]\n"
-                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black]\n",
+                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event]\n",
           msg.c_str());
   exit(2);
 }
@@ -171,6 +171,7 @@ Cli parse(int argc, char** argv) {
     else if (a == "--unbiased-light-pick") c.flags |= YART_FLAG_UNBIASED_LIGHT_PICK;
     else if (a == "--russian-roulette") c.flags |= YART_FLAG_RUSSIAN_ROULETTE;
     else if (a == "--depth-zero-black") c.flags |= YART_FLAG_DEPTH_ZERO_BLACK;
+    else if (a == "--next-event") c.flags |= YART_FLAG_NEXT_EVENT;
     else if (a == "--dry-run") c.dry_run = true;
     else if (a == "--list-scenes") c.list_scenes = true;
     else if (a == "--help" || a == "-h") {
