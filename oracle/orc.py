@@ -47,12 +47,19 @@ _lib = None
 
 
 def lib():
+    """The default build, oracle/_build/liboracle.so (built on first use)."""
     global _lib
-    if _lib is not None:
-        return _lib
-    if not LIB_PATH.exists():
-        build()
-    L = C.CDLL(str(LIB_PATH))
+    if _lib is None:
+        if not LIB_PATH.exists():
+            build()
+        _lib = load(LIB_PATH)
+    return _lib
+
+
+def load(path):
+    """A library of the oracle's API at `path` (the default build or a variant of it, tests/perturbed_oracle.py),
+    with its signatures declared."""
+    L = C.CDLL(str(path))
     P, vp, u32, u64, f64, i32 = C.POINTER, C.c_void_p, C.c_uint32, C.c_uint64, C.c_double, C.c_int
     sig = {
         "orc_last_error": (C.c_char_p, []),
@@ -86,13 +93,12 @@ def lib():
         fn = getattr(L, name)
         fn.restype = res
         fn.argtypes = args
-    _lib = L
     return L
 
 
-def _check(rc):
+def _check(rc, L=None):
     if rc != 0:
-        raise RuntimeError("oracle error %d: %s" % (rc, lib().orc_last_error().decode()))
+        raise RuntimeError("oracle error %d: %s" % (rc, (L or lib()).orc_last_error().decode()))
 
 
 def _opts(width, height, sample_begin, sample_end, max_depth, seed, order, flags=0):
@@ -105,29 +111,33 @@ def _opts(width, height, sample_begin, sample_end, max_depth, seed, order, flags
 
 class Scene:
     """The oracle's view of a scene description (a ctypes POINTER(SceneDesc) or a ScenePreset-like
-    object with a `.desc`)."""
+    object with a `.desc`).  `L`: the library to use (default: lib())."""
 
-    def __init__(self, scene):
+    def __init__(self, scene, L=None):
         self._keep = scene
+        self._L = L or lib()
         desc = getattr(scene, "desc", scene)
         self._h = C.c_void_p()
-        _check(lib().orc_scene_create(desc, C.byref(self._h)))
+        self._check(self._L.orc_scene_create(desc, C.byref(self._h)))
+
+    def _check(self, rc):
+        _check(rc, self._L)
 
     def qbvh_info(self, mesh=0):
         info = QbvhInfo()
-        _check(lib().orc_qbvh_info_get(self._h, mesh, C.byref(info)))
+        self._check(self._L.orc_qbvh_info_get(self._h, mesh, C.byref(info)))
         return info
 
     def qbvh_node(self, mesh, i):
         boxes = np.empty(24, dtype=np.float64)
         children = np.empty(4, dtype=np.uint32)
         axes = np.empty(3, dtype=np.uint32)
-        _check(lib().orc_qbvh_node(self._h, mesh, i, boxes.ctypes.data, children.ctypes.data, axes.ctypes.data))
+        self._check(self._L.orc_qbvh_node(self._h, mesh, i, boxes.ctypes.data, children.ctypes.data, axes.ctypes.data))
         return boxes, children, axes
 
     def tri_order(self, mesh=0):
         out = np.empty(self.qbvh_info(mesh).n_tris, dtype=np.uint32)
-        _check(lib().orc_qbvh_tri_order(self._h, mesh, out.ctypes.data))
+        self._check(self._L.orc_qbvh_tri_order(self._h, mesh, out.ctypes.data))
         return out
 
     def closest_hit(self, rays, target=abi.TARGET_WORLD, t_min=0.001, t_max=float("inf"), order=abi.ORDER_REFERENCE,
@@ -135,23 +145,23 @@ class Scene:
         rays = np.ascontiguousarray(rays, dtype=abi.RAY_DTYPE)
         hits = np.empty(rays.shape[0], dtype=abi.HIT_DTYPE)
         cnt = Counters()
-        _check(lib().orc_closest_hit(self._h, target, rays.ctypes.data, rays.shape[0], t_min, t_max, order,
-                                     hits.ctypes.data, C.byref(cnt), n_threads))
+        self._check(self._L.orc_closest_hit(self._h, target, rays.ctypes.data, rays.shape[0], t_min, t_max, order,
+                                            hits.ctypes.data, C.byref(cnt), n_threads))
         return hits, cnt
 
     def brute_force_hit(self, rays, mesh=0, t_min=0.001, t_max=float("inf")):
         rays = np.ascontiguousarray(rays, dtype=abi.RAY_DTYPE)
         hits = np.empty(rays.shape[0], dtype=abi.HIT_DTYPE)
         ties = np.empty(rays.shape[0], dtype=np.uint32)
-        _check(lib().orc_brute_force_hit(self._h, mesh, rays.ctypes.data, rays.shape[0], t_min, t_max,
-                                         hits.ctypes.data, ties.ctypes.data))
+        self._check(self._L.orc_brute_force_hit(self._h, mesh, rays.ctypes.data, rays.shape[0], t_min, t_max,
+                                                hits.ctypes.data, ties.ctypes.data))
         return hits, ties
 
     def tie_set(self, ray, mesh=0, t_min=0.001, t_max=float("inf")):
         ray = np.ascontiguousarray(ray, dtype=abi.RAY_DTYPE).reshape(1)
         ids = np.empty(64, dtype=np.uint32)
         n = C.c_uint32()
-        _check(lib().orc_tie_set(self._h, mesh, ray.ctypes.data, t_min, t_max, ids.ctypes.data, 64, C.byref(n)))
+        self._check(self._L.orc_tie_set(self._h, mesh, ray.ctypes.data, t_min, t_max, ids.ctypes.data, 64, C.byref(n)))
         return ids[:min(n.value, 64)].copy()
 
     def render(self, camera, width, height, sample_begin, sample_end, max_depth=50, seed=1, order=abi.ORDER_REFERENCE,
@@ -160,35 +170,36 @@ class Scene:
             film = np.zeros((height, width, 3), dtype=np.float64)
         st = abi.Stats()
         o = _opts(width, height, sample_begin, sample_end, max_depth, seed, order, flags)
-        _check(lib().orc_render_tiles(self._h, C.byref(camera), C.byref(o), film.ctypes.data, C.byref(st), n_threads,
-                                      tiles[0], tiles[1]))
+        self._check(self._L.orc_render_tiles(self._h, C.byref(camera), C.byref(o), film.ctypes.data, C.byref(st), n_threads,
+                                             tiles[0], tiles[1]))
         return film, st
 
     def dump_path_rays(self, camera, width, height, sample_begin, sample_end, cap, max_depth=50, seed=1):
         rays = np.empty(cap, dtype=abi.RAY_DTYPE)
         n = C.c_uint64()
         o = _opts(width, height, sample_begin, sample_end, max_depth, seed, abi.ORDER_REFERENCE)
-        _check(lib().orc_dump_path_rays(self._h, C.byref(camera), C.byref(o), rays.ctypes.data, cap, C.byref(n)))
+        self._check(self._L.orc_dump_path_rays(self._h, C.byref(camera), C.byref(o), rays.ctypes.data, cap, C.byref(n)))
         return rays[:n.value].copy()
 
-    def sample_path(self, camera, width, height, pixel, sample, max_depth=50, seed=1):
+    def sample_path(self, camera, width, height, pixel, sample, max_depth=50, seed=1, order=abi.ORDER_REFERENCE, flags=0):
         rays = np.empty(max_depth + 1, dtype=abi.RAY_DTYPE)
         n = C.c_uint64()
-        o = _opts(width, height, sample, sample + 1, max_depth, seed, abi.ORDER_REFERENCE)
-        _check(lib().orc_sample_path(self._h, C.byref(camera), C.byref(o), pixel, sample, rays.ctypes.data, len(rays),
-                                     C.byref(n)))
+        o = _opts(width, height, sample, sample + 1, max_depth, seed, order, flags)
+        self._check(self._L.orc_sample_path(self._h, C.byref(camera), C.byref(o), pixel, sample, rays.ctypes.data, len(rays),
+                                            C.byref(n)))
         return rays[:n.value].copy()
 
-    def sample(self, camera, width, height, pixel, sample, max_depth=50, seed=1):
+    def sample(self, camera, width, height, pixel, sample, max_depth=50, seed=1, order=abi.ORDER_REFERENCE, flags=0):
+        """(unsanitised XYZ, ray count) of one (pixel, sample), pixel = y * width + x."""
         xyz = np.empty(3, dtype=np.float64)
         nr = C.c_uint32()
-        o = _opts(width, height, sample, sample + 1, max_depth, seed, abi.ORDER_REFERENCE)
-        _check(lib().orc_sample(self._h, C.byref(camera), C.byref(o), pixel, sample, xyz.ctypes.data, C.byref(nr)))
+        o = _opts(width, height, sample, sample + 1, max_depth, seed, order, flags)
+        self._check(self._L.orc_sample(self._h, C.byref(camera), C.byref(o), pixel, sample, xyz.ctypes.data, C.byref(nr)))
         return xyz, nr.value
 
     def __del__(self):
-        if getattr(self, "_h", None) and _lib is not None:
-            _lib.orc_scene_free(self._h)
+        if getattr(self, "_h", None) and getattr(self, "_L", None) is not None:
+            self._L.orc_scene_free(self._h)
             self._h = None
 
 

@@ -32,6 +32,50 @@ const double kF64Max = std::numeric_limits<double>::max();
 thread_local std::string g_err;
 
 // ---------------------------------------------------------------------------------------
+// The transcendentals on the film path (sphere uv, ConstantMedium, noise textures, cone and cosine sampling).  CUDA's
+// sin/cos/acos/atan2 (2 ulp) and log (1 ulp) may differ from glibc's in the last bits, so the tests build variants
+// of this file that move each result by a few ulp, to tell a sample that flips on such a difference from a real
+// divergence (tests/perturbed_oracle.py).  YART_ORACLE_LIBM_PERTURB undefined: plain libm.  Defined as k: every
+// result moves k ulp (0: the hook is compiled in and moves nothing); with YART_ORACLE_LIBM_SEED also defined, a hash
+// of (seed, function, input bits) picks a move in [-|k|, |k|] per call.  Zero and non-finite results stay.
+// ---------------------------------------------------------------------------------------
+enum LibmFn : uint64_t { LM_SIN = 1, LM_COS, LM_ACOS, LM_ATAN2, LM_LOG };
+#ifndef YART_ORACLE_LIBM_PERTURB
+inline double libm_result(LibmFn, double, double, double r) { return r; }
+#else
+inline uint64_t libm_bits(double x) {
+  uint64_t b;
+  memcpy(&b, &x, sizeof b);
+  return b;
+}
+inline double libm_result(LibmFn fn, double a, double b, double r) {
+  if (r == 0.0 || !std::isfinite(r)) return r;
+#ifdef YART_ORACLE_LIBM_SEED
+  uint64_t h = (uint64_t)(YART_ORACLE_LIBM_SEED) * 0x9e3779b97f4a7c15ull ^ fn;
+  for (uint64_t w : {libm_bits(a), libm_bits(b)}) { // splitmix64 steps
+    h += w + 0x9e3779b97f4a7c15ull;
+    h = (h ^ (h >> 30)) * 0xbf58476d1ce4e5b9ull;
+    h = (h ^ (h >> 27)) * 0x94d049bb133111ebull;
+    h ^= h >> 31;
+  }
+  const int span = (YART_ORACLE_LIBM_PERTURB) < 0 ? -(YART_ORACLE_LIBM_PERTURB) : (YART_ORACLE_LIBM_PERTURB);
+  const int k = (int)(h % (uint64_t)(2 * span + 1)) - span;
+#else
+  (void)fn; (void)a; (void)b;
+  const int k = YART_ORACLE_LIBM_PERTURB;
+#endif
+  for (int i = 0; i < (k < 0 ? -k : k); ++i) r = std::nextafter(r, k < 0 ? -INFINITY : INFINITY);
+  if (fn == LM_SIN || fn == LM_COS) r = r > 1.0 ? 1.0 : (r < -1.0 ? -1.0 : r); // (as both libraries bound them)
+  return r;
+}
+#endif
+inline double lm_sin(double x) { return libm_result(LM_SIN, x, 0.0, std::sin(x)); }
+inline double lm_cos(double x) { return libm_result(LM_COS, x, 0.0, std::cos(x)); }
+inline double lm_acos(double x) { return libm_result(LM_ACOS, x, 0.0, std::acos(x)); }
+inline double lm_atan2(double y, double x) { return libm_result(LM_ATAN2, y, x, std::atan2(y, x)); }
+inline double lm_log(double x) { return libm_result(LM_LOG, x, 0.0, std::log(x)); }
+
+// ---------------------------------------------------------------------------------------
 // Vec3 (vec3.rs:8-247)
 // ---------------------------------------------------------------------------------------
 struct V3 {
@@ -508,8 +552,8 @@ struct Scene {
 };
 
 inline void get_sphere_uv(V3 p, double& u, double& v) { // sphere.rs:213-220
-  double theta = std::acos(-p.y);
-  double phi = std::atan2(-p.z, p.x) + kPi;
+  double theta = lm_acos(-p.y);
+  double phi = lm_atan2(-p.z, p.x) + kPi;
   u = phi / (2.0 * kPi);
   v = theta / kPi;
 }
@@ -771,7 +815,7 @@ bool hit_object(const HitCtx& c, const yart_object& o, uint32_t obj_index, const
   const double distance_inside = (rec2.t - rec1.t) * ray_length;
   double u0 = 0.5, u1;
   if (rng) rng->draw(bounce, YART_SLOT_MEDIUM + obj_index, u0, u1);
-  const double hit_distance = o.neg_inv_density * std::log(u0);
+  const double hit_distance = o.neg_inv_density * lm_log(u0);
   if (!(hit_distance < distance_inside)) return false;
   rec.t = rec1.t + hit_distance / ray_length;
   rec.p = ray_at(ray, rec.t);
@@ -870,7 +914,7 @@ double texture_value(const Scene& s, uint32_t tex, const Ray& ray_in, const HitR
   switch (t.kind) {
     case YART_TEX_SOLID: return rgb_reflect(t.rgb_a, ray_in.wl); // texture.rs:36-40
     case YART_TEX_CHECKER: {                                     // texture.rs:57-68
-      double sines = std::sin(10.0 * rec.p.x) * std::sin(10.0 * rec.p.y) * std::sin(10.0 * rec.p.z);
+      double sines = lm_sin(10.0 * rec.p.x) * lm_sin(10.0 * rec.p.y) * lm_sin(10.0 * rec.p.z);
       return sines < 0.0 ? rgb_reflect(t.rgb_a, ray_in.wl) : rgb_reflect(t.rgb_b, ray_in.wl);
     }
     case YART_TEX_NOISE: { // texture.rs:260-284
@@ -879,7 +923,7 @@ double texture_value(const Scene& s, uint32_t tex, const Ray& ray_in, const HitR
         return rgb_reflect(white, ray_in.wl) * perlin_turb(pn, t.noise_type, rec.p * t.scale, 7);
       if (t.noise_type == YART_NOISE_MARBLE)
         return rgb_reflect(white, ray_in.wl) * 0.5 *
-               (1.0 + std::sin(t.scale * rec.p.z + 10.0 * perlin_turb(pn, t.noise_type, rec.p, 7)));
+               (1.0 + lm_sin(t.scale * rec.p.z + 10.0 * perlin_turb(pn, t.noise_type, rec.p, 7)));
       return rgb_reflect(white, ray_in.wl) * 0.5 * (1.0 + perlin_noise(pn, t.noise_type, rec.p * t.scale));
     }
     case YART_TEX_IMAGE: { // texture.rs:313-345
@@ -947,8 +991,8 @@ V3 light_random(const yart_object& l, V3 origin, double r1, double r2) {
     Onb uvw = onb_from_w(direction);
     double z = 1.0 + r2 * (std::sqrt(1.0 - radius * radius / distance_squared) - 1.0);
     double phi = 2.0 * kPi * r1;
-    double x = std::cos(phi) * std::sqrt(1.0 - z * z);
-    double y = std::sin(phi) * std::sqrt(1.0 - z * z);
+    double x = lm_cos(phi) * std::sqrt(1.0 - z * z);
+    double y = lm_sin(phi) * std::sqrt(1.0 - z * z);
     return onb_local(uvw, v3(x, y, z));
   }
   if (l.wrap == 0 && l.kind == YART_OBJ_XZ_RECT) { // aarect.rs:164-171
@@ -1107,8 +1151,8 @@ double ray_reflectance(const HitCtx& c, Ray ray, const Rng& rng, uint32_t max_de
     auto cosine_dir = [&]() { // random_cosine_direction (pdf.rs:15-25)
       double z = std::sqrt(1.0 - r2);
       double phi = 2.0 * kPi * r1;
-      double x = std::cos(phi) * std::sqrt(r2);
-      double y = std::sin(phi) * std::sqrt(r2);
+      double x = lm_cos(phi) * std::sqrt(r2);
+      double y = lm_sin(phi) * std::sqrt(r2);
       return onb_local(uvw, v3(x, y, z));
     };
     V3 dir;

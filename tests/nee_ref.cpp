@@ -132,8 +132,8 @@ double ray_reflectance_nee(const HitCtx& c, Ray ray, const Rng& rng, uint32_t ma
     auto cosine_dir = [&]() {
       double z = std::sqrt(1.0 - r2);
       double phi = 2.0 * kPi * r1;
-      double x = std::cos(phi) * std::sqrt(r2);
-      double y = std::sin(phi) * std::sqrt(r2);
+      double x = lm_cos(phi) * std::sqrt(r2);
+      double y = lm_sin(phi) * std::sqrt(r2);
       return onb_local(uvw, v3(x, y, z));
     };
     const bool have_lights = !s.lights.empty();

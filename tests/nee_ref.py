@@ -27,46 +27,59 @@ FLAGS = ["-O3", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-
 _lib = None
 
 
-def lib():
-    global _lib
-    if _lib is not None:
-        return _lib
+def compile_shared(stem, source, deps, flags):
+    """Compile `source` with `flags` into <tmp>/yart_nee_ref_<uid>/<stem>_<digest>.so, the digest taken over the
+    compiler, the flags and `deps`; built once, replaced atomically (parallel test workers may build it at the same
+    time).  Returns the path."""
     cxx = os.environ.get("CXX", "g++")
-    h = hashlib.sha256(" ".join([cxx] + FLAGS).encode())
-    for f in SOURCES:
+    h = hashlib.sha256(" ".join([cxx] + flags).encode())
+    for f in deps:
         h.update(f.read_bytes())
     out_dir = Path(tempfile.gettempdir()) / ("yart_nee_ref_%d" % os.getuid())
     out_dir.mkdir(exist_ok=True)
-    so = out_dir / ("nee_ref_%s.so" % h.hexdigest()[:16])
+    so = out_dir / ("%s_%s.so" % (stem, h.hexdigest()[:16]))
     if not so.exists():
         tmp = so.with_suffix(".tmp%d.so" % os.getpid())
-        res = subprocess.run([cxx] + FLAGS + ["-o", str(tmp), str(HERE / "nee_ref.cpp")], capture_output=True, text=True)
+        res = subprocess.run([cxx] + flags + ["-o", str(tmp), str(source)], capture_output=True, text=True)
         if res.returncode != 0:
-            raise RuntimeError("next-event reference build failed:\n" + res.stdout + res.stderr)
-        os.replace(tmp, so)  # (atomic: parallel test workers may build it at the same time)
-    L = C.CDLL(str(so))
+            raise RuntimeError("%s build failed:\n%s%s" % (stem, res.stdout, res.stderr))
+        os.replace(tmp, so)
+    return so
+
+
+def load(path):
+    """A build of nee_ref.cpp at `path` (the default one or a variant, tests/perturbed_oracle.py)."""
+    L = C.CDLL(str(path))
     vp = C.c_void_p
     L.neeref_last_error.restype, L.neeref_last_error.argtypes = C.c_char_p, []
     L.neeref_scene_create.restype, L.neeref_scene_create.argtypes = C.c_int, [C.POINTER(abi.SceneDesc), C.POINTER(vp)]
     L.neeref_scene_free.restype, L.neeref_scene_free.argtypes = None, [vp]
     L.neeref_render.restype = C.c_int
     L.neeref_render.argtypes = [vp, C.POINTER(abi.Camera), C.POINTER(abi.RenderOpts), vp, C.POINTER(abi.Stats), C.c_int]
-    _lib = L
     return L
 
 
-def _check(rc):
+def lib():
+    global _lib
+    if _lib is None:
+        _lib = load(compile_shared("nee_ref", HERE / "nee_ref.cpp", SOURCES, FLAGS))
+    return _lib
+
+
+def _check(rc, L=None):
     if rc != 0:
-        raise RuntimeError("next-event reference error %d: %s" % (rc, lib().neeref_last_error().decode()))
+        raise RuntimeError("next-event reference error %d: %s" % (rc, (L or lib()).neeref_last_error().decode()))
 
 
 class Scene:
-    """The reference's view of a scene description (a ctypes POINTER(SceneDesc) or an object with a `.desc`)."""
+    """The reference's view of a scene description (a ctypes POINTER(SceneDesc) or an object with a `.desc`).
+    `L`: the library to use (default: lib())."""
 
-    def __init__(self, scene):
+    def __init__(self, scene, L=None):
         self._keep = scene
+        self._L = L or lib()
         self._h = C.c_void_p()
-        _check(lib().neeref_scene_create(getattr(scene, "desc", scene), C.byref(self._h)))
+        _check(self._L.neeref_scene_create(getattr(scene, "desc", scene), C.byref(self._h)), self._L)
 
     def render(self, camera, width, height, sample_begin, sample_end, max_depth=50, seed=1, order=abi.ORDER_REFERENCE,
                n_threads=1, flags=abi.FLAG_NEXT_EVENT):
@@ -77,10 +90,10 @@ class Scene:
         o.width, o.height, o.sample_begin, o.sample_end = width, height, sample_begin, sample_end
         o.max_depth, o.order, o.batch_spp, o.flags, o.seed = max_depth, order, 0, flags, seed
         st = abi.Stats()
-        _check(lib().neeref_render(self._h, C.byref(camera), C.byref(o), film.ctypes.data, C.byref(st), n_threads))
+        _check(self._L.neeref_render(self._h, C.byref(camera), C.byref(o), film.ctypes.data, C.byref(st), n_threads), self._L)
         return film, st
 
     def __del__(self):
-        if getattr(self, "_h", None) and _lib is not None:
-            _lib.neeref_scene_free(self._h)
+        if getattr(self, "_h", None) and getattr(self, "_L", None) is not None:
+            self._L.neeref_scene_free(self._h)
             self._h = None
