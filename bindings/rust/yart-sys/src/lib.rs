@@ -120,6 +120,13 @@ pub struct yart_hit_f32 { pub t: f32, pub u: f32, pub v: f32, pub prim_id: u32 }
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct yart_hit { pub t: f64, pub u: f64, pub v: f64, pub prim_id: u32, pub obj_id: u32, pub front_face: u32, pub _pad: u32 }
 
+/// The whole `HitRecord` (hittable.rs:37-45) of `yart_closest_hit_records`, 88 bytes.
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct yart_hit_record {
+    pub t: f64, pub p: [f64; 3], pub normal: [f64; 3], pub u: f64, pub v: f64,
+    pub material: u32, pub front_face: u32, pub obj_id: u32, pub prim_id: u32,
+}
+
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct yart_stats {
     pub rays: u64, pub paths: u64, pub node_visits: u64, pub tri_tests: u64, pub kernel_launches: u64,
@@ -180,6 +187,9 @@ extern "C" {
                             order: u32, flags: u32, hits: *mut yart_hit, stats: *mut yart_stats) -> c_int;
     pub fn yart_closest_hit_f32(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray_f32, n: u64, t_min: f32, t_max: f32,
                                 order: u32, flags: u32, hits: *mut yart_hit_f32, stats: *mut yart_stats) -> c_int;
+    pub fn yart_closest_hit_records(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray, times: *const f64, n: u64,
+                                    t_min: f64, t_max: f64, order: u32, flags: u32, records: *mut yart_hit_record,
+                                    stats: *mut yart_stats) -> c_int;
     pub fn yart_occluded(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray, n: u64, t_min: f64, t_max: f64,
                          flags: u32, occluded: *mut u8, stats: *mut yart_stats) -> c_int;
     pub fn yart_occluded_f32(ctx: *mut yart_ctx, target: u32, rays: *const yart_ray_f32, n: u64, t_min: f32, t_max: f32,

@@ -3,7 +3,7 @@
 //!
 //! `GpuScene` plays the part of `world: Arc<HittableList>` (main.rs:434-446): `hit` has the shape of
 //! `Hittable::hit(&self, &Ray, t_min, t_max) -> Option<HitRecord>` (hittable.rs:24) for drop-in testing, `hit_many`
-//! is the batched form the GPU is for, `render` replaces the tile loop of `render()` (main.rs:629-760).
+//! is the batched form the GPU is for, `hit_records` / `hit_record` return the whole `HitRecord`, `render` replaces the tile loop of `render()` (main.rs:629-760).
 use std::ffi::{CStr, CString};
 use std::ptr;
 use yart_sys as sys;
@@ -18,6 +18,15 @@ pub struct Ray { pub origin: [f64; 3], pub direction: [f64; 3] }
 /// The part of the reference's `HitRecord` the closest-hit query returns (the shade stage rebuilds the rest).
 #[derive(Clone, Copy, Debug)]
 pub struct Hit { pub t: f64, pub u: f64, pub v: f64, pub prim_id: u32, pub obj_id: u32, pub front_face: bool }
+
+/// The reference's whole `HitRecord` (hittable.rs:37-45) as `world.hit` returns it, plus the ids of `Hit`:
+/// `p`, the stored (face-oriented, unnormalised) normal, the texture `u, v`, and `material`, an index into the scene's
+/// material table (a group hit: the member's; `YART_MISS` for a bare mesh).
+#[derive(Clone, Copy, Debug)]
+pub struct Record {
+    pub t: f64, pub p: [f64; 3], pub normal: [f64; 3], pub u: f64, pub v: f64,
+    pub material: u32, pub front_face: bool, pub obj_id: u32, pub prim_id: u32,
+}
 
 pub struct GpuScene { ctx: *mut sys::yart_ctx, preset: *mut sys::yart_preset }
 
@@ -62,6 +71,30 @@ impl GpuScene {
         Ok(hits.iter().map(|h| if h.obj_id == sys::YART_MISS { None } else {
             Some(Hit { t: h.t, u: h.u, v: h.v, prim_id: h.prim_id, obj_id: h.obj_id, front_face: h.front_face != 0 })
         }).collect())
+    }
+
+    /// Batched `world.hit(ray, t_min, t_max)` returning whole records (`yart_closest_hit_records`), each ray traced at
+    /// its own `Ray.time` (`times`: one per ray; `None` = every ray at time 0).  `None` in the result = miss.
+    pub fn hit_records(&self, rays: &[Ray], times: Option<&[f64]>, t_min: f64, t_max: f64) -> Result<Vec<Option<Record>>> {
+        if let Some(t) = times { assert_eq!(t.len(), rays.len()); }
+        let raw: Vec<sys::yart_ray> = rays.iter().map(|r| sys::yart_ray { origin: r.origin, direction: r.direction }).collect();
+        let mut recs = vec![sys::yart_hit_record { t: 0.0, p: [0.0; 3], normal: [0.0; 3], u: 0.0, v: 0.0, material: 0,
+                                                   front_face: 0, obj_id: 0, prim_id: 0 }; rays.len()];
+        let rc = unsafe {
+            sys::yart_closest_hit_records(self.ctx, sys::YART_TARGET_WORLD, raw.as_ptr(), times.map_or(ptr::null(), |t| t.as_ptr()),
+                                          raw.len() as u64, t_min, t_max, sys::YART_ORDER_NEAR, 0, recs.as_mut_ptr(),
+                                          ptr::null_mut())
+        };
+        if rc != 0 { return Err(self.ctx_err(rc)); }
+        Ok(recs.iter().map(|r| if r.obj_id == sys::YART_MISS { None } else {
+            Some(Record { t: r.t, p: r.p, normal: r.normal, u: r.u, v: r.v, material: r.material, front_face: r.front_face != 0,
+                          obj_id: r.obj_id, prim_id: r.prim_id })
+        }).collect())
+    }
+
+    /// `Hittable::hit` for a single ray at time `time` with the whole record -- for drop-in tests; use `hit_records` for work.
+    pub fn hit_record(&self, ray: &Ray, time: f64, t_min: f64, t_max: f64) -> Result<Option<Record>> {
+        Ok(self.hit_records(std::slice::from_ref(ray), Some(std::slice::from_ref(&time)), t_min, t_max)?.pop().flatten())
     }
 
     /// Batched occlusion query (`yart_occluded`): `true` where the ray hits anything of the world in (t_min, t_max) --

@@ -206,6 +206,23 @@ typedef struct yart_hit {
   uint32_t _pad;
 } yart_hit;
 
+/* The whole HitRecord (hittable.rs:37-45) as world.hit returns it, plus the ids of yart_hit: for
+ * yart_closest_hit_records.  88 bytes. */
+typedef struct yart_hit_record {
+  double t;          /* HitRecord.t; +inf on a miss                                                    */
+  double p[3];       /* HitRecord.p: ray.at(t) in the primitive's space, then the wrappers' transforms   */
+                     /* (RotateY rotates it, Translate adds the offset); 0 on a miss                     */
+  double normal[3];  /* HitRecord.normal exactly as the reference stores it: face-oriented, NOT          */
+                     /* normalised (mesh / triangle: the interpolated vertex normals); 0 on a miss       */
+  double u, v;       /* TEXTURE coordinates: mesh / triangle: the interpolated uvs; sphere and moving    */
+                     /* sphere: get_sphere_uv; rect / box: the rect coordinates; medium: 0; 0 on a miss  */
+  uint32_t material; /* index into yart_scene_desc.materials (a group hit: the member's material);
+                        YART_MISS on a miss and for a mesh target (a bare mesh has no material)          */
+  uint32_t front_face;
+  uint32_t obj_id;   /* as yart_hit.obj_id; YART_MISS on a miss                                          */
+  uint32_t prim_id;  /* as yart_hit.prim_id; YART_MISS on a miss                                         */
+} yart_hit_record;
+
 /* Single-precision ray / hit records for yart_closest_hit_f32: 24 + 16 bytes per ray instead of 48 + 40. */
 typedef struct yart_ray_f32 {
   float origin[3];
@@ -402,6 +419,26 @@ int yart_closest_hit(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint6
 int yart_closest_hit_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* rays, uint64_t n,
                          float t_min, float t_max, uint32_t order, uint32_t flags,
                          yart_hit_f32* hits, yart_stats* stats /* may be NULL */);
+
+/* The same query returning the whole HitRecord (hittable.rs:37-45) -- p, the stored normal, the texture u, v and the
+ * material -- for hosts that shade on the CPU, and tracing each ray at its own Ray.time (ray.rs:4-9).
+ *   t, obj_id, prim_id and front_face equal yart_closest_hit's for the same rays, target, order, t_min and t_max when
+ *   `times` is NULL, bit for bit, in both orders and with all its documented quirks (constant media draw from the same
+ *   Philox stream: pixel = ray index, sample 0, bounce 1).
+ *   times: NULL (every ray at time 0, as yart_closest_hit traces) or n doubles, times[i] = ray i's Ray.time; it reaches
+ *   MovingSphere::hit / center(time) (sphere.rs:149-198) both in the traversal and in the record.
+ *   Every other field is what the reference's world.hit stores: wrappers applied (RotateY, Translate, FlipFace), the
+ *   mesh's interpolated normals and uvs, a group member's own material, the constant-medium record (p = ray.at(t),
+ *   normal (1,0,0), front_face 1, u = v = 0, the medium's phase-function material).  Sphere u, v are always computed.
+ *   Fields from a libm call differ from the reference's glibc by its last bits: sphere u, v (acos / atan2) and the t
+ *   and p of a constant-medium hit (log).
+ * flags: YART_FLAG_DEVICE_PTRS (rays, times and records are device arrays; rays 16-byte aligned, times and records
+ * 8-byte aligned) and YART_FLAG_COUNT_VISITS; any other bit is YART_ERR_INVALID.  Host arrays go through the chunk
+ * pipeline of yart_closest_hit, the times uploaded with the rays.  stats as in yart_closest_hit: the one record export
+ * launch per chunk counts in kernel_launches, not in trace_launches.  There is no f32 variant. */
+int yart_closest_hit_records(yart_ctx* ctx, uint32_t target, const yart_ray* rays, const double* times /* may be NULL */,
+                             uint64_t n, double t_min, double t_max, uint32_t order, uint32_t flags,
+                             yart_hit_record* records, yart_stats* stats /* may be NULL */);
 
 /* Batched occlusion query (Embree's rtcOccluded, an OptiX any-hit that terminates on the first hit): occluded[i] = 1
  * if ray i hits anything of `target` (a mesh index or YART_TARGET_WORLD) that yart_closest_hit(..., YART_ORDER_REFERENCE,

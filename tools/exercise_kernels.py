@@ -20,9 +20,10 @@ for scene, w, h, spp in (("david", 48, 32, 2), ("cornell-box-smoke", 32, 32, 2),
     film, st = ctx.render(cam, w, h, 0, spp, 50, 1)
     ctx.render(cam, w, h, 0, spp, 50, 1, flags=y.FLAG_NEXT_EVENT)
     rgba = ctx.film_finalize(film, spp)
-    rays, _, _ = ctx.camera_rays(cam, w, h, 0, 1)
+    rays, _, times = ctx.camera_rays(cam, w, h, 0, 1)
     for order in (0, 1):
         ctx.closest_hit(rays, y.TARGET_WORLD, 0.001, float("inf"), order, count_visits=True)
+        ctx.closest_hit_records(rays, times, y.TARGET_WORLD, 0.001, float("inf"), order)  # k_export_record
     ctx.occluded(rays, y.TARGET_WORLD, 0.001, float("inf"))  # k_occlude + k_analytic_occluded
     print(scene, st.rays, int(rgba.sum()))
 p = y.ScenePreset("david"); ctx.set_scene(p)
@@ -32,6 +33,7 @@ weird = y.make_rays([(0, 0, 0), (0, 0, 5), (np.nan, 0, 0), (0, 0, 5)], [(0, 0, 0
 for r in (rays, weird, rays[:1], rays[:33]):
     for order in (0, 1):
         ctx.closest_hit(r, 0, 0.0, float("inf"), order)
+        ctx.closest_hit_records(r, None, 0, 0.0, float("inf"), order)
     ctx.occluded(r, 0, 0.0, float("inf"))
 # round-2 entry points: f32 records, sampling flags, path-ray dump, device films + a one-rank communicator
 r32 = np.empty(len(rays), dtype=y.abi.RAY_F32_DTYPE)
@@ -78,6 +80,7 @@ for seed in range(6):
     o, d = sc.rays(20000)
     for order in (0, 1):
         ctx.closest_hit(y.make_rays(o, d), y.TARGET_WORLD, 0.001, float("inf"), order, count_visits=bool(order))
+        ctx.closest_hit_records(y.make_rays(o, d), np.linspace(0.0, 1.0, len(o)), y.TARGET_WORLD, 0.001, float("inf"), order)
     ctx.render(sc.camera(32, 24), 32, 24, 0, 3, 12, 1, flags=flags if seed % 2 else 0)
     ctx.render(sc.camera(32, 24), 32, 24, 0, 3, 12, 1, flags=y.FLAG_NEXT_EVENT)
 for seed, n_tris in ((1, 6), (2, 33), (3, 1000)):

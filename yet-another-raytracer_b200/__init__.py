@@ -19,8 +19,8 @@ import numpy as np
 
 from . import _abi as abi
 from ._abi import (FLAG_COUNT_VISITS, FLAG_DEPTH_ZERO_BLACK, FLAG_DEVICE_PTRS, FLAG_NEXT_EVENT, FLAG_RUSSIAN_ROULETTE,
-                   FLAG_UNBIASED_LIGHT_PICK, HIT_DTYPE, MISS, ORDER_NEAR, ORDER_REFERENCE, RAY_DTYPE, TARGET_WORLD,
-                   make_rays)
+                   FLAG_UNBIASED_LIGHT_PICK, HIT_DTYPE, MISS, ORDER_NEAR, ORDER_REFERENCE, RAY_DTYPE, RECORD_DTYPE,
+                   TARGET_WORLD, make_rays)
 
 PKG_DIR = Path(__file__).resolve().parent
 REPO_ROOT = PKG_DIR.parent
@@ -88,6 +88,7 @@ def load_library():
         "yart_ctx_set_scene": (i32, [vp, P(abi.SceneDesc)]),
         "yart_closest_hit": (i32, [vp, u32, vp, u64, f64, f64, u32, u32, vp, P(abi.Stats)]),
         "yart_closest_hit_f32": (i32, [vp, u32, vp, u64, C.c_float, C.c_float, u32, u32, vp, P(abi.Stats)]),
+        "yart_closest_hit_records": (i32, [vp, u32, vp, vp, u64, f64, f64, u32, u32, vp, P(abi.Stats)]),
         "yart_occluded": (i32, [vp, u32, vp, u64, f64, f64, u32, vp, P(abi.Stats)]),
         "yart_occluded_f32": (i32, [vp, u32, vp, u64, C.c_float, C.c_float, u32, vp, P(abi.Stats)]),
         "yart_render": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, P(abi.Stats)]),
@@ -125,6 +126,7 @@ EXPORTED_SYMBOLS = [
     "yart_comm_destroy", "yart_comm_info", "yart_comm_last_error", "yart_film_reduce", "yart_film_create",
     "yart_film_clear", "yart_film_read", "yart_film_destroy", "yart_preset_note", "yart_closest_hit_f32",
     "yart_dump_path_rays", "yart_host_register", "yart_host_unregister", "yart_occluded", "yart_occluded_f32",
+    "yart_closest_hit_records",
 ]
 
 
@@ -360,6 +362,38 @@ class Context:
         flags = FLAG_DEVICE_PTRS | (FLAG_COUNT_VISITS if count_visits else 0)
         self._check(_lib.yart_closest_hit_f32(self._h, target, C.c_void_p(rays_ptr), n, t_min, t_max, order, flags,
                                               C.c_void_p(hits_ptr), C.byref(st)))
+        return st
+
+    def closest_hit_records(self, rays, times=None, target=TARGET_WORLD, t_min=0.001, t_max=float("inf"),
+                            order=ORDER_REFERENCE, count_visits=False, out=None):
+        """The whole HitRecord per ray (yart_closest_hit_records) with host buffers: (RECORD_DTYPE array, stats).
+        times: None (every ray at time 0) or one f64 Ray.time per ray.  `out`: an optional preallocated (e.g. pinned)
+        RECORD_DTYPE array as long as rays."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        n = rays.shape[0]
+        if times is not None:
+            times = np.ascontiguousarray(times, dtype=np.float64)
+            if times.shape != (n,):
+                raise ValueError("times must hold one f64 per ray")
+        if out is None:
+            out = np.empty(n, dtype=RECORD_DTYPE)
+        elif out.dtype != RECORD_DTYPE or out.shape != (n,) or not out.flags.c_contiguous:
+            raise ValueError("out must be a contiguous RECORD_DTYPE array as long as rays")
+        st = abi.Stats()
+        flags = FLAG_COUNT_VISITS if count_visits else 0
+        self._check(_lib.yart_closest_hit_records(self._h, target, rays.ctypes.data,
+                                                  None if times is None else times.ctypes.data, n, t_min, t_max, order,
+                                                  flags, out.ctypes.data, C.byref(st)))
+        return out, st
+
+    def closest_hit_records_device(self, rays_ptr, times_ptr, n, out_ptr, target=TARGET_WORLD, t_min=0.001,
+                                   t_max=float("inf"), order=ORDER_REFERENCE, count_visits=False):
+        """Same with device pointers: rays (yart_ray), times (n f64, or 0 for every ray at time 0) and out
+        (yart_hit_record) on this context's GPU."""
+        st = abi.Stats()
+        flags = FLAG_DEVICE_PTRS | (FLAG_COUNT_VISITS if count_visits else 0)
+        self._check(_lib.yart_closest_hit_records(self._h, target, C.c_void_p(rays_ptr), C.c_void_p(times_ptr or None), n,
+                                                  t_min, t_max, order, flags, C.c_void_p(out_ptr), C.byref(st)))
         return st
 
     def host_register(self, array):

@@ -104,11 +104,14 @@ class PresetInfo(C.Structure):
                 ("output_filename", C.c_char * 64)]
 
 
-# numpy views of the two array-of-struct types that cross the ABI in bulk
+# numpy views of the array-of-struct types that cross the ABI in bulk
 RAY_DTYPE = np.dtype([("origin", "<f8", 3), ("direction", "<f8", 3)])
 HIT_DTYPE = np.dtype([("t", "<f8"), ("u", "<f8"), ("v", "<f8"), ("prim_id", "<u4"), ("obj_id", "<u4"),
                       ("front_face", "<u4"), ("_pad", "<u4")])
 assert RAY_DTYPE.itemsize == 48 and HIT_DTYPE.itemsize == 40
+RECORD_DTYPE = np.dtype([("t", "<f8"), ("p", "<f8", 3), ("normal", "<f8", 3), ("u", "<f8"), ("v", "<f8"),
+                         ("material", "<u4"), ("front_face", "<u4"), ("obj_id", "<u4"), ("prim_id", "<u4")])
+assert RECORD_DTYPE.itemsize == 88
 RAY_F32_DTYPE = np.dtype([("origin", "<f4", 3), ("direction", "<f4", 3)])
 HIT_F32_DTYPE = np.dtype([("t", "<f4"), ("u", "<f4"), ("v", "<f4"), ("prim_id", "<u4")])
 assert RAY_F32_DTYPE.itemsize == 24 and HIT_F32_DTYPE.itemsize == 16

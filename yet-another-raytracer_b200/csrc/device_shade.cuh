@@ -102,14 +102,19 @@ YART_DEV void rect_record(int kaxis, double a0, double a1, double b0, double b1,
     rec.normal = -outward; rec.front_face = false;
   }
 }
-// record of an un-wrapped primitive in its own space
+// record of an un-wrapped primitive in its own space.  ALL_UV = false: the renderer's record, which leaves a sphere's u, v
+// at 0 where its material cannot read them; true: every field as the reference computes it (yart_closest_hit_records).
+template <bool ALL_UV = false>
 YART_DEV void prim_record(const DevScene& S, const yart_object& o, D3 ro, D3 rd, double time, double t, uint32_t prim,
                           double bu, double bv, HitRec& rec) {
   rec.t = t;
   rec.material = o.material;
   // get_sphere_uv (acos + atan2) only feeds ImageTexture::value; skip it when this material cannot read u, v
-  const yart_material& pm = S.materials[o.material];
-  const bool need_uv = pm.kind != YART_MAT_NONE && pm.kind != YART_MAT_DIELECTRIC && S.textures[pm.texture].kind == YART_TEX_IMAGE;
+  bool need_uv = true;
+  if (!ALL_UV) {
+    const yart_material& pm = S.materials[o.material];
+    need_uv = pm.kind != YART_MAT_NONE && pm.kind != YART_MAT_DIELECTRIC && S.textures[pm.texture].kind == YART_TEX_IMAGE;
+  }
   switch (o.kind) {
     case YART_OBJ_SPHERE: { // sphere.rs:68-85
       const D3 center = d3(o.p[0], o.p[1], o.p[2]);
@@ -188,7 +193,8 @@ YART_DEV void prim_record(const DevScene& S, const yart_object& o, D3 ro, D3 rd,
   }
 }
 
-// the HitRecord world.hit returns for (object, t): wrappers applied outside-in
+// the HitRecord world.hit returns for (object, t): wrappers applied outside-in (ALL_UV: as for prim_record)
+template <bool ALL_UV = false>
 YART_DEV void world_record(const DevScene& S, const DevHit& h, D3 wo, D3 wd, double time, HitRec& rec) {
   const yart_object& o = S.objects[h.obj];
   if (o.wrap & YART_WRAP_MEDIUM) { // hittable.rs:296-308
@@ -204,9 +210,9 @@ YART_DEV void world_record(const DevScene& S, const DevHit& h, D3 wo, D3 wd, dou
   to_object_space(o, ro, rd);
   if (o.kind == YART_OBJ_GROUP) {
     const DevGroup g = S.groups[o.index];
-    prim_record(S, g.members[h.prim >> 3], ro, rd, time, h.t, h.prim & 7u, h.bu, h.bv, rec);
+    prim_record<ALL_UV>(S, g.members[h.prim >> 3], ro, rd, time, h.t, h.prim & 7u, h.bu, h.bv, rec);
   } else {
-    prim_record(S, o, ro, rd, time, h.t, h.prim, h.bu, h.bv, rec);
+    prim_record<ALL_UV>(S, o, ro, rd, time, h.t, h.prim, h.bu, h.bv, rec);
   }
   if (o.wrap & YART_WRAP_FLIP_FACE) rec.front_face = !rec.front_face;
   if (o.wrap & YART_WRAP_ROTATE_Y) { // hittable.rs:232-246

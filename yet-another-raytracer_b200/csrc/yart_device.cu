@@ -1,5 +1,5 @@
 // yart_device.cu -- the device half of the C ABI (include/yart.h): context, scene upload,
-// yart_closest_hit, yart_occluded, yart_render, yart_film_finalize, yart_generate_camera_rays.
+// yart_closest_hit, yart_closest_hit_records, yart_occluded, yart_render, yart_film_finalize, yart_generate_camera_rays.
 //
 // There is no CPU fallback anywhere in this file: every entry point launches the sm_100a
 // kernels of device_trace.cuh / device_shade.cuh or fails with YART_ERR_CUDA.
@@ -21,6 +21,15 @@
 #include "host_common.h"
 
 namespace yart {
+
+// yart_hit.prim_id of a hit on object o: 0 for a medium, the ORIGINAL triangle index of a mesh (FlatTri.orig), the
+// member's index in its yart_group for a group, else the primitive's own id
+YART_DEV uint32_t export_prim_id(const DevScene& S, const yart_object& o, uint32_t prim) {
+  if (o.wrap & YART_WRAP_MEDIUM) return 0;
+  if (o.kind == YART_OBJ_MESH) return __float_as_uint(__ldg(S.meshes[o.index].tris + (size_t)prim * 3).w);
+  if (o.kind == YART_OBJ_GROUP) return S.groups[o.index].member_orig[prim >> 3];
+  return prim;
+}
 
 // ---------------------------------------------------------------------------------------------
 // k_export: DevHit -> yart_hit for yart_closest_hit: original triangle id and front_face as the
@@ -44,16 +53,7 @@ __global__ void __launch_bounds__(256) k_export(const DevScene S, const yart_ray
     HitRec rec; // rebuild the HitRecord of this object to get front_face exactly as the reference computes it
     world_record(S, h, wo, wd, 0.0, rec);
     out.t = h.t; out.u = h.bu; out.v = h.bv; out.obj_id = h.obj; out.front_face = rec.front_face ? 1u : 0u; out._pad = 0;
-    if (o.wrap & YART_WRAP_MEDIUM) {
-      out.prim_id = 0;
-    } else if (o.kind == YART_OBJ_MESH) {
-      const DevMesh m = S.meshes[o.index];
-      out.prim_id = __float_as_uint(__ldg(m.tris + (size_t)h.prim * 3).w); // FlatTri.orig
-    } else if (o.kind == YART_OBJ_GROUP) {
-      out.prim_id = S.groups[o.index].member_orig[h.prim >> 3];
-    } else {
-      out.prim_id = h.prim;
-    }
+    out.prim_id = export_prim_id(S, o, h.prim);
     out_hits[i] = out;
   }
 }
@@ -67,14 +67,42 @@ __global__ void __launch_bounds__(256) k_export_f32(const DevScene S, const yart
     if (h.obj == YART_MISS) {
       out.t = __int_as_float(0x7f800000); out.u = 0.f; out.v = 0.f; out.prim_id = YART_MISS;
     } else {
-      const yart_object& o = objects[h.obj];
       out.t = (float)h.t; out.u = (float)h.bu; out.v = (float)h.bv;
-      if (o.wrap & YART_WRAP_MEDIUM) out.prim_id = 0;
-      else if (o.kind == YART_OBJ_MESH) out.prim_id = __float_as_uint(__ldg(S.meshes[o.index].tris + (size_t)h.prim * 3).w);
-      else if (o.kind == YART_OBJ_GROUP) out.prim_id = S.groups[o.index].member_orig[h.prim >> 3];
-      else out.prim_id = h.prim;
+      out.prim_id = export_prim_id(S, objects[h.obj], h.prim);
     }
     out_hits[i] = out;
+  }
+}
+
+// yart_closest_hit_records: DevHit -> the whole yart_hit_record, rebuilt at each ray's own time (times may be null:
+// time 0) with every field the reference computes (world_record<true>).  A mesh target has no material.
+__global__ void __launch_bounds__(256) k_export_record(const DevScene S, const yart_ray* rays, const double* times,
+                                                        const DevHit* hits, yart_hit_record* out_recs, uint64_t n,
+                                                        uint32_t mesh_target) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+    const DevHit h = hits[i];
+    yart_hit_record out;
+    if (h.obj == YART_MISS) {
+      out.t = d_inf();
+      for (int k = 0; k < 3; ++k) { out.p[k] = 0.0; out.normal[k] = 0.0; }
+      out.u = 0.0; out.v = 0.0;
+      out.material = YART_MISS; out.front_face = 0; out.obj_id = YART_MISS; out.prim_id = YART_MISS;
+      out_recs[i] = out;
+      continue;
+    }
+    D3 wo, wd;
+    load_ray(rays + i, wo, wd);
+    HitRec rec;
+    world_record<true>(S, h, wo, wd, times ? times[i] : 0.0, rec);
+    out.t = rec.t;
+    out.p[0] = rec.p.x; out.p[1] = rec.p.y; out.p[2] = rec.p.z;
+    out.normal[0] = rec.normal.x; out.normal[1] = rec.normal.y; out.normal[2] = rec.normal.z;
+    out.u = rec.u; out.v = rec.v;
+    out.material = mesh_target ? YART_MISS : rec.material;
+    out.front_face = rec.front_face ? 1u : 0u;
+    out.obj_id = h.obj;
+    out.prim_id = export_prim_id(S, S.objects[h.obj], h.prim);
+    out_recs[i] = out;
   }
 }
 
@@ -390,6 +418,7 @@ struct yart_ctx {
   DevBuf rays, hits_export, time, wavelength, throughput, hits, queue_a, queue_b, counts, work, counters, film, rgba;
   DevBuf nee_rays, nee_pending, nee_sum, nee_w, queue_s; // YART_FLAG_NEXT_EVENT's per-path state (NeeState)
   DevBuf occluded; // staging of yart_occluded's flags for host arrays
+  DevBuf ray_times; // staging of yart_closest_hit_records' ray times for host arrays
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> ev_pool;
   // host-buffer closest-hit queries: copy streams + events of the chunk pipeline (made on first use)
@@ -688,9 +717,12 @@ int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launch
 // run(off, len) enqueues on ctx->stream the kernels that read the ray records at d_in + off * in_bytes and leave
 // out_bytes per ray at d_out + off * out_bytes.  Everything is enqueued on return; after a synchronisation of
 // ctx->stream, chunked_kernel_ms gives the kernels' time.
+// An optional second per-ray input (in2, in2_bytes per ray; null = none) goes up with the rays, chunk by chunk on the
+// same copy stream, into d_in2 (host arrays only: with device arrays run() reads it where it is).
 template <class Run>
 int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* out, size_t out_bytes, uint64_t n,
-                const char* d_in, char* d_out, Run&& run, uint64_t* n_chunks_out) {
+                const char* d_in, char* d_out, Run&& run, uint64_t* n_chunks_out, const void* in2 = nullptr,
+                size_t in2_bytes = 0, char* d_in2 = nullptr) {
   const int chunk_env = tune_env("YART_TUNE_HOST_CHUNK", 1 << 19); // (rays per chunk, read per call; 2^19 measured best: tools/host_chunk_probe.py)
   const uint64_t chunk = dev ? n : (uint64_t)std::max(chunk_env, 1024);
   const uint64_t n_chunks = (n + chunk - 1) / chunk;
@@ -698,6 +730,7 @@ int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* 
   char* stage_in = const_cast<char*>(d_in); // (host arrays: d_in is the context's staging buffer)
   if (dev || n_chunks == 1) {
     if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(stage_in, in, n * in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (!dev && in2) CUDA_TRY(ctx, cudaMemcpyAsync(d_in2, in2, n * in2_bytes, cudaMemcpyHostToDevice, ctx->stream));
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream)); // (stats->gpu_ms: the kernels, not the copies)
     const int rc = run(0, n);
     if (rc) return rc;
@@ -722,6 +755,9 @@ int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* 
       const uint64_t off = i * chunk, len = std::min(chunk, n - off);
       CUDA_TRY(ctx, cudaMemcpyAsync(stage_in + off * in_bytes, static_cast<const char*>(in) + off * in_bytes,
                                     len * in_bytes, cudaMemcpyHostToDevice, ctx->copy_in));
+      if (in2)
+        CUDA_TRY(ctx, cudaMemcpyAsync(d_in2 + off * in2_bytes, static_cast<const char*>(in2) + off * in2_bytes,
+                                      len * in2_bytes, cudaMemcpyHostToDevice, ctx->copy_in));
       CUDA_TRY(ctx, cudaEventRecord(up[i], ctx->copy_in));
       return YART_OK;
     };
@@ -832,7 +868,7 @@ void yart_ctx_destroy(yart_ctx* ctx) {
   ctx->free_scene();
   DevBuf* bufs[] = {&ctx->rays, &ctx->hits_export, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits,
                     &ctx->queue_a, &ctx->queue_b, &ctx->counts, &ctx->work, &ctx->counters, &ctx->film, &ctx->rgba,
-                    &ctx->occluded};
+                    &ctx->occluded, &ctx->ray_times};
   for (DevBuf* b : bufs) b->release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->chunk_events) cudaEventDestroy(e);
@@ -1258,9 +1294,13 @@ int yart_ctx_set_scene(yart_ctx* ctx, const yart_scene_desc* d) {
   YART_ABI_GUARD_END(ctx, "yart_ctx_set_scene")
 }
 
-static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bool f32, uint64_t n, double t_min, double t_max,
-                            uint32_t order, uint32_t flags, void* hits, yart_stats* stats) {
-  const char* fn = f32 ? "yart_closest_hit_f32" : "yart_closest_hit";
+// What a closest-hit query returns per ray: yart_hit, yart_hit_f32 (from f32 rays) or yart_hit_record.
+enum class HitFormat { F64, F32, RECORD };
+
+static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, const double* times, HitFormat fmt, uint64_t n,
+                            double t_min, double t_max, uint32_t order, uint32_t flags, void* hits, yart_stats* stats) {
+  const bool f32 = fmt == HitFormat::F32, record = fmt == HitFormat::RECORD;
+  const char* fn = f32 ? "yart_closest_hit_f32" : (record ? "yart_closest_hit_records" : "yart_closest_hit");
   if (!ctx->have_scene) {
     ctx->err = std::string(fn) + ": no scene (call yart_ctx_set_scene first)";
     return YART_ERR_INVALID;
@@ -1269,9 +1309,17 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bo
     ctx->err = std::string(fn) + ": bad argument";
     return YART_ERR_INVALID;
   }
+  if (record && (flags & ~(uint32_t)(YART_FLAG_DEVICE_PTRS | YART_FLAG_COUNT_VISITS))) {
+    ctx->err = std::string(fn) + ": the only flags it takes are YART_FLAG_DEVICE_PTRS and YART_FLAG_COUNT_VISITS";
+    return YART_ERR_INVALID;
+  }
   const uintptr_t ray_align = f32 ? 7u : 15u, hit_align = f32 ? 3u : 7u;
   if ((flags & YART_FLAG_DEVICE_PTRS) && ((reinterpret_cast<uintptr_t>(rays) & ray_align) || (reinterpret_cast<uintptr_t>(hits) & hit_align))) {
     ctx->err = std::string(fn) + (f32 ? ": device ray arrays must be 8-byte aligned (hits: 4)" : ": device ray arrays must be 16-byte aligned (hits: 8)");
+    return YART_ERR_INVALID;
+  }
+  if ((flags & YART_FLAG_DEVICE_PTRS) && (reinterpret_cast<uintptr_t>(times) & 7u)) {
+    ctx->err = std::string(fn) + ": device time arrays must be 8-byte aligned";
     return YART_ERR_INVALID;
   }
   if (target != YART_TARGET_WORLD && target >= ctx->n_meshes) {
@@ -1281,16 +1329,22 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bo
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if (stats) memset(stats, 0, sizeof(*stats));
   if (n == 0) return YART_OK;
-  const size_t ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray), hit_bytes = f32 ? sizeof(yart_hit_f32) : sizeof(yart_hit);
+  const size_t ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray);
+  const size_t hit_bytes = f32 ? sizeof(yart_hit_f32) : (record ? sizeof(yart_hit_record) : sizeof(yart_hit));
   const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
   const bool count = (flags & YART_FLAG_COUNT_VISITS) != 0;
   const char* d_rays = static_cast<const char*>(rays);
   char* d_hits = static_cast<char*>(hits);
+  const double* d_times = times;
   if (!dev) {
     CUDA_TRY(ctx, ctx->rays.reserve(n * ray_bytes));
     CUDA_TRY(ctx, ctx->hits_export.reserve(n * hit_bytes));
     d_rays = ctx->rays.as<char>();
     d_hits = ctx->hits_export.as<char>();
+    if (times) {
+      CUDA_TRY(ctx, ctx->ray_times.reserve(n * sizeof(double)));
+      d_times = ctx->ray_times.as<double>();
+    }
   }
   const uint32_t n_list = (target == YART_TARGET_WORLD) ? ctx->scene.n_objects : 1u;
   const size_t work_bytes = ((size_t)n_list + 2) * sizeof(uint32_t);
@@ -1337,11 +1391,16 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bo
     q.c.n_rays = (uint32_t)len;
     q.c.hits = ctx->hits.as<DevHit>() + off;
     q.pixel_base = (uint32_t)off; // (keeps a ray's Philox stream = its index in the caller's array)
+    q.ray_time = d_times ? d_times + off : nullptr;
     const int rc = run_passes(ctx, q, &launches);
     if (rc) return rc;
     if (f32)
       k_export_f32<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, export_scene.objects, q.c.hits,
                                                                reinterpret_cast<yart_hit_f32*>(d_hits + off * hit_bytes), len);
+    else if (record)
+      k_export_record<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, q.c.rays, q.ray_time, q.c.hits,
+                                                                  reinterpret_cast<yart_hit_record*>(d_hits + off * hit_bytes), len,
+                                                                  target != YART_TARGET_WORLD ? 1u : 0u);
     else
       k_export<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, q.c.rays, q.c.hits,
                                                            reinterpret_cast<yart_hit*>(d_hits + off * hit_bytes), len);
@@ -1350,7 +1409,8 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, bo
     return YART_OK;
   };
   uint64_t n_chunks = 0;
-  const int rc = run_chunked(ctx, dev, rays, ray_bytes, hits, hit_bytes, n, d_rays, d_hits, run_range, &n_chunks);
+  const int rc = run_chunked(ctx, dev, rays, ray_bytes, hits, hit_bytes, n, d_rays, d_hits, run_range, &n_chunks, times,
+                             sizeof(double), ctx->ray_times.as<char>());
   if (rc) return rc;
   unsigned long long c[2] = {0, 0};
   if (count) CUDA_TRY(ctx, cudaMemcpyAsync(c, ctx->counters.p, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1374,7 +1434,7 @@ int yart_closest_hit(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint6
                      uint32_t order, uint32_t flags, yart_hit* hits, yart_stats* stats) {
   if (!ctx) return YART_ERR_INVALID;
   YART_ABI_GUARD_BEGIN
-  return closest_hit_impl(ctx, target, rays, false, n, t_min, t_max, order, flags, hits, stats);
+  return closest_hit_impl(ctx, target, rays, nullptr, HitFormat::F64, n, t_min, t_max, order, flags, hits, stats);
   YART_ABI_GUARD_END(ctx, "yart_closest_hit")
 }
 
@@ -1382,8 +1442,16 @@ int yart_closest_hit_f32(yart_ctx* ctx, uint32_t target, const yart_ray_f32* ray
                          uint32_t order, uint32_t flags, yart_hit_f32* hits, yart_stats* stats) {
   if (!ctx) return YART_ERR_INVALID;
   YART_ABI_GUARD_BEGIN
-  return closest_hit_impl(ctx, target, rays, true, n, (double)t_min, (double)t_max, order, flags, hits, stats);
+  return closest_hit_impl(ctx, target, rays, nullptr, HitFormat::F32, n, (double)t_min, (double)t_max, order, flags, hits, stats);
   YART_ABI_GUARD_END(ctx, "yart_closest_hit_f32")
+}
+
+int yart_closest_hit_records(yart_ctx* ctx, uint32_t target, const yart_ray* rays, const double* times, uint64_t n, double t_min,
+                             double t_max, uint32_t order, uint32_t flags, yart_hit_record* records, yart_stats* stats) {
+  if (!ctx) return YART_ERR_INVALID;
+  YART_ABI_GUARD_BEGIN
+  return closest_hit_impl(ctx, target, rays, times, HitFormat::RECORD, n, t_min, t_max, order, flags, records, stats);
+  YART_ABI_GUARD_END(ctx, "yart_closest_hit_records")
 }
 
 static int occluded_impl(yart_ctx* ctx, uint32_t target, const void* rays, bool f32, uint64_t n, double t_min, double t_max,
