@@ -4,7 +4,6 @@ must be IDENTICAL -- the kernel does the reference's f64 arithmetic in the refer
 losslessly stored f32 geometry (north_star asks for exact prim id and 1e-5 relative t).
 """
 import os
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -177,34 +176,6 @@ def test_full_size_sweep_properties(yart, orc, ctx, mesh_scene):
     idx = np.random.Generator(np.random.Philox(3)).choice(n, 1 << 16, replace=False)
     want, _ = s.closest_hit(rays[idx], 0, 0.0, INF, 0, n_threads=os.cpu_count())
     assert_same_hits(a[idx], want, "subset")
-
-
-def test_all_f64_slab_path_gives_the_same_hits(yart, orc, mesh_scene, tmp_path):
-    """YART_TUNE_MIXED=0 selects the all-f64 slab tests (no conservative f32 stage).  It must return exactly what
-    the default mixed-precision kernel returns -- run it in a fresh process (the knob is read once)."""
-    import subprocess
-    import sys
-    _, ms, s = mesh_scene("sycee")
-    rays = mesh_rays(orc, s.qbvh_info(0), 100000, seed_shift=9)
-    want, _ = s.closest_hit(rays, 0, 0.001, INF, 0, n_threads=os.cpu_count())
-    np.save(tmp_path / "rays.npy", rays)
-    code = (
-        "import importlib, sys, numpy as np\n"
-        "sys.path.insert(0, %r)\n"
-        "from oracle import orc\n"
-        "y = importlib.import_module('yet-another-raytracer_b200')\n"
-        "m = y.TriangleMesh.from_obj(y.assets_dir() + '/sycee.obj')\n"
-        "ms = orc.MeshScene(m.positions(), m.normals(), m.uvs())\n"
-        "ctx = y.Context(0); ctx.set_scene(ms.desc)\n"
-        "rays = np.load(%r)\n"
-        "for order in (0, 1):\n"
-        "    hits, st = ctx.closest_hit(rays, 0, 0.001, float('inf'), order, count_visits=True)\n"
-        "    np.save(%r %% order, hits)\n"
-    ) % (str(Path(__file__).resolve().parent.parent), str(tmp_path / "rays.npy"), str(tmp_path / "hits%d.npy"))
-    env = dict(os.environ, YART_TUNE_MIXED="0")
-    subprocess.run([sys.executable, "-c", code], check=True, env=env)
-    for order in (0, 1):
-        assert_same_hits(np.load(tmp_path / ("hits%d.npy" % order)), want, "f64 path order %d" % order)
 
 
 def test_fetch_peak_diagnostic(yart, ctx):

@@ -472,35 +472,6 @@ def test_one_process_per_gpu_comm_from_id(yart, ctx, tmp_path):
 
 
 # ---------------------------------------------------------------------------------------------------------
-# the compact-node experiment (YART_TUNE_COMPACT=1): off by default because it is slower, but it has to stay bit-exact
-# ---------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("name", ["sycee", "david"])
-def test_compact_nodes_are_bit_identical(yart, orc, ctx, mesh_scene, name, monkeypatch):
-    _, ms, s = mesh_scene(name)
-    info = s.qbvh_info(0)
-    lo, hi = np.array(info.bbox_min), np.array(info.bbox_max)
-    o, d = raysets.uniform(400000, lo, hi, 77)
-    o2, d2 = raysets.axis(20000, lo, hi, 5)
-    rays = orc.abi.make_rays(np.concatenate([o, o2]), np.concatenate([d, d2]))
-    want, _ = s.closest_hit(rays, 0, 0.001, INF, yart.ORDER_REFERENCE, n_threads=os.cpu_count())
-    monkeypatch.setenv("YART_TUNE_COMPACT", "2")  # 2: pack even where the grid is coarse against the triangles
-    ctx.set_scene(ms.desc)
-    try:
-        got, st = ctx.closest_hit(rays, 0, 0.001, INF, yart.ORDER_NEAR)
-        for f in ("prim_id", "t", "u", "v"):
-            assert np.array_equal(got[f], want[f]), f
-        # rays that start far outside, graze the bounding box, or run along a grid plane
-        far = orc.abi.make_rays(o * 1000.0, -o * 1000.0 + (lo + hi) / 2)
-        w2, _ = s.closest_hit(far, 0, 0.0, INF, yart.ORDER_REFERENCE, n_threads=os.cpu_count())
-        g2, _ = ctx.closest_hit(far, 0, 0.0, INF, yart.ORDER_NEAR)
-        for f in ("prim_id", "t", "u", "v"):
-            assert np.array_equal(g2[f], w2[f]), f
-    finally:
-        monkeypatch.delenv("YART_TUNE_COMPACT")
-        ctx.set_scene(ms.desc)
-
-
-# ---------------------------------------------------------------------------------------------------------
 # host-buffer queries run as a chunk pipeline (upload / kernels / download overlapped): same answers as one piece
 # ---------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("scene", ["cornell-box-smoke", "david"])

@@ -111,8 +111,7 @@ def test_random_scene_sampling_flags_and_f32_records(yart, orc, ctx, seed):
 
 
 @pytest.mark.parametrize("seed,n_tris", [(s, n) for s, n in enumerate([5, 6, 7, 8, 9, 12, 13, 16, 17, 31, 33, 64, 100, 257, 1000, 3001, 20000, 4, 11, 500])])
-@pytest.mark.parametrize("compact", [0, 2])
-def test_random_soup_build_and_closest_hit(yart, orc, ctx, seed, n_tris, compact, monkeypatch):
+def test_random_soup_build_and_closest_hit(yart, orc, ctx, seed, n_tris):
     """Random triangle soups: device-built tree == host-built tree byte for byte, and L4QBVH::hit bit-exact against the
     oracle (both orders, with and without visit counting, two [t_min, t_max] windows)."""
     from scene_fuzz import fuzz_soup, fuzz_mesh_rays
@@ -128,7 +127,6 @@ def test_random_soup_build_and_closest_hit(yart, orc, ctx, seed, n_tris, compact
     assert_same_tree(yart, ctx, t, keep)
     ms = orc.MeshScene(pos, nrm, uv)
     s = orc.Scene(ms)
-    monkeypatch.setenv("YART_TUNE_COMPACT", str(compact))  # 2: the compact-node experiment, on whatever the grid is like
     ctx.set_scene(ms.desc)
     o, d = fuzz_mesh_rays(seed, pos, 40000)
     rays = yart.make_rays(o, d)

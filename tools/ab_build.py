@@ -36,8 +36,8 @@ def one(spec):
     info = []
     lines = text.splitlines()
     for i, ln in enumerate(lines):
-        if "Compiling entry function" in ln and ("k_traverseILb1ELb0ELi32ELb1E" in ln or "k_shade" in ln or "k_traverseILb1ELb0ELi24ELb1E" in ln):
-            name = "k_shade" if "k_shade" in ln else "k_traverse<near>"
+        if "Compiling entry function" in ln and ("k_traverseILb0ELb0ELi32E" in ln or "k_shade" in ln):
+            name = "k_shade" if "k_shade" in ln else "k_traverse<reference>"
             info.append("%s: %s | %s" % (name, lines[i + 2].strip() if i + 2 < len(lines) else "", lines[i + 3].strip() if i + 3 < len(lines) else ""))
     return tag, "\n  ".join(info)
 

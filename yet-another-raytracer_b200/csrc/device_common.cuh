@@ -149,13 +149,22 @@ struct DevMesh {
   uint32_t max_stack;
   uint32_t n_nodes, n_tris;
   double bound[3];      // max |coordinate| per axis
-  // Compact nodes (k_pack_nodes): the same tree, node for node, as 64-byte records -- the 24 box planes as 16-bit
-  // offsets from the mesh's bounding-box corner in units of cscale (lower planes rounded down, upper planes up: the
-  // quantised box CONTAINS the exact one and is at most one unit larger on each side) + the four child words.
-  // Null when the mesh is not eligible (see set_scene).
-  const uint4* cnodes;
-  float corigin[3];     // the corner (an exact f32)
-  float cscale;         // 2^e
+};
+
+// The mesh instance one pass of a traversal kernel (k_traverse, k_traverse_lean, k_occlude) walks: the tree of its
+// DevMesh, the instance's wrappers, and the scheduling of the persistent kernels.
+struct MeshPass {
+  const float4* nodes;
+  const float4* tris;
+  const float4* leafgeo;      // packed per-leaf vertex blocks (DevMesh::leafgeo)
+  uint32_t root;
+  uint32_t n_nodes, n_tris;   // array lengths (bounds-checked build)
+  uint32_t wrap;              // YART_WRAP_ROTATE_Y / TRANSLATE of this instance
+  double sin_theta, cos_theta, offset[3];
+  double bound[3];            // max |coordinate| of the mesh per axis (for the f32 slab error bound)
+  uint32_t refill_threshold;  // run the retire/fetch phase once this many lanes wait for it
+  uint32_t node_threshold;    // leave the inner-node loop once fewer lanes than this are in it
+  uint32_t* work_counter;     // zero before launch
 };
 
 // A flat 4-wide tree over the members of a BVHNode group (spheres / boxes).  Same 128-byte node

@@ -17,17 +17,7 @@ struct OccludeCommon {
 // one mesh instance (k_occlude)
 struct OccludeParams {
   OccludeCommon c;
-  const float4* nodes;
-  const float4* tris;
-  const float4* leafgeo;      // packed per-leaf vertex blocks (DevMesh::leafgeo)
-  uint32_t root;
-  uint32_t wrap;              // YART_WRAP_ROTATE_Y / TRANSLATE of this instance
-  uint32_t refill_threshold;  // run the retire/fetch phase once this many lanes wait for it
-  uint32_t node_threshold;    // leave the inner-node loop once fewer lanes than this are in it
-  uint32_t n_nodes, n_tris;   // array lengths (bounds-checked build)
-  double sin_theta, cos_theta, offset[3];
-  double bound[3];            // max |coordinate| of the mesh per axis (for the f32 slab error bound)
-  uint32_t* work_counter;     // zero before launch
+  MeshPass m;
 };
 
 // a run of consecutive analytic / media-wrapped objects of the world list (k_analytic_occluded)

@@ -103,10 +103,10 @@ YART_DEV bool triangle_t(const double* p, D3 ro, D3 rd, double t_min, double t_m
 }
 
 // ray into the space of Translate(RotateY(.)) (hittable.rs:137-143, 218-227)
-YART_DEV void to_object_space(const yart_object& o, D3& ro, D3& rd) {
-  if (o.wrap & YART_WRAP_TRANSLATE) ro = ro - d3(o.offset[0], o.offset[1], o.offset[2]);
-  if (o.wrap & YART_WRAP_ROTATE_Y) {
-    const double ct = o.cos_theta, st = o.sin_theta;
+YART_DEV void instance_to_object(uint32_t wrap, const double* offset, double sin_theta, double cos_theta, D3& ro, D3& rd) {
+  if (wrap & YART_WRAP_TRANSLATE) ro = ro - d3(offset[0], offset[1], offset[2]);
+  if (wrap & YART_WRAP_ROTATE_Y) {
+    const double ct = cos_theta, st = sin_theta;
     D3 org = ro, dir = rd;
     org.x = ct * ro.x - st * ro.z;
     org.z = st * ro.x + ct * ro.z;
@@ -115,6 +115,9 @@ YART_DEV void to_object_space(const yart_object& o, D3& ro, D3& rd) {
     ro = org;
     rd = dir;
   }
+}
+YART_DEV void to_object_space(const yart_object& o, D3& ro, D3& rd) {
+  instance_to_object(o.wrap, o.offset, o.sin_theta, o.cos_theta, ro, rd);
 }
 
 // one primitive record without wrappers; `prim` encodes what the shade stage needs
@@ -279,21 +282,8 @@ struct PassCommon {
 
 struct TraverseParams {
   PassCommon c;
-  const float4* nodes;
-  const float4* tris;
-  const float4* leafgeo;      // packed per-leaf vertex blocks (DevMesh::leafgeo)
-  const uint4* cnodes;        // compact 64-byte nodes (DevMesh::cnodes), null = not available
-  float corigin[3], cscale;
-  uint32_t root;
+  MeshPass m;
   uint32_t obj_index;         // world object index recorded with a hit
-  uint32_t wrap;              // YART_WRAP_ROTATE_Y / TRANSLATE of this instance
-  uint32_t refill_threshold;  // run the retire/fetch phase once this many lanes wait for it
-  uint32_t node_threshold;    // leave the inner-node loop once fewer lanes than this are in it
-  uint32_t _pad;
-  uint32_t n_nodes, n_tris;   // array lengths (bounds-checked build)
-  double sin_theta, cos_theta, offset[3];
-  double bound[3];            // max |coordinate| of the mesh per axis (for the f32 slab error bound)
-  uint32_t* work_counter;     // zero before launch
   unsigned long long* counters; // [0] node visits, [1] triangle tests, [2] exact-fallback nodes (COUNT only)
 };
 
@@ -311,11 +301,6 @@ struct AnalyticParams {
   uint32_t media_mask;
   uint32_t _pad;
 };
-
-// min / max for values that cannot be NaN: one DSETP + selects instead of the IEEE minNum/maxNum
-// sequence (DSETP.MIN + SEL + FSEL + NaN quieting) the compiler emits for fmin/fmax on doubles
-YART_DEV double min_nn(double a, double b) { return a < b ? a : b; }
-YART_DEV double max_nn(double a, double b) { return a > b ? a : b; }
 
 // The four slab tests of one node exactly as qbvh.rs:495-519 with IEEE minNum/maxNum folds -- the
 // path for rays with a zero or non-finite component, whose slabs can be NaN (0 * inf).  Out of line:
@@ -347,69 +332,360 @@ __device__ __noinline__ uint32_t box4_ieee(const float4* nd, double ox, double o
 }
 
 // ---------------------------------------------------------------------------------------------
+// the steps of the QBVH walk (qbvh.rs:381-543) that k_traverse, k_traverse_lean and k_occlude share
+// ---------------------------------------------------------------------------------------------
+// Phase A's hand-out of work items to the lanes of a persistent warp.
+// Work distribution: warp w starts with items [32w, 32w+32) without touching the counter and only then
+// fetches dynamically from total_warps*32 + atomicAdd(counter).  Warps whose first slice is already past
+// the end leave at once -- a nearly empty queue (the deep bounces) costs no same-address atomics.
+// A short queue is spread thinly (rpw < 32 rays per warp): a warp's run time is the serialised work of
+// its most divergent rays, so a deep bounce with a few hundred rays finishes sooner on many warps.
+// Work items reach the lanes through a two-deep pipeline of 32-item chunks, so that neither the claim
+// (an atomic), nor the queue read, nor the DRAM miss of the ray record sits on the warp's critical path:
+//   chunk "cur": ids held one per lane (id_cur), handed to fetching lanes by shuffle;
+//   chunk "nxt": claimed when cur was started (stage 1: atomic in flight), ids loaded one retire/fetch phase
+//   later (stage 2), ray / hit records prefetched into L2 the phase after (stage 3).
+// The first chunk of a warp is its static slice; all later ones come from the global counter.  Item counts are
+// 32-bit: yart_closest_hit and yart_occluded cap n below 2^32, the renderer's queues hold at most 2^28 paths.
+// `queue` maps items to ray ids (null = identity); `counter` is zero at launch.
+struct ChunkQueue {
+  uint32_t n_items, dyn_base;
+  // the warp-uniform counters of the pipeline share ONE register (bit fields of a 32-bit word)
+  struct {
+    uint32_t cur_cnt : 6, cur_used : 6, nxt_cnt : 6, nxt_stage : 2, dyn_done : 1;
+  } w;
+  uint32_t id_cur, id_nxt, claim_raw;
+
+  // false: the warp's static slice lies past the end of the queue, it has nothing to do
+  YART_DEV bool start(uint32_t n, const uint32_t* queue, uint32_t* counter, uint32_t lane) {
+    n_items = n;
+    const uint32_t warp_global = (blockIdx.x * kTraceThreads + threadIdx.x) >> 5;
+    const uint32_t total_warps = gridDim.x * (kTraceThreads / 32);
+    const uint32_t rpw = max(1u, min(32u, (uint32_t)(((uint64_t)n_items + total_warps - 1) / total_warps)));
+    dyn_base = total_warps * rpw; // (<= 2^17: at most a few thousand resident warps)
+    if ((uint64_t)warp_global * rpw >= n_items) return false;
+    const uint32_t cur_base = warp_global * rpw;
+    w.cur_cnt = min(rpw, n_items - cur_base);
+    w.cur_used = 0;
+    id_cur = YART_MISS;
+    id_nxt = YART_MISS;
+    claim_raw = 0;
+    if (lane < w.cur_cnt) id_cur = queue ? queue[cur_base + lane] : (uint32_t)(cur_base + lane);
+    w.dyn_done = dyn_base >= n_items; // nothing beyond the static slices: never touch the counter
+    w.nxt_cnt = 0;
+    w.nxt_stage = 0;
+    if (!w.dyn_done) {
+      if (lane == 0) claim_raw = atomicAdd(counter, 32u);
+      w.nxt_stage = 1;
+    }
+    return true;
+  }
+
+  // stage 1 -> 2: the claim has come back, read the chunk's ids
+  YART_DEV void load_next(uint32_t lane, const uint32_t* queue) {
+    const uint64_t nb = (uint64_t)dyn_base + __shfl_sync(0xffffffffu, claim_raw, 0);
+    w.nxt_cnt = nb < n_items ? min(32u, n_items - (uint32_t)nb) : 0u;
+    id_nxt = YART_MISS;
+    if (lane < w.nxt_cnt) id_nxt = queue ? queue[nb + lane] : (uint32_t)(nb + lane);
+    if (w.nxt_cnt < 32u) w.dyn_done = 1; // the counter has passed the end of the queue
+    w.nxt_stage = 2;
+  }
+
+  // One retire/fetch phase (warp-uniform; all lanes take part in the shuffles): advance the pipeline by one stage
+  // and hand an item to each fetching lane that can get one.  True with `id` for those lanes; `exhausted` is set for
+  // a fetching lane that got nothing, which happens only once the queue is used up.  `second` is the other per-ray
+  // record the kernel reads on fetch, prefetched with the ray (null = none).
+  template <class Second>
+  YART_DEV bool next(bool fetching, uint32_t lane, const uint32_t* queue, uint32_t* counter, const yart_ray* rays,
+                     const yart_ray_f32* rays32, const Second* second, uint32_t n_rays, uint32_t& id, bool& exhausted) {
+    if (w.nxt_stage == 2) {
+      if (id_nxt != YART_MISS) {
+        YART_CHECK(id_nxt < n_rays);
+        if (rays32) {
+          const char* rp = reinterpret_cast<const char*>(rays32 + id_nxt);
+          prefetch_l2(rp);
+          prefetch_l2(rp + 23); // a 24-byte record may straddle two 32-byte sectors
+        } else {
+          const char* rp = reinterpret_cast<const char*>(rays + id_nxt);
+          prefetch_l2(rp);
+          prefetch_l2(rp + 32); // a 48-byte record always spans two 32-byte sectors
+        }
+        if (second) prefetch_l2(second + id_nxt);
+      }
+      w.nxt_stage = 3;
+    }
+    const uint32_t fmask = __ballot_sync(0xffffffffu, fetching);
+    const uint32_t need = (uint32_t)__popc(fmask);
+    const uint32_t rank = (uint32_t)__popc(fmask & ((1u << lane) - 1u));
+    const uint32_t take1 = min(need, (uint32_t)w.cur_cnt - (uint32_t)w.cur_used);
+    uint32_t new_id = __shfl_sync(0xffffffffu, id_cur, ((uint32_t)w.cur_used + rank) & 31u);
+    bool got = fetching && rank < take1;
+    w.cur_used = w.cur_used + take1;
+    if (need > take1) { // the current chunk ran out: the next one becomes current, and another is claimed
+      if (w.nxt_stage == 1) load_next(lane, queue);
+      if (w.nxt_stage >= 2) {
+        id_cur = id_nxt;
+        w.cur_cnt = w.nxt_cnt;
+      } else {
+        w.cur_cnt = 0;
+      }
+      w.cur_used = 0;
+      w.nxt_stage = 0;
+      w.nxt_cnt = 0;
+      if (!w.dyn_done) {
+        if (lane == 0) claim_raw = atomicAdd(counter, 32u);
+        w.nxt_stage = 1;
+      }
+      const uint32_t rank2 = rank - take1; // (meaningful for the lanes that are still waiting)
+      const uint32_t take2 = min(need - take1, (uint32_t)w.cur_cnt);
+      const uint32_t id2 = __shfl_sync(0xffffffffu, id_cur, rank2 & 31u);
+      if (fetching && !got && rank2 < take2) {
+        new_id = id2;
+        got = true;
+      }
+      w.cur_used = take2;
+      if (fetching && !got) exhausted = true;
+    } else if (w.nxt_stage == 1) { // no swap this time: use the phase to resolve the claim and load the ids
+      load_next(lane, queue);
+    }
+    id = new_id;
+    return got;
+  }
+};
+
+// The ray in the mesh's space as the conservative f32 slab test below sees it.
+struct SlabRay {
+  float ixf, iyf, izf, cxf, cyf, czf; // per axis t = fma(b, inv, c)
+  float amax2;                        // the absolute part of the error bound
+  uint32_t pos; // bit a set: direction component a is >= 0 (qbvh.rs:388-392); bit 3: `weird`, exact tests throughout
+  uint32_t sgn; // ORDER_TABLE sign bits, mirrored for near-first
+};
+YART_DEV SlabRay slab_ray(D3 o, D3 d, const double* bound, bool near) {
+  SlabRay r;
+  const double ix = 1.0 / d.x, iy = 1.0 / d.y, iz = 1.0 / d.z; // qbvh.rs:403-407
+  r.pos = (d.x >= 0.0 ? 1u : 0u) | (d.y >= 0.0 ? 2u : 0u) | (d.z >= 0.0 ? 4u : 0u); // qbvh.rs:388-392
+  r.sgn = near ? (r.pos ^ 7u) : r.pos;
+  // (b - o) * (1/d) can only be NaN when 1/d is infinite or the ray itself is not finite
+  if (!(isfinite(ix) && isfinite(iy) && isfinite(iz) && isfinite(o.x) && isfinite(o.y) && isfinite(o.z))) r.pos |= 8u;
+  r.ixf = (float)ix; r.iyf = (float)iy; r.izf = (float)iz;
+  r.cxf = (float)(-(o.x * ix)); r.cyf = (float)(-(o.y * iy)); r.czf = (float)(-(o.z * iz));
+  // |t32 - t64| <= 2^-24 (|b| + |o|) |inv| + 2^-24 |t32| (+ f64 roundings); doubled for margin:
+  // absolute part A = 2^-23 (B + |o|) |inv| maximised over the axes, kept as 2A (rounded up)
+  const double a = fmax(fmax((bound[0] + fabs(o.x)) * fabs(ix), (bound[1] + fabs(o.y)) * fabs(iy)),
+                        (bound[2] + fabs(o.z)) * fabs(iz));
+  r.amax2 = __double2float_ru(a * (1.0 / 4194304.0)); // 2A = 2^-22 * a
+  // rays whose f32 image is not well inside the normal range take the exact path throughout
+  const float lo = 1e-30f, hi = 1e30f;
+  const bool ok = fabsf(r.ixf) > lo && fabsf(r.ixf) < hi && fabsf(r.iyf) > lo && fabsf(r.iyf) < hi && fabsf(r.izf) > lo &&
+                  fabsf(r.izf) < hi && fabsf(r.cxf) < hi && fabsf(r.cyf) < hi && fabsf(r.czf) < hi && r.amax2 < hi;
+  if (!ok) r.pos |= 8u;
+  return r;
+}
+
+// node `cur` of the pass's tree
+YART_DEV const float4* node_at(const MeshPass& P, uint32_t cur) {
+  YART_CHECK(cur < P.n_nodes);
+  return P.nodes + (size_t)cur * 8;
+}
+
+// one 128-byte node (FlatNode) in four 256-bit loads, all in flight together
+struct QNode {
+  F8 x, y, z;     // per axis: the four children's lower planes, then their upper planes
+  uint4 child;
+  uint32_t axes;  // split axes of the top, left and right pair (2 bits each)
+};
+YART_DEV QNode load_node(const float4* nd) {
+  QNode n;
+  n.x = ldg256(nd + 0);
+  n.y = ldg256(nd + 2);
+  n.z = ldg256(nd + 4);
+  const F8 cm8 = ldg256(nd + 6);
+  n.child = make_uint4(__float_as_uint(cm8.lo.x), __float_as_uint(cm8.lo.y), __float_as_uint(cm8.lo.z), __float_as_uint(cm8.lo.w));
+  n.axes = __float_as_uint(cm8.hi.x);
+  return n;
+}
+
+// Which children of node `nd` the walk enters: the same hit mask as qbvh.rs:495-532.
+// Conservative f32 test.  Per slab t32 = fma(b, inv32, c32); near32 / far32 are the max / min over
+// the entry / exit planes with t_min / t_best folded in.  With R = 2^-22 and A as in slab_ray,
+// |near32 - near64| <= R|near32| + A and the same for far, so
+//   far32 - near32 >  R(|far32| + |near32|) + 2A  =>  far64 > near64   (the reference pushes)
+//   far32 - near32 < -R(|far32| + |near32|) - 2A  =>  far64 < near64   (the reference does not)
+// and everything in between (also any inf / NaN) is settled by the exact f64 test, which `weird` rays take for
+// every box.  The f64 ray (o, d) is read from ray[0], ray[stride], .., ray[5 stride] only for that exact test.
+// `undecided`: the children the exact test settled.
+template <bool NEAR>
+YART_DEV uint32_t node_hits(const float4* nd, const QNode& n, const SlabRay& r, float t_min_f, float t_best_f,
+                            const double* ray, int stride, double t_min, double t_best, uint32_t& undecided) {
+  undecided = 0;
+  if (!(r.pos & 8u)) {
+    const bool px = (r.pos & 1u) != 0, py = (r.pos & 2u) != 0, pz = (r.pos & 4u) != 0;
+#define YART_SEL4(P_, A, B) make_float4((P_) ? A.x : B.x, (P_) ? A.y : B.y, (P_) ? A.z : B.z, (P_) ? A.w : B.w)
+    const float4 nx = YART_SEL4(px, n.x.lo, n.x.hi), fx = YART_SEL4(px, n.x.hi, n.x.lo);
+    const float4 ny = YART_SEL4(py, n.y.lo, n.y.hi), fy = YART_SEL4(py, n.y.hi, n.y.lo);
+    const float4 nz = YART_SEL4(pz, n.z.lo, n.z.hi), fz = YART_SEL4(pz, n.z.hi, n.z.lo);
+#undef YART_SEL4
+    const float nxs[4] = {nx.x, nx.y, nx.z, nx.w}, nys[4] = {ny.x, ny.y, ny.z, ny.w}, nzs[4] = {nz.x, nz.y, nz.z, nz.w};
+    const float fxs[4] = {fx.x, fx.y, fx.z, fx.w}, fys[4] = {fy.x, fy.y, fy.z, fy.w}, fzs[4] = {fz.x, fz.y, fz.z, fz.w};
+    uint32_t hitmask = 0, amb = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const float tn = fmaxf(fmaxf(t_min_f, fmaf(nxs[k], r.ixf, r.cxf)), fmaxf(fmaf(nys[k], r.iyf, r.cyf), fmaf(nzs[k], r.izf, r.czf)));
+      const float tf = fminf(fminf(t_best_f, fmaf(fxs[k], r.ixf, r.cxf)), fminf(fmaf(fys[k], r.iyf, r.cyf), fmaf(fzs[k], r.izf, r.czf)));
+      const float g = tf - tn;
+      const float e = fmaf(fabsf(tf) + fabsf(tn), 2.384185791015625e-7f, r.amax2);
+      hitmask |= (g > e) ? (1u << k) : 0u;
+      amb |= ((g > e) || (g < -e)) ? 0u : (1u << k);
+    }
+    if (amb) {
+      undecided = amb;
+      const uint32_t exact = box4_ieee<NEAR>(nd, ray[0], ray[stride], ray[2 * stride], 1.0 / ray[3 * stride],
+                                             1.0 / ray[4 * stride], 1.0 / ray[5 * stride], t_min, t_best);
+      hitmask = (hitmask & ~amb) | (exact & amb);
+    }
+    return hitmask;
+  }
+  return box4_ieee<NEAR>(nd, ray[0], ray[stride], ray[2 * stride], 1.0 / ray[3 * stride], 1.0 / ray[4 * stride],
+                         1.0 / ray[5 * stride], t_min, t_best);
+}
+
+// push_hit_children (qbvh.rs:18-31) in the order ORDER_TABLE[4*pos[top] + 2*pos[left] + pos[right]]
+// (qbvh.rs:14-16, 521-524) gives; near-first walks pass mirrored sign bits, so the nearest child ends up on top.
+// The table has structure: bit `top` says whether the left pair {0,1} is pushed before the right pair {2,3};
+// `left` whether 0 goes before 1, `right` whether 2 goes before 3.  So every hit child's stack slot is a closed
+// form of the hit bits -- four predicated stores, no table, no serial loop.  One stack column per lane.
+template <int STACK>
+YART_DEV void push_children(uint32_t (*s_stack)[kTraceThreads], int tid, int& sp, uint32_t hitmask, uint32_t sgn,
+                            const QNode& n) {
+  const uint32_t T = (sgn >> (n.axes & 3u)) & 1u, L = (sgn >> ((n.axes >> 2) & 3u)) & 1u,
+                 Rr = (sgn >> ((n.axes >> 4) & 3u)) & 1u;
+  const uint32_t h0 = hitmask & 1u, h1 = (hitmask >> 1) & 1u, h2 = (hitmask >> 2) & 1u, h3 = (hitmask >> 3) & 1u;
+  const uint32_t nl = h0 + h1, nr = h2 + h3;
+  const uint32_t bl = T ? 0u : nr, br = T ? nl : 0u; // slots taken by the pair pushed first
+  if (h0) s_stack[sp + bl + (L ? 0u : h1)][tid] = n.child.x;
+  if (h1) s_stack[sp + bl + (L ? h0 : 0u)][tid] = n.child.y;
+  if (h2) s_stack[sp + br + (Rr ? 0u : h3)][tid] = n.child.z;
+  if (h3) s_stack[sp + br + (Rr ? h2 : 0u)][tid] = n.child.w;
+  sp += (int)(nl + nr);
+  YART_CHECK(sp <= STACK + 1);
+}
+// the lane's next node or leaf, kSentinel once its stack is empty
+YART_DEV uint32_t pop(uint32_t (*s_stack)[kTraceThreads], int tid, int& sp) {
+  if (sp == 0) return kSentinel;
+  sp--;
+  return s_stack[sp][tid];
+}
+
+// one triangle as 9 floats: v0, v1, v2
+struct Tri9 {
+  float x0, y0, z0, x1, y1, z1, x2, y2, z2;
+};
+// Moeller-Trumbore exactly as qbvh.rs:419-489: true when the ray passes the edge tests and t >= t_min, with the
+// hit's t and barycentrics u, v.  The test against t_max / the best hit so far is the caller's.
+YART_DEV bool mt_hit(const Tri9& p, D3 o, D3 d, double t_min, double& t, double& u, double& v) {
+  const double v0x = (double)p.x0, v0y = (double)p.y0, v0z = (double)p.z0;
+  const double e1x = (double)p.x1 - v0x, e1y = (double)p.y1 - v0y, e1z = (double)p.z1 - v0z;
+  const double e2x = (double)p.x2 - v0x, e2y = (double)p.y2 - v0y, e2z = (double)p.z2 - v0z;
+  const double hx = d.y * e2z - d.z * e2y, hy = d.z * e2x - d.x * e2z, hz = d.x * e2y - d.y * e2x;
+  const double a = e1x * hx + e1y * hy + e1z * hz;
+  bool ok = !((a > -kF64Eps) && (a < kF64Eps));
+  const double f = 1.0 / a;
+  const double sx = o.x - v0x, sy = o.y - v0y, sz = o.z - v0z;
+  u = f * (sx * hx + sy * hy + sz * hz);
+  ok = ok && (u >= 0.0) && (u <= 1.0);
+  const double qx = sy * e1z - sz * e1y, qy = sz * e1x - sx * e1z, qz = sx * e1y - sy * e1x;
+  v = f * (d.x * qx + d.y * qy + d.z * qz);
+  ok = ok && (v >= 0.0) && ((u + v) <= 1.0);
+  t = f * (e2x * qx + e2y * qy + e2z * qz);
+  return ok && (t >= t_min);
+}
+
+// One leaf (qbvh.rs:413-490): test(i, tri) for its triangles first + i, from the last one backwards when REVERSE;
+// a test that returns true ends the leaf.  A leaf of up to three triangles is one packed block (36 B each, 32-byte
+// aligned): 2 / 3 / 4 sector loads for 1 / 2 / 3 triangles instead of 3 loads per triangle, at most three sectors in
+// registers at a time, the next one requested one test ahead.  4-triangle leaves are read one 48-byte record at a
+// time, the next one requested before the current is tested.
+template <bool REVERSE, class Test>
+YART_DEV void visit_leaf(const float4* leafgeo, const float4* tris, uint32_t first, uint32_t count, Test&& test) {
+  if (count <= 3u) {
+    const float4* lp = leafgeo + (size_t)first * 4;
+#define YART_TRI0 Tri9{s0.lo.x, s0.lo.y, s0.lo.z, s0.lo.w, s0.hi.x, s0.hi.y, s0.hi.z, s0.hi.w, s1.lo.x}
+#define YART_TRI1 Tri9{s1.lo.y, s1.lo.z, s1.lo.w, s1.hi.x, s1.hi.y, s1.hi.z, s1.hi.w, s2.lo.x, s2.lo.y}
+#define YART_TRI2 Tri9{s2.lo.z, s2.lo.w, s2.hi.x, s2.hi.y, s2.hi.z, s2.hi.w, s3.lo.x, s3.lo.y, s3.lo.z}
+    if (REVERSE) { // from the last sector backwards
+      F8 s1 = ldg256(lp + 2), s2, s3;
+      s2.lo = s2.hi = s3.lo = s3.hi = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (count >= 2u) s2 = ldg256(lp + 4);
+      if (count >= 3u) {
+        s3 = ldg256(lp + 6);
+        if (test(2u, YART_TRI2)) return;
+      }
+      const F8 s0 = ldg256(lp);
+      if (count >= 2u && test(1u, YART_TRI1)) return;
+      test(0u, YART_TRI0);
+    } else {
+      const F8 s0 = ldg256(lp), s1 = ldg256(lp + 2);
+      F8 s2, s3;
+      s2.lo = s2.hi = s3.lo = s3.hi = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (count >= 2u) s2 = ldg256(lp + 4);
+      if (test(0u, YART_TRI0)) return;
+      if (count >= 3u) s3 = ldg256(lp + 6);
+      if (count >= 2u && test(1u, YART_TRI1)) return;
+      if (count >= 3u) test(2u, YART_TRI2);
+    }
+#undef YART_TRI0
+#undef YART_TRI1
+#undef YART_TRI2
+  } else {
+    float4 n0, n1, n2;
+    {
+      const float4* tp = tris + (size_t)(first + (REVERSE ? (count - 1u) : 0u)) * 3;
+      n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
+    }
+    for (uint32_t j = 0; j < count; ++j) {
+      const uint32_t i = REVERSE ? (count - 1u - j) : j;
+      const float4 a0 = n0, a1 = n1, a2 = n2;
+      if (j + 1u < count) {
+        const float4* tp = tris + (size_t)(first + (REVERSE ? (i - 1u) : (i + 1u))) * 3;
+        n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
+      }
+      if (test(i, Tri9{a0.x, a0.y, a0.z, a1.x, a1.y, a1.z, a2.x, a2.y, a2.z})) return;
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 // k_traverse: one TriangleMesh instance against the whole ray queue
 // ---------------------------------------------------------------------------------------------
 #ifndef YART_TRAVERSE_MIN_BLOCKS
 #define YART_TRAVERSE_MIN_BLOCKS 4
 #endif
 
-// MIXED selects how the four slab tests of a node are evaluated:
-//   false: f64 in the reference's operation order (after 24 f32->f64 conversions per node);
-//   true : a conservative f32 evaluation decides every box that is clearly hit or clearly missed
-//          and only the (rare) undecided ones are re-evaluated exactly in f64.  Both give the SAME
-//          hit mask as qbvh.rs:495-532 -- see the error bound at the f32 test below.
-template <bool NEAR, bool COUNT, int STACK, bool MIXED>
+// The reference order, and visit counting in either order.  (Near-first without counting is k_traverse_lean,
+// device_trace_lean.cu: the same walk with the f64 ray in shared memory.)  Here the f64 ray and the best hit's
+// barycentrics stay in registers.
+template <bool NEAR, bool COUNT, int STACK>
 __global__ void __launch_bounds__(kTraceThreads, YART_TRAVERSE_MIN_BLOCKS) k_traverse(const TraverseParams P) {
   __shared__ uint32_t s_stack[STACK + 1][kTraceThreads];
   const int tid = threadIdx.x;
   const uint32_t lane = tid & 31;
-  const uint64_t n_items = P.c.n_items_dev ? (uint64_t)*P.c.n_items_dev : P.c.n_items;
-  // Work distribution: warp w starts with items [32w, 32w+32) without touching the counter and only then
-  // fetches dynamically from total_warps*32 + atomicAdd(counter).  Warps whose first slice is already past
-  // the end leave at once -- a nearly empty queue (the deep bounces) costs no same-address atomics.
-  // A short queue is spread thinly (rpw < 32 rays per warp): a warp's run time is the serialised work of
-  // its most divergent rays, so a deep bounce with a few hundred rays finishes sooner on many warps.
-  const uint32_t warp_global = (blockIdx.x * kTraceThreads + tid) >> 5;
-  const uint64_t total_warps = (uint64_t)gridDim.x * (kTraceThreads / 32);
-  const uint32_t rpw = (uint32_t)max((unsigned long long)1, min((unsigned long long)32, (unsigned long long)((n_items + total_warps - 1) / total_warps)));
-  const uint64_t dyn_base = total_warps * rpw;
-  if ((uint64_t)warp_global * rpw >= n_items) return;
-  // Work items reach the lanes through a two-deep pipeline of 32-item chunks, so that neither the claim
-  // (an atomic), nor the queue read, nor the DRAM miss of the ray record sits on the warp's critical path:
-  //   chunk "cur": ids held one per lane (id_cur), handed to fetching lanes by shuffle;
-  //   chunk "nxt": claimed when cur was started (stage 1: atomic in flight), ids loaded one retire/fetch phase
-  //   later (stage 2), ray / hit records prefetched into L2 the phase after (stage 3).
-  // The first chunk of a warp is its static slice; all later ones come from the global counter.
-  uint64_t cur_base = (uint64_t)warp_global * rpw;
-  uint32_t cur_cnt = (uint32_t)min((unsigned long long)rpw, (unsigned long long)(n_items - cur_base));
-  uint32_t cur_used = 0;
-  uint32_t id_cur = YART_MISS, id_nxt = YART_MISS, claim_raw = 0;
-  if (lane < cur_cnt) id_cur = P.c.queue ? P.c.queue[cur_base + lane] : (uint32_t)(cur_base + lane);
-  bool dyn_done = dyn_base >= n_items; // nothing beyond the static slices: never touch the counter
-  uint32_t nxt_cnt = 0, nxt_stage = 0;
-  if (!dyn_done) {
-    if (lane == 0) claim_raw = atomicAdd(P.work_counter, 32u);
-    nxt_stage = 1;
-  }
-  const uint32_t RT = P.refill_threshold, NT = P.node_threshold;
-  const float4* __restrict__ nodes = P.nodes;
-  const float4* __restrict__ tris = P.tris;
+  ChunkQueue q;
+  if (!q.start(P.c.n_items_dev ? *P.c.n_items_dev : (uint32_t)P.c.n_items, P.c.queue, P.m.work_counter, lane)) return;
+  const uint32_t RT = P.m.refill_threshold, NT = P.m.node_threshold;
   const double t_min = P.c.t_min;
+  const float t_min_f = (float)t_min;
 
   // ---- lane state ----
   uint32_t ray_id = YART_MISS; // YART_MISS = idle
   uint32_t cur = kSentinel;    // current stack top (node or leaf id), kSentinel = not traversing
   int sp = 0;
-  double ox = 0, oy = 0, oz = 0, dx = 0, dy = 0, dz = 0, ix = 0, iy = 0, iz = 0; // ray in the mesh's space
-  uint32_t sgn = 0;  // ORDER_TABLE sign bits (mirrored when NEAR)
-  uint32_t pos = 0;  // bit a set: direction component a is >= 0 (qbvh.rs:388-392); bit 3: `weird`
+  double ray[6] = {0, 0, 0, 0, 0, 0}; // the ray (o, d) in the mesh's space
+  SlabRay r = {};
   double t_best = 0, best_bu = 0, best_bv = 0;
+  float t_best_f = 0;
   uint32_t best_prim = YART_MISS; // YART_MISS = this mesh has not produced a hit
   bool exhausted = false;         // the global queue is empty
   unsigned long long n_nodes = 0, n_tris = 0, n_exact = 0;
-  // MIXED: the ray as f32 slab coefficients t = b*inv + c, and the absolute part of the error bound
-  float ixf = 0, iyf = 0, izf = 0, cxf = 0, cyf = 0, czf = 0, amax2 = 0, t_best_f = 0;
-  const float t_min_f = (float)t_min;
 
   for (;;) {
     // =============== phase A: retire finished rays, fetch new ones ================================
@@ -430,119 +706,25 @@ __global__ void __launch_bounds__(kTraceThreads, YART_TRAVERSE_MIN_BLOCKS) k_tra
         }
         ray_id = YART_MISS;
       }
-      // ---- advance the chunk pipeline by one stage (warp-uniform) ----
-      if (nxt_stage == 2) {
-        if (id_nxt != YART_MISS) {
-          YART_CHECK(id_nxt < P.c.n_rays);
-          if (P.c.rays32) {
-            const char* rp = reinterpret_cast<const char*>(P.c.rays32 + id_nxt);
-            prefetch_l2(rp);
-            prefetch_l2(rp + 23); // a 24-byte record may straddle two 32-byte sectors
-          } else {
-            const char* rp = reinterpret_cast<const char*>(P.c.rays + id_nxt);
-            prefetch_l2(rp);
-            prefetch_l2(rp + 32); // a 48-byte record always spans two 32-byte sectors
-          }
-          if (!P.c.first_pass) prefetch_l2(P.c.hits + id_nxt);
-        }
-        nxt_stage = 3;
-      }
-      // ---- hand out items (all lanes take part in the shuffles) ----
-      const bool fetching = want_a && !exhausted;
-      const uint32_t fmask = __ballot_sync(0xffffffffu, fetching);
-      const uint32_t need = (uint32_t)__popc(fmask);
-      const uint32_t rank = (uint32_t)__popc(fmask & ((1u << lane) - 1u));
-      const uint32_t take1 = min(need, cur_cnt - cur_used);
-      uint32_t new_id = __shfl_sync(0xffffffffu, id_cur, (cur_used + rank) & 31u);
-      bool got = fetching && rank < take1;
-      cur_used += take1;
-      if (need > take1) { // the current chunk ran out: the next one becomes current, and another is claimed
-        if (nxt_stage == 1) { // its claim has come back by now: read its ids
-          const uint64_t nb = dyn_base + __shfl_sync(0xffffffffu, claim_raw, 0);
-          nxt_cnt = nb < n_items ? (uint32_t)min((unsigned long long)32, (unsigned long long)(n_items - nb)) : 0u;
-          id_nxt = YART_MISS;
-          if (lane < nxt_cnt) id_nxt = P.c.queue ? P.c.queue[nb + lane] : (uint32_t)(nb + lane);
-          if (nxt_cnt < 32u) dyn_done = true; // the counter has passed the end of the queue
-          nxt_stage = 2;
-        }
-        if (nxt_stage >= 2) {
-          id_cur = id_nxt;
-          cur_cnt = nxt_cnt;
-        } else {
-          cur_cnt = 0;
-        }
-        cur_used = 0;
-        nxt_stage = 0;
-        nxt_cnt = 0;
-        if (!dyn_done) {
-          if (lane == 0) claim_raw = atomicAdd(P.work_counter, 32u);
-          nxt_stage = 1;
-        }
-        const uint32_t rank2 = rank - take1; // (meaningful for the lanes that are still waiting)
-        const uint32_t take2 = min(need - take1, cur_cnt);
-        const uint32_t id2 = __shfl_sync(0xffffffffu, id_cur, rank2 & 31u);
-        if (fetching && !got && rank2 < take2) {
-          new_id = id2;
-          got = true;
-        }
-        cur_used = take2;
-        if (fetching && !got) exhausted = true; // only possible once the queue is used up
-      } else if (nxt_stage == 1) { // no swap this time: use the phase to resolve the claim and load the ids
-        const uint64_t nb = dyn_base + __shfl_sync(0xffffffffu, claim_raw, 0);
-        nxt_cnt = nb < n_items ? (uint32_t)min((unsigned long long)32, (unsigned long long)(n_items - nb)) : 0u;
-        id_nxt = YART_MISS;
-        if (lane < nxt_cnt) id_nxt = P.c.queue ? P.c.queue[nb + lane] : (uint32_t)(nb + lane);
-        if (nxt_cnt < 32u) dyn_done = true;
-        nxt_stage = 2;
-      }
-      if (got) {
-        {
-          ray_id = new_id;
-          YART_CHECK(ray_id < P.c.n_rays);
-          D3 ro, rd;
-          if (P.c.rays32) load_ray_f32(P.c.rays32 + ray_id, ro, rd);
-          else load_ray(P.c.rays + ray_id, ro, rd);
-          t_best = P.c.first_pass ? P.c.t_max : fmin(P.c.hits[ray_id].t, P.c.t_max);
-          if (NEAR) t_best = just_below(t_best); // strict against earlier objects / the caller's t_max (device_common.cuh)
-          // ray into the instance's space (hittable.rs:137-143, 218-227); uniform across the launch
-          if (P.wrap & YART_WRAP_TRANSLATE) ro = ro - d3(P.offset[0], P.offset[1], P.offset[2]);
-          if (P.wrap & YART_WRAP_ROTATE_Y) {
-            const double ct = P.cos_theta, st = P.sin_theta;
-            D3 org = ro, dir = rd;
-            org.x = ct * ro.x - st * ro.z;
-            org.z = st * ro.x + ct * ro.z;
-            dir.x = ct * rd.x - st * rd.z;
-            dir.z = st * rd.x + ct * rd.z;
-            ro = org;
-            rd = dir;
-          }
-          ox = ro.x; oy = ro.y; oz = ro.z;
-          dx = rd.x; dy = rd.y; dz = rd.z;
-          ix = 1.0 / dx; iy = 1.0 / dy; iz = 1.0 / dz; // qbvh.rs:403-407
-          pos = (dx >= 0.0 ? 1u : 0u) | (dy >= 0.0 ? 2u : 0u) | (dz >= 0.0 ? 4u : 0u); // qbvh.rs:388-392
-          sgn = NEAR ? (pos ^ 7u) : pos;
-          // (b - o) * (1/d) can only be NaN when 1/d is infinite or the ray itself is not finite
-          if (!(isfinite(ix) && isfinite(iy) && isfinite(iz) && isfinite(ox) && isfinite(oy) && isfinite(oz))) pos |= 8u;
-          if (MIXED) {
-            ixf = (float)ix; iyf = (float)iy; izf = (float)iz;
-            cxf = (float)(-(ox * ix)); cyf = (float)(-(oy * iy)); czf = (float)(-(oz * iz));
-            // |t32 - t64| <= 2^-24 (|b| + |o|) |inv| + 2^-24 |t32| (+ f64 roundings); doubled for margin:
-            // absolute part A = 2^-23 (B + |o|) |inv| maximised over the axes, kept as 2A (rounded up)
-            const double a = fmax(fmax((P.bound[0] + fabs(ox)) * fabs(ix), (P.bound[1] + fabs(oy)) * fabs(iy)),
-                                  (P.bound[2] + fabs(oz)) * fabs(iz));
-            amax2 = __double2float_ru(a * (1.0 / 4194304.0)); // 2A = 2^-22 * a
-            // rays whose f32 image is not well inside the normal range take the exact path throughout
-            const float lo = 1e-30f, hi = 1e30f;
-            const bool ok = fabsf(ixf) > lo && fabsf(ixf) < hi && fabsf(iyf) > lo && fabsf(iyf) < hi && fabsf(izf) > lo &&
-                            fabsf(izf) < hi && fabsf(cxf) < hi && fabsf(cyf) < hi && fabsf(czf) < hi && amax2 < hi;
-            if (!ok) pos |= 8u;
-            t_best_f = (float)t_best;
-          }
-          cur = P.root;
-          sp = 0;
-          best_prim = YART_MISS;
-          best_bu = best_bv = 0.0;
-        }
+      uint32_t id;
+      if (q.next(want_a && !exhausted, lane, P.c.queue, P.m.work_counter, P.c.rays, P.c.rays32,
+                 P.c.first_pass ? nullptr : P.c.hits, P.c.n_rays, id, exhausted)) {
+        ray_id = id;
+        YART_CHECK(ray_id < P.c.n_rays);
+        D3 ro, rd;
+        if (P.c.rays32) load_ray_f32(P.c.rays32 + ray_id, ro, rd);
+        else load_ray(P.c.rays + ray_id, ro, rd);
+        t_best = P.c.first_pass ? P.c.t_max : fmin(P.c.hits[ray_id].t, P.c.t_max);
+        if (NEAR) t_best = just_below(t_best); // strict against earlier objects / the caller's t_max (device_common.cuh)
+        instance_to_object(P.m.wrap, P.m.offset, P.m.sin_theta, P.m.cos_theta, ro, rd); // uniform across the launch
+        ray[0] = ro.x; ray[1] = ro.y; ray[2] = ro.z;
+        ray[3] = rd.x; ray[4] = rd.y; ray[5] = rd.z;
+        r = slab_ray(ro, rd, P.m.bound, NEAR);
+        t_best_f = (float)t_best;
+        cur = P.m.root;
+        sp = 0;
+        best_prim = YART_MISS;
+        best_bu = best_bv = 0.0;
       }
     }
     if (!__any_sync(0xffffffffu, ray_id != YART_MISS)) break;
@@ -560,101 +742,14 @@ __global__ void __launch_bounds__(kTraceThreads, YART_TRAVERSE_MIN_BLOCKS) k_tra
         if (lm != 0 || (uint32_t)__popc(wm) >= RT) break;
       }
       if (has_node) {
-        YART_CHECK(cur < P.n_nodes);
-        const float4* nd = nodes + (size_t)cur * 8;
-        // the whole 128-byte node in four 256-bit loads, all in flight together
-        const F8 sx8 = ldg256(nd + 0), sy8 = ldg256(nd + 2), sz8 = ldg256(nd + 4), cm8 = ldg256(nd + 6);
-        const uint4 ch = make_uint4(__float_as_uint(cm8.lo.x), __float_as_uint(cm8.lo.y), __float_as_uint(cm8.lo.z),
-                                    __float_as_uint(cm8.lo.w));
-        const uint32_t axes = __float_as_uint(cm8.hi.x);
+        const float4* nd = node_at(P.m, cur);
+        const QNode n = load_node(nd);
         if (COUNT) n_nodes++;
-        uint32_t hitmask = 0;
-        if (MIXED && !(pos & 8u)) {
-          // Conservative f32 test.  Per slab t32 = fma(b, inv32, c32); near32 / far32 are the max / min over
-          // the entry / exit planes with t_min / t_best folded in.  With R = 2^-22 and A as above,
-          // |near32 - near64| <= R|near32| + A and the same for far, so
-          //   far32 - near32 >  R(|far32| + |near32|) + 2A  =>  far64 > near64   (the reference pushes)
-          //   far32 - near32 < -R(|far32| + |near32|) - 2A  =>  far64 < near64   (the reference does not)
-          // and everything in between (also any inf / NaN) is settled by the exact f64 test.
-          const bool px = (pos & 1u) != 0, py = (pos & 2u) != 0, pz = (pos & 4u) != 0;
-#define YART_SEL4(P_, A, B) make_float4((P_) ? A.x : B.x, (P_) ? A.y : B.y, (P_) ? A.z : B.z, (P_) ? A.w : B.w)
-          const float4 nx = YART_SEL4(px, sx8.lo, sx8.hi), fx = YART_SEL4(px, sx8.hi, sx8.lo);
-          const float4 ny = YART_SEL4(py, sy8.lo, sy8.hi), fy = YART_SEL4(py, sy8.hi, sy8.lo);
-          const float4 nz = YART_SEL4(pz, sz8.lo, sz8.hi), fz = YART_SEL4(pz, sz8.hi, sz8.lo);
-#undef YART_SEL4
-          uint32_t amb = 0;
-#define YART_BOX_F32(K, C)                                                                                  \
-  {                                                                                                         \
-    const float tn = fmaxf(fmaxf(t_min_f, fmaf(nx.C, ixf, cxf)), fmaxf(fmaf(ny.C, iyf, cyf), fmaf(nz.C, izf, czf))); \
-    const float tf = fminf(fminf(t_best_f, fmaf(fx.C, ixf, cxf)), fminf(fmaf(fy.C, iyf, cyf), fmaf(fz.C, izf, czf))); \
-    const float g = tf - tn;                                                                                \
-    const float e = fmaf(fabsf(tf) + fabsf(tn), 2.384185791015625e-7f, amax2);                              \
-    hitmask |= (g > e) ? (1u << (K)) : 0u;                                                                  \
-    amb |= ((g > e) || (g < -e)) ? 0u : (1u << (K));                                                        \
-  }
-          YART_BOX_F32(0, x)
-          YART_BOX_F32(1, y)
-          YART_BOX_F32(2, z)
-          YART_BOX_F32(3, w)
-#undef YART_BOX_F32
-          if (amb) {
-            if (COUNT) n_exact++;
-            const uint32_t exact = box4_ieee<NEAR>(nd, ox, oy, oz, 1.0 / dx, 1.0 / dy, 1.0 / dz, t_min, t_best);
-            hitmask = (hitmask & ~amb) | (exact & amb);
-          }
-        } else if (!MIXED && !(pos & 8u)) {
-          // Fast f64 path.  All slab values are finite or +-inf, never NaN, and b_min <= b_max, so
-          // min(t0,t1) is the plane on the side the ray comes from and max(t0,t1) the other one:
-          // identical values to qbvh.rs:495-519 with half the min/max work and no NaN handling.
-          const bool px = (pos & 1u) != 0, py = (pos & 2u) != 0, pz = (pos & 4u) != 0;
-#define YART_SEL4(P_, A, B) make_float4((P_) ? A.x : B.x, (P_) ? A.y : B.y, (P_) ? A.z : B.z, (P_) ? A.w : B.w)
-          const float4 nx = YART_SEL4(px, sx8.lo, sx8.hi), fx = YART_SEL4(px, sx8.hi, sx8.lo);
-          const float4 ny = YART_SEL4(py, sy8.lo, sy8.hi), fy = YART_SEL4(py, sy8.hi, sy8.lo);
-          const float4 nz = YART_SEL4(pz, sz8.lo, sz8.hi), fz = YART_SEL4(pz, sz8.hi, sz8.lo);
-#undef YART_SEL4
-#define YART_BOX_FAST(K, C)                                                                              \
-  {                                                                                                      \
-    double tn = max_nn(t_min, ((double)nx.C - ox) * ix);                                                 \
-    tn = max_nn(tn, ((double)ny.C - oy) * iy);                                                           \
-    tn = max_nn(tn, ((double)nz.C - oz) * iz);                                                           \
-    double tf = NEAR ? ((double)fx.C - ox) * ix : min_nn(t_best, ((double)fx.C - ox) * ix);             \
-    tf = min_nn(tf, ((double)fy.C - oy) * iy);                                                           \
-    tf = min_nn(tf, ((double)fz.C - oz) * iz);                                                           \
-    const bool h = NEAR ? ((tf > tn) && (t_best >= tn)) : (tf > tn);                                     \
-    hitmask |= h ? (1u << (K)) : 0u;                                                                     \
-  }
-          YART_BOX_FAST(0, x)
-          YART_BOX_FAST(1, y)
-          YART_BOX_FAST(2, z)
-          YART_BOX_FAST(3, w)
-#undef YART_BOX_FAST
-        } else {
-          hitmask = box4_ieee<NEAR>(nd, ox, oy, oz, 1.0 / dx, 1.0 / dy, 1.0 / dz, t_min, t_best);
-        }
-        // push_hit_children (qbvh.rs:18-31) in the order ORDER_TABLE[4*pos[top] + 2*pos[left] + pos[right]]
-        // (qbvh.rs:14-16, 521-524) gives.  The table has structure: bit `top` says whether the left pair
-        // {0,1} is pushed before the right pair {2,3}; `left` whether 0 goes before 1, `right` whether 2 goes
-        // before 3.  So every hit child's stack slot is a closed form of the hit bits -- four predicated
-        // stores, no table, no serial loop.
-        {
-          const uint32_t T = (sgn >> (axes & 3u)) & 1u, L = (sgn >> ((axes >> 2) & 3u)) & 1u,
-                         Rr = (sgn >> ((axes >> 4) & 3u)) & 1u;
-          const uint32_t h0 = hitmask & 1u, h1 = (hitmask >> 1) & 1u, h2 = (hitmask >> 2) & 1u, h3 = (hitmask >> 3) & 1u;
-          const uint32_t nl = h0 + h1, nr = h2 + h3;
-          const uint32_t bl = T ? 0u : nr, br = T ? nl : 0u; // slots taken by the pair pushed first
-          if (h0) s_stack[sp + bl + (L ? 0u : h1)][tid] = ch.x;
-          if (h1) s_stack[sp + bl + (L ? h0 : 0u)][tid] = ch.y;
-          if (h2) s_stack[sp + br + (Rr ? 0u : h3)][tid] = ch.z;
-          if (h3) s_stack[sp + br + (Rr ? h2 : 0u)][tid] = ch.w;
-          sp += (int)(nl + nr);
-          YART_CHECK(sp <= STACK + 1);
-        }
-        if (sp == 0) {
-          cur = kSentinel;
-        } else {
-          sp--;
-          cur = s_stack[sp][tid];
-        }
+        uint32_t undecided;
+        const uint32_t hitmask = node_hits<NEAR>(nd, n, r, t_min_f, t_best_f, ray, 1, t_min, t_best, undecided);
+        if (COUNT && undecided) n_exact++;
+        push_children<STACK>(s_stack, tid, sp, hitmask, r.sgn, n);
+        cur = pop(s_stack, tid, sp);
       }
     }
 
@@ -663,74 +758,20 @@ __global__ void __launch_bounds__(kTraceThreads, YART_TRAVERSE_MIN_BLOCKS) k_tra
       const uint32_t count = (cur >> 27) & 0xFu;
       const uint32_t first = cur & 0x7FFFFFFu;
       if (COUNT) n_tris += count;
-      YART_CHECK(count >= 1 && count <= 4 && first + count <= P.n_tris);
-      // Moeller-Trumbore exactly as qbvh.rs:419-489 on one triangle given as 9 floats
-#define YART_TRI_TEST(I_, F0, F1, F2, F3, F4, F5, F6, F7, F8)                                                       \
-  {                                                                                                                 \
-    const double v0x = (double)(F0), v0y = (double)(F1), v0z = (double)(F2);                                        \
-    const double e1x = (double)(F3) - v0x, e1y = (double)(F4) - v0y, e1z = (double)(F5) - v0z;                      \
-    const double e2x = (double)(F6) - v0x, e2y = (double)(F7) - v0y, e2z = (double)(F8) - v0z;                      \
-    const double hx = dy * e2z - dz * e2y, hy = dz * e2x - dx * e2z, hz = dx * e2y - dy * e2x;                      \
-    const double a = e1x * hx + e1y * hy + e1z * hz;                                                                \
-    bool ok = !((a > -kF64Eps) && (a < kF64Eps));                                                                   \
-    const double f = 1.0 / a;                                                                                       \
-    const double sx = ox - v0x, sy = oy - v0y, sz = oz - v0z;                                                       \
-    const double u = f * (sx * hx + sy * hy + sz * hz);                                                             \
-    ok = ok && (u >= 0.0) && (u <= 1.0);                                                                            \
-    const double qx = sy * e1z - sz * e1y, qy = sz * e1x - sx * e1z, qz = sx * e1y - sy * e1x;                      \
-    const double v = f * (dx * qx + dy * qy + dz * qz);                                                             \
-    ok = ok && (v >= 0.0) && ((u + v) <= 1.0);                                                                      \
-    const double t = f * (e2x * qx + e2y * qy + e2z * qz);                                                          \
-    ok = ok && (t >= t_min);                                                                                        \
-    /* REFERENCE: first found wins (`t_max > t`, qbvh.rs:478).  NEAR: mirrored -- last found wins among this */    \
-    /* mesh's equal-t hits; strictness against earlier objects comes from the start value just_below(t_max).  */    \
-    ok = ok && (NEAR ? (t <= t_best) : (t_best > t));                                                               \
-    if (ok) {                                                                                                       \
-      t_best = t; best_prim = first + (I_); best_bu = u; best_bv = v;                                               \
-      if (MIXED) t_best_f = (float)t;                                                                               \
-    }                                                                                                               \
-  }
-      if (count <= 3u) {
-        // The leaf's triangles as one packed block (36 B each, 32-byte aligned): 2 / 3 / 4 sector loads for
-        // 1 / 2 / 3 triangles instead of 3 loads per triangle, all in flight together.
-        const float4* lp = P.leafgeo + (size_t)first * 4;
-        F8 s0 = ldg256(lp), s1 = ldg256(lp + 2), s2, s3;
-        s2.lo = s2.hi = s3.lo = s3.hi = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (count >= 2u) s2 = ldg256(lp + 4);
-        if (count >= 3u) s3 = ldg256(lp + 6);
-        if (NEAR) { // lanes in reverse order (mirrored tie rule)
-          if (count >= 3u) YART_TRI_TEST(2u, s2.lo.z, s2.lo.w, s2.hi.x, s2.hi.y, s2.hi.z, s2.hi.w, s3.lo.x, s3.lo.y, s3.lo.z)
-          if (count >= 2u) YART_TRI_TEST(1u, s1.lo.y, s1.lo.z, s1.lo.w, s1.hi.x, s1.hi.y, s1.hi.z, s1.hi.w, s2.lo.x, s2.lo.y)
-          YART_TRI_TEST(0u, s0.lo.x, s0.lo.y, s0.lo.z, s0.lo.w, s0.hi.x, s0.hi.y, s0.hi.z, s0.hi.w, s1.lo.x)
-        } else {
-          YART_TRI_TEST(0u, s0.lo.x, s0.lo.y, s0.lo.z, s0.lo.w, s0.hi.x, s0.hi.y, s0.hi.z, s0.hi.w, s1.lo.x)
-          if (count >= 2u) YART_TRI_TEST(1u, s1.lo.y, s1.lo.z, s1.lo.w, s1.hi.x, s1.hi.y, s1.hi.z, s1.hi.w, s2.lo.x, s2.lo.y)
-          if (count >= 3u) YART_TRI_TEST(2u, s2.lo.z, s2.lo.w, s2.hi.x, s2.hi.y, s2.hi.z, s2.hi.w, s3.lo.x, s3.lo.y, s3.lo.z)
+      YART_CHECK(count >= 1 && count <= 4 && first + count <= P.m.n_tris);
+      const D3 o = d3(ray[0], ray[1], ray[2]), d = d3(ray[3], ray[4], ray[5]);
+      // NEAR tests the leaf's triangles in reverse order (the mirrored tie rule)
+      visit_leaf<NEAR>(P.m.leafgeo, P.m.tris, first, count, [&](uint32_t i, const Tri9& tri) {
+        double t, u, v;
+        // REFERENCE: first found wins (`t_max > t`, qbvh.rs:478).  NEAR: mirrored -- last found wins among this
+        // mesh's equal-t hits; strictness against earlier objects comes from the start value just_below(t_max).
+        if (mt_hit(tri, o, d, t_min, t, u, v) && (NEAR ? (t <= t_best) : (t_best > t))) {
+          t_best = t; best_prim = first + i; best_bu = u; best_bv = v;
+          t_best_f = (float)t;
         }
-      } else {
-        // 4-triangle leaves: one 48-byte record at a time, the next one requested before the current is tested
-        float4 n0, n1, n2;
-        {
-          const float4* tp = tris + (size_t)(first + (NEAR ? (count - 1u) : 0u)) * 3;
-          n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
-        }
-        for (uint32_t j = 0; j < count; ++j) {
-          const uint32_t i = NEAR ? (count - 1u - j) : j;
-          const float4 a0 = n0, a1 = n1, a2 = n2;
-          if (j + 1u < count) {
-            const float4* tp = tris + (size_t)(first + (NEAR ? (i - 1u) : (i + 1u))) * 3;
-            n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
-          }
-          YART_TRI_TEST(i, a0.x, a0.y, a0.z, a1.x, a1.y, a1.z, a2.x, a2.y, a2.z)
-        }
-      }
-#undef YART_TRI_TEST
-      if (sp == 0) {
-        cur = kSentinel;
-      } else {
-        sp--;
-        cur = s_stack[sp][tid];
-      }
+        return false;
+      });
+      cur = pop(s_stack, tid, sp);
     }
   }
   if (COUNT) {
@@ -739,6 +780,9 @@ __global__ void __launch_bounds__(kTraceThreads, YART_TRAVERSE_MIN_BLOCKS) k_tra
     atomicAdd(&P.counters[2], n_exact);
   }
 }
+
+typedef void (*TraverseKernel)(const TraverseParams);
+TraverseKernel lean_traverse_kernel(uint32_t max_stack); // device_trace_lean.cu
 
 // ---------------------------------------------------------------------------------------------
 // k_analytic: a run of consecutive non-mesh objects of the list, one thread per queued ray

@@ -1,40 +1,19 @@
-// device_trace_lean.cu -- k_traverse_lean: the closest-hit traversal of device_trace.cuh (same phases, same arithmetic,
-// same results bit for bit) on a register diet, so that five instead of four 128-thread CTAs fit an SM (20 warps).
+// device_trace_lean.cu -- k_traverse_lean: the near-first closest-hit traversal of device_trace.cuh (same phases, same
+// arithmetic, same results bit for bit) on a register diet, so that five instead of four 128-thread CTAs fit an SM (20 warps).
 //
 // k_traverse is bound by the latency of its node / leaf fetches at 16 warps per SM (DESIGN.md section 7); its 128
 // registers are the price of keeping the f64 ray next to the f32 slab coefficients.  Here everything only the exact
 // f64 code touches -- the ray (o, d) and the best hit's barycentrics -- lives in shared memory (one column per
-// lane, conflict-free) and is loaded when a leaf test or a (rare) exact box test needs it, and a leaf's sectors are
-// requested one test ahead instead of all at once.  Measured: +7 % on the render step, +6 % on the sweep; at 20 warps
-// the L1 data pipe (82-94 % busy) is the limiter.
+// lane, conflict-free) and is loaded when a leaf test or a (rare) exact box test needs it.  Measured: +7 % on the
+// render step, +6 % on the sweep; at 20 warps the L1 data pipe (82-94 % busy) is the limiter.  The reference order
+// stays with k_traverse: this kernel spills there and was 5 % slower on the sweep (2,074 vs 2,188 Mrays/s).
 #define YART_TRACE_NO_ANALYTIC_KERNEL
 #include "device_trace.cuh"
 
 namespace yart {
 
-// COMPACT (an experiment, off unless YART_TUNE_COMPACT=1; bit-exact but 20-29 % slower -- DESIGN.md section 7):
-// inner nodes are read from DevMesh::cnodes (64 bytes = TWO sectors per visit instead of four; the kernel is
-// bound by L1 data-pipe wavefronts once 20 warps are resident).  The 24 planes of a node are 16-bit offsets q from the
-// mesh's bounding-box corner G in units of s = 2^e: plane = G + q s.  Per ray and axis the slab value is one FMA,
-//     t = fma(m, A, B),   m = float(2^23 + q) (one PRMT builds it from the 16-bit field),  A = s inv32,
-//     B = fma(-2^23, A, fma(G, inv32, c32)),
-// and it differs from the exact-real slab value of that quantised plane by at most
-//     2^-24 |t| + 2^-21 (Bmax + |o|) |inv| + |A| / 2
-// (inv32, c32 carry 2^-24 relative each; the fma that forms B rounds a number of size 2^23 |A|, i.e. by up to |A| / 2; the
-// 2^23 A in m A cancels against it exactly).  The quantised box CONTAINS the exact f32 box, and the same box shrunk by
-// one grid step (|A| in t) on every side is CONTAINED in it (k_pack_nodes).  Per node and axis four shifted constants
-//     B - |A| (entry, outer)   B + 3|A| (entry, inner)   B + |A| (exit, outer)   B - 3|A| (exit, inner)
-// (each rounds by another |A| / 2 at most) give slab values that bracket the exact box's PER AXIS -- the grid step in t
-// is s / |d_a|, huge on an axis the ray is nearly parallel to, so one common margin would be useless:
-//     outer entry <= exact entry <= inner entry,   inner exit <= exact exit <= outer exit   (up to the first two terms),
-// and with E = R (|far| + |near|) + 2^-20 max (Bmax + |o|) |inv|  (R = 2^-22; margins doubled like in k_traverse):
-//     far_outer - near_outer < -E   =>  even the containing box is missed  =>  the reference's far > near fails;
-//     far_inner - near_inner >  E   =>  even the contained box is hit      =>  the reference's test passes;
-// only what lies in between -- the ray passes within ~4 grid steps of deciding otherwise -- is settled by the exact f64
-// test on the exact 128-byte node.  Results are bit-identical to the reference either way.
-template <bool NEAR, int STACK, int MIN_BLOCKS, bool COMPACT>
-__global__ void __launch_bounds__(kTraceThreads, MIN_BLOCKS) k_traverse_lean(const TraverseParams P) {
-  constexpr bool MIXED = true;
+template <int STACK>
+__global__ void __launch_bounds__(kTraceThreads, 5) k_traverse_lean(const TraverseParams P) {
   __shared__ uint32_t s_stack[STACK + 1][kTraceThreads];
   // what only the exact f64 code needs lives in shared memory, one column per lane: the ray in the mesh's space
   // (o, d) and the barycentrics of the best hit
@@ -42,58 +21,21 @@ __global__ void __launch_bounds__(kTraceThreads, MIN_BLOCKS) k_traverse_lean(con
   __shared__ double s_buv[2][kTraceThreads];
   const int tid = threadIdx.x;
   const uint32_t lane = tid & 31;
-  const uint32_t n_items = P.c.n_items_dev ? *P.c.n_items_dev : (uint32_t)P.c.n_items; // (yart_closest_hit caps n below 2^32)
-  // Work distribution: warp w starts with items [32w, 32w+32) without touching the counter and only then
-  // fetches dynamically from total_warps*32 + atomicAdd(counter).  Warps whose first slice is already past
-  // the end leave at once -- a nearly empty queue (the deep bounces) costs no same-address atomics.
-  // A short queue is spread thinly (rpw < 32 rays per warp): a warp's run time is the serialised work of
-  // its most divergent rays, so a deep bounce with a few hundred rays finishes sooner on many warps.
-  const uint32_t warp_global = (blockIdx.x * kTraceThreads + tid) >> 5;
-  const uint32_t total_warps = gridDim.x * (kTraceThreads / 32);
-  const uint32_t rpw = max(1u, min(32u, (uint32_t)(((uint64_t)n_items + total_warps - 1) / total_warps)));
-  const uint32_t dyn_base = total_warps * rpw; // (<= 2^17: at most a few thousand resident warps)
-  if ((uint64_t)warp_global * rpw >= n_items) return;
-  // Work items reach the lanes through a two-deep pipeline of 32-item chunks, so that neither the claim
-  // (an atomic), nor the queue read, nor the DRAM miss of the ray record sits on the warp's critical path:
-  //   chunk "cur": ids held one per lane (id_cur), handed to fetching lanes by shuffle;
-  //   chunk "nxt": claimed when cur was started (stage 1: atomic in flight), ids loaded one retire/fetch phase
-  //   later (stage 2), ray / hit records prefetched into L2 the phase after (stage 3).
-  // The first chunk of a warp is its static slice; all later ones come from the global counter.
-  const uint32_t cur_base = warp_global * rpw;
-  // the warp-uniform counters of the chunk pipeline share ONE register (bit fields of a 32-bit word)
-  struct {
-    uint32_t cur_cnt : 6, cur_used : 6, nxt_cnt : 6, nxt_stage : 2, dyn_done : 1;
-  } w;
-  w.cur_cnt = min(rpw, n_items - cur_base);
-  w.cur_used = 0;
-  uint32_t id_cur = YART_MISS, id_nxt = YART_MISS, claim_raw = 0;
-  if (lane < w.cur_cnt) id_cur = P.c.queue ? P.c.queue[cur_base + lane] : (uint32_t)(cur_base + lane);
-  w.dyn_done = dyn_base >= n_items; // nothing beyond the static slices: never touch the counter
-  w.nxt_cnt = 0;
-  w.nxt_stage = 0;
-  if (!w.dyn_done) {
-    if (lane == 0) claim_raw = atomicAdd(P.work_counter, 32u);
-    w.nxt_stage = 1;
-  }
-  const uint32_t RT = P.refill_threshold, NT = P.node_threshold;
-  const float4* __restrict__ nodes = P.nodes;
-  const float4* __restrict__ tris = P.tris;
+  ChunkQueue q;
+  if (!q.start(P.c.n_items_dev ? *P.c.n_items_dev : (uint32_t)P.c.n_items, P.c.queue, P.m.work_counter, lane)) return;
+  const uint32_t RT = P.m.refill_threshold, NT = P.m.node_threshold;
   const double t_min = P.c.t_min;
+  const float t_min_f = (float)t_min;
 
   // ---- lane state ----
   uint32_t ray_id = YART_MISS; // YART_MISS = idle
   uint32_t cur = kSentinel;    // current stack top (node or leaf id), kSentinel = not traversing
   int sp = 0;
-  uint32_t sgn = 0;  // ORDER_TABLE sign bits (mirrored when NEAR)
-  uint32_t pos = 0;  // bit a set: direction component a is >= 0 (qbvh.rs:388-392); bit 3: `weird`
+  SlabRay r = {};
   double t_best = 0;
+  float t_best_f = 0;
   uint32_t best_prim = YART_MISS; // YART_MISS = this mesh has not produced a hit
   bool exhausted = false;         // the global queue is empty
-  // MIXED: the ray as f32 slab coefficients t = b*inv + c, and the absolute part of the error bound
-  // !COMPACT: t = fma(b, ixf, cxf) per slab, amax2 = the absolute error term.  COMPACT: ixf.. hold A, cxf.. hold B,
-  // amax2 the constant part of E.
-  float ixf = 0, iyf = 0, izf = 0, cxf = 0, cyf = 0, czf = 0, amax2 = 0, t_best_f = 0;
-  const float t_min_f = (float)t_min;
 
   for (;;) {
     // =============== phase A: retire finished rays, fetch new ones ================================
@@ -114,134 +56,26 @@ __global__ void __launch_bounds__(kTraceThreads, MIN_BLOCKS) k_traverse_lean(con
         }
         ray_id = YART_MISS;
       }
-      // ---- advance the chunk pipeline by one stage (warp-uniform) ----
-      if (w.nxt_stage == 2) {
-        if (id_nxt != YART_MISS) {
-          YART_CHECK(id_nxt < P.c.n_rays);
-          if (P.c.rays32) {
-            const char* rp = reinterpret_cast<const char*>(P.c.rays32 + id_nxt);
-            prefetch_l2(rp);
-            prefetch_l2(rp + 23); // a 24-byte record may straddle two 32-byte sectors
-          } else {
-            const char* rp = reinterpret_cast<const char*>(P.c.rays + id_nxt);
-            prefetch_l2(rp);
-            prefetch_l2(rp + 32); // a 48-byte record always spans two 32-byte sectors
-          }
-          if (!P.c.first_pass) prefetch_l2(P.c.hits + id_nxt);
-        }
-        w.nxt_stage = 3;
-      }
-      // ---- hand out items (all lanes take part in the shuffles) ----
-      const bool fetching = want_a && !exhausted;
-      const uint32_t fmask = __ballot_sync(0xffffffffu, fetching);
-      const uint32_t need = (uint32_t)__popc(fmask);
-      const uint32_t rank = (uint32_t)__popc(fmask & ((1u << lane) - 1u));
-      const uint32_t take1 = min(need, (uint32_t)w.cur_cnt - (uint32_t)w.cur_used);
-      uint32_t new_id = __shfl_sync(0xffffffffu, id_cur, ((uint32_t)w.cur_used + rank) & 31u);
-      bool got = fetching && rank < take1;
-      w.cur_used = w.cur_used + take1;
-      if (need > take1) { // the current chunk ran out: the next one becomes current, and another is claimed
-        if (w.nxt_stage == 1) { // its claim has come back by now: read its ids
-          const uint64_t nb = (uint64_t)dyn_base + __shfl_sync(0xffffffffu, claim_raw, 0);
-          w.nxt_cnt = nb < n_items ? min(32u, n_items - (uint32_t)nb) : 0u;
-          id_nxt = YART_MISS;
-          if (lane < w.nxt_cnt) id_nxt = P.c.queue ? P.c.queue[nb + lane] : (uint32_t)(nb + lane);
-          if (w.nxt_cnt < 32u) w.dyn_done = 1; // the counter has passed the end of the queue
-          w.nxt_stage = 2;
-        }
-        if (w.nxt_stage >= 2) {
-          id_cur = id_nxt;
-          w.cur_cnt = w.nxt_cnt;
-        } else {
-          w.cur_cnt = 0;
-        }
-        w.cur_used = 0;
-        w.nxt_stage = 0;
-        w.nxt_cnt = 0;
-        if (!w.dyn_done) {
-          if (lane == 0) claim_raw = atomicAdd(P.work_counter, 32u);
-          w.nxt_stage = 1;
-        }
-        const uint32_t rank2 = rank - take1; // (meaningful for the lanes that are still waiting)
-        const uint32_t take2 = min(need - take1, (uint32_t)w.cur_cnt);
-        const uint32_t id2 = __shfl_sync(0xffffffffu, id_cur, rank2 & 31u);
-        if (fetching && !got && rank2 < take2) {
-          new_id = id2;
-          got = true;
-        }
-        w.cur_used = take2;
-        if (fetching && !got) exhausted = true; // only possible once the queue is used up
-      } else if (w.nxt_stage == 1) { // no swap this time: use the phase to resolve the claim and load the ids
-        const uint64_t nb = (uint64_t)dyn_base + __shfl_sync(0xffffffffu, claim_raw, 0);
-        w.nxt_cnt = nb < n_items ? min(32u, n_items - (uint32_t)nb) : 0u;
-        id_nxt = YART_MISS;
-        if (lane < w.nxt_cnt) id_nxt = P.c.queue ? P.c.queue[nb + lane] : (uint32_t)(nb + lane);
-        if (w.nxt_cnt < 32u) w.dyn_done = 1;
-        w.nxt_stage = 2;
-      }
-      if (got) {
-        {
-          ray_id = new_id;
-          YART_CHECK(ray_id < P.c.n_rays);
-          D3 ro, rd;
-          if (P.c.rays32) load_ray_f32(P.c.rays32 + ray_id, ro, rd);
-          else load_ray(P.c.rays + ray_id, ro, rd);
-          t_best = P.c.first_pass ? P.c.t_max : fmin(P.c.hits[ray_id].t, P.c.t_max);
-          if (NEAR) t_best = just_below(t_best); // strict against earlier objects / the caller's t_max (device_common.cuh)
-          // ray into the instance's space (hittable.rs:137-143, 218-227); uniform across the launch
-          if (P.wrap & YART_WRAP_TRANSLATE) ro = ro - d3(P.offset[0], P.offset[1], P.offset[2]);
-          if (P.wrap & YART_WRAP_ROTATE_Y) {
-            const double ct = P.cos_theta, st = P.sin_theta;
-            D3 org = ro, dir = rd;
-            org.x = ct * ro.x - st * ro.z;
-            org.z = st * ro.x + ct * ro.z;
-            dir.x = ct * rd.x - st * rd.z;
-            dir.z = st * rd.x + ct * rd.z;
-            ro = org;
-            rd = dir;
-          }
-          const double ox = ro.x, oy = ro.y, oz = ro.z, dx = rd.x, dy = rd.y, dz = rd.z;
-          const double ix = 1.0 / dx, iy = 1.0 / dy, iz = 1.0 / dz; // qbvh.rs:403-407
-          s_ray[0][tid] = ox; s_ray[1][tid] = oy; s_ray[2][tid] = oz;
-          s_ray[3][tid] = dx; s_ray[4][tid] = dy; s_ray[5][tid] = dz;
-          pos = (dx >= 0.0 ? 1u : 0u) | (dy >= 0.0 ? 2u : 0u) | (dz >= 0.0 ? 4u : 0u); // qbvh.rs:388-392
-          sgn = NEAR ? (pos ^ 7u) : pos;
-          // (b - o) * (1/d) can only be NaN when 1/d is infinite or the ray itself is not finite
-          if (!(isfinite(ix) && isfinite(iy) && isfinite(iz) && isfinite(ox) && isfinite(oy) && isfinite(oz))) pos |= 8u;
-          if (MIXED) {
-            ixf = (float)ix; iyf = (float)iy; izf = (float)iz;
-            cxf = (float)(-(ox * ix)); cyf = (float)(-(oy * iy)); czf = (float)(-(oz * iz));
-            // |t32 - t64| <= 2^-24 (|b| + |o|) |inv| + 2^-24 |t32| (+ f64 roundings); doubled for margin:
-            // absolute part A = 2^-23 (B + |o|) |inv| maximised over the axes, kept as 2A (rounded up)
-            const double a = fmax(fmax((P.bound[0] + fabs(ox)) * fabs(ix), (P.bound[1] + fabs(oy)) * fabs(iy)),
-                                  (P.bound[2] + fabs(oz)) * fabs(iz));
-            amax2 = __double2float_ru(a * (1.0 / 4194304.0)); // 2A = 2^-22 * a
-            // rays whose f32 image is not well inside the normal range take the exact path throughout
-            const float lo = 1e-30f, hi = 1e30f;
-            const bool ok = fabsf(ixf) > lo && fabsf(ixf) < hi && fabsf(iyf) > lo && fabsf(iyf) < hi && fabsf(izf) > lo &&
-                            fabsf(izf) < hi && fabsf(cxf) < hi && fabsf(cyf) < hi && fabsf(czf) < hi && amax2 < hi;
-            if (!ok) pos |= 8u;
-            if (COMPACT) {
-              const float ax = P.cscale * ixf, ay = P.cscale * iyf, az = P.cscale * izf; // (exact: a power of two)
-              const float bx = fmaf(-8388608.f, ax, fmaf(P.corigin[0], ixf, cxf));
-              const float by = fmaf(-8388608.f, ay, fmaf(P.corigin[1], iyf, cyf));
-              const float bz = fmaf(-8388608.f, az, fmaf(P.corigin[2], izf, czf));
-              const float q = fmaxf(fabsf(ax), fmaxf(fabsf(ay), fabsf(az)));
-              const float aterm = __double2float_ru(a * (1.0 / 1048576.0)); // 2^-20 * a
-              const bool okc = fabsf(bx) < hi && fabsf(by) < hi && fabsf(bz) < hi && q < hi && q > 0.f && aterm < hi;
-              if (!okc) pos |= 8u;
-              ixf = ax; iyf = ay; izf = az;
-              cxf = bx; cyf = by; czf = bz;
-              amax2 = aterm;
-            }
-            t_best_f = (float)t_best;
-          }
-          cur = P.root;
-          sp = 0;
-          best_prim = YART_MISS;
-          s_buv[0][tid] = 0.0;
-          s_buv[1][tid] = 0.0;
-        }
+      uint32_t id;
+      if (q.next(want_a && !exhausted, lane, P.c.queue, P.m.work_counter, P.c.rays, P.c.rays32,
+                 P.c.first_pass ? nullptr : P.c.hits, P.c.n_rays, id, exhausted)) {
+        ray_id = id;
+        YART_CHECK(ray_id < P.c.n_rays);
+        D3 ro, rd;
+        if (P.c.rays32) load_ray_f32(P.c.rays32 + ray_id, ro, rd);
+        else load_ray(P.c.rays + ray_id, ro, rd);
+        t_best = P.c.first_pass ? P.c.t_max : fmin(P.c.hits[ray_id].t, P.c.t_max);
+        t_best = just_below(t_best); // strict against earlier objects / the caller's t_max (device_common.cuh)
+        instance_to_object(P.m.wrap, P.m.offset, P.m.sin_theta, P.m.cos_theta, ro, rd); // uniform across the launch
+        s_ray[0][tid] = ro.x; s_ray[1][tid] = ro.y; s_ray[2][tid] = ro.z;
+        s_ray[3][tid] = rd.x; s_ray[4][tid] = rd.y; s_ray[5][tid] = rd.z;
+        r = slab_ray(ro, rd, P.m.bound, true);
+        t_best_f = (float)t_best;
+        cur = P.m.root;
+        sp = 0;
+        best_prim = YART_MISS;
+        s_buv[0][tid] = 0.0;
+        s_buv[1][tid] = 0.0;
       }
     }
     if (!__any_sync(0xffffffffu, ray_id != YART_MISS)) break;
@@ -259,239 +93,42 @@ __global__ void __launch_bounds__(kTraceThreads, MIN_BLOCKS) k_traverse_lean(con
         if (lm != 0 || (uint32_t)__popc(wm) >= RT) break;
       }
       if (has_node) {
-        YART_CHECK(cur < P.n_nodes);
-        uint4 ch;
-        uint32_t axes, hitmask = 0;
-        if (COMPACT) {
-          const float4* cn = reinterpret_cast<const float4*>(P.cnodes) + (size_t)cur * 4;
-          const F8 c0 = ldg256(cn), c1 = ldg256(cn + 2); // the whole 64-byte node: two sectors
-          // child words: ids with the node's axes in bits 29-30 of the first three (k_pack_nodes)
-          const uint32_t w0 = __float_as_uint(c1.hi.x), w1 = __float_as_uint(c1.hi.y), w2 = __float_as_uint(c1.hi.z),
-                         w3 = __float_as_uint(c1.hi.w);
-          ch = make_uint4(w0 & 0x9FFFFFFFu, w1 & 0x9FFFFFFFu, w2 & 0x9FFFFFFFu, w3);
-          axes = ((w0 >> 29) & 3u) | (((w1 >> 29) & 3u) << 2) | (((w2 >> 29) & 3u) << 4);
-          const uint32_t present = ((w0 | 0x60000000u) != 0xFFFFFFFFu ? 1u : 0u) | ((w1 | 0x60000000u) != 0xFFFFFFFFu ? 2u : 0u) |
-                                   ((w2 | 0x60000000u) != 0xFFFFFFFFu ? 4u : 0u) | (w3 != 0xFFFFFFFFu ? 8u : 0u);
-          if (!(pos & 8u)) {
-            const bool px = (pos & 1u) != 0, py = (pos & 2u) != 0, pz = (pos & 4u) != 0;
-            // entry / exit planes: the lower or the upper 16-bit fields, by the sign of the direction (12 selects)
-            const uint32_t xl01 = __float_as_uint(c0.lo.x), xl23 = __float_as_uint(c0.lo.y), xh01 = __float_as_uint(c0.lo.z),
-                           xh23 = __float_as_uint(c0.lo.w), yl01 = __float_as_uint(c0.hi.x), yl23 = __float_as_uint(c0.hi.y),
-                           yh01 = __float_as_uint(c0.hi.z), yh23 = __float_as_uint(c0.hi.w), zl01 = __float_as_uint(c1.lo.x),
-                           zl23 = __float_as_uint(c1.lo.y), zh01 = __float_as_uint(c1.lo.z), zh23 = __float_as_uint(c1.lo.w);
-            const uint32_t nx01 = px ? xl01 : xh01, nx23 = px ? xl23 : xh23, fx01 = px ? xh01 : xl01, fx23 = px ? xh23 : xl23;
-            const uint32_t ny01 = py ? yl01 : yh01, ny23 = py ? yl23 : yh23, fy01 = py ? yh01 : yl01, fy23 = py ? yh23 : yl23;
-            const uint32_t nz01 = pz ? zl01 : zh01, nz23 = pz ? zl23 : zh23, fz01 = pz ? zh01 : zl01, fz23 = pz ? zh23 : zl23;
-            uint32_t amb = 0;
-            // the four shifted constants per axis (see the bound above)
-            const float hx = fabsf(ixf), hy = fabsf(iyf), hz = fabsf(izf);
-            const float bxno = cxf - hx, bxni = fmaf(3.f, hx, cxf), bxfo = cxf + hx, bxfi = fmaf(-3.f, hx, cxf);
-            const float byno = cyf - hy, byni = fmaf(3.f, hy, cyf), byfo = cyf + hy, byfi = fmaf(-3.f, hy, cyf);
-            const float bzno = czf - hz, bzni = fmaf(3.f, hz, czf), bzfo = czf + hz, bzfi = fmaf(-3.f, hz, czf);
-            // float(2^23 + q) from a 16-bit field: bytes {q.lo, q.hi, 0x00, 0x4B}
-#define YART_MAGIC(W, HALF) __uint_as_float(__byte_perm((W), 0x4B000000u, (HALF) ? 0x7432u : 0x7410u))
-#define YART_BOX_Q(K, NXW, NYW, NZW, FXW, FYW, FZW, HALF)                                                              \
-  {                                                                                                                    \
-    const float mnx = YART_MAGIC(NXW, HALF), mny = YART_MAGIC(NYW, HALF), mnz = YART_MAGIC(NZW, HALF);                 \
-    const float mfx = YART_MAGIC(FXW, HALF), mfy = YART_MAGIC(FYW, HALF), mfz = YART_MAGIC(FZW, HALF);                 \
-    const float tno = fmaxf(fmaxf(t_min_f, fmaf(mnx, ixf, bxno)), fmaxf(fmaf(mny, iyf, byno), fmaf(mnz, izf, bzno)));  \
-    const float tfo = fminf(fminf(t_best_f, fmaf(mfx, ixf, bxfo)), fminf(fmaf(mfy, iyf, byfo), fmaf(mfz, izf, bzfo))); \
-    const float tni = fmaxf(fmaxf(t_min_f, fmaf(mnx, ixf, bxni)), fmaxf(fmaf(mny, iyf, byni), fmaf(mnz, izf, bzni)));  \
-    const float tfi = fminf(fminf(t_best_f, fmaf(mfx, ixf, bxfi)), fminf(fmaf(mfy, iyf, byfi), fmaf(mfz, izf, bzfi))); \
-    const float e = fmaf(fabsf(tfo) + fabsf(tno), 2.384185791015625e-7f, amax2);                                       \
-    const bool hit = (tfi - tni) > e, miss = (tfo - tno) < -e;                                                         \
-    hitmask |= hit ? (1u << (K)) : 0u;                                                                                 \
-    amb |= (hit || miss) ? 0u : (1u << (K));                                                                           \
-  }
-            YART_BOX_Q(0, nx01, ny01, nz01, fx01, fy01, fz01, 0)
-            YART_BOX_Q(1, nx01, ny01, nz01, fx01, fy01, fz01, 1)
-            YART_BOX_Q(2, nx23, ny23, nz23, fx23, fy23, fz23, 0)
-            YART_BOX_Q(3, nx23, ny23, nz23, fx23, fy23, fz23, 1)
-#undef YART_BOX_Q
-#undef YART_MAGIC
-            hitmask &= present;
-            amb &= present;
-            if (amb) {
-              const uint32_t exact = box4_ieee<NEAR>(nodes + (size_t)cur * 8, s_ray[0][tid], s_ray[1][tid], s_ray[2][tid], 1.0 / s_ray[3][tid],
-                                                     1.0 / s_ray[4][tid], 1.0 / s_ray[5][tid], t_min, t_best);
-              hitmask = (hitmask & ~amb) | (exact & amb);
-            }
-          } else {
-            hitmask = box4_ieee<NEAR>(nodes + (size_t)cur * 8, s_ray[0][tid], s_ray[1][tid], s_ray[2][tid], 1.0 / s_ray[3][tid],
-                                      1.0 / s_ray[4][tid], 1.0 / s_ray[5][tid], t_min, t_best);
-          }
-        } else {
-          const float4* nd = nodes + (size_t)cur * 8;
-          // the whole 128-byte node in four 256-bit loads, all in flight together
-          const F8 sx8 = ldg256(nd + 0), sy8 = ldg256(nd + 2), sz8 = ldg256(nd + 4), cm8 = ldg256(nd + 6);
-          ch = make_uint4(__float_as_uint(cm8.lo.x), __float_as_uint(cm8.lo.y), __float_as_uint(cm8.lo.z), __float_as_uint(cm8.lo.w));
-          axes = __float_as_uint(cm8.hi.x);
-          if (MIXED && !(pos & 8u)) {
-            // Conservative f32 test.  Per slab t32 = fma(b, inv32, c32); near32 / far32 are the max / min over
-            // the entry / exit planes with t_min / t_best folded in.  With R = 2^-22 and A as above,
-            // |near32 - near64| <= R|near32| + A and the same for far, so
-            //   far32 - near32 >  R(|far32| + |near32|) + 2A  =>  far64 > near64   (the reference pushes)
-            //   far32 - near32 < -R(|far32| + |near32|) - 2A  =>  far64 < near64   (the reference does not)
-            // and everything in between (also any inf / NaN) is settled by the exact f64 test.
-            const bool px = (pos & 1u) != 0, py = (pos & 2u) != 0, pz = (pos & 4u) != 0;
-  #define YART_SEL4(P_, A, B) make_float4((P_) ? A.x : B.x, (P_) ? A.y : B.y, (P_) ? A.z : B.z, (P_) ? A.w : B.w)
-            const float4 nx = YART_SEL4(px, sx8.lo, sx8.hi), fx = YART_SEL4(px, sx8.hi, sx8.lo);
-            const float4 ny = YART_SEL4(py, sy8.lo, sy8.hi), fy = YART_SEL4(py, sy8.hi, sy8.lo);
-            const float4 nz = YART_SEL4(pz, sz8.lo, sz8.hi), fz = YART_SEL4(pz, sz8.hi, sz8.lo);
-  #undef YART_SEL4
-            uint32_t amb = 0;
-  #define YART_BOX_F32(K, C)                                                                                  \
-    {                                                                                                         \
-      const float tn = fmaxf(fmaxf(t_min_f, fmaf(nx.C, ixf, cxf)), fmaxf(fmaf(ny.C, iyf, cyf), fmaf(nz.C, izf, czf))); \
-      const float tf = fminf(fminf(t_best_f, fmaf(fx.C, ixf, cxf)), fminf(fmaf(fy.C, iyf, cyf), fmaf(fz.C, izf, czf))); \
-      const float g = tf - tn;                                                                                \
-      const float e = fmaf(fabsf(tf) + fabsf(tn), 2.384185791015625e-7f, amax2);                              \
-      hitmask |= (g > e) ? (1u << (K)) : 0u;                                                                  \
-      amb |= ((g > e) || (g < -e)) ? 0u : (1u << (K));                                                        \
-    }
-            YART_BOX_F32(0, x)
-            YART_BOX_F32(1, y)
-            YART_BOX_F32(2, z)
-            YART_BOX_F32(3, w)
-  #undef YART_BOX_F32
-            if (amb) {
-              const uint32_t exact = box4_ieee<NEAR>(nd, s_ray[0][tid], s_ray[1][tid], s_ray[2][tid], 1.0 / s_ray[3][tid], 1.0 / s_ray[4][tid],
-                                                     1.0 / s_ray[5][tid], t_min, t_best);
-              hitmask = (hitmask & ~amb) | (exact & amb);
-            }
-          } else {
-            hitmask = box4_ieee<NEAR>(nd, s_ray[0][tid], s_ray[1][tid], s_ray[2][tid], 1.0 / s_ray[3][tid], 1.0 / s_ray[4][tid],
-                                      1.0 / s_ray[5][tid], t_min, t_best);
-          }
-        }
-        // push_hit_children (qbvh.rs:18-31) in the order ORDER_TABLE[4*pos[top] + 2*pos[left] + pos[right]]
-        // (qbvh.rs:14-16, 521-524) gives.  The table has structure: bit `top` says whether the left pair
-        // {0,1} is pushed before the right pair {2,3}; `left` whether 0 goes before 1, `right` whether 2 goes
-        // before 3.  So every hit child's stack slot is a closed form of the hit bits -- four predicated
-        // stores, no table, no serial loop.
-        {
-          const uint32_t T = (sgn >> (axes & 3u)) & 1u, L = (sgn >> ((axes >> 2) & 3u)) & 1u,
-                         Rr = (sgn >> ((axes >> 4) & 3u)) & 1u;
-          const uint32_t h0 = hitmask & 1u, h1 = (hitmask >> 1) & 1u, h2 = (hitmask >> 2) & 1u, h3 = (hitmask >> 3) & 1u;
-          const uint32_t nl = h0 + h1, nr = h2 + h3;
-          const uint32_t bl = T ? 0u : nr, br = T ? nl : 0u; // slots taken by the pair pushed first
-          if (h0) s_stack[sp + bl + (L ? 0u : h1)][tid] = ch.x;
-          if (h1) s_stack[sp + bl + (L ? h0 : 0u)][tid] = ch.y;
-          if (h2) s_stack[sp + br + (Rr ? 0u : h3)][tid] = ch.z;
-          if (h3) s_stack[sp + br + (Rr ? h2 : 0u)][tid] = ch.w;
-          sp += (int)(nl + nr);
-          YART_CHECK(sp <= STACK + 1);
-        }
-        if (sp == 0) {
-          cur = kSentinel;
-        } else {
-          sp--;
-          cur = s_stack[sp][tid];
-        }
+        const float4* nd = node_at(P.m, cur);
+        const QNode n = load_node(nd);
+        uint32_t undecided;
+        const uint32_t hitmask = node_hits<true>(nd, n, r, t_min_f, t_best_f, &s_ray[0][tid], kTraceThreads, t_min, t_best, undecided);
+        push_children<STACK>(s_stack, tid, sp, hitmask, r.sgn, n);
+        cur = pop(s_stack, tid, sp);
       }
     }
 
     // =============== phase C: one leaf (qbvh.rs:413-490) ========================================
     if (cur >= 0x80000000u) {
-      const uint32_t count = COMPACT ? ((cur >> 27) & 3u) + 1u : (cur >> 27) & 0xFu; // (compact child words keep count - 1)
+      const uint32_t count = (cur >> 27) & 0xFu;
       const uint32_t first = cur & 0x7FFFFFFu;
-      YART_CHECK(count >= 1 && count <= 4 && first + count <= P.n_tris);
-      const double ox = s_ray[0][tid], oy = s_ray[1][tid], oz = s_ray[2][tid];
-      const double dx = s_ray[3][tid], dy = s_ray[4][tid], dz = s_ray[5][tid];
-      // Moeller-Trumbore exactly as qbvh.rs:419-489 on one triangle given as 9 floats
-#define YART_TRI_TEST(I_, F0, F1, F2, F3, F4, F5, F6, F7, F8)                                                       \
-  {                                                                                                                 \
-    const double v0x = (double)(F0), v0y = (double)(F1), v0z = (double)(F2);                                        \
-    const double e1x = (double)(F3) - v0x, e1y = (double)(F4) - v0y, e1z = (double)(F5) - v0z;                      \
-    const double e2x = (double)(F6) - v0x, e2y = (double)(F7) - v0y, e2z = (double)(F8) - v0z;                      \
-    const double hx = dy * e2z - dz * e2y, hy = dz * e2x - dx * e2z, hz = dx * e2y - dy * e2x;                      \
-    const double a = e1x * hx + e1y * hy + e1z * hz;                                                                \
-    bool ok = !((a > -kF64Eps) && (a < kF64Eps));                                                                   \
-    const double f = 1.0 / a;                                                                                       \
-    const double sx = ox - v0x, sy = oy - v0y, sz = oz - v0z;                                                       \
-    const double u = f * (sx * hx + sy * hy + sz * hz);                                                             \
-    ok = ok && (u >= 0.0) && (u <= 1.0);                                                                            \
-    const double qx = sy * e1z - sz * e1y, qy = sz * e1x - sx * e1z, qz = sx * e1y - sy * e1x;                      \
-    const double v = f * (dx * qx + dy * qy + dz * qz);                                                             \
-    ok = ok && (v >= 0.0) && ((u + v) <= 1.0);                                                                      \
-    const double t = f * (e2x * qx + e2y * qy + e2z * qz);                                                          \
-    ok = ok && (t >= t_min);                                                                                        \
-    /* REFERENCE: first found wins (`t_max > t`, qbvh.rs:478).  NEAR: mirrored -- last found wins among this */    \
-    /* mesh's equal-t hits, still strictly closer than what earlier objects left.                            */    \
-    ok = ok && (NEAR ? (t <= t_best) : (t_best > t));                                                               \
-    if (ok) {                                                                                                       \
-      t_best = t; best_prim = first + (I_); s_buv[0][tid] = u; s_buv[1][tid] = v;                                   \
-      if (MIXED) t_best_f = (float)t;                                                                               \
-    }                                                                                                               \
-  }
-      if (count <= 3u) {
-        // The leaf's triangles as one packed block (36 B each, 32-byte aligned): 2 / 3 / 4 sector loads for
-        // 1 / 2 / 3 triangles instead of 3 loads per triangle, all in flight together.
-        const float4* lp = P.leafgeo + (size_t)first * 4;
-        // at most three sectors in registers at a time: the next one is requested one test ahead
-        if (NEAR) { // lanes in reverse order (mirrored tie rule): from the last sector backwards
-          F8 s1 = ldg256(lp + 2), s2, s3;
-          s2.lo = s2.hi = s3.lo = s3.hi = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (count >= 2u) s2 = ldg256(lp + 4);
-          if (count >= 3u) {
-            s3 = ldg256(lp + 6);
-            YART_TRI_TEST(2u, s2.lo.z, s2.lo.w, s2.hi.x, s2.hi.y, s2.hi.z, s2.hi.w, s3.lo.x, s3.lo.y, s3.lo.z)
-          }
-          const F8 s0 = ldg256(lp);
-          if (count >= 2u) YART_TRI_TEST(1u, s1.lo.y, s1.lo.z, s1.lo.w, s1.hi.x, s1.hi.y, s1.hi.z, s1.hi.w, s2.lo.x, s2.lo.y)
-          YART_TRI_TEST(0u, s0.lo.x, s0.lo.y, s0.lo.z, s0.lo.w, s0.hi.x, s0.hi.y, s0.hi.z, s0.hi.w, s1.lo.x)
-        } else {
-          const F8 s0 = ldg256(lp), s1 = ldg256(lp + 2);
-          F8 s2, s3;
-          s2.lo = s2.hi = s3.lo = s3.hi = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (count >= 2u) s2 = ldg256(lp + 4);
-          YART_TRI_TEST(0u, s0.lo.x, s0.lo.y, s0.lo.z, s0.lo.w, s0.hi.x, s0.hi.y, s0.hi.z, s0.hi.w, s1.lo.x)
-          if (count >= 3u) s3 = ldg256(lp + 6);
-          if (count >= 2u) YART_TRI_TEST(1u, s1.lo.y, s1.lo.z, s1.lo.w, s1.hi.x, s1.hi.y, s1.hi.z, s1.hi.w, s2.lo.x, s2.lo.y)
-          if (count >= 3u) YART_TRI_TEST(2u, s2.lo.z, s2.lo.w, s2.hi.x, s2.hi.y, s2.hi.z, s2.hi.w, s3.lo.x, s3.lo.y, s3.lo.z)
+      YART_CHECK(count >= 1 && count <= 4 && first + count <= P.m.n_tris);
+      const D3 o = d3(s_ray[0][tid], s_ray[1][tid], s_ray[2][tid]), d = d3(s_ray[3][tid], s_ray[4][tid], s_ray[5][tid]);
+      // triangles in reverse order: the last found wins among this mesh's equal-t hits (the mirrored tie rule), still
+      // strictly closer than what earlier objects left
+      visit_leaf<true>(P.m.leafgeo, P.m.tris, first, count, [&](uint32_t i, const Tri9& tri) {
+        double t, u, v;
+        if (mt_hit(tri, o, d, t_min, t, u, v) && t <= t_best) {
+          t_best = t; best_prim = first + i; s_buv[0][tid] = u; s_buv[1][tid] = v;
+          t_best_f = (float)t;
         }
-      } else {
-        // 4-triangle leaves: one 48-byte record at a time, the next one requested before the current is tested
-        float4 n0, n1, n2;
-        {
-          const float4* tp = tris + (size_t)(first + (NEAR ? (count - 1u) : 0u)) * 3;
-          n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
-        }
-        for (uint32_t j = 0; j < count; ++j) {
-          const uint32_t i = NEAR ? (count - 1u - j) : j;
-          const float4 a0 = n0, a1 = n1, a2 = n2;
-          if (j + 1u < count) {
-            const float4* tp = tris + (size_t)(first + (NEAR ? (i - 1u) : (i + 1u))) * 3;
-            n0 = __ldg(tp); n1 = __ldg(tp + 1); n2 = __ldg(tp + 2);
-          }
-          YART_TRI_TEST(i, a0.x, a0.y, a0.z, a1.x, a1.y, a1.z, a2.x, a2.y, a2.z)
-        }
-      }
-#undef YART_TRI_TEST
-      if (sp == 0) {
-        cur = kSentinel;
-      } else {
-        sp--;
-        cur = s_stack[sp][tid];
-      }
+        return false;
+      });
+      cur = pop(s_stack, tid, sp);
     }
   }
 }
 
-
-typedef void (*TraverseKernel)(const TraverseParams);
-// (visit counting and the all-f64 slab variant stay with k_traverse)
-// ctas_per_sm: 5 (96 registers, 20 warps per SM) or 6 (80 registers, 24 warps).  The stack is sized to the tree:
-// 24 entries cover 7 node levels (3 * height + 1 = 22: david, sycee), 32 cover 10, 64 the reference's own limit.
-template <int MIN_BLOCKS, bool COMPACT>
-static TraverseKernel pick_lean(bool near, uint32_t max_stack) {
-  if (max_stack <= 24) return near ? k_traverse_lean<true, 24, MIN_BLOCKS, COMPACT> : k_traverse_lean<false, 24, MIN_BLOCKS, COMPACT>;
-  if (max_stack <= 32) return near ? k_traverse_lean<true, 32, MIN_BLOCKS, COMPACT> : k_traverse_lean<false, 32, MIN_BLOCKS, COMPACT>;
-  return near ? k_traverse_lean<true, 64, MIN_BLOCKS, COMPACT> : k_traverse_lean<false, 64, MIN_BLOCKS, COMPACT>;
-}
-TraverseKernel lean_traverse_kernel(bool near, uint32_t max_stack, int ctas_per_sm, bool compact) {
-  if (compact) return pick_lean<5, true>(near, max_stack);
-  return ctas_per_sm >= 6 ? pick_lean<6, false>(near, max_stack) : pick_lean<5, false>(near, max_stack);
+// The stack is sized to the tree: 24 entries cover 7 node levels (3 * height + 1 = 22: david, sycee), 32 cover 10,
+// 64 the reference's own limit.
+TraverseKernel lean_traverse_kernel(uint32_t max_stack) {
+  if (max_stack <= 24) return k_traverse_lean<24>;
+  if (max_stack <= 32) return k_traverse_lean<32>;
+  return k_traverse_lean<64>;
 }
 
 } // namespace yart

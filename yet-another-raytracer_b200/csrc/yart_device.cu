@@ -142,47 +142,6 @@ __global__ void __launch_bounds__(256) k_pack_leaves(const FlatNode* __restrict_
   }
 }
 
-// DevMesh::cnodes from the flattened tree, one thread per node.  Word layout of a 64-byte compact node (two 32-byte
-// sectors; every 32-bit word holds the 16-bit values of two children, child 2j in the low half, 2j+1 in the high half):
-//   sector 0: x lower planes (children 01, 23), x upper planes (01, 23), y lower (01, 23), y upper (01, 23)
-//   sector 1: z lower (01, 23), z upper (01, 23), then the four child words exactly as in FlatNode::child, with the node's
-//             three split axes stowed in the otherwise unused bits 29-30 of the first three words (child ids use bits
-//             0-26 + the leaf flag 31 + the leaf count 27-28 as count-1).  0xFFFFFFFF = absent child, as in FlatNode.
-// Quantisation, exact in f64: lower plane -> floor((b - origin) / scale), upper plane -> ceil(...): the quantised box
-// contains the exact box, and shrinking it by one unit on every side gives a box contained in the exact one.
-__global__ void __launch_bounds__(256) k_pack_nodes(const FlatNode* __restrict__ nodes, uint32_t n_nodes, float ox, float oy, float oz,
-                                                     float scale, uint4* __restrict__ out) {
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_nodes) return;
-  const FlatNode nd = nodes[i];
-  const double o[3] = {(double)ox, (double)oy, (double)oz}, inv = 1.0 / (double)scale; // (scale is a power of two)
-  const float* lo[3] = {nd.min_x, nd.min_y, nd.min_z};
-  const float* hi[3] = {nd.max_x, nd.max_y, nd.max_z};
-  uint32_t w[16];
-  for (int a = 0; a < 3; ++a)
-    for (int pair = 0; pair < 2; ++pair) {
-      uint32_t ql[2], qh[2];
-      for (int h = 0; h < 2; ++h) {
-        const int k = pair * 2 + h;
-        const bool present = nd.child[k] != 0xFFFFFFFFu;
-        const double l = floor(((double)lo[a][k] - o[a]) * inv), u = ceil(((double)hi[a][k] - o[a]) * inv);
-        ql[h] = present ? (uint32_t)fmin(fmax(l, 0.0), 65535.0) : 65535u; // (an absent child: an inverted box)
-        qh[h] = present ? (uint32_t)fmin(fmax(u, 0.0), 65535.0) : 0u;
-      }
-      w[a * 4 + pair] = ql[0] | (ql[1] << 16);
-      w[a * 4 + 2 + pair] = qh[0] | (qh[1] << 16);
-    }
-  for (int k = 0; k < 4; ++k) {
-    uint32_t c = nd.child[k];
-    if (c != 0xFFFFFFFFu) {
-      if (c >> 31) c = 0x80000000u | ((((c >> 27) & 0xFu) - 1u) << 27) | (c & 0x7FFFFFFu); // leaf count 1..4 -> 2 bits
-      if (k < 3) c |= ((nd.axes >> (2 * k)) & 3u) << 29;                                    // top, left, right axis
-    }
-    w[12 + k] = c;
-  }
-  for (int j = 0; j < 4; ++j) out[(size_t)i * 4 + j] = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-}
-
 // yart_measure_fetch_peak: independent random 128-byte line fetches (one QBVH node visit = four LDG.E.256)
 template <int THREADS, int MIN_BLOCKS>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) k_fetch_peak(const float4* __restrict__ table, uint32_t n_lines, uint32_t iters,
@@ -492,23 +451,50 @@ DevCamera make_camera(const yart_camera& c) { // Camera::new (camera.rs:41-80), 
   return k;
 }
 
-typedef void (*TraverseKernel)(const TraverseParams);
-} // namespace
-namespace yart {
-TraverseKernel lean_traverse_kernel(bool near, uint32_t max_stack, int ctas_per_sm, bool compact); // device_trace_lean.cu
+// The closest-hit kernel of one mesh pass: near-first without visit counting is k_traverse_lean (device_trace_lean.cu):
+// 96 registers, FIVE 128-thread CTAs per SM (20 warps) instead of four, +7 % on the david render, +6 % on the sweep.
+// The reference order and every counted query take k_traverse.
+TraverseKernel traverse_kernel(bool near, bool count, uint32_t max_stack) {
+  if (near && !count) return lean_traverse_kernel(max_stack);
+  if (max_stack <= 32) return near ? k_traverse<true, true, 32> : count ? k_traverse<false, true, 32> : k_traverse<false, false, 32>;
+  return near ? k_traverse<true, true, 64> : count ? k_traverse<false, true, 64> : k_traverse<false, false, 64>;
 }
-namespace {
-template <bool MIXED>
-TraverseKernel pick_traverse_kernel_m(bool near, bool count, uint32_t max_stack) {
-  if (max_stack <= 32) {
-    if (near) return count ? k_traverse<true, true, 32, MIXED> : k_traverse<true, false, 32, MIXED>;
-    return count ? k_traverse<false, true, 32, MIXED> : k_traverse<false, false, 32, MIXED>;
+
+// One mesh instance of the world list for a traversal pass; work_counter must be zero at launch.
+MeshPass mesh_pass(const yart_object& o, const DevMesh& m, uint32_t* work_counter) {
+  static const int rt = tune_env("YART_TUNE_RT", 8), nt = tune_env("YART_TUNE_NT", 12);
+  MeshPass p;
+  memset(&p, 0, sizeof(p));
+  p.nodes = m.nodes;
+  p.tris = m.tris;
+  p.leafgeo = m.leafgeo;
+  p.root = m.root;
+  p.n_nodes = m.n_nodes;
+  p.n_tris = m.n_tris;
+  p.wrap = o.wrap & (YART_WRAP_ROTATE_Y | YART_WRAP_TRANSLATE);
+  p.sin_theta = o.sin_theta;
+  p.cos_theta = o.cos_theta;
+  for (int k = 0; k < 3; ++k) p.offset[k] = o.offset[k];
+  for (int k = 0; k < 3; ++k) p.bound[k] = m.bound[k];
+  p.refill_threshold = (uint32_t)std::max(1, std::min(32, rt));
+  p.node_threshold = (uint32_t)std::max(1, std::min(32, nt));
+  p.work_counter = work_counter;
+  return p;
+}
+
+// A persistent traversal kernel: one resident wave of CTAs.  The carveout leaves everything the stacks do not need
+// to L1, where the tree's upper levels live.  It and the occupancy query are set once per kernel: they cost tens of
+// microseconds of host time, which is the whole budget of a deep bounce.
+template <class Params>
+int launch_persistent(yart_ctx* ctx, void (*k)(const Params), int carveout, const Params& p) {
+  int& per_sm = ctx->traverse_blocks[(const void*)k];
+  if (per_sm == 0) {
+    cudaFuncSetAttribute(reinterpret_cast<const void*>(k), cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
+    CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(k), kTraceThreads, 0));
+    per_sm = std::max(per_sm, 1);
   }
-  if (near) return count ? k_traverse<true, true, 64, MIXED> : k_traverse<true, false, 64, MIXED>;
-  return count ? k_traverse<false, true, 64, MIXED> : k_traverse<false, false, 64, MIXED>;
-}
-TraverseKernel pick_traverse_kernel(bool near, bool count, uint32_t max_stack, bool mixed) {
-  return mixed ? pick_traverse_kernel_m<true>(near, count, max_stack) : pick_traverse_kernel_m<false>(near, count, max_stack);
+  k<<<per_sm * ctx->sm_count, kTraceThreads, 0, ctx->stream>>>(p);
+  return YART_OK;
 }
 
 // What is the same for every pass of one closest-hit query.
@@ -528,10 +514,8 @@ struct QueryArgs {
 // HittableList::hit (hittable.rs:66-79) as passes over the ray queue, in list order: one k_traverse per
 // mesh instance, one k_analytic per run of consecutive analytic objects.
 int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
-  static const int rt = tune_env("YART_TUNE_RT", 8), nt = tune_env("YART_TUNE_NT", 12);
   static const int carve = tune_env("YART_TUNE_CARVEOUT", 35);
   static const int carve_lean = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
-  static const int mixed = tune_env("YART_TUNE_MIXED", 1); // 0: all-f64 slab tests (same results, slower)
   bool first = true;
   uint32_t i = 0, n_trav = 0;
   auto is_mesh = [&](uint32_t k) {
@@ -551,54 +535,16 @@ int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
   while (i < q.n_objects) {
     if (is_mesh(i)) {
       const yart_object& o = q.h_objects[i];
-      const DevMesh& m = ctx->h_meshes[o.index];
       TraverseParams T;
       memset(&T, 0, sizeof(T));
       T.c = q.c;
       T.c.first_pass = first ? 1u : 0u;
-      T.nodes = m.nodes;
-      T.tris = m.tris;
-      T.leafgeo = m.leafgeo;
-      T.cnodes = m.cnodes;
-      T.cscale = m.cscale;
-      for (int k = 0; k < 3; ++k) T.corigin[k] = m.corigin[k];
-      T.root = m.root;
-      T.n_nodes = m.n_nodes;
-      T.n_tris = m.n_tris;
+      T.m = mesh_pass(o, ctx->h_meshes[o.index], q.work_counters + n_trav++);
       T.obj_index = i;
-      T.wrap = o.wrap & (YART_WRAP_ROTATE_Y | YART_WRAP_TRANSLATE);
-      T.refill_threshold = (uint32_t)std::max(1, std::min(32, rt));
-      T.node_threshold = (uint32_t)std::max(1, std::min(32, nt));
-      T.sin_theta = o.sin_theta;
-      T.cos_theta = o.cos_theta;
-      for (int k = 0; k < 3; ++k) T.offset[k] = o.offset[k];
-      T.work_counter = q.work_counters + n_trav++;
       T.counters = q.counters;
-      for (int k = 0; k < 3; ++k) T.bound[k] = m.bound[k];
-      // k_traverse_lean (device_trace_lean.cu): the same traversal with the f64-only state in shared memory -- 96
-      // registers, FIVE 128-thread CTAs per SM (20 warps) instead of four: +7 % on the david render, +6 % on the sweep.
-      // YART_TUNE_LEAN=0 selects k_traverse (which also serves visit counting and the all-f64 slab variant).
-      static const int lean = tune_env("YART_TUNE_LEAN", 5);
-      static const int lean_stack24 = tune_env("YART_TUNE_LEAN_STACK24", 1);
-      // (the reference-order instantiation of the lean kernel spills 150 B at 96 registers and is 5 % SLOWER than
-      // k_traverse on the sweep -- 2,074 vs 2,188 Mrays/s -- so only the near-first order, the default everywhere, uses it;
-      // YART_TUNE_LEAN_REF=1 forces it for both)
-      static const int lean_ref = tune_env("YART_TUNE_LEAN_REF", 0);
-      const bool use_lean = lean && mixed && !q.count && (q.near || lean_ref);
-      TraverseKernel k = use_lean ? yart::lean_traverse_kernel(q.near, (lean_stack24 || ctx->max_stack > 24) ? ctx->max_stack : 25u, lean,
-                                                                 m.cnodes != nullptr && q.near)
-                                  : pick_traverse_kernel(q.near, q.count, ctx->max_stack, mixed != 0);
-      // occupancy query + carveout once per kernel variant (they cost tens of microseconds of host time,
-      // which is the whole budget of a deep bounce)
-      int& per_sm = ctx->traverse_blocks[(const void*)k];
-      if (per_sm == 0) {
-        // leave everything the stacks do not need to L1: the tree's upper levels live there
-        // (the lean kernel keeps 22-42 KB of shared memory per CTA: five CTAs need the 132 KB configuration)
-        cudaFuncSetAttribute(reinterpret_cast<const void*>(k), cudaFuncAttributePreferredSharedMemoryCarveout, use_lean ? carve_lean : carve);
-        CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(k), kTraceThreads, 0));
-        per_sm = std::max(per_sm, 1);
-      }
-      k<<<per_sm * ctx->sm_count, kTraceThreads, 0, ctx->stream>>>(T); // persistent: one resident wave
+      // (the lean kernel keeps 22-42 KB of shared memory per CTA: five CTAs need the 132 KB configuration)
+      const int carveout = q.near && !q.count ? carve_lean : carve;
+      if (int rc = launch_persistent(ctx, traverse_kernel(q.near, q.count, ctx->max_stack), carveout, T)) return rc;
       i++;
     } else {
       uint32_t j = i;
@@ -642,7 +588,6 @@ struct OcclusionArgs {
 // k_analytic_occluded per run of consecutive analytic objects.  c.occluded must be zeroed: a pass only ever writes 1,
 // and the passes after the first skip the rays already marked.  An empty world launches nothing.
 int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launches) {
-  static const int rt = tune_env("YART_TUNE_RT", 8), nt = tune_env("YART_TUNE_NT", 12);
   static const int carve = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
   // A closest-hit pass starts a ray that nothing has hit yet from t_max if it is the first mesh pass, and from
   // fmin(+inf, t_max) otherwise (the recorded miss is +inf).  The two differ only for a NaN t_max.
@@ -655,34 +600,13 @@ int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launch
   while (i < q.n_objects) {
     if (is_mesh(i)) {
       const yart_object& o = q.h_objects[i];
-      const DevMesh& m = ctx->h_meshes[o.index];
       OccludeParams T;
       memset(&T, 0, sizeof(T));
       T.c = q.c;
       T.c.first_pass = first ? 1u : 0u;
       T.c.t_max = first ? q.c.t_max : t_max_later;
-      T.nodes = m.nodes;
-      T.tris = m.tris;
-      T.leafgeo = m.leafgeo;
-      T.root = m.root;
-      T.n_nodes = m.n_nodes;
-      T.n_tris = m.n_tris;
-      T.wrap = o.wrap & (YART_WRAP_ROTATE_Y | YART_WRAP_TRANSLATE);
-      T.refill_threshold = (uint32_t)std::max(1, std::min(32, rt));
-      T.node_threshold = (uint32_t)std::max(1, std::min(32, nt));
-      T.sin_theta = o.sin_theta;
-      T.cos_theta = o.cos_theta;
-      for (int k = 0; k < 3; ++k) T.offset[k] = o.offset[k];
-      for (int k = 0; k < 3; ++k) T.bound[k] = m.bound[k];
-      T.work_counter = q.work_counters + n_trav++;
-      const OccludeKernel k = yart::occlude_kernel(ctx->max_stack);
-      int& per_sm = ctx->traverse_blocks[(const void*)k]; // (occupancy query + carveout once per variant, as above)
-      if (per_sm == 0) {
-        cudaFuncSetAttribute(reinterpret_cast<const void*>(k), cudaFuncAttributePreferredSharedMemoryCarveout, carve);
-        CUDA_TRY(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(k), kTraceThreads, 0));
-        per_sm = std::max(per_sm, 1);
-      }
-      k<<<per_sm * ctx->sm_count, kTraceThreads, 0, ctx->stream>>>(T); // persistent: one resident wave
+      T.m = mesh_pass(o, ctx->h_meshes[o.index], q.work_counters + n_trav++);
+      if (int rc = launch_persistent(ctx, yart::occlude_kernel(ctx->max_stack), carve, T)) return rc;
       i++;
     } else {
       uint32_t j = i;
@@ -1106,47 +1030,6 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
       k_pack_leaves<<<(q.n_nodes * 4u + 255u) / 256u, 256, 0, ctx->stream>>>(dn, q.n_nodes, dt, dl);
       CUDA_TRY(ctx, cudaGetLastError());
       meshes[i].leafgeo = reinterpret_cast<const float4*>(dl);
-    }
-    {
-      // Compact 64-byte nodes: an EXPERIMENT, off unless YART_TUNE_COMPACT=1 (2 = also for fine meshes).  It is
-      // bit-identical (tests/test_gpu_flags_and_abi.py runs the parity cases with it on) and cuts L1 wavefronts by 40 %,
-      // but costs ~55 % more instructions and loses ~20 % on the B200 (DESIGN.md section 7).  Eligible when inner node
-      // ids fit 27 bits, the bounding box is finite, and the 16-bit grid is fine against the mesh: the grid step is
-      // (largest extent) / 65534, and a mesh whose AVERAGE triangle is smaller than ~32 steps would send too many box
-      // tests to the exact fallback.  (Read per scene, not cached, so that one process can compare both.)
-      meshes[i].cnodes = nullptr;
-      meshes[i].cscale = 0.f;
-      for (int a = 0; a < 3; ++a) meshes[i].corigin[a] = 0.f;
-      const int compact = tune_env("YART_TUNE_COMPACT", 0);
-      double ext = 0.0;
-      bool finite = true;
-      for (int a = 0; a < 3; ++a) {
-        ext = std::fmax(ext, q.bbox_max[a] - q.bbox_min[a]);
-        finite = finite && std::isfinite(q.bbox_min[a]) && std::isfinite(q.bbox_max[a]) && std::fabs(q.bbox_min[a]) < 1e30 && std::fabs(q.bbox_max[a]) < 1e30;
-      }
-      if (compact && finite && ext > 0.0 && q.n_nodes < (1u << 27) && q.n_nodes > 0) {
-        int e = 0;
-        std::frexp(ext / 65534.0, &e); // ext / 65534 = m * 2^e with m in [0.5, 1): 2^e >= ext / 65534
-        const double step = std::ldexp(1.0, e);
-        const double avg_tri = ext / std::cbrt((double)std::max<uint32_t>(q.n_tris, 1u)); // a crude length scale of one triangle
-        if (e > -100 && e < 100 && (avg_tri / step >= 32.0 || compact > 1)) {
-          uint4* dc = nullptr;
-          CUDA_TRY(ctx, cudaMalloc((void**)&dc, (size_t)q.n_nodes * 64));
-          ctx->scene_allocs.push_back(dc);
-          // (the corner is the f32 image of the f64 bounding box's minimum, rounded DOWN so that every plane lies above it)
-          float org[3];
-          for (int a = 0; a < 3; ++a) {
-            float f = (float)q.bbox_min[a];
-            if ((double)f > q.bbox_min[a]) f = nextafterf(f, -INFINITY);
-            org[a] = f;
-          }
-          k_pack_nodes<<<(q.n_nodes + 255u) / 256u, 256, 0, ctx->stream>>>(dn, q.n_nodes, org[0], org[1], org[2], (float)step, dc);
-          CUDA_TRY(ctx, cudaGetLastError());
-          meshes[i].cnodes = dc;
-          meshes[i].cscale = (float)step;
-          for (int a = 0; a < 3; ++a) meshes[i].corigin[a] = org[a];
-        }
-      }
     }
     meshes[i].root = q.root;
     meshes[i].max_stack = q.max_stack;
