@@ -139,6 +139,10 @@ pub struct yart_render_opts {
     pub order: u32, pub batch_spp: u32, pub flags: u32, pub seed: u64,
 }
 
+/// The denoiser planes of `yart_render_aovs`: each a `[height][width][3]` f64 film or null.
+#[repr(C)] #[derive(Clone, Copy)]
+pub struct yart_aov_planes { pub albedo: *mut f64, pub normal: *mut f64, pub depth: *mut f64 }
+
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct yart_qbvh_info {
     pub n_nodes: u32, pub n_leaves: u32, pub n_tris: u32, pub height: u32, pub root: u32, pub max_stack: u32,
@@ -198,6 +202,10 @@ extern "C" {
                        stats: *mut yart_stats) -> c_int;
     pub fn yart_film_finalize(ctx: *mut yart_ctx, film_xyz: *const f64, width: u32, height: u32, spp: u32, flags: u32,
                               rgba8: *mut u8) -> c_int;
+    pub fn yart_film_finalize_linear(ctx: *mut yart_ctx, film_xyz: *const f64, width: u32, height: u32, spp: u32,
+                                     flags: u32, rgb: *mut f32) -> c_int;
+    pub fn yart_render_aovs(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,
+                            planes: *const yart_aov_planes, stats: *mut yart_stats) -> c_int;
     pub fn yart_generate_camera_rays(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,
                                      rays_host: *mut yart_ray, wavelength_host: *mut f64, time_host: *mut f64) -> c_int;
     pub fn yart_dump_path_rays(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,

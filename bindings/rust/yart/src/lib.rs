@@ -3,7 +3,7 @@
 //!
 //! `GpuScene` plays the part of `world: Arc<HittableList>` (main.rs:434-446): `hit` has the shape of
 //! `Hittable::hit(&self, &Ray, t_min, t_max) -> Option<HitRecord>` (hittable.rs:24) for drop-in testing, `hit_many`
-//! is the batched form the GPU is for, `hit_records` / `hit_record` return the whole `HitRecord`, `render` replaces the tile loop of `render()` (main.rs:629-760).
+//! is the batched form the GPU is for, `hit_records` / `hit_record` return the whole `HitRecord`, `render` replaces the tile loop of `render()` (main.rs:629-760), `render_aovs` gives a denoiser its inputs.
 use std::ffi::{CStr, CString};
 use std::ptr;
 use yart_sys as sys;
@@ -169,7 +169,49 @@ impl GpuScene {
         }
         Ok(rgba)
     }
+
+    /// Denoiser inputs for the image `render(width, height, spp, ..)` makes: the film as linear RGB
+    /// (`yart_film_finalize_linear`) from samples `[0, spp)`, and the first-hit means of samples `[0, aov_spp)`
+    /// (`yart_render_aovs`) -- albedo and normal per pixel (`[h][w][3]`), and the mean distance of the samples that
+    /// hit (`[h][w]`, 0 where none did).  The two calls draw the same camera samples, so the planes line up with the
+    /// beauty image.
+    pub fn render_aovs(&self, width: u32, height: u32, spp: u32, aov_spp: u32, max_depth: u32, seed: u64) -> Result<Aovs> {
+        let mut cam: sys::yart_camera = unsafe { std::mem::zeroed() };
+        let rc = unsafe { sys::yart_preset_camera(self.preset, width, height, -1.0, -1.0, &mut cam) };
+        if rc != 0 { return Err(Self::global_err(rc)); }
+        let n = (width as usize) * (height as usize);
+        let mut opts = sys::yart_render_opts { width, height, sample_begin: 0, sample_end: spp, max_depth,
+                                               order: sys::YART_ORDER_NEAR, seed, ..Default::default() };
+        let mut film = vec![0f64; n * 3];
+        let (mut albedo, mut normal, mut depth) = (vec![0f64; n * 3], vec![0f64; n * 3], vec![0f64; n * 3]);
+        let mut color = vec![0f32; n * 3];
+        unsafe {
+            let rc = sys::yart_render(self.ctx, &cam, &opts, film.as_mut_ptr(), ptr::null_mut());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+            let rc = sys::yart_film_finalize_linear(self.ctx, film.as_ptr(), width, height, spp, 0, color.as_mut_ptr());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+            opts.sample_end = aov_spp;
+            let planes = sys::yart_aov_planes { albedo: albedo.as_mut_ptr(), normal: normal.as_mut_ptr(), depth: depth.as_mut_ptr() };
+            let rc = sys::yart_render_aovs(self.ctx, &cam, &opts, &planes, ptr::null_mut());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+        }
+        let mut out = Aovs { color, albedo: vec![0f32; n * 3], normal: vec![0f32; n * 3], depth: vec![0f32; n] };
+        for i in 0..n {
+            let (hits, samples) = (depth[i * 3 + 1], depth[i * 3 + 2]);
+            for k in 0..3 {
+                if samples > 0.0 {
+                    out.albedo[i * 3 + k] = (albedo[i * 3 + k] / samples) as f32;
+                    out.normal[i * 3 + k] = (normal[i * 3 + k] / samples) as f32;
+                }
+            }
+            if hits > 0.0 { out.depth[i] = (depth[i * 3] / hits) as f32; }
+        }
+        Ok(out)
+    }
 }
+
+/// What `GpuScene::render_aovs` returns: row-major images, top row first.
+pub struct Aovs { pub color: Vec<f32>, pub albedo: Vec<f32>, pub normal: Vec<f32>, pub depth: Vec<f32> }
 
 /// A page-locked view of a caller's slice (see `GpuScene::pin`).
 pub struct Pinned<'a, T> {

@@ -470,6 +470,50 @@ int yart_render(yart_ctx* ctx, const yart_camera* camera, const yart_render_opts
 int yart_film_finalize(yart_ctx* ctx, const double* film_xyz, uint32_t width, uint32_t height,
                        uint32_t spp, uint32_t flags, uint8_t* rgba8);
 
+/* The film as LINEAR RGB, the HDR colour input of a denoiser: yart_film_finalize's (r, g, b) after into_rgb and
+ * before the sRGB OETF and the clamp, i.e. XYZ * (720-360)/(106.856895*spp) -> into_rgb, computed in f64 and
+ * rounded to f32.  Pixels outside the reference's 8x8 tiles are 0.  rgb: [height][width][3].  flags:
+ * YART_FLAG_DEVICE_PTRS (film_xyz and rgb are device arrays). */
+int yart_film_finalize_linear(yart_ctx* ctx, const double* film_xyz, uint32_t width, uint32_t height,
+                              uint32_t spp, uint32_t flags, float* rgb);
+
+/* Auxiliary images (AOVs) for a denoiser.  Each plane is a film: [height][width][3] f64, added to like film_xyz. */
+typedef struct yart_aov_planes {
+  double* albedo;  /* [height][width][3] or NULL */
+  double* normal;  /* [height][width][3] or NULL */
+  double* depth;   /* [height][width][3] or NULL: {sum of distance over the samples that hit, samples that hit, samples} */
+} yart_aov_planes;
+
+/* What each camera sample of yart_render first hits, summed per pixel: the albedo, normal and distance planes that
+ * denoisers (Open Image Denoise, the OptiX denoiser) take beside the linear colour of yart_film_finalize_linear.
+ *   Samples: [sample_begin, sample_end) of every pixel, with yart_render's camera rays: the same Philox (pixel, sample)
+ *   draws for jitter, lens, wavelength and time, and the same 8x8 tiles.  Pixels the reference never samples get
+ *   nothing, not even a sample count.
+ *   First hit: the render's bounce-1 world.hit(ray, 0.001, inf), bit for bit: the same `order`, the ray's own time
+ *   (MovingSphere), constant media drawing at (pixel, sample, bounce 1).  AOV sample s of pixel p describes exactly
+ *   the surface beauty sample s reached first.
+ *   Accumulation: per pixel and in sample order, like the film.  Chaining calls over consecutive sample ranges, and
+ *   any batch_spp, give the same bits as one call.  yart_film_create / _read / _reduce work on the planes unchanged.
+ *   Per sample, with h the first hit's HitRecord:
+ *     albedo  an RGB from h's material, each channel clamped to [0, 1] (NaN to 0): Lambertian, Metal and Isotropic:
+ *             the RGB their texture hands to RGB::reflect at (u, v, p) -- checker a / b, the image texel, the solid
+ *             colour, or the noise scalar times white; Dielectric: (1, 1, 1); DiffuseLight: its emit texture's RGB
+ *             when h.front_face, else 0; no material: 0; a miss: background_rgb.
+ *     normal  h.normal / |h.normal| (world space, face-oriented as the reference stores it); 0 for a miss, a
+ *             constant-medium hit, and a zero or non-finite length.  |n| = sqrt(x*x + y*y + z*z), in that order.
+ *     depth   {t * |d|, 1, 1} for a hit, {0, 0, 1} for a miss: the Euclidean distance from the ray's origin on the
+ *             lens (d is the camera ray's direction, not normalised; |d| as for the normal).
+ *   Values from a libm call differ from the reference's glibc in the last bits where they feed the planes: sphere u, v
+ *   read by an image texture (acos / atan2), a checker's sin, noise, and a constant medium's log.
+ * opts: the struct of the beauty call may be passed as it is.  The sampling flags are accepted and change nothing
+ * (none of them changes a camera ray or its first hit); max_depth is validated as in yart_render and otherwise unused.
+ * Flags: YART_FLAG_DEVICE_PTRS (the planes are device arrays, 8-byte aligned), YART_FLAG_COUNT_VISITS as in yart_render.
+ * All three planes NULL is YART_ERR_INVALID.
+ * stats (may be NULL): rays = camera rays traced, paths = samples started, trace_ms / trace_launches = the closest-hit
+ * passes; max_bounce is 1 when anything was traced. */
+int yart_render_aovs(yart_ctx* ctx, const yart_camera* camera, const yart_render_opts* opts,
+                     const yart_aov_planes* planes, yart_stats* stats /* may be NULL */);
+
 /* Camera rays exactly as the render loop generates them (main.rs:690-698, camera.rs:82-94):
  * one ray per (pixel, sample) in [sample_begin, sample_end), pixel-major.  For parity tests
  * and for dumping the ray distribution the renderer really sees. */

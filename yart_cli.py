@@ -6,6 +6,7 @@
                        [--seed S] [--order near|reference] [--device D] [--gpus N]   (additions)
                        [--preview-every N] [--checkpoint FILE] [--resume]    (additions)
                        [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event]   (better sampling, off by default)
+                       [--aovs [--aov-samples N]]                            (denoiser inputs)
 
 `--workers` is accepted for compatibility and ignored (the render runs on the GPU).  Option resolution
 follows resolve_render_options / resolve_dimensions (main.rs:166-209); the image is finalised exactly like
@@ -21,6 +22,13 @@ the same moments; `--resume` continues from FILE if it matches the request.
 films are combined by the library's NCCL reduce (yet-another-raytracer_b200/sharding.py, yart_film_reduce).  The three
 sampling flags change the ESTIMATOR (SURVEY.md 8(f) row 4) and are off unless asked for; they are part of a
 checkpoint's identity.
+
+`--aovs` also writes the inputs of a denoiser such as Open Image Denoise (`oidnDenoise --hdr <stem>.color.pfm --alb
+<stem>.albedo.pfm --nrm <stem>.normal.pfm`) next to the PNG: <stem>.color.pfm is the film as linear RGB
+(yart_film_finalize_linear), and <stem>.albedo.pfm, <stem>.normal.pfm and <stem>.depth.pfm (one channel: the mean
+distance of the samples that hit, 0 where none did) are the first-hit means of samples [0, --aov-samples) (default
+min(16, --samples)), the very camera samples the beauty pass started with (yart_render_aovs).  They are rendered once,
+after the beauty pass, on the first GPU, and are not part of a checkpoint.
 """
 import argparse
 import importlib
@@ -71,6 +79,10 @@ def build_parser(scene_names):
                     help="write the image after every N samples per pixel")
     ap.add_argument("--checkpoint", default=None, help=".npz file holding the film and the samples done so far")
     ap.add_argument("--resume", action="store_true", help="continue from --checkpoint if it matches this render")
+    ap.add_argument("--aovs", action="store_true",
+                    help="also write <stem>.color/.albedo/.normal/.depth.pfm next to the PNG (denoiser inputs)")
+    ap.add_argument("--aov-samples", type=positive_int, default=None, dest="aov_samples",
+                    help="samples per pixel of the albedo / normal / depth images (default min(16, --samples))")
     return ap
 
 
@@ -111,6 +123,44 @@ def write_png(ctx, film, spp_done, path):
         os.makedirs(parent, exist_ok=True)
     from PIL import Image
     Image.fromarray(ctx.film_finalize(film, spp_done), "RGBA").save(path)
+
+
+def write_pfm(path, img):
+    """A portable float map: (H, W, 3) -> "PF", (H, W) -> "Pf"; little-endian f32, rows bottom to top."""
+    import numpy as np
+    img = np.asarray(img, dtype="<f4")
+    with open(path, "wb") as f:
+        f.write(b"%s\n%d %d\n-1.0\n" % (b"PF" if img.ndim == 3 else b"Pf", img.shape[1], img.shape[0]))
+        f.write(np.ascontiguousarray(img[::-1]).tobytes())
+
+
+def read_pfm(path):
+    """write_pfm's inverse (either byte order)."""
+    import numpy as np
+    with open(path, "rb") as f:
+        kind = f.readline().strip()
+        w, h = (int(v) for v in f.readline().split())
+        scale = float(f.readline())
+        data = np.frombuffer(f.read(), dtype="<f4" if scale < 0 else ">f4")
+    shape = (h, w, 3) if kind == b"PF" else (h, w)
+    return data.reshape(shape)[::-1].astype(np.float32)
+
+
+def aov_paths(output_path):
+    stem = os.path.splitext(output_path)[0]
+    return {k: "%s.%s.pfm" % (stem, k) for k in ("color", "albedo", "normal", "depth")}
+
+
+def write_aovs(y, ctx, cam, o, args, order, flags, film, spp):
+    """The four denoiser inputs of --aovs; returns their paths."""
+    n = args.aov_samples or min(16, spp)
+    planes, _ = ctx.render_aovs(cam, o["width"], o["height"], 0, n, o["max_depth"], args.seed, order, flags=flags)
+    means = y.aov_means(planes)
+    paths = aov_paths(o["output_path"])
+    write_pfm(paths["color"], ctx.film_finalize_linear(film, spp))
+    for k in ("albedo", "normal", "depth"):
+        write_pfm(paths[k], means[k])
+    return paths
 
 
 def main(argv=None):
@@ -172,6 +222,8 @@ def main(argv=None):
     if film is None:  # (resumed a finished render)
         raise SystemExit("nothing to do")
     write_png(ctx, film, total, o["output_path"])
+    if args.aovs:
+        write_aovs(y, ctx, cam, o, args, order, flags, film, total)
     if multi is not None:
         multi.close()
     print("%s rendered in %d seconds" % (o["output_path"], int(time.time() - start)))  # main.rs:763-767

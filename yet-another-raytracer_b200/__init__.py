@@ -31,6 +31,23 @@ SCENE_NAMES = ["random-scene", "two-spheres", "two-perlin-spheres", "earth", "si
 
 
 BUILDER_HOST, BUILDER_DEVICE = 0, 1
+AOV_PLANES = ("albedo", "normal", "depth")  # the fields of yart_aov_planes, in order
+
+
+def aov_means(planes):
+    """Per-pixel averages of render_aovs' sums: albedo / samples and normal / samples, (H, W, 3), and distance / hits,
+    (H, W), 0 where nothing was hit.  Reads only the planes given; the sample count is in the depth plane, so the
+    albedo and normal means need it."""
+    depth = planes["depth"]
+    n = depth[..., 2:3]
+    out = {}
+    with np.errstate(invalid="ignore", divide="ignore"):
+        for k in ("albedo", "normal"):
+            if k in planes:
+                out[k] = np.where(n > 0, planes[k] / np.where(n > 0, n, 1.0), 0.0)
+        hits = depth[..., 1]
+        out["depth"] = np.where(hits > 0, depth[..., 0] / np.where(hits > 0, hits, 1.0), 0.0)
+    return out
 
 
 class YartError(RuntimeError):
@@ -93,6 +110,8 @@ def load_library():
         "yart_occluded_f32": (i32, [vp, u32, vp, u64, C.c_float, C.c_float, u32, vp, P(abi.Stats)]),
         "yart_render": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, P(abi.Stats)]),
         "yart_film_finalize": (i32, [vp, vp, u32, u32, u32, u32, vp]),
+        "yart_film_finalize_linear": (i32, [vp, vp, u32, u32, u32, u32, vp]),
+        "yart_render_aovs": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), P(abi.AovPlanes), P(abi.Stats)]),
         "yart_generate_camera_rays": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, vp, vp]),
         "yart_dump_path_rays": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, u64, P(u64)]),
         "yart_comm_unique_id": (i32, [vp]),
@@ -126,7 +145,7 @@ EXPORTED_SYMBOLS = [
     "yart_comm_destroy", "yart_comm_info", "yart_comm_last_error", "yart_film_reduce", "yart_film_create",
     "yart_film_clear", "yart_film_read", "yart_film_destroy", "yart_preset_note", "yart_closest_hit_f32",
     "yart_dump_path_rays", "yart_host_register", "yart_host_unregister", "yart_occluded", "yart_occluded_f32",
-    "yart_closest_hit_records",
+    "yart_closest_hit_records", "yart_render_aovs", "yart_film_finalize_linear",
 ]
 
 
@@ -494,6 +513,42 @@ class Context:
         """Same with device pointers (film: [h][w][3] f64, rgba: [h][w][4] u8); asynchronous work is synchronised."""
         self._check(_lib.yart_film_finalize(self._h, C.c_void_p(film_ptr), width, height, spp, FLAG_DEVICE_PTRS,
                                             C.c_void_p(rgba_ptr)))
+
+    def film_finalize_linear(self, film, spp):
+        """The film as linear RGB (yart_film_finalize_linear): (H, W, 3) f32, 0 outside the reference's tiles."""
+        film = np.ascontiguousarray(film, dtype=np.float64)
+        h, w = film.shape[:2]
+        rgb = np.empty((h, w, 3), dtype=np.float32)
+        self._check(_lib.yart_film_finalize_linear(self._h, film.ctypes.data, w, h, spp, 0, rgb.ctypes.data))
+        return rgb
+
+    def render_aovs(self, camera, width, height, sample_begin, sample_end, max_depth=50, seed=1, order=ORDER_NEAR,
+                    batch_spp=0, flags=0, planes=None, count_visits=False):
+        """First-hit albedo, normal and depth of samples [sample_begin, sample_end) (yart_render_aovs).  Returns
+        (planes, stats): a dict of (H, W, 3) f64 sums "albedo", "normal", "depth" (depth = {distance over the samples
+        that hit, samples that hit, samples}).  Given `planes` (a dict holding any of the three), those arrays are added
+        to in place and only they are computed.  aov_means() turns the sums into averages."""
+        if planes is None:
+            planes = {k: np.zeros((height, width, 3), dtype=np.float64) for k in AOV_PLANES}
+        ap = abi.AovPlanes()
+        for k, arr in planes.items():
+            assert k in AOV_PLANES, k
+            assert arr.dtype == np.float64 and arr.shape == (height, width, 3) and arr.flags.c_contiguous
+            setattr(ap, k, arr.ctypes.data)
+        st = abi.Stats()
+        o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, order, batch_spp,
+                       (FLAG_COUNT_VISITS if count_visits else 0) | (flags & ~FLAG_DEVICE_PTRS))
+        self._check(_lib.yart_render_aovs(self._h, C.byref(camera), C.byref(o), C.byref(ap), C.byref(st)))
+        return planes, st
+
+    def render_aovs_device(self, camera, width, height, sample_begin, sample_end, albedo_ptr=None, normal_ptr=None,
+                           depth_ptr=None, max_depth=50, seed=1, order=ORDER_NEAR, batch_spp=0, flags=0):
+        """The same into device planes ([h][w][3] f64 each, e.g. from film_create); a missing plane is skipped."""
+        ap = abi.AovPlanes(albedo_ptr, normal_ptr, depth_ptr)
+        st = abi.Stats()
+        o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, order, batch_spp, FLAG_DEVICE_PTRS | flags)
+        self._check(_lib.yart_render_aovs(self._h, C.byref(camera), C.byref(o), C.byref(ap), C.byref(st)))
+        return st
 
     def camera_rays(self, camera, width, height, sample_begin, sample_end, seed=1):
         n = width * height * (sample_end - sample_begin)

@@ -322,6 +322,47 @@ __device__ __noinline__ double texture_value(const DevScene& S, uint32_t tex, do
   }
 }
 
+// The RGB a texture hands to rgb_reflect in texture_value (noise: its scalar times white; an image without texels:
+// white).  A function of its own, not the first half of texture_value: for noise, rgb_reflect(white) * s and
+// rgb_reflect(s * white) are different doubles, and the renderer keeps texture_value's.
+YART_DEV void texture_rgb(const DevScene& S, uint32_t tex, const HitRec& rec, double rgb[3]) {
+  const yart_texture& t = S.textures[tex];
+  const double* c = nullptr;
+  double s = 0.0;
+  switch (t.kind) {
+    case YART_TEX_SOLID: c = t.rgb_a; break;
+    case YART_TEX_CHECKER: {
+      double sines = sin(10.0 * rec.p.x) * sin(10.0 * rec.p.y) * sin(10.0 * rec.p.z);
+      c = sines < 0.0 ? t.rgb_a : t.rgb_b;
+      break;
+    }
+    case YART_TEX_NOISE: {
+      const yart_perlin& pn = S.perlins[t.perlin];
+      if (t.noise_type == YART_NOISE_NET) s = perlin_turb(pn, t.noise_type, rec.p * t.scale, 7);
+      else if (t.noise_type == YART_NOISE_MARBLE) s = 0.5 * (1.0 + sin(t.scale * rec.p.z + 10.0 * perlin_turb(pn, t.noise_type, rec.p, 7)));
+      else s = 0.5 * (1.0 + perlin_noise(pn, t.noise_type, rec.p * t.scale));
+      break;
+    }
+    case YART_TEX_IMAGE: {
+      const DevImage im = S.images[t.image];
+      if (im.rgb8 == nullptr) { s = 1.0; break; }
+      double uu = rec.u < 0.0 ? 0.0 : (rec.u > 1.0 ? 1.0 : rec.u);
+      double vc = rec.v < 0.0 ? 0.0 : (rec.v > 1.0 ? 1.0 : rec.v);
+      double vv = 1.0 - vc;
+      uint32_t i = f64_as_u32(uu * (double)im.width);
+      uint32_t j = f64_as_u32(vv * (double)im.height);
+      if (i >= im.width) i = im.width - 1;
+      if (j >= im.height) j = im.height - 1;
+      const double cs = 1.0 / 255.0;
+      const size_t px = (size_t)j * 3 * im.width + (size_t)i * 3;
+      for (int k = 0; k < 3; ++k) rgb[k] = cs * (double)im.rgb8[px + k];
+      return;
+    }
+    default: break;
+  }
+  for (int k = 0; k < 3; ++k) rgb[k] = c ? c[k] : s;
+}
+
 // ---------------------------------------------------------------------------------------------
 // ONB, PDFs, light sampling (onb.rs, pdf.rs, sphere.rs:95-118, aarect.rs:148-171)
 // ---------------------------------------------------------------------------------------------
@@ -922,6 +963,14 @@ YART_DEV uint8_t clamp_display_channel(double c) { // main.rs:461-463
   if (v != v) return 0;
   return (uint8_t)v;
 }
+// main.rs:710-712: one pixel's XYZ sum * (720-360) / (106.856895*spp), then into_rgb -- linear RGB
+YART_DEV void film_linear_rgb(const double* f, uint32_t spp, double& r, double& g, double& b) {
+  const double mul = 720.0 - 360.0, den = 106.856895 * (double)spp;
+  const D3 c = vdiv(d3(f[0] * mul, f[1] * mul, f[2] * mul), den);
+  r = 2.6896552 * c.x - 1.2758621 * c.y - 0.4137931 * c.z;
+  g = -1.0221082 * c.x + 1.9782866 * c.y + 0.0438216 * c.z;
+  b = 0.0612245 * c.x - 0.2244898 * c.y + 1.1632653 * c.z;
+}
 // main.rs:710-718
 __global__ void __launch_bounds__(256) k_film_finalize(const double* film, uint32_t W, uint32_t H, uint32_t spp, uint8_t* rgba) {
   const uint32_t n = W * H;
@@ -932,15 +981,82 @@ __global__ void __launch_bounds__(256) k_film_finalize(const double* film, uint3
       o[0] = o[1] = o[2] = o[3] = 0;
       continue;
     }
-    const double mul = 720.0 - 360.0, den = 106.856895 * (double)spp;
-    const D3 c = vdiv(d3(film[(size_t)p * 3] * mul, film[(size_t)p * 3 + 1] * mul, film[(size_t)p * 3 + 2] * mul), den);
-    const double r = 2.6896552 * c.x - 1.2758621 * c.y - 0.4137931 * c.z;
-    const double g = -1.0221082 * c.x + 1.9782866 * c.y + 0.0438216 * c.z;
-    const double b = 0.0612245 * c.x - 0.2244898 * c.y + 1.1632653 * c.z;
+    double r, g, b;
+    film_linear_rgb(film + (size_t)p * 3, spp, r, g, b);
     o[0] = clamp_display_channel(gamma_channel(r));
     o[1] = clamp_display_channel(gamma_channel(g));
     o[2] = clamp_display_channel(gamma_channel(b));
     o[3] = 255;
+  }
+}
+
+// yart_film_finalize_linear: the (r, g, b) k_film_finalize gamma-encodes, rounded to f32; 0 outside the tiles
+__global__ void __launch_bounds__(256) k_film_finalize_linear(const double* film, uint32_t W, uint32_t H, uint32_t spp, float* rgb) {
+  const uint32_t n = W * H;
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+    float* o = rgb + (size_t)p * 3;
+    if (!pixel_is_rendered(p % W, W) || !pixel_is_rendered(p / W, H)) {
+      o[0] = o[1] = o[2] = 0.f;
+      continue;
+    }
+    double r, g, b;
+    film_linear_rgb(film + (size_t)p * 3, spp, r, g, b);
+    o[0] = (float)r; o[1] = (float)g; o[2] = (float)b;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// yart_render_aovs: the first hit of every camera sample as denoiser inputs
+// ---------------------------------------------------------------------------------------------
+YART_DEV double clamp01(double x) { return x > 0.0 ? (x < 1.0 ? x : 1.0) : 0.0; } // (NaN -> 0)
+
+// One batch of k_raygen<false> samples after the bounce-1 passes over ALL objects (no k_shade, so no tail fold): adds,
+// per rendered pixel and in sample order, each sample's albedo, unit normal and {distance, hit, 1} to the planes
+// (null planes are skipped).  Pixels outside the tiles get nothing.
+__global__ void __launch_bounds__(256) k_aov_accumulate(const RenderParams R, double* albedo, double* normal, double* depth) {
+  const DevScene& S = R.scene;
+  for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < R.n_pixels; p += gridDim.x * blockDim.x) {
+    const uint32_t pixel = R.pixel_base + p;
+    if (!pixel_is_rendered(pixel % R.width, R.width) || !pixel_is_rendered(pixel / R.width, R.height)) continue;
+    double a[3] = {0.0, 0.0, 0.0}, nm[3] = {0.0, 0.0, 0.0}, dp[3] = {0.0, 0.0, 0.0};
+    for (int k = 0; k < 3; ++k) {
+      if (albedo) a[k] = albedo[(size_t)pixel * 3 + k];
+      if (normal) nm[k] = normal[(size_t)pixel * 3 + k];
+      if (depth) dp[k] = depth[(size_t)pixel * 3 + k];
+    }
+    for (uint32_t s = 0; s < R.spp_batch; ++s) {
+      const size_t id = (size_t)p * R.spp_batch + s;
+      const DevHit h = R.st.hits[id];
+      double alb[3] = {0.0, 0.0, 0.0}, n[3] = {0.0, 0.0, 0.0}, dist = 0.0;
+      if (h.obj == YART_MISS) {
+        for (int k = 0; k < 3; ++k) alb[k] = S.background[k];
+      } else {
+        YART_CHECK(h.obj < S.n_objects);
+        D3 wo, wd;
+        load_ray(R.st.rays + id, wo, wd);
+        HitRec rec;
+        world_record<true>(S, h, wo, wd, R.st.time[id], rec);
+        const yart_material& mat = S.materials[rec.material];
+        if (mat.kind == YART_MAT_LAMBERTIAN || mat.kind == YART_MAT_METAL || mat.kind == YART_MAT_ISOTROPIC ||
+            (mat.kind == YART_MAT_DIFFUSE_LIGHT && rec.front_face)) {
+          texture_rgb(S, mat.texture, rec, alb);
+        } else if (mat.kind == YART_MAT_DIELECTRIC) {
+          alb[0] = alb[1] = alb[2] = 1.0;
+        }
+        if (!(S.objects[h.obj].wrap & YART_WRAP_MEDIUM)) {
+          const double len = sqrt(rec.normal.x * rec.normal.x + rec.normal.y * rec.normal.y + rec.normal.z * rec.normal.z);
+          if (len > 0.0 && isfinite(len)) { n[0] = rec.normal.x / len; n[1] = rec.normal.y / len; n[2] = rec.normal.z / len; }
+        }
+        dist = rec.t * sqrt(wd.x * wd.x + wd.y * wd.y + wd.z * wd.z);
+      }
+      for (int k = 0; k < 3; ++k) { a[k] += clamp01(alb[k]); nm[k] += n[k]; }
+      dp[0] += dist; dp[1] += h.obj == YART_MISS ? 0.0 : 1.0; dp[2] += 1.0;
+    }
+    for (int k = 0; k < 3; ++k) {
+      if (albedo) albedo[(size_t)pixel * 3 + k] = a[k];
+      if (normal) normal[(size_t)pixel * 3 + k] = nm[k];
+      if (depth) depth[(size_t)pixel * 3 + k] = dp[k];
+    }
   }
 }
 

@@ -1,5 +1,6 @@
 // yart_device.cu -- the device half of the C ABI (include/yart.h): context, scene upload,
-// yart_closest_hit, yart_closest_hit_records, yart_occluded, yart_render, yart_film_finalize, yart_generate_camera_rays.
+// yart_closest_hit, yart_closest_hit_records, yart_occluded, yart_render, yart_render_aovs, yart_film_finalize(_linear),
+// yart_generate_camera_rays.
 //
 // There is no CPU fallback anywhere in this file: every entry point launches the sm_100a
 // kernels of device_trace.cuh / device_shade.cuh or fails with YART_ERR_CUDA.
@@ -378,6 +379,7 @@ struct yart_ctx {
   DevBuf nee_rays, nee_pending, nee_sum, nee_w, queue_s; // YART_FLAG_NEXT_EVENT's per-path state (NeeState)
   DevBuf occluded; // staging of yart_occluded's flags for host arrays
   DevBuf ray_times; // staging of yart_closest_hit_records' ray times for host arrays
+  DevBuf aov[3];    // staging of yart_render_aovs' host planes
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> ev_pool;
   // host-buffer closest-hit queries: copy streams + events of the chunk pipeline (made on first use)
@@ -792,7 +794,7 @@ void yart_ctx_destroy(yart_ctx* ctx) {
   ctx->free_scene();
   DevBuf* bufs[] = {&ctx->rays, &ctx->hits_export, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits,
                     &ctx->queue_a, &ctx->queue_b, &ctx->counts, &ctx->work, &ctx->counters, &ctx->film, &ctx->rgba,
-                    &ctx->occluded, &ctx->ray_times};
+                    &ctx->occluded, &ctx->ray_times, &ctx->aov[0], &ctx->aov[1], &ctx->aov[2]};
   for (DevBuf* b : bufs) b->release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->chunk_events) cudaEventDestroy(e);
@@ -1518,6 +1520,64 @@ int yart_dump_path_rays(yart_ctx* ctx, const yart_camera* cam, const yart_render
   YART_ABI_GUARD_END(ctx, "yart_dump_path_rays")
 }
 
+// The batch shape of a sample loop over o's samples (yart_render, yart_render_aovs): whole frame x *spp_batch, or
+// pixel chunks of *pix_chunk when the frame alone is too large; the path state of pix_chunk * spp_batch paths (ray,
+// time, wavelength, throughput, hit, two queues) is reserved.  staging_bytes: device memory the call needs besides
+// (the host films' device copies).
+// Big batches: every batch pays ~12 ms of fixed cost (the nearly empty tail bounces run at the latency of
+// their longest ray), so put up to 256 Mi paths in flight -- 112 B of state each (48 ray + 8 time + 8 wavelength
+// + 8 throughput + 32 hit + 2 x 4 queue) = 30 GB of the 180 GB: david 1080p at 32 / 64 / 128 spp per batch
+// = 1121 / 1146 / 1158 Mrays/s.  The cap is also bounded by what is actually FREE on the device right now
+// (minus a margin), so that a busy GPU gets smaller batches instead of a failed cudaMalloc.
+static int size_path_batches(yart_ctx* ctx, const yart_render_opts* o, bool nee, uint64_t staging_bytes, uint32_t* spp_batch_out,
+                             uint32_t* pix_chunk_out) {
+  const uint32_t n_pixels_total = o->width * o->height;
+  const uint32_t n_samples = o->sample_end - o->sample_begin;
+  static const int max_paths_log2 = std::max(10, std::min(30, tune_env("YART_TUNE_MAX_PATHS_LOG2", 28)));
+  uint64_t kMaxPaths = 1ull << max_paths_log2;
+  {
+    // YART_FLAG_NEXT_EVENT adds 76 B: 48 shadow ray + 8 pending + 8 light-sample sum + 8 emission weight + 4 shadow queue
+    // (the shadow passes write their hits into the path hits, which are dead from k_shade to the next bounce's passes)
+    const uint64_t kNeeBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(uint32_t);
+    const uint64_t kStateBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(DevHit) + 2 * sizeof(uint32_t) +
+                                        (nee ? kNeeBytesPerPath : 0);
+    if (!nee) // a flag-off render does not keep an earlier NEE render's state alive (no-op when there is none)
+      for (DevBuf* b : {&ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s}) b->release();
+    size_t free_b = 0, total_b = 0;
+    CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
+    const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b,
+                            &ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s};
+    uint64_t avail = free_b; // what the state buffers may grow into: free memory + what they already hold
+    for (const DevBuf* b : held) avail += b->cap;
+    const uint64_t margin = (256ull << 20) + staging_bytes;
+    const uint64_t fit = avail > margin ? (avail - margin) / kStateBytesPerPath : 0;
+    kMaxPaths = std::min<uint64_t>(kMaxPaths, fit);
+    static const int mem_cap_mb = tune_env("YART_TUNE_STATE_MB", 0); // testing: pretend only this much is free
+    if (mem_cap_mb > 0) kMaxPaths = std::min<uint64_t>(kMaxPaths, ((uint64_t)mem_cap_mb << 20) / kStateBytesPerPath);
+    if (kMaxPaths < 1024) {
+      ctx->err = "yart_render: not enough free device memory for the path state (" + std::to_string(free_b >> 20) +
+                 " MiB free of " + std::to_string(total_b >> 20) + " MiB; " + std::to_string(kStateBytesPerPath) +
+                 " bytes per path in flight)";
+      return YART_ERR_NOMEM;
+    }
+  }
+  uint32_t spp_batch = o->batch_spp ? o->batch_spp : (uint32_t)std::max<uint64_t>(1, kMaxPaths / n_pixels_total);
+  spp_batch = std::min(spp_batch, n_samples);
+  uint32_t pix_chunk = n_pixels_total;
+  if ((uint64_t)pix_chunk * spp_batch > kMaxPaths) pix_chunk = (uint32_t)std::max<uint64_t>(1, kMaxPaths / spp_batch);
+  const uint64_t cap = (uint64_t)pix_chunk * spp_batch;
+  CUDA_TRY(ctx, ctx->rays.reserve(cap * sizeof(yart_ray)));
+  CUDA_TRY(ctx, ctx->time.reserve(cap * sizeof(double)));
+  CUDA_TRY(ctx, ctx->wavelength.reserve(cap * sizeof(double)));
+  CUDA_TRY(ctx, ctx->throughput.reserve(cap * sizeof(double)));
+  CUDA_TRY(ctx, ctx->hits.reserve(cap * sizeof(DevHit)));
+  CUDA_TRY(ctx, ctx->queue_a.reserve(cap * sizeof(uint32_t)));
+  CUDA_TRY(ctx, ctx->queue_b.reserve(cap * sizeof(uint32_t)));
+  *spp_batch_out = spp_batch;
+  *pix_chunk_out = pix_chunk;
+  return YART_OK;
+}
+
 // film_xyz == nullptr (yart_dump_path_rays): the samples are traced exactly as for a render, the film is a scratch
 // buffer that is thrown away, and every bounce's rays are copied to dump_out.
 static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, double* film_xyz, yart_stats* stats,
@@ -1548,53 +1608,10 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
   double trace_ms = 0.0;
   uint32_t deepest = 0;
   if (n_samples > 0) {
-    // Batch shape: whole frame x spp_batch, or pixel chunks when the frame alone is too large.
-    // Big batches: every batch pays ~12 ms of fixed cost (the nearly empty tail bounces run at the latency of
-    // their longest ray), so put up to 256 Mi paths in flight -- 112 B of state each (48 ray + 8 time + 8 wavelength
-    // + 8 throughput + 32 hit + 2 x 4 queue) = 30 GB of the 180 GB: david 1080p at 32 / 64 / 128 spp per batch
-    // = 1121 / 1146 / 1158 Mrays/s.  The cap is also bounded by what is actually FREE on the device right now
-    // (minus a margin), so that a busy GPU gets smaller batches instead of a failed cudaMalloc.
-    static const int max_paths_log2 = std::max(10, std::min(30, tune_env("YART_TUNE_MAX_PATHS_LOG2", 28)));
-    uint64_t kMaxPaths = 1ull << max_paths_log2;
     const bool nee = (R.flags & YART_FLAG_NEXT_EVENT) != 0;
-    {
-      // YART_FLAG_NEXT_EVENT adds 76 B: 48 shadow ray + 8 pending + 8 light-sample sum + 8 emission weight + 4 shadow queue
-      // (the shadow passes write their hits into the path hits, which are dead from k_shade to the next bounce's passes)
-      const uint64_t kNeeBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(uint32_t);
-      const uint64_t kStateBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(DevHit) + 2 * sizeof(uint32_t) +
-                                          (nee ? kNeeBytesPerPath : 0);
-      if (!nee) // a flag-off render does not keep an earlier NEE render's state alive (no-op when there is none)
-        for (DevBuf* b : {&ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s}) b->release();
-      size_t free_b = 0, total_b = 0;
-      CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
-      const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b,
-                              &ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s};
-      uint64_t avail = free_b; // what the state buffers may grow into: free memory + what they already hold
-      for (const DevBuf* b : held) avail += b->cap;
-      const uint64_t margin = (256ull << 20) + (dev ? 0 : film_bytes);
-      const uint64_t fit = avail > margin ? (avail - margin) / kStateBytesPerPath : 0;
-      kMaxPaths = std::min<uint64_t>(kMaxPaths, fit);
-      static const int mem_cap_mb = tune_env("YART_TUNE_STATE_MB", 0); // testing: pretend only this much is free
-      if (mem_cap_mb > 0) kMaxPaths = std::min<uint64_t>(kMaxPaths, ((uint64_t)mem_cap_mb << 20) / kStateBytesPerPath);
-      if (kMaxPaths < 1024) {
-        ctx->err = "yart_render: not enough free device memory for the path state (" + std::to_string(free_b >> 20) +
-                   " MiB free of " + std::to_string(total_b >> 20) + " MiB; " + std::to_string(kStateBytesPerPath) +
-                   " bytes per path in flight)";
-        return YART_ERR_NOMEM;
-      }
-    }
-    uint32_t spp_batch = o->batch_spp ? o->batch_spp : (uint32_t)std::max<uint64_t>(1, kMaxPaths / n_pixels_total);
-    spp_batch = std::min(spp_batch, n_samples);
-    uint32_t pix_chunk = n_pixels_total;
-    if ((uint64_t)pix_chunk * spp_batch > kMaxPaths) pix_chunk = (uint32_t)std::max<uint64_t>(1, kMaxPaths / spp_batch);
+    uint32_t spp_batch = 0, pix_chunk = 0;
+    if ((rc = size_path_batches(ctx, o, nee, dev ? 0 : film_bytes, &spp_batch, &pix_chunk)) != YART_OK) return rc;
     const uint64_t cap = (uint64_t)pix_chunk * spp_batch;
-    CUDA_TRY(ctx, ctx->rays.reserve(cap * sizeof(yart_ray)));
-    CUDA_TRY(ctx, ctx->time.reserve(cap * sizeof(double)));
-    CUDA_TRY(ctx, ctx->wavelength.reserve(cap * sizeof(double)));
-    CUDA_TRY(ctx, ctx->throughput.reserve(cap * sizeof(double)));
-    CUDA_TRY(ctx, ctx->hits.reserve(cap * sizeof(DevHit)));
-    CUDA_TRY(ctx, ctx->queue_a.reserve(cap * sizeof(uint32_t)));
-    CUDA_TRY(ctx, ctx->queue_b.reserve(cap * sizeof(uint32_t)));
     const uint32_t D = o->max_depth;
     // with NEE: path counts [0, D+2), then the shadow queue's count of bounce b at D+2+b; path work counters, then the
     // shadow passes' ones
@@ -1800,6 +1817,172 @@ int yart_film_finalize(yart_ctx* ctx, const double* film_xyz, uint32_t width, ui
   if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(rgba8, d_rgba, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   return YART_OK;
+}
+
+int yart_film_finalize_linear(yart_ctx* ctx, const double* film_xyz, uint32_t width, uint32_t height, uint32_t spp,
+                              uint32_t flags, float* rgb) {
+  if (!ctx) return YART_ERR_INVALID;
+  if (!film_xyz || !rgb || !width || !height || !spp || (uint64_t)width * height > 0xFFFFFFFFull) {
+    ctx->err = "yart_film_finalize_linear: bad argument";
+    return YART_ERR_INVALID;
+  }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const size_t n = (size_t)width * height;
+  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
+  const double* d_film = film_xyz;
+  float* d_rgb = rgb;
+  if (!dev) {
+    CUDA_TRY(ctx, ctx->film.reserve(n * 3 * sizeof(double)));
+    CUDA_TRY(ctx, ctx->rgba.reserve(n * 3 * sizeof(float)));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->film.p, film_xyz, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    d_film = ctx->film.as<double>();
+    d_rgb = ctx->rgba.as<float>();
+  }
+  k_film_finalize_linear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_film, width, height, spp, d_rgb);
+  CUDA_TRY(ctx, cudaGetLastError());
+  if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(rgb, d_rgb, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  return YART_OK;
+}
+
+// k_raygen<false> and the bounce-1 passes of yart_render over all objects, then k_aov_accumulate, batch by batch.
+static int render_aovs_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, const yart_aov_planes* planes,
+                            yart_stats* stats) {
+  if (!ctx->have_scene || !cam || !o || !planes) {
+    ctx->err = "yart_render_aovs: missing scene or null argument";
+    return YART_ERR_INVALID;
+  }
+  double* user[3] = {planes->albedo, planes->normal, planes->depth};
+  if (!user[0] && !user[1] && !user[2]) {
+    ctx->err = "yart_render_aovs: all three planes are null";
+    return YART_ERR_INVALID;
+  }
+  const bool dev = (o->flags & YART_FLAG_DEVICE_PTRS) != 0;
+  for (double* p : user)
+    if (dev && (reinterpret_cast<uintptr_t>(p) & 7u)) {
+      ctx->err = "yart_render_aovs: device planes must be 8-byte aligned";
+      return YART_ERR_INVALID;
+    }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  RenderParams R;
+  int rc = fill_render_params(ctx, cam, o, R);
+  if (rc) return rc;
+  if (stats) memset(stats, 0, sizeof(*stats));
+  const uint32_t n_pixels_total = o->width * o->height;
+  const size_t plane_bytes = (size_t)n_pixels_total * 3 * sizeof(double);
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  double* d_plane[3] = {nullptr, nullptr, nullptr};
+  uint64_t staging = 0;
+  for (int k = 0; k < 3; ++k) {
+    if (!user[k]) continue;
+    d_plane[k] = user[k];
+    if (dev) continue;
+    CUDA_TRY(ctx, ctx->aov[k].reserve(plane_bytes));
+    d_plane[k] = ctx->aov[k].as<double>();
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_plane[k], user[k], plane_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    staging += plane_bytes;
+  }
+  uint64_t total_rays = 0, launches = 0, trace_launches = 0;
+  double trace_ms = 0.0;
+  if (o->sample_end > o->sample_begin) {
+    uint32_t spp_batch = 0, pix_chunk = 0;
+    if ((rc = size_path_batches(ctx, o, false, staging, &spp_batch, &pix_chunk)) != YART_OK) return rc;
+    const size_t n_obj_slots = (size_t)ctx->scene.n_objects + 1;
+    CUDA_TRY(ctx, ctx->counts.reserve(2 * sizeof(uint32_t)));
+    CUDA_TRY(ctx, ctx->work.reserve(n_obj_slots * sizeof(uint32_t)));
+    CUDA_TRY(ctx, ctx->counters.reserve(64));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->counters.p, 0, 64, ctx->stream));
+    while (ctx->ev_pool.size() < 2) {
+      cudaEvent_t e;
+      CUDA_TRY(ctx, cudaEventCreate(&e));
+      ctx->ev_pool.push_back(e);
+    }
+    R.st.rays = ctx->rays.as<yart_ray>();
+    R.st.time = ctx->time.as<double>();
+    R.st.wavelength = ctx->wavelength.as<double>();
+    R.st.throughput = ctx->throughput.as<double>();
+    R.st.hits = ctx->hits.as<DevHit>();
+    uint32_t* counts = ctx->counts.as<uint32_t>();
+    NeeState N;
+    memset(&N, 0, sizeof(N));
+    const int stream_grid = ctx->sm_count * 8;
+    for (uint32_t s0 = o->sample_begin; s0 < o->sample_end; s0 += spp_batch) {
+      const uint32_t spp = std::min(spp_batch, o->sample_end - s0);
+      for (uint32_t p0 = 0; p0 < n_pixels_total; p0 += pix_chunk) {
+        R.pixel_base = p0;
+        R.n_pixels = std::min(pix_chunk, n_pixels_total - p0);
+        R.sample_base = s0;
+        R.spp_batch = spp;
+        CUDA_TRY(ctx, cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), ctx->stream));
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, n_obj_slots * sizeof(uint32_t), ctx->stream));
+        k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, ctx->queue_a.as<uint32_t>(), counts + 1, N);
+        QueryArgs q;
+        memset(&q, 0, sizeof(q));
+        q.c.rays = R.st.rays;
+        q.c.queue = ctx->queue_a.as<uint32_t>();
+        q.c.n_items_dev = counts + 1;
+        q.c.n_rays = R.n_pixels * spp;
+        q.c.hits = R.st.hits;
+        q.c.t_min = 0.001; // the render's bounce 1: world.hit(ray, 0.001, f64::INFINITY) (main.rs:548)
+        q.c.t_max = INFINITY;
+        q.d_objects = ctx->scene.objects;
+        q.h_objects = ctx->h_objects.data();
+        q.n_objects = ctx->scene.n_objects; // all of them: there is no k_shade to intersect R.tail_begin..
+        q.ray_time = R.st.time;
+        q.seed = o->seed;
+        q.bounce = 1;
+        q.spp_batch = spp;
+        q.sample_base = s0;
+        q.pixel_base = p0;
+        q.work_counters = ctx->work.as<uint32_t>();
+        q.counters = ctx->counters.as<unsigned long long>();
+        q.near = o->order == YART_ORDER_NEAR;
+        q.count = (o->flags & YART_FLAG_COUNT_VISITS) != 0;
+        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[0], ctx->stream));
+        if ((rc = run_passes(ctx, q, &trace_launches)) != YART_OK) return rc;
+        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[1], ctx->stream));
+        k_aov_accumulate<<<stream_grid, 256, 0, ctx->stream>>>(R, d_plane[0], d_plane[1], d_plane[2]);
+        launches += 2;
+        CUDA_TRY(ctx, cudaGetLastError());
+        uint32_t n_rays = 0;
+        CUDA_TRY(ctx, cudaMemcpyAsync(&n_rays, counts + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        float ms = 0.f;
+        CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[0], ctx->ev_pool[1]));
+        trace_ms += ms;
+        total_rays += n_rays;
+      }
+    }
+  }
+  for (int k = 0; k < 3; ++k)
+    if (user[k] && !dev) CUDA_TRY(ctx, cudaMemcpyAsync(user[k], d_plane[k], plane_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  unsigned long long visit[2] = {0, 0};
+  if ((o->flags & YART_FLAG_COUNT_VISITS) && o->sample_end > o->sample_begin)
+    CUDA_TRY(ctx, cudaMemcpyAsync(visit, ctx->counters.p, sizeof(visit), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (stats) {
+    float ms = 0.f;
+    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    stats->node_visits = visit[0];
+    stats->tri_tests = visit[1];
+    stats->rays = total_rays;
+    stats->paths = total_rays;
+    stats->kernel_launches = launches + trace_launches;
+    stats->trace_launches = (uint32_t)trace_launches;
+    stats->gpu_ms = ms;
+    stats->trace_ms = trace_ms;
+    stats->max_bounce = total_rays ? 1u : 0u;
+  }
+  return YART_OK;
+}
+
+int yart_render_aovs(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, const yart_aov_planes* planes,
+                     yart_stats* stats) {
+  if (!ctx) return YART_ERR_INVALID;
+  YART_ABI_GUARD_BEGIN
+  return render_aovs_impl(ctx, cam, o, planes, stats);
+  YART_ABI_GUARD_END(ctx, "yart_render_aovs")
 }
 
 int yart_generate_camera_rays(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, yart_ray* rays_host,

@@ -10,8 +10,8 @@
 // Additions: --seed S (the reference is OS-seeded), --device D, --gpus N (N GPUs of this box: one host thread per
 // context, yart_comm_init + yart_film_reduce = one in-place ncclReduce of the f64 film), --order near|reference,
 // --unbiased-light-pick / --russian-roulette / --depth-zero-black / --next-event (better sampling, OFF by default), --assets DIR,
-// --dry-run (print the resolved options as one JSON line and exit: what the reference's unit tests check,
-// main.rs:868-915), --list-scenes.  `--workers` is accepted and ignored.  There is no CPU mode.
+// --aovs [--aov-samples N] (denoiser inputs next to the PNG, as yart_cli.py writes them), --dry-run (print the
+// resolved options as one JSON line and exit: what the reference's unit tests check, main.rs:868-915), --list-scenes.  `--workers` is accepted and ignored.  There is no CPU mode.
 //
 // build (build.py does this): g++ -std=c++17 -O2 -Iinclude host/yart_main.cpp -o yart -L. -lyart_b200 -Wl,-rpath,'$ORIGIN' -pthread
 #include <algorithm>
@@ -99,6 +99,17 @@ bool write_png(const std::string& path, const uint8_t* rgba, uint32_t w, uint32_
   return fclose(f) == 0 && ok;
 }
 
+// a portable float map: "PF" (3 channels) or "Pf" (1), little-endian f32 (scale -1), rows bottom to top -- what
+// Open Image Denoise's oidnDenoise reads
+bool write_pfm(const std::string& path, const std::vector<float>& px, uint32_t w, uint32_t h, int channels) {
+  FILE* f = fopen(path.c_str(), "wb");
+  if (!f) return false;
+  bool ok = fprintf(f, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", w, h) > 0;
+  for (uint32_t y = h; ok && y-- > 0;)
+    ok = fwrite(px.data() + (size_t)y * w * channels, sizeof(float), (size_t)w * channels, f) == (size_t)w * channels;
+  return fclose(f) == 0 && ok;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // command line (clap's behaviour where the reference's tests pin it: main.rs:831-842)
 // ---------------------------------------------------------------------------------------------------------
@@ -111,13 +122,15 @@ struct Cli {
   int device = 0, gpus = 1;
   uint32_t flags = 0;
   bool dry_run = false, list_scenes = false;
+  bool aovs = false;
+  uint32_t aov_samples = 0; // 0 = min(16, samples)
 };
 
 [[noreturn]] void usage_error(const std::string& msg) { // clap exits with status 2 on a usage error
   fprintf(stderr, "error: %s\n\nUsage: yart --scene <SCENE> [--output <OUTPUT>] [--width <WIDTH>] [--height <HEIGHT>] "
                   "[--samples <SAMPLES>] [--max-depth <MAX_DEPTH>] [--workers <WORKERS>] [--vfov <VFOV>] [--aperture <APERTURE>]\n"
                   "            [--seed S] [--device D] [--gpus N] [--order near|reference] [--assets DIR] [--dry-run] [--list-scenes]\n"
-                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event]\n",
+                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event] [--aovs] [--aov-samples N]\n",
           msg.c_str());
   exit(2);
 }
@@ -172,6 +185,8 @@ Cli parse(int argc, char** argv) {
     else if (a == "--russian-roulette") c.flags |= YART_FLAG_RUSSIAN_ROULETTE;
     else if (a == "--depth-zero-black") c.flags |= YART_FLAG_DEPTH_ZERO_BLACK;
     else if (a == "--next-event") c.flags |= YART_FLAG_NEXT_EVENT;
+    else if (a == "--aovs") c.aovs = true;
+    else if (a == "--aov-samples") c.aov_samples = positive("--aov-samples", value());
     else if (a == "--dry-run") c.dry_run = true;
     else if (a == "--list-scenes") c.list_scenes = true;
     else if (a == "--help" || a == "-h") {
@@ -300,6 +315,42 @@ int main(int argc, char** argv) {
   if (!write_png(output, rgba.data(), width, height)) {
     fprintf(stderr, "yart: cannot write %s\n", output.c_str());
     return 1;
+  }
+  if (cli.aovs) { // denoiser inputs next to the PNG: linear colour + first-hit means of samples [0, aov_samples)
+    const size_t np = (size_t)width * height;
+    std::vector<float> color(np * 3), albedo(np * 3), normal(np * 3), depth(np);
+    if (yart_film_finalize_linear(ctxs[0], film.data(), width, height, spp, 0, color.data()) != YART_OK)
+      return die("yart_film_finalize_linear", ctxs[0]);
+    std::vector<double> pa(np * 3, 0.0), pn(np * 3, 0.0), pd(np * 3, 0.0);
+    yart_aov_planes planes = {pa.data(), pn.data(), pd.data()};
+    yart_render_opts o;
+    memset(&o, 0, sizeof o);
+    o.width = width;
+    o.height = height;
+    o.sample_end = cli.aov_samples ? cli.aov_samples : std::min<uint32_t>(16, spp);
+    o.max_depth = max_depth;
+    o.order = cli.order == "near" ? YART_ORDER_NEAR : YART_ORDER_REFERENCE;
+    o.flags = cli.flags;
+    o.seed = cli.seed;
+    if (yart_render_aovs(ctxs[0], &cam, &o, &planes, nullptr) != YART_OK) return die("yart_render_aovs", ctxs[0]);
+    for (size_t i = 0; i < np; ++i) { // the means of aov_means() in the Python package
+      const double n = pd[i * 3 + 2], hits = pd[i * 3 + 1];
+      for (int k = 0; k < 3; ++k) {
+        albedo[i * 3 + k] = n > 0 ? (float)(pa[i * 3 + k] / n) : 0.f;
+        normal[i * 3 + k] = n > 0 ? (float)(pn[i * 3 + k] / n) : 0.f;
+      }
+      depth[i] = hits > 0 ? (float)(pd[i * 3] / hits) : 0.f;
+    }
+    const std::string stem = (std::filesystem::path(output).parent_path() / std::filesystem::path(output).stem()).string();
+    const struct { const char* name; const std::vector<float>& px; int ch; } files[] = {
+        {"color", color, 3}, {"albedo", albedo, 3}, {"normal", normal, 3}, {"depth", depth, 1}};
+    for (const auto& f : files) {
+      const std::string path = stem + "." + f.name + ".pfm";
+      if (!write_pfm(path, f.px, width, height, f.ch)) {
+        fprintf(stderr, "yart: cannot write %s\n", path.c_str());
+        return 1;
+      }
+    }
   }
   if (comm) yart_comm_destroy(comm);
   for (int r = 0; r < n; ++r) {
