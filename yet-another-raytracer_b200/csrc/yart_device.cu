@@ -215,9 +215,14 @@ int tune_env(const char* name, int dflt) { // tuning / debugging knobs from the 
   return v ? atoi(v) : dflt;
 }
 
+// A growable device allocation that frees itself.
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { release(); }
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFree(p); // (cudaFree synchronises the device: work still using the old buffer has finished)
@@ -237,6 +242,21 @@ struct DevBuf {
     return reinterpret_cast<T*>(p);
   }
 };
+
+// Grows an event list to at least n events.
+cudaError_t ensure_events(std::vector<cudaEvent_t>& events, size_t n) {
+  while (events.size() < n) {
+    cudaEvent_t e;
+    if (cudaError_t err = cudaEventCreate(&e)) return err;
+    events.push_back(e);
+  }
+  return cudaSuccess;
+}
+
+// YART_FLAG_NEXT_EVENT's bytes per path in flight, one entry per buffer of yart_ctx::nee in NeeState's order: 48 shadow
+// ray + 8 pending + 8 light-sample sum + 8 emission weight + 4 shadow queue (the shadow passes write their hits into the
+// path hits, which are dead from k_shade to the next bounce's passes)
+constexpr size_t kNeeBytes[5] = {sizeof(yart_ray), sizeof(double), sizeof(double), sizeof(double), sizeof(uint32_t)};
 
 // flat 4-wide tree over the members of a BVHNode group (median split on the longest centroid
 // axis; the shape is free -- closest-hit results do not depend on it)
@@ -365,7 +385,8 @@ struct yart_ctx {
   DevScene scene;
   yart_object* d_solo = nullptr; // one un-wrapped MESH object per mesh, for mesh-only queries
   std::map<const void*, int> traverse_blocks; // resident CTAs per SM of each k_traverse variant
-  std::vector<yart_object> h_objects; // host copy of the world list: the pass plan is made on the host
+  std::vector<yart_object> h_objects; // host copies of the world list and of d_solo: the pass plan is made on the host
+  std::vector<yart_object> h_solo;
   std::vector<DevMesh> h_meshes;
   uint32_t n_meshes = 0;
   uint32_t max_stack = 0;
@@ -376,7 +397,7 @@ struct yart_ctx {
 
   // work buffers
   DevBuf rays, hits_export, time, wavelength, throughput, hits, queue_a, queue_b, counts, work, counters, film, rgba;
-  DevBuf nee_rays, nee_pending, nee_sum, nee_w, queue_s; // YART_FLAG_NEXT_EVENT's per-path state (NeeState)
+  DevBuf nee[5]; // YART_FLAG_NEXT_EVENT's per-path state, as kNeeBytes lists it
   DevBuf occluded; // staging of yart_occluded's flags for host arrays
   DevBuf ray_times; // staging of yart_closest_hit_records' ray times for host arrays
   DevBuf aov[3];    // staging of yart_render_aovs' host planes
@@ -499,12 +520,41 @@ int launch_persistent(yart_ctx* ctx, void (*k)(const Params), int carveout, cons
   return YART_OK;
 }
 
+// The shared-memory carveout of a persistent traversal kernel: k_traverse's, or that of k_traverse_lean and k_occlude
+// (the lean kernel keeps 22-42 KB of shared memory per CTA: five CTAs need the 132 KB configuration).
+int carveout(bool lean) {
+  static const int carve = tune_env("YART_TUNE_CARVEOUT", 35), carve_lean = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
+  return lean ? carve_lean : carve;
+}
+
+// The pass plan of a world list, in list order: one traversal pass per mesh instance (a mesh wrapped in a medium is
+// not one), one analytic pass per run of consecutive other objects.
+bool is_mesh_pass(const yart_object& o) { return o.kind == YART_OBJ_MESH && !(o.wrap & YART_WRAP_MEDIUM); }
+
+// The end of the pass that starts at list position i.
+uint32_t pass_end(const yart_object* objects, uint32_t n_objects, uint32_t i) {
+  if (is_mesh_pass(objects[i])) return i + 1;
+  while (i < n_objects && !is_mesh_pass(objects[i])) ++i;
+  return i;
+}
+
+// The list a query walks: device copy, host copy (the plan is made on the host) and length.
+struct ObjectList {
+  const yart_object* d;
+  const yart_object* h;
+  uint32_t n;
+};
+
+// The world, or (target = a mesh index) that mesh alone, un-wrapped.
+ObjectList target_objects(const yart_ctx* ctx, uint32_t target) {
+  if (target == YART_TARGET_WORLD) return {ctx->scene.objects, ctx->h_objects.data(), ctx->scene.n_objects};
+  return {ctx->d_solo + target, ctx->h_solo.data() + target, 1u};
+}
+
 // What is the same for every pass of one closest-hit query.
 struct QueryArgs {
   PassCommon c;
-  const yart_object* d_objects; // device copy of the list the host plan walks
-  const yart_object* h_objects;
-  uint32_t n_objects;
+  ObjectList objects;
   const double* ray_time;
   uint64_t seed;
   uint32_t bounce, spp_batch, sample_base, pixel_base;
@@ -516,47 +566,38 @@ struct QueryArgs {
 // HittableList::hit (hittable.rs:66-79) as passes over the ray queue, in list order: one k_traverse per
 // mesh instance, one k_analytic per run of consecutive analytic objects.
 int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
-  static const int carve = tune_env("YART_TUNE_CARVEOUT", 35);
-  static const int carve_lean = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
-  bool first = true;
-  uint32_t i = 0, n_trav = 0;
-  auto is_mesh = [&](uint32_t k) {
-    return q.h_objects[k].kind == YART_OBJ_MESH && !(q.h_objects[k].wrap & YART_WRAP_MEDIUM);
-  };
-  if (q.n_objects == 0) { // an empty world: every ray misses
+  const ObjectList& L = q.objects;
+  if (L.n == 0) { // an empty world: every ray misses
     AnalyticParams A;
     memset(&A, 0, sizeof(A));
     A.c = q.c;
     A.c.first_pass = 1;
     A.scene = ctx->scene;
-    A.objects = q.d_objects;
+    A.objects = L.d;
     A.spp_batch = 1;
     k_analytic<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(A);
     if (launches) (*launches)++;
   }
-  while (i < q.n_objects) {
-    if (is_mesh(i)) {
-      const yart_object& o = q.h_objects[i];
+  uint32_t n_trav = 0;
+  for (uint32_t i = 0, j; i < L.n; i = j) {
+    j = pass_end(L.h, L.n, i);
+    if (is_mesh_pass(L.h[i])) {
       TraverseParams T;
       memset(&T, 0, sizeof(T));
       T.c = q.c;
-      T.c.first_pass = first ? 1u : 0u;
-      T.m = mesh_pass(o, ctx->h_meshes[o.index], q.work_counters + n_trav++);
+      T.c.first_pass = i == 0 ? 1u : 0u;
+      T.m = mesh_pass(L.h[i], ctx->h_meshes[L.h[i].index], q.work_counters + n_trav++);
       T.obj_index = i;
       T.counters = q.counters;
-      // (the lean kernel keeps 22-42 KB of shared memory per CTA: five CTAs need the 132 KB configuration)
-      const int carveout = q.near && !q.count ? carve_lean : carve;
-      if (int rc = launch_persistent(ctx, traverse_kernel(q.near, q.count, ctx->max_stack), carveout, T)) return rc;
-      i++;
+      const bool lean = q.near && !q.count;
+      if (int rc = launch_persistent(ctx, traverse_kernel(q.near, q.count, ctx->max_stack), carveout(lean), T)) return rc;
     } else {
-      uint32_t j = i;
-      while (j < q.n_objects && !is_mesh(j)) ++j;
       AnalyticParams A;
       memset(&A, 0, sizeof(A));
       A.c = q.c;
-      A.c.first_pass = first ? 1u : 0u;
+      A.c.first_pass = i == 0 ? 1u : 0u;
       A.scene = ctx->scene;
-      A.objects = q.d_objects;
+      A.objects = L.d;
       A.obj_begin = i;
       A.obj_end = j;
       A.ray_time = q.ray_time;
@@ -567,9 +608,7 @@ int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
       A.pixel_base = q.pixel_base;
       A.media_mask = ctx->has_media ? 1u : 0u;
       k_analytic<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(A);
-      i = j;
     }
-    first = false;
     if (launches) (*launches)++;
   }
   CUDA_TRY(ctx, cudaGetLastError());
@@ -579,9 +618,7 @@ int run_passes(yart_ctx* ctx, const QueryArgs& q, uint64_t* launches) {
 // What is the same for every pass of one occlusion query.
 struct OcclusionArgs {
   OccludeCommon c;
-  const yart_object* d_objects;
-  const yart_object* h_objects;
-  uint32_t n_objects;
+  ObjectList objects;
   uint32_t pixel_base;
   uint32_t* work_counters; // one zeroed u32 per mesh pass (at least n_objects)
 };
@@ -590,44 +627,35 @@ struct OcclusionArgs {
 // k_analytic_occluded per run of consecutive analytic objects.  c.occluded must be zeroed: a pass only ever writes 1,
 // and the passes after the first skip the rays already marked.  An empty world launches nothing.
 int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launches) {
-  static const int carve = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
+  const ObjectList& L = q.objects;
   // A closest-hit pass starts a ray that nothing has hit yet from t_max if it is the first mesh pass, and from
   // fmin(+inf, t_max) otherwise (the recorded miss is +inf).  The two differ only for a NaN t_max.
   const double t_max_later = std::fmin(INFINITY, q.c.t_max);
-  bool first = true;
-  uint32_t i = 0, n_trav = 0;
-  auto is_mesh = [&](uint32_t k) {
-    return q.h_objects[k].kind == YART_OBJ_MESH && !(q.h_objects[k].wrap & YART_WRAP_MEDIUM);
-  };
-  while (i < q.n_objects) {
-    if (is_mesh(i)) {
-      const yart_object& o = q.h_objects[i];
+  uint32_t n_trav = 0;
+  for (uint32_t i = 0, j; i < L.n; i = j) {
+    j = pass_end(L.h, L.n, i);
+    if (is_mesh_pass(L.h[i])) {
       OccludeParams T;
       memset(&T, 0, sizeof(T));
       T.c = q.c;
-      T.c.first_pass = first ? 1u : 0u;
-      T.c.t_max = first ? q.c.t_max : t_max_later;
-      T.m = mesh_pass(o, ctx->h_meshes[o.index], q.work_counters + n_trav++);
-      if (int rc = launch_persistent(ctx, yart::occlude_kernel(ctx->max_stack), carve, T)) return rc;
-      i++;
+      T.c.first_pass = i == 0 ? 1u : 0u;
+      T.c.t_max = i == 0 ? q.c.t_max : t_max_later;
+      T.m = mesh_pass(L.h[i], ctx->h_meshes[L.h[i].index], q.work_counters + n_trav++);
+      if (int rc = launch_persistent(ctx, yart::occlude_kernel(ctx->max_stack), carveout(true), T)) return rc;
     } else {
-      uint32_t j = i;
-      while (j < q.n_objects && !is_mesh(j)) ++j;
       AnalyticOccludedParams A;
       memset(&A, 0, sizeof(A));
       A.c = q.c;
-      A.c.first_pass = first ? 1u : 0u;
+      A.c.first_pass = i == 0 ? 1u : 0u;
       A.c.t_max = t_max_later;
       A.scene = ctx->scene;
-      A.objects = q.d_objects;
+      A.objects = L.d;
       A.obj_begin = i;
       A.obj_end = j;
       A.pixel_base = q.pixel_base;
       A.media = ctx->has_media ? 1u : 0u;
       yart::analytic_occluded_kernel()<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(A);
-      i = j;
     }
-    first = false;
     if (launches) (*launches)++;
   }
   CUDA_TRY(ctx, cudaGetLastError());
@@ -642,7 +670,7 @@ int run_occlusion_passes(yart_ctx* ctx, const OcclusionArgs& q, uint64_t* launch
 // the next upload is issued; with pinned memory everything is asynchronous.
 // run(off, len) enqueues on ctx->stream the kernels that read the ray records at d_in + off * in_bytes and leave
 // out_bytes per ray at d_out + off * out_bytes.  Everything is enqueued on return; after a synchronisation of
-// ctx->stream, chunked_kernel_ms gives the kernels' time.
+// ctx->stream, finish_query gives the kernels' time.
 // An optional second per-ray input (in2, in2_bytes per ray; null = none) goes up with the rays, chunk by chunk on the
 // same copy stream, into d_in2 (host arrays only: with device arrays run() reads it where it is).
 template <class Run>
@@ -665,11 +693,7 @@ int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* 
   } else {
     if (!ctx->copy_in) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_in, cudaStreamNonBlocking));
     if (!ctx->copy_out) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_out, cudaStreamNonBlocking));
-    while (ctx->chunk_events.size() < 3 * n_chunks + 1) {
-      cudaEvent_t e;
-      CUDA_TRY(ctx, cudaEventCreate(&e));
-      ctx->chunk_events.push_back(e);
-    }
+    CUDA_TRY(ctx, ensure_events(ctx->chunk_events, 3 * n_chunks + 1));
     cudaEvent_t* up = ctx->chunk_events.data();                   // up[i]: chunk i is on the device
     cudaEvent_t* done = ctx->chunk_events.data() + n_chunks;      // done[i]: chunk i's results are in d_out
     cudaEvent_t* begun = ctx->chunk_events.data() + 2 * n_chunks; // begun[i]: chunk i's kernels start (its upload is in)
@@ -713,18 +737,211 @@ int run_chunked(yart_ctx* ctx, bool dev, const void* in, size_t in_bytes, void* 
   return YART_OK;
 }
 
-// the kernels of a finished run_chunked call: ev0 -> ev1, or the chunks without the waits for their uploads in between
-int chunked_kernel_ms(yart_ctx* ctx, uint64_t n_chunks, bool dev, float* ms) {
-  *ms = 0.f;
-  if (dev || n_chunks == 1) {
-    CUDA_TRY(ctx, cudaEventElapsedTime(ms, ctx->ev0, ctx->ev1));
-  } else {
-    for (uint64_t i = 0; i < n_chunks; ++i) {
-      float part = 0.f;
-      CUDA_TRY(ctx, cudaEventElapsedTime(&part, ctx->chunk_events[2 * n_chunks + i], ctx->chunk_events[n_chunks + i]));
-      *ms += part;
+// One batched query (yart_closest_hit*, yart_occluded*) after begin_query: where its arrays are on the device and what
+// its passes walk.
+struct BatchQuery {
+  uint64_t n;
+  bool dev;             // YART_FLAG_DEVICE_PTRS: the caller's arrays are on the device
+  size_t ray_bytes;
+  const char* d_rays;   // the caller's rays, or the staging buffer run_chunked uploads them into
+  const double* d_times;
+  char* d_out;          // the caller's results, or the staging buffer run_chunked downloads
+  ObjectList objects;
+  size_t work_bytes;    // the passes' work counters: one per object, zeroed before each chunk
+  uint64_t n_chunks = 0, launches = 0;
+};
+
+// The argument checks and set-up the batched queries share.  bad_arg: the caller's own argument check failed;
+// allowed_flags / flags_err: the flags the call takes and the message that rejects any other; out_bytes / out_align:
+// one result and the alignment a device result array needs (0: any); out_stage: the staging buffer of host results;
+// times: an optional per-ray input that is staged with the rays.  YART_OK with q.n == 0: there is nothing to run.
+int begin_query(yart_ctx* ctx, const char* fn, uint32_t target, bool f32, const void* rays, const double* times, void* out,
+                size_t out_bytes, uintptr_t out_align, DevBuf& out_stage, uint64_t n, bool bad_arg, uint32_t flags,
+                uint32_t allowed_flags, const char* flags_err, yart_stats* stats, BatchQuery& q) {
+  if (!ctx->have_scene) {
+    ctx->err = std::string(fn) + ": no scene (call yart_ctx_set_scene first)";
+    return YART_ERR_INVALID;
+  }
+  if ((n && (!rays || !out)) || n > 0xFFFFFFF0ull || bad_arg) {
+    ctx->err = std::string(fn) + ": bad argument";
+    return YART_ERR_INVALID;
+  }
+  if (flags & ~allowed_flags) {
+    ctx->err = std::string(fn) + flags_err;
+    return YART_ERR_INVALID;
+  }
+  q.dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
+  const uintptr_t ray_align = f32 ? 7u : 15u;
+  if (q.dev && ((reinterpret_cast<uintptr_t>(rays) & ray_align) || (reinterpret_cast<uintptr_t>(out) & out_align))) {
+    ctx->err = std::string(fn) + ": device ray arrays must be " + std::to_string(ray_align + 1) + "-byte aligned" +
+               (out_align ? " (hits: " + std::to_string(out_align + 1) + ")" : "");
+    return YART_ERR_INVALID;
+  }
+  if (q.dev && (reinterpret_cast<uintptr_t>(times) & 7u)) {
+    ctx->err = std::string(fn) + ": device time arrays must be 8-byte aligned";
+    return YART_ERR_INVALID;
+  }
+  if (target != YART_TARGET_WORLD && target >= ctx->n_meshes) {
+    ctx->err = std::string(fn) + ": target is neither a mesh index nor YART_TARGET_WORLD";
+    return YART_ERR_INVALID;
+  }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (stats) memset(stats, 0, sizeof(*stats));
+  q.n = n;
+  if (n == 0) return YART_OK;
+  q.ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray);
+  q.d_rays = static_cast<const char*>(rays);
+  q.d_times = times;
+  q.d_out = static_cast<char*>(out);
+  if (!q.dev) {
+    CUDA_TRY(ctx, ctx->rays.reserve(n * q.ray_bytes));
+    CUDA_TRY(ctx, out_stage.reserve(n * out_bytes));
+    q.d_rays = ctx->rays.as<char>();
+    q.d_out = out_stage.as<char>();
+    if (times) {
+      CUDA_TRY(ctx, ctx->ray_times.reserve(n * sizeof(double)));
+      q.d_times = ctx->ray_times.as<double>();
     }
   }
+  q.objects = target_objects(ctx, target);
+  q.work_bytes = ((size_t)q.objects.n + 2) * sizeof(uint32_t);
+  CUDA_TRY(ctx, ctx->work.reserve(q.work_bytes));
+  return YART_OK;
+}
+
+// After run_chunked: waits for the query and fills stats.  gpu_ms and trace_ms are the kernels' time: ev0 -> ev1, or
+// the chunks without the waits for their uploads in between.
+int finish_query(yart_ctx* ctx, const BatchQuery& q, uint64_t trace_launches, const unsigned long long visits[2],
+                 yart_stats* stats) {
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (!stats) return YART_OK;
+  float ms = 0.f;
+  if (q.dev || q.n_chunks == 1) {
+    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+  } else {
+    for (uint64_t i = 0; i < q.n_chunks; ++i) {
+      float part = 0.f;
+      CUDA_TRY(ctx, cudaEventElapsedTime(&part, ctx->chunk_events[2 * q.n_chunks + i], ctx->chunk_events[q.n_chunks + i]));
+      ms += part;
+    }
+  }
+  stats->rays = q.n;
+  stats->node_visits = visits[0];
+  stats->tri_tests = visits[1];
+  stats->kernel_launches = q.launches;
+  stats->trace_launches = (uint32_t)trace_launches;
+  stats->gpu_ms = ms;
+  stats->trace_ms = ms;
+  return YART_OK;
+}
+
+// The closest-hit query of bounce b of the batch R describes, over `queue` (its length at *count) and the world list's
+// first n_objects objects; work: one zeroed u32 per object.
+QueryArgs bounce_query(yart_ctx* ctx, const yart_render_opts* o, const RenderParams& R, uint32_t* queue, uint32_t* count,
+                       uint32_t b, uint32_t n_objects, uint32_t* work) {
+  QueryArgs q;
+  memset(&q, 0, sizeof(q));
+  q.c.rays = R.st.rays;
+  q.c.queue = queue;
+  q.c.n_items_dev = count;
+  q.c.n_rays = R.n_pixels * R.spp_batch;
+  q.c.hits = R.st.hits;
+  q.c.t_min = 0.001; // world.hit(ray_in, 0.001, f64::INFINITY) (main.rs:548)
+  q.c.t_max = INFINITY;
+  q.objects = {ctx->scene.objects, ctx->h_objects.data(), n_objects};
+  q.ray_time = R.st.time;
+  q.seed = o->seed;
+  q.bounce = b;
+  q.spp_batch = R.spp_batch;
+  q.sample_base = R.sample_base;
+  q.pixel_base = R.pixel_base;
+  q.work_counters = work;
+  q.counters = ctx->counters.as<unsigned long long>();
+  q.near = o->order == YART_ORDER_NEAR;
+  q.count = (o->flags & YART_FLAG_COUNT_VISITS) != 0;
+  return q;
+}
+
+// What the sample loop of yart_render and yart_render_aovs adds up for yart_stats.
+struct RenderTotals {
+  uint64_t rays = 0, paths = 0, launches = 0, trace_launches = 0;
+  double trace_ms = 0.0;
+  uint32_t deepest = 0;
+};
+
+// The sample loop of yart_render and yart_render_aovs over the path state size_path_batches reserved: the visit
+// counters are zeroed once, then batch() runs for each pixel chunk of each range of spp_batch samples, with R's batch
+// fields set and the first n_counts u32 of ctx->counts and n_work of ctx->work zeroed.
+template <class Batch>
+int for_each_batch(yart_ctx* ctx, const yart_render_opts* o, uint32_t spp_batch, uint32_t pix_chunk, size_t n_counts,
+                   size_t n_work, RenderParams& R, Batch&& batch) {
+  R.st.rays = ctx->rays.as<yart_ray>();
+  R.st.time = ctx->time.as<double>();
+  R.st.wavelength = ctx->wavelength.as<double>();
+  R.st.throughput = ctx->throughput.as<double>();
+  R.st.hits = ctx->hits.as<DevHit>();
+  CUDA_TRY(ctx, ctx->counters.reserve(64));
+  CUDA_TRY(ctx, cudaMemsetAsync(ctx->counters.p, 0, 64, ctx->stream));
+  const uint32_t n_pixels_total = o->width * o->height;
+  for (uint32_t s0 = o->sample_begin; s0 < o->sample_end; s0 += spp_batch) {
+    for (uint32_t p0 = 0; p0 < n_pixels_total; p0 += pix_chunk) {
+      R.pixel_base = p0;
+      R.n_pixels = std::min(pix_chunk, n_pixels_total - p0);
+      R.sample_base = s0;
+      R.spp_batch = std::min(spp_batch, o->sample_end - s0);
+      CUDA_TRY(ctx, cudaMemsetAsync(ctx->counts.p, 0, n_counts * sizeof(uint32_t), ctx->stream));
+      CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, n_work * sizeof(uint32_t), ctx->stream));
+      if (int rc = batch()) return rc;
+    }
+  }
+  return YART_OK;
+}
+
+// The end of yart_render / yart_render_aovs, after their results are queued for download: the visit counters, the
+// call's time since ctx->ev0 and the totals into stats.
+int finish_render(yart_ctx* ctx, const yart_render_opts* o, const RenderTotals& t, yart_stats* stats) {
+  unsigned long long visit[2] = {0, 0};
+  if ((o->flags & YART_FLAG_COUNT_VISITS) && o->sample_end > o->sample_begin)
+    CUDA_TRY(ctx, cudaMemcpyAsync(visit, ctx->counters.p, sizeof(visit), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (!stats) return YART_OK;
+  float ms = 0.f;
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+  stats->node_visits = visit[0];
+  stats->tri_tests = visit[1];
+  stats->rays = t.rays;
+  stats->paths = t.paths;
+  stats->kernel_launches = t.launches + t.trace_launches;
+  stats->trace_launches = (uint32_t)t.trace_launches;
+  stats->gpu_ms = ms;
+  stats->trace_ms = t.trace_ms;
+  stats->max_bounce = t.deepest;
+  return YART_OK;
+}
+
+// yart_film_finalize(_linear) once the arguments are checked: kernel writes `channels` values of T per pixel; host
+// arrays are staged through ctx->film and ctx->rgba.
+template <class T>
+int film_finalize_impl(yart_ctx* ctx, void (*kernel)(const double*, uint32_t, uint32_t, uint32_t, T*), size_t channels,
+                       const double* film_xyz, uint32_t width, uint32_t height, uint32_t spp, uint32_t flags, T* out) {
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const size_t n = (size_t)width * height;
+  const size_t out_bytes = n * channels * sizeof(T);
+  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
+  const double* d_film = film_xyz;
+  T* d_out = out;
+  if (!dev) {
+    CUDA_TRY(ctx, ctx->film.reserve(n * 3 * sizeof(double)));
+    CUDA_TRY(ctx, ctx->rgba.reserve(out_bytes));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->film.p, film_xyz, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    d_film = ctx->film.as<double>();
+    d_out = ctx->rgba.as<T>();
+  }
+  kernel<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_film, width, height, spp, d_out);
+  CUDA_TRY(ctx, cudaGetLastError());
+  if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   return YART_OK;
 }
 
@@ -792,10 +1009,6 @@ void yart_ctx_destroy(yart_ctx* ctx) {
   cudaSetDevice(ctx->device);
   cudaDeviceSynchronize();
   ctx->free_scene();
-  DevBuf* bufs[] = {&ctx->rays, &ctx->hits_export, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits,
-                    &ctx->queue_a, &ctx->queue_b, &ctx->counts, &ctx->work, &ctx->counters, &ctx->film, &ctx->rgba,
-                    &ctx->occluded, &ctx->ray_times, &ctx->aov[0], &ctx->aov[1], &ctx->aov[2]};
-  for (DevBuf* b : bufs) b->release();
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->chunk_events) cudaEventDestroy(e);
   if (ctx->copy_in) cudaStreamDestroy(ctx->copy_in);
@@ -995,7 +1208,6 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
       DeviceQbvh dq;
       if (!build_qbvh_device(ctx->stream, d->meshes[i], dq, err)) {
         ctx->err = "yart_ctx_set_scene: mesh " + std::to_string(i) + " (device build): " + err;
-        ctx->free_scene();
         return err.find("cuda") != std::string::npos ? YART_ERR_CUDA : YART_ERR_INVALID;
       }
       dn = dq.nodes; dt = dq.tris; ds = dq.shade;
@@ -1008,15 +1220,12 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
       FlatQbvh hq;
       if (!build_qbvh(d->meshes[i], hq, err)) {
         ctx->err = "yart_ctx_set_scene: mesh " + std::to_string(i) + ": " + err;
-        ctx->free_scene();
         return YART_ERR_INVALID;
       }
       int rc;
       if ((rc = upload(ctx, hq.nodes.data(), hq.nodes.size(), &dn)) || (rc = upload(ctx, hq.tris.data(), hq.tris.size(), &dt)) ||
-          (rc = upload(ctx, hq.shade.data(), hq.shade.size(), &ds))) {
-        ctx->free_scene();
+          (rc = upload(ctx, hq.shade.data(), hq.shade.size(), &ds)))
         return rc;
-      }
       CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); // hq goes out of scope
       q.root = hq.root; q.max_stack = hq.max_stack; q.n_nodes = (uint32_t)hq.nodes.size(); q.n_tris = (uint32_t)hq.tris.size();
       for (int a = 0; a < 3; ++a) { q.bbox_min[a] = hq.bbox_min[a]; q.bbox_max[a] = hq.bbox_max[a]; }
@@ -1046,7 +1255,6 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
   }
   if (ctx->max_stack > 64) {
     ctx->err = "yart_ctx_set_scene: QBVH deeper than the 64-entry traversal stack (qbvh.rs:382)";
-    ctx->free_scene();
     return YART_ERR_UNSUPPORTED;
   }
   // ---- groups ----
@@ -1060,12 +1268,10 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
     for (uint32_t k = 0; k < g.n_members; ++k)
       if (const char* m = check_obj(g.members[k], true)) {
         ctx->err = std::string("yart_ctx_set_scene: group member: ") + m;
-        ctx->free_scene();
         return YART_ERR_INVALID;
       }
     if (g.n_members > 65536u) { // tree height <= 7 keeps the traversal within its 24-entry stack (3 * height + 1)
       ctx->err = "yart_ctx_set_scene: a group holds more than 65536 members";
-      ctx->free_scene();
       return YART_ERR_UNSUPPORTED;
     }
     std::vector<yart_object> members(g.members, g.members + g.n_members);
@@ -1086,10 +1292,8 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
     uint32_t* dorig;
     int rc;
     if ((rc = upload(ctx, gb.nodes.data(), gb.nodes.size(), &dn)) || (rc = upload(ctx, members.data(), members.size(), &dm)) ||
-        (rc = upload(ctx, orig.data(), orig.size(), &dorig))) {
-      ctx->free_scene();
+        (rc = upload(ctx, orig.data(), orig.size(), &dorig)))
       return rc;
-    }
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     groups[i].nodes = reinterpret_cast<const float4*>(dn);
     groups[i].members = dm;
@@ -1110,11 +1314,7 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
   for (uint32_t i = 0; i < d->n_images; ++i) {
     uint8_t* dp;
     const size_t img_bytes = d->images[i].rgb8 ? (size_t)d->images[i].width * d->images[i].height * 3 : 0;
-    int rc = upload(ctx, d->images[i].rgb8, img_bytes, &dp);
-    if (rc) {
-      ctx->free_scene();
-      return rc;
-    }
+    if (int rc = upload(ctx, d->images[i].rgb8, img_bytes, &dp)) return rc;
     images[i].rgb8 = dp;
     images[i].width = d->images[i].width;
     images[i].height = d->images[i].height;
@@ -1134,10 +1334,8 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
       (rc = upload(ctx, meshes.data(), meshes.size(), &dmeshes)) || (rc = upload(ctx, groups.data(), groups.size(), &dgroups)) ||
       (rc = upload(ctx, d->materials, d->n_materials, &dmat)) || (rc = upload(ctx, d->textures, d->n_textures, &dtex)) ||
       (rc = upload(ctx, d->perlins, d->n_perlins, &dper)) || (rc = upload(ctx, images.data(), images.size(), &dimg)) ||
-      (rc = upload(ctx, solo.data(), solo.size(), &ctx->d_solo))) {
-    ctx->free_scene();
+      (rc = upload(ctx, solo.data(), solo.size(), &ctx->d_solo)))
     return rc;
-  }
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   S.objects = dobj;
   S.lights = dlights;
@@ -1154,6 +1352,7 @@ static int set_scene_impl(yart_ctx* ctx, const yart_scene_desc* d) {
   for (int k = 0; k < 3; ++k) S.background[k] = d->background_rgb[k];
   ctx->n_meshes = d->n_meshes;
   ctx->h_objects.assign(d->objects, d->objects + d->n_objects);
+  ctx->h_solo = solo;
   ctx->h_meshes = meshes;
   ctx->have_scene = true;
   return YART_OK;
@@ -1186,78 +1385,26 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, co
                             double t_min, double t_max, uint32_t order, uint32_t flags, void* hits, yart_stats* stats) {
   const bool f32 = fmt == HitFormat::F32, record = fmt == HitFormat::RECORD;
   const char* fn = f32 ? "yart_closest_hit_f32" : (record ? "yart_closest_hit_records" : "yart_closest_hit");
-  if (!ctx->have_scene) {
-    ctx->err = std::string(fn) + ": no scene (call yart_ctx_set_scene first)";
-    return YART_ERR_INVALID;
-  }
-  if ((n && (!rays || !hits)) || n > 0xFFFFFFF0ull || order > YART_ORDER_NEAR) {
-    ctx->err = std::string(fn) + ": bad argument";
-    return YART_ERR_INVALID;
-  }
-  if (record && (flags & ~(uint32_t)(YART_FLAG_DEVICE_PTRS | YART_FLAG_COUNT_VISITS))) {
-    ctx->err = std::string(fn) + ": the only flags it takes are YART_FLAG_DEVICE_PTRS and YART_FLAG_COUNT_VISITS";
-    return YART_ERR_INVALID;
-  }
-  const uintptr_t ray_align = f32 ? 7u : 15u, hit_align = f32 ? 3u : 7u;
-  if ((flags & YART_FLAG_DEVICE_PTRS) && ((reinterpret_cast<uintptr_t>(rays) & ray_align) || (reinterpret_cast<uintptr_t>(hits) & hit_align))) {
-    ctx->err = std::string(fn) + (f32 ? ": device ray arrays must be 8-byte aligned (hits: 4)" : ": device ray arrays must be 16-byte aligned (hits: 8)");
-    return YART_ERR_INVALID;
-  }
-  if ((flags & YART_FLAG_DEVICE_PTRS) && (reinterpret_cast<uintptr_t>(times) & 7u)) {
-    ctx->err = std::string(fn) + ": device time arrays must be 8-byte aligned";
-    return YART_ERR_INVALID;
-  }
-  if (target != YART_TARGET_WORLD && target >= ctx->n_meshes) {
-    ctx->err = std::string(fn) + ": target is neither a mesh index nor YART_TARGET_WORLD";
-    return YART_ERR_INVALID;
-  }
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (stats) memset(stats, 0, sizeof(*stats));
-  if (n == 0) return YART_OK;
-  const size_t ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray);
+  const uint32_t allowed_flags = record ? (uint32_t)(YART_FLAG_DEVICE_PTRS | YART_FLAG_COUNT_VISITS) : ~0u;
   const size_t hit_bytes = f32 ? sizeof(yart_hit_f32) : (record ? sizeof(yart_hit_record) : sizeof(yart_hit));
-  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
+  BatchQuery s;
+  if (int rc = begin_query(ctx, fn, target, f32, rays, times, hits, hit_bytes, f32 ? 3u : 7u, ctx->hits_export, n,
+                           order > YART_ORDER_NEAR, flags, allowed_flags,
+                           ": the only flags it takes are YART_FLAG_DEVICE_PTRS and YART_FLAG_COUNT_VISITS", stats, s))
+    return rc;
+  if (n == 0) return YART_OK;
   const bool count = (flags & YART_FLAG_COUNT_VISITS) != 0;
-  const char* d_rays = static_cast<const char*>(rays);
-  char* d_hits = static_cast<char*>(hits);
-  const double* d_times = times;
-  if (!dev) {
-    CUDA_TRY(ctx, ctx->rays.reserve(n * ray_bytes));
-    CUDA_TRY(ctx, ctx->hits_export.reserve(n * hit_bytes));
-    d_rays = ctx->rays.as<char>();
-    d_hits = ctx->hits_export.as<char>();
-    if (times) {
-      CUDA_TRY(ctx, ctx->ray_times.reserve(n * sizeof(double)));
-      d_times = ctx->ray_times.as<double>();
-    }
-  }
-  const uint32_t n_list = (target == YART_TARGET_WORLD) ? ctx->scene.n_objects : 1u;
-  const size_t work_bytes = ((size_t)n_list + 2) * sizeof(uint32_t);
-  CUDA_TRY(ctx, ctx->work.reserve(work_bytes));
   CUDA_TRY(ctx, ctx->counters.reserve(64));
   CUDA_TRY(ctx, ctx->hits.reserve(n * sizeof(DevHit)));
   CUDA_TRY(ctx, cudaMemsetAsync(ctx->counters.p, 0, 64, ctx->stream));
 
-  yart_object solo;
-  memset(&solo, 0, sizeof(solo));
-  solo.kind = YART_OBJ_MESH;
-  solo.cos_theta = 1.0;
   QueryArgs q;
   memset(&q, 0, sizeof(q));
   q.c.t_min = t_min;
   q.c.t_max = t_max;
+  q.objects = s.objects;
   DevScene export_scene = ctx->scene;
-  if (target == YART_TARGET_WORLD) {
-    q.d_objects = ctx->scene.objects;
-    q.h_objects = ctx->h_objects.data();
-    q.n_objects = ctx->scene.n_objects;
-  } else {
-    solo.index = target;
-    q.d_objects = ctx->d_solo + target;
-    q.h_objects = &solo;
-    q.n_objects = 1;
-    export_scene.objects = ctx->d_solo + target;
-  }
+  export_scene.objects = s.objects.d;
   q.seed = 0;
   q.bounce = 1;
   q.spp_batch = 1; // media inside world.hit: Philox stream of pixel = ray index, sample 0, bounce 1
@@ -1265,54 +1412,39 @@ static int closest_hit_impl(yart_ctx* ctx, uint32_t target, const void* rays, co
   q.counters = ctx->counters.as<unsigned long long>();
   q.near = order == YART_ORDER_NEAR;
   q.count = count;
-  uint64_t launches = 0;
   // The passes + the export over rays [off, off + len), on the context's stream.
   auto run_range = [&](uint64_t off, uint64_t len) -> int {
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, work_bytes, ctx->stream));
-    const char* r = d_rays + off * ray_bytes;
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, s.work_bytes, ctx->stream));
+    const char* r = s.d_rays + off * s.ray_bytes;
     q.c.rays = f32 ? nullptr : reinterpret_cast<const yart_ray*>(r);
     q.c.rays32 = f32 ? reinterpret_cast<const yart_ray_f32*>(r) : nullptr;
     q.c.n_items = len;
     q.c.n_rays = (uint32_t)len;
     q.c.hits = ctx->hits.as<DevHit>() + off;
     q.pixel_base = (uint32_t)off; // (keeps a ray's Philox stream = its index in the caller's array)
-    q.ray_time = d_times ? d_times + off : nullptr;
-    const int rc = run_passes(ctx, q, &launches);
+    q.ray_time = s.d_times ? s.d_times + off : nullptr;
+    const int rc = run_passes(ctx, q, &s.launches);
     if (rc) return rc;
+    char* out = s.d_out + off * hit_bytes;
     if (f32)
       k_export_f32<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, export_scene.objects, q.c.hits,
-                                                               reinterpret_cast<yart_hit_f32*>(d_hits + off * hit_bytes), len);
+                                                               reinterpret_cast<yart_hit_f32*>(out), len);
     else if (record)
       k_export_record<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, q.c.rays, q.ray_time, q.c.hits,
-                                                                  reinterpret_cast<yart_hit_record*>(d_hits + off * hit_bytes), len,
+                                                                  reinterpret_cast<yart_hit_record*>(out), len,
                                                                   target != YART_TARGET_WORLD ? 1u : 0u);
     else
-      k_export<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, q.c.rays, q.c.hits,
-                                                           reinterpret_cast<yart_hit*>(d_hits + off * hit_bytes), len);
-    launches++;
+      k_export<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(export_scene, q.c.rays, q.c.hits, reinterpret_cast<yart_hit*>(out), len);
+    s.launches++;
     CUDA_TRY(ctx, cudaGetLastError());
     return YART_OK;
   };
-  uint64_t n_chunks = 0;
-  const int rc = run_chunked(ctx, dev, rays, ray_bytes, hits, hit_bytes, n, d_rays, d_hits, run_range, &n_chunks, times,
-                             sizeof(double), ctx->ray_times.as<char>());
-  if (rc) return rc;
+  if (int rc = run_chunked(ctx, s.dev, rays, s.ray_bytes, hits, hit_bytes, n, s.d_rays, s.d_out, run_range, &s.n_chunks,
+                           times, sizeof(double), ctx->ray_times.as<char>()))
+    return rc;
   unsigned long long c[2] = {0, 0};
   if (count) CUDA_TRY(ctx, cudaMemcpyAsync(c, ctx->counters.p, sizeof(c), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  if (stats) {
-    float ms = 0.f;
-    const int erc = chunked_kernel_ms(ctx, n_chunks, dev, &ms);
-    if (erc) return erc;
-    stats->rays = n;
-    stats->node_visits = c[0];
-    stats->tri_tests = c[1];
-    stats->kernel_launches = launches;
-    stats->trace_launches = (uint32_t)(launches - (dev ? 1 : n_chunks)); // (one export kernel per chunk)
-    stats->gpu_ms = ms;
-    stats->trace_ms = ms;
-  }
-  return YART_OK;
+  return finish_query(ctx, s, s.launches - (s.dev ? 1 : s.n_chunks), c, stats); // (one export kernel per chunk)
 }
 
 int yart_closest_hit(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint64_t n, double t_min, double t_max,
@@ -1342,90 +1474,34 @@ int yart_closest_hit_records(yart_ctx* ctx, uint32_t target, const yart_ray* ray
 static int occluded_impl(yart_ctx* ctx, uint32_t target, const void* rays, bool f32, uint64_t n, double t_min, double t_max,
                          uint32_t flags, uint8_t* occluded, yart_stats* stats) {
   const char* fn = f32 ? "yart_occluded_f32" : "yart_occluded";
-  if (!ctx->have_scene) {
-    ctx->err = std::string(fn) + ": no scene (call yart_ctx_set_scene first)";
-    return YART_ERR_INVALID;
-  }
-  if ((n && (!rays || !occluded)) || n > 0xFFFFFFF0ull) {
-    ctx->err = std::string(fn) + ": bad argument";
-    return YART_ERR_INVALID;
-  }
-  if (flags & ~(uint32_t)YART_FLAG_DEVICE_PTRS) {
-    ctx->err = std::string(fn) + ": the only flag it takes is YART_FLAG_DEVICE_PTRS";
-    return YART_ERR_INVALID;
-  }
-  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
-  if (dev && (reinterpret_cast<uintptr_t>(rays) & (f32 ? 7u : 15u))) {
-    ctx->err = std::string(fn) + (f32 ? ": device ray arrays must be 8-byte aligned" : ": device ray arrays must be 16-byte aligned");
-    return YART_ERR_INVALID;
-  }
-  if (target != YART_TARGET_WORLD && target >= ctx->n_meshes) {
-    ctx->err = std::string(fn) + ": target is neither a mesh index nor YART_TARGET_WORLD";
-    return YART_ERR_INVALID;
-  }
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  if (stats) memset(stats, 0, sizeof(*stats));
+  BatchQuery s; // (no export pass: the kernels write the flags straight into the staging buffer that is downloaded)
+  if (int rc = begin_query(ctx, fn, target, f32, rays, nullptr, occluded, 1, 0, ctx->occluded, n, false, flags,
+                           YART_FLAG_DEVICE_PTRS, ": the only flag it takes is YART_FLAG_DEVICE_PTRS", stats, s))
+    return rc;
   if (n == 0) return YART_OK;
-  const size_t ray_bytes = f32 ? sizeof(yart_ray_f32) : sizeof(yart_ray);
-  const char* d_rays = static_cast<const char*>(rays);
-  char* d_out = reinterpret_cast<char*>(occluded);
-  if (!dev) { // (no export pass: the kernels write the flags straight into the staging buffer that is downloaded)
-    CUDA_TRY(ctx, ctx->rays.reserve(n * ray_bytes));
-    CUDA_TRY(ctx, ctx->occluded.reserve(n));
-    d_rays = ctx->rays.as<char>();
-    d_out = ctx->occluded.as<char>();
-  }
-  const uint32_t n_list = (target == YART_TARGET_WORLD) ? ctx->scene.n_objects : 1u;
-  const size_t work_bytes = ((size_t)n_list + 2) * sizeof(uint32_t);
-  CUDA_TRY(ctx, ctx->work.reserve(work_bytes));
 
-  yart_object solo;
-  memset(&solo, 0, sizeof(solo));
-  solo.kind = YART_OBJ_MESH;
-  solo.cos_theta = 1.0;
   OcclusionArgs q;
   memset(&q, 0, sizeof(q));
   q.c.t_min = t_min;
   q.c.t_max = t_max;
-  if (target == YART_TARGET_WORLD) {
-    q.d_objects = ctx->scene.objects;
-    q.h_objects = ctx->h_objects.data();
-    q.n_objects = ctx->scene.n_objects;
-  } else {
-    solo.index = target;
-    q.d_objects = ctx->d_solo + target;
-    q.h_objects = &solo;
-    q.n_objects = 1;
-  }
+  q.objects = s.objects;
   q.work_counters = ctx->work.as<uint32_t>();
-  uint64_t launches = 0;
   // the passes over rays [off, off + len), on the context's stream
   auto run_range = [&](uint64_t off, uint64_t len) -> int {
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, work_bytes, ctx->stream));
-    CUDA_TRY(ctx, cudaMemsetAsync(d_out + off, 0, len, ctx->stream));
-    const char* r = d_rays + off * ray_bytes;
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, s.work_bytes, ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(s.d_out + off, 0, len, ctx->stream));
+    const char* r = s.d_rays + off * s.ray_bytes;
     q.c.rays = f32 ? nullptr : reinterpret_cast<const yart_ray*>(r);
     q.c.rays32 = f32 ? reinterpret_cast<const yart_ray_f32*>(r) : nullptr;
-    q.c.occluded = reinterpret_cast<uint8_t*>(d_out + off);
+    q.c.occluded = reinterpret_cast<uint8_t*>(s.d_out + off);
     q.c.n_rays = (uint32_t)len;
     q.pixel_base = (uint32_t)off; // (keeps a ray's Philox stream = its index in the caller's array)
-    return run_occlusion_passes(ctx, q, &launches);
+    return run_occlusion_passes(ctx, q, &s.launches);
   };
-  uint64_t n_chunks = 0;
-  const int rc = run_chunked(ctx, dev, rays, ray_bytes, occluded, 1, n, d_rays, d_out, run_range, &n_chunks);
-  if (rc) return rc;
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  if (stats) {
-    float ms = 0.f;
-    const int erc = chunked_kernel_ms(ctx, n_chunks, dev, &ms);
-    if (erc) return erc;
-    stats->rays = n;
-    stats->kernel_launches = launches;
-    stats->trace_launches = (uint32_t)launches;
-    stats->gpu_ms = ms;
-    stats->trace_ms = ms;
-  }
-  return YART_OK;
+  if (int rc = run_chunked(ctx, s.dev, rays, s.ray_bytes, occluded, 1, n, s.d_rays, s.d_out, run_range, &s.n_chunks))
+    return rc;
+  const unsigned long long no_visits[2] = {0, 0};
+  return finish_query(ctx, s, s.launches, no_visits, stats);
 }
 
 int yart_occluded(yart_ctx* ctx, uint32_t target, const yart_ray* rays, uint64_t n, double t_min, double t_max,
@@ -1462,12 +1538,10 @@ static int fill_render_params(yart_ctx* ctx, const yart_camera* cam, const yart_
   {
     // A trailing run of plain spheres that directly follows a mesh pass is intersected inside k_shade (which
     // reads the ray and the hit anyway) -- saves one read-modify-write pass over the queue per bounce.
-    static const int fold = tune_env("YART_TUNE_FOLD_TAIL", 1);
     const uint32_t n_obj = ctx->scene.n_objects;
     uint32_t tb = n_obj;
     while (tb > 0 && ctx->h_objects[tb - 1].kind == YART_OBJ_SPHERE && ctx->h_objects[tb - 1].wrap == 0) tb--;
-    const bool after_mesh = tb > 0 && ctx->h_objects[tb - 1].kind == YART_OBJ_MESH && !(ctx->h_objects[tb - 1].wrap & YART_WRAP_MEDIUM);
-    if (!fold || !after_mesh || n_obj - tb > 16) tb = n_obj;
+    if (tb == 0 || !is_mesh_pass(ctx->h_objects[tb - 1]) || n_obj - tb > 16) tb = n_obj;
     R.tail_begin = tb;
     R.tail_end = n_obj;
   }
@@ -1522,8 +1596,8 @@ int yart_dump_path_rays(yart_ctx* ctx, const yart_camera* cam, const yart_render
 
 // The batch shape of a sample loop over o's samples (yart_render, yart_render_aovs): whole frame x *spp_batch, or
 // pixel chunks of *pix_chunk when the frame alone is too large; the path state of pix_chunk * spp_batch paths (ray,
-// time, wavelength, throughput, hit, two queues) is reserved.  staging_bytes: device memory the call needs besides
-// (the host films' device copies).
+// time, wavelength, throughput, hit, two queues, and with nee YART_FLAG_NEXT_EVENT's) is reserved.  staging_bytes:
+// device memory the call needs besides (the host films' device copies).
 // Big batches: every batch pays ~12 ms of fixed cost (the nearly empty tail bounces run at the latency of
 // their longest ray), so put up to 256 Mi paths in flight -- 112 B of state each (48 ray + 8 time + 8 wavelength
 // + 8 throughput + 32 hit + 2 x 4 queue) = 30 GB of the 180 GB: david 1080p at 32 / 64 / 128 spp per batch
@@ -1536,19 +1610,16 @@ static int size_path_batches(yart_ctx* ctx, const yart_render_opts* o, bool nee,
   static const int max_paths_log2 = std::max(10, std::min(30, tune_env("YART_TUNE_MAX_PATHS_LOG2", 28)));
   uint64_t kMaxPaths = 1ull << max_paths_log2;
   {
-    // YART_FLAG_NEXT_EVENT adds 76 B: 48 shadow ray + 8 pending + 8 light-sample sum + 8 emission weight + 4 shadow queue
-    // (the shadow passes write their hits into the path hits, which are dead from k_shade to the next bounce's passes)
-    const uint64_t kNeeBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(uint32_t);
     const uint64_t kStateBytesPerPath = sizeof(yart_ray) + 3 * sizeof(double) + sizeof(DevHit) + 2 * sizeof(uint32_t) +
-                                        (nee ? kNeeBytesPerPath : 0);
+                                        (nee ? std::accumulate(std::begin(kNeeBytes), std::end(kNeeBytes), size_t(0)) : 0);
     if (!nee) // a flag-off render does not keep an earlier NEE render's state alive (no-op when there is none)
-      for (DevBuf* b : {&ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s}) b->release();
+      for (DevBuf& b : ctx->nee) b.release();
     size_t free_b = 0, total_b = 0;
     CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
-    const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b,
-                            &ctx->nee_rays, &ctx->nee_pending, &ctx->nee_sum, &ctx->nee_w, &ctx->queue_s};
+    const DevBuf* held[] = {&ctx->rays, &ctx->time, &ctx->wavelength, &ctx->throughput, &ctx->hits, &ctx->queue_a, &ctx->queue_b};
     uint64_t avail = free_b; // what the state buffers may grow into: free memory + what they already hold
     for (const DevBuf* b : held) avail += b->cap;
+    for (const DevBuf& b : ctx->nee) avail += b.cap;
     const uint64_t margin = (256ull << 20) + staging_bytes;
     const uint64_t fit = avail > margin ? (avail - margin) / kStateBytesPerPath : 0;
     kMaxPaths = std::min<uint64_t>(kMaxPaths, fit);
@@ -1573,6 +1644,8 @@ static int size_path_batches(yart_ctx* ctx, const yart_render_opts* o, bool nee,
   CUDA_TRY(ctx, ctx->hits.reserve(cap * sizeof(DevHit)));
   CUDA_TRY(ctx, ctx->queue_a.reserve(cap * sizeof(uint32_t)));
   CUDA_TRY(ctx, ctx->queue_b.reserve(cap * sizeof(uint32_t)));
+  if (nee)
+    for (int k = 0; k < 5; ++k) CUDA_TRY(ctx, ctx->nee[k].reserve(cap * kNeeBytes[k]));
   *spp_batch_out = spp_batch;
   *pix_chunk_out = pix_chunk;
   return YART_OK;
@@ -1604,14 +1677,11 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
     if (dumping) CUDA_TRY(ctx, cudaMemsetAsync(d_film, 0, film_bytes, ctx->stream));
     else CUDA_TRY(ctx, cudaMemcpyAsync(d_film, film_xyz, film_bytes, cudaMemcpyHostToDevice, ctx->stream));
   }
-  uint64_t total_rays = 0, total_paths = 0, launches = 0, trace_launches = 0;
-  double trace_ms = 0.0;
-  uint32_t deepest = 0;
+  RenderTotals t;
   if (n_samples > 0) {
     const bool nee = (R.flags & YART_FLAG_NEXT_EVENT) != 0;
     uint32_t spp_batch = 0, pix_chunk = 0;
     if ((rc = size_path_batches(ctx, o, nee, dev ? 0 : film_bytes, &spp_batch, &pix_chunk)) != YART_OK) return rc;
-    const uint64_t cap = (uint64_t)pix_chunk * spp_batch;
     const uint32_t D = o->max_depth;
     // with NEE: path counts [0, D+2), then the shadow queue's count of bounce b at D+2+b; path work counters, then the
     // shadow passes' ones
@@ -1620,177 +1690,104 @@ static int render_impl(yart_ctx* ctx, const yart_camera* cam, const yart_render_
     const size_t n_work = n_obj_slots * D * (nee ? 2 : 1);
     CUDA_TRY(ctx, ctx->counts.reserve(n_counts * sizeof(uint32_t)));
     CUDA_TRY(ctx, ctx->work.reserve(n_work * sizeof(uint32_t)));
+    uint32_t* counts = ctx->counts.as<uint32_t>();
+    uint32_t* work = ctx->work.as<uint32_t>();
     NeeState N;
     memset(&N, 0, sizeof(N));
     if (nee) {
-      CUDA_TRY(ctx, ctx->nee_rays.reserve(cap * sizeof(yart_ray)));
-      CUDA_TRY(ctx, ctx->nee_pending.reserve(cap * sizeof(double)));
-      CUDA_TRY(ctx, ctx->nee_sum.reserve(cap * sizeof(double)));
-      CUDA_TRY(ctx, ctx->nee_w.reserve(cap * sizeof(double)));
-      CUDA_TRY(ctx, ctx->queue_s.reserve(cap * sizeof(uint32_t)));
-      N.rays = ctx->nee_rays.as<yart_ray>();
-      N.pending = ctx->nee_pending.as<double>();
-      N.sum = ctx->nee_sum.as<double>();
-      N.w_emit = ctx->nee_w.as<double>();
-      N.queue = ctx->queue_s.as<uint32_t>();
-      N.counts = ctx->counts.as<uint32_t>() + D + 2;
+      N.rays = ctx->nee[0].as<yart_ray>();
+      N.pending = ctx->nee[1].as<double>();
+      N.sum = ctx->nee[2].as<double>();
+      N.w_emit = ctx->nee[3].as<double>();
+      N.queue = ctx->nee[4].as<uint32_t>();
+      N.counts = counts + D + 2;
     }
     // events: [0, 2D) closest-hit passes per bounce, [2D, 4D) YART_DEBUG_BOUNCES's shade timing, [4D, 6D) shadow passes
-    while (ctx->ev_pool.size() < (nee ? 6 : 2) * (size_t)D) {
-      cudaEvent_t e;
-      CUDA_TRY(ctx, cudaEventCreate(&e));
-      ctx->ev_pool.push_back(e);
-    }
-    R.st.rays = ctx->rays.as<yart_ray>();
-    R.st.time = ctx->time.as<double>();
-    R.st.wavelength = ctx->wavelength.as<double>();
-    R.st.throughput = ctx->throughput.as<double>();
-    R.st.hits = ctx->hits.as<DevHit>();
-    uint32_t* counts = ctx->counts.as<uint32_t>();
-    uint32_t* work = ctx->work.as<uint32_t>();
+    static const int debug_bounces = tune_env("YART_DEBUG_BOUNCES", 0);
+    CUDA_TRY(ctx, ensure_events(ctx->ev_pool, (nee ? 6 : debug_bounces ? 4 : 2) * (size_t)D));
     std::vector<uint32_t> h_counts(n_counts);
-    const bool near = o->order == YART_ORDER_NEAR;
-    const bool count = (o->flags & YART_FLAG_COUNT_VISITS) != 0;
     const int stream_grid = ctx->sm_count * 8;
-    CUDA_TRY(ctx, ctx->counters.reserve(64));
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->counters.p, 0, 64, ctx->stream));
 
-    for (uint32_t s0 = o->sample_begin; s0 < o->sample_end; s0 += spp_batch) {
-      const uint32_t spp = std::min(spp_batch, o->sample_end - s0);
-      for (uint32_t p0 = 0; p0 < n_pixels_total; p0 += pix_chunk) {
-        R.pixel_base = p0;
-        R.n_pixels = std::min(pix_chunk, n_pixels_total - p0);
-        R.sample_base = s0;
-        R.spp_batch = spp;
-        CUDA_TRY(ctx, cudaMemsetAsync(counts, 0, n_counts * sizeof(uint32_t), ctx->stream));
-        CUDA_TRY(ctx, cudaMemsetAsync(work, 0, n_work * sizeof(uint32_t), ctx->stream));
-        uint32_t* qa = ctx->queue_a.as<uint32_t>();
-        uint32_t* qb = ctx->queue_b.as<uint32_t>();
-        if (nee) k_raygen<true><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
-        else k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
-        launches++;
-        uint32_t b_done = 0;
-        for (uint32_t b = 1; b <= D; ++b) {
-          QueryArgs q;
-          memset(&q, 0, sizeof(q));
-          q.c.rays = R.st.rays;
-          q.c.queue = qa;
-          q.c.n_items_dev = counts + b;
-          q.c.n_rays = R.n_pixels * spp;
-          q.c.hits = R.st.hits;
-          q.c.t_min = 0.001; // world.hit(ray_in, 0.001, f64::INFINITY) (main.rs:548)
-          q.c.t_max = INFINITY;
-          q.d_objects = ctx->scene.objects;
-          q.h_objects = ctx->h_objects.data();
-          q.n_objects = R.tail_begin; // (== n_objects unless k_shade takes a trailing run of spheres)
-          q.ray_time = R.st.time;
-          q.seed = o->seed;
-          q.bounce = b;
-          q.spp_batch = spp;
-          q.sample_base = s0;
-          q.pixel_base = p0;
-          q.work_counters = work + (size_t)(b - 1) * n_obj_slots;
-          q.counters = ctx->counters.as<unsigned long long>();
-          q.near = near;
-          q.count = count;
-          if (dump_out) {
-            k_dump_rays<<<stream_grid, 256, 0, ctx->stream>>>(R.st.rays, qa, counts, b, total_rays, dump_out, dump_cap);
-            launches++;
-          }
-          CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * (b - 1)], ctx->stream));
-          rc = run_passes(ctx, q, &trace_launches);
-          if (rc) return rc;
-          CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * (b - 1) + 1], ctx->stream));
-          static const int dbg_shade_ev = tune_env("YART_DEBUG_BOUNCES", 0);
-          if (dbg_shade_ev) {
-            while (ctx->ev_pool.size() < 4 * (size_t)D) {
-              cudaEvent_t e;
-              CUDA_TRY(ctx, cudaEventCreate(&e));
-              ctx->ev_pool.push_back(e);
-            }
-            CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->stream));
-          }
-          const int shade_grid = std::max(1, stream_grid * 256 / kShadeThreads);
-          if (nee) k_shade<true><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
-          else k_shade<false><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
-          launches += 1;
-          if (dbg_shade_ev) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1) + 1], ctx->stream));
-          if (nee && b < D) { // the shadow rays k_shade queued: the same world query, on their own queue and Philox stream
-            QueryArgs sq = q;
-            sq.c.rays = N.rays;
-            sq.c.queue = N.queue;
-            sq.c.n_items_dev = N.counts + b;
-            sq.bounce = YART_NEE_BOUNCE_BASE + b;
-            sq.work_counters = work + (size_t)(D + b - 1) * n_obj_slots;
-            CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->stream));
-            rc = run_passes(ctx, sq, &trace_launches);
-            if (rc) return rc;
-            CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1) + 1], ctx->stream));
-            k_nee_resolve<<<stream_grid, 256, 0, ctx->stream>>>(R, b, N);
-            launches += 1;
-          }
-          std::swap(qa, qb);
-          b_done = b;
-          // the tail of the bounce loop is nearly empty: look at the live count now and then
-          if (b >= 4 && (b % 4) == 0 && b < D) {
-            uint32_t live = 0;
-            CUDA_TRY(ctx, cudaMemcpyAsync(&live, counts + b + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-            CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-            if (live == 0) break;
-          }
+    rc = for_each_batch(ctx, o, spp_batch, pix_chunk, n_counts, n_work, R, [&]() -> int {
+      uint32_t* qa = ctx->queue_a.as<uint32_t>();
+      uint32_t* qb = ctx->queue_b.as<uint32_t>();
+      if (nee) k_raygen<true><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
+      else k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, qa, counts + 1, N);
+      t.launches++;
+      uint32_t b_done = 0;
+      for (uint32_t b = 1; b <= D; ++b) {
+        // (R.tail_begin == n_objects unless k_shade takes a trailing run of spheres)
+        const QueryArgs q = bounce_query(ctx, o, R, qa, counts + b, b, R.tail_begin, work + (size_t)(b - 1) * n_obj_slots);
+        if (dump_out) {
+          k_dump_rays<<<stream_grid, 256, 0, ctx->stream>>>(R.st.rays, qa, counts, b, t.rays, dump_out, dump_cap);
+          t.launches++;
         }
-        if (nee) k_film_accumulate<true><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
-        else k_film_accumulate<false><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
-        launches++;
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaMemcpyAsync(h_counts.data(), counts, n_counts * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-        total_paths += h_counts[1];
-        static const int debug_bounces = tune_env("YART_DEBUG_BOUNCES", 0);
-        for (uint32_t b = 1; b <= b_done; ++b) {
-          total_rays += h_counts[b];
-          if (h_counts[b]) deepest = std::max(deepest, b);
-          float ms = 0.f;
-          CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[2 * (b - 1)], ctx->ev_pool[2 * (b - 1) + 1]));
-          trace_ms += ms;
-          if (nee && b < D) {
-            float shadow_ms = 0.f;
-            CUDA_TRY(ctx, cudaEventElapsedTime(&shadow_ms, ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->ev_pool[4 * D + 2 * (b - 1) + 1]));
-            trace_ms += shadow_ms;
-          }
-          if (debug_bounces) {
-            float gap = 0.f; // from the end of this bounce's closest-hit stage to the start of the next one
-            if (b < b_done) cudaEventElapsedTime(&gap, ctx->ev_pool[2 * (b - 1) + 1], ctx->ev_pool[2 * b]);
-            float shade = 0.f;
-            cudaEventElapsedTime(&shade, ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->ev_pool[2 * D + 2 * (b - 1) + 1]);
-            fprintf(stderr, "bounce %2u: rays %9u  closest-hit %8.3f ms  shade %8.3f ms  shade+gap %8.3f ms", b, h_counts[b], ms, shade, gap);
-            if (nee) fprintf(stderr, "  shadow rays %9u", b < D ? h_counts[D + 2 + b] : 0u);
-            fprintf(stderr, "\n");
-          }
+        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * (b - 1)], ctx->stream));
+        if (int prc = run_passes(ctx, q, &t.trace_launches)) return prc;
+        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * (b - 1) + 1], ctx->stream));
+        if (debug_bounces) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->stream));
+        const int shade_grid = std::max(1, stream_grid * 256 / kShadeThreads);
+        if (nee) k_shade<true><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
+        else k_shade<false><<<shade_grid, kShadeThreads, 0, ctx->stream>>>(R, qa, counts + b, qb, counts + b + 1, b, N);
+        t.launches += 1;
+        if (debug_bounces) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[2 * D + 2 * (b - 1) + 1], ctx->stream));
+        if (nee && b < D) { // the shadow rays k_shade queued: the same world query, on their own queue and Philox stream
+          QueryArgs sq = q;
+          sq.c.rays = N.rays;
+          sq.c.queue = N.queue;
+          sq.c.n_items_dev = N.counts + b;
+          sq.bounce = YART_NEE_BOUNCE_BASE + b;
+          sq.work_counters = work + (size_t)(D + b - 1) * n_obj_slots;
+          CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->stream));
+          if (int prc = run_passes(ctx, sq, &t.trace_launches)) return prc;
+          CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[4 * D + 2 * (b - 1) + 1], ctx->stream));
+          k_nee_resolve<<<stream_grid, 256, 0, ctx->stream>>>(R, b, N);
+          t.launches += 1;
+        }
+        std::swap(qa, qb);
+        b_done = b;
+        // the tail of the bounce loop is nearly empty: look at the live count now and then
+        if (b >= 4 && (b % 4) == 0 && b < D) {
+          uint32_t live = 0;
+          CUDA_TRY(ctx, cudaMemcpyAsync(&live, counts + b + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+          CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+          if (live == 0) break;
         }
       }
-    }
+      if (nee) k_film_accumulate<true><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
+      else k_film_accumulate<false><<<stream_grid, 256, 0, ctx->stream>>>(R, d_film, N);
+      t.launches++;
+      CUDA_TRY(ctx, cudaGetLastError());
+      CUDA_TRY(ctx, cudaMemcpyAsync(h_counts.data(), counts, n_counts * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+      CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+      t.paths += h_counts[1];
+      for (uint32_t b = 1; b <= b_done; ++b) {
+        t.rays += h_counts[b];
+        if (h_counts[b]) t.deepest = std::max(t.deepest, b);
+        float ms = 0.f;
+        CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[2 * (b - 1)], ctx->ev_pool[2 * (b - 1) + 1]));
+        t.trace_ms += ms;
+        if (nee && b < D) {
+          float shadow_ms = 0.f;
+          CUDA_TRY(ctx, cudaEventElapsedTime(&shadow_ms, ctx->ev_pool[4 * D + 2 * (b - 1)], ctx->ev_pool[4 * D + 2 * (b - 1) + 1]));
+          t.trace_ms += shadow_ms;
+        }
+        if (debug_bounces) {
+          float gap = 0.f; // from the end of this bounce's closest-hit stage to the start of the next one
+          if (b < b_done) cudaEventElapsedTime(&gap, ctx->ev_pool[2 * (b - 1) + 1], ctx->ev_pool[2 * b]);
+          float shade = 0.f;
+          cudaEventElapsedTime(&shade, ctx->ev_pool[2 * D + 2 * (b - 1)], ctx->ev_pool[2 * D + 2 * (b - 1) + 1]);
+          fprintf(stderr, "bounce %2u: rays %9u  closest-hit %8.3f ms  shade %8.3f ms  shade+gap %8.3f ms", b, h_counts[b], ms, shade, gap);
+          if (nee) fprintf(stderr, "  shadow rays %9u", b < D ? h_counts[D + 2 + b] : 0u);
+          fprintf(stderr, "\n");
+        }
+      }
+      return YART_OK;
+    });
+    if (rc) return rc;
   }
   if (!dev && !dumping) CUDA_TRY(ctx, cudaMemcpyAsync(film_xyz, d_film, film_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  unsigned long long visit[2] = {0, 0};
-  if ((o->flags & YART_FLAG_COUNT_VISITS) && n_samples > 0)
-    CUDA_TRY(ctx, cudaMemcpyAsync(visit, ctx->counters.p, sizeof(visit), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  if (stats) {
-    float ms = 0.f;
-    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    stats->node_visits = visit[0];
-    stats->tri_tests = visit[1];
-    stats->rays = total_rays;
-    stats->paths = total_paths;
-    stats->kernel_launches = launches + trace_launches;
-    stats->trace_launches = (uint32_t)trace_launches;
-    stats->gpu_ms = ms;
-    stats->trace_ms = trace_ms;
-    stats->max_bounce = deepest;
-  }
-  return YART_OK;
+  return finish_render(ctx, o, t, stats);
 }
 
 int yart_film_finalize(yart_ctx* ctx, const double* film_xyz, uint32_t width, uint32_t height, uint32_t spp, uint32_t flags,
@@ -1800,23 +1797,7 @@ int yart_film_finalize(yart_ctx* ctx, const double* film_xyz, uint32_t width, ui
     ctx->err = "yart_film_finalize: bad argument";
     return YART_ERR_INVALID;
   }
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  const size_t n = (size_t)width * height;
-  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
-  const double* d_film = film_xyz;
-  uint8_t* d_rgba = rgba8;
-  if (!dev) {
-    CUDA_TRY(ctx, ctx->film.reserve(n * 3 * sizeof(double)));
-    CUDA_TRY(ctx, ctx->rgba.reserve(n * 4));
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->film.p, film_xyz, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    d_film = ctx->film.as<double>();
-    d_rgba = ctx->rgba.as<uint8_t>();
-  }
-  k_film_finalize<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_film, width, height, spp, d_rgba);
-  CUDA_TRY(ctx, cudaGetLastError());
-  if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(rgba8, d_rgba, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  return YART_OK;
+  return film_finalize_impl(ctx, k_film_finalize, 4, film_xyz, width, height, spp, flags, rgba8);
 }
 
 int yart_film_finalize_linear(yart_ctx* ctx, const double* film_xyz, uint32_t width, uint32_t height, uint32_t spp,
@@ -1826,23 +1807,7 @@ int yart_film_finalize_linear(yart_ctx* ctx, const double* film_xyz, uint32_t wi
     ctx->err = "yart_film_finalize_linear: bad argument";
     return YART_ERR_INVALID;
   }
-  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  const size_t n = (size_t)width * height;
-  const bool dev = (flags & YART_FLAG_DEVICE_PTRS) != 0;
-  const double* d_film = film_xyz;
-  float* d_rgb = rgb;
-  if (!dev) {
-    CUDA_TRY(ctx, ctx->film.reserve(n * 3 * sizeof(double)));
-    CUDA_TRY(ctx, ctx->rgba.reserve(n * 3 * sizeof(float)));
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->film.p, film_xyz, n * 3 * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-    d_film = ctx->film.as<double>();
-    d_rgb = ctx->rgba.as<float>();
-  }
-  k_film_finalize_linear<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d_film, width, height, spp, d_rgb);
-  CUDA_TRY(ctx, cudaGetLastError());
-  if (!dev) CUDA_TRY(ctx, cudaMemcpyAsync(rgb, d_rgb, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  return YART_OK;
+  return film_finalize_impl(ctx, k_film_finalize_linear, 3, film_xyz, width, height, spp, flags, rgb);
 }
 
 // k_raygen<false> and the bounce-1 passes of yart_render over all objects, then k_aov_accumulate, batch by batch.
@@ -1882,99 +1847,45 @@ static int render_aovs_impl(yart_ctx* ctx, const yart_camera* cam, const yart_re
     CUDA_TRY(ctx, cudaMemcpyAsync(d_plane[k], user[k], plane_bytes, cudaMemcpyHostToDevice, ctx->stream));
     staging += plane_bytes;
   }
-  uint64_t total_rays = 0, launches = 0, trace_launches = 0;
-  double trace_ms = 0.0;
+  RenderTotals t;
   if (o->sample_end > o->sample_begin) {
     uint32_t spp_batch = 0, pix_chunk = 0;
     if ((rc = size_path_batches(ctx, o, false, staging, &spp_batch, &pix_chunk)) != YART_OK) return rc;
     const size_t n_obj_slots = (size_t)ctx->scene.n_objects + 1;
     CUDA_TRY(ctx, ctx->counts.reserve(2 * sizeof(uint32_t)));
     CUDA_TRY(ctx, ctx->work.reserve(n_obj_slots * sizeof(uint32_t)));
-    CUDA_TRY(ctx, ctx->counters.reserve(64));
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->counters.p, 0, 64, ctx->stream));
-    while (ctx->ev_pool.size() < 2) {
-      cudaEvent_t e;
-      CUDA_TRY(ctx, cudaEventCreate(&e));
-      ctx->ev_pool.push_back(e);
-    }
-    R.st.rays = ctx->rays.as<yart_ray>();
-    R.st.time = ctx->time.as<double>();
-    R.st.wavelength = ctx->wavelength.as<double>();
-    R.st.throughput = ctx->throughput.as<double>();
-    R.st.hits = ctx->hits.as<DevHit>();
+    CUDA_TRY(ctx, ensure_events(ctx->ev_pool, 2));
     uint32_t* counts = ctx->counts.as<uint32_t>();
     NeeState N;
     memset(&N, 0, sizeof(N));
     const int stream_grid = ctx->sm_count * 8;
-    for (uint32_t s0 = o->sample_begin; s0 < o->sample_end; s0 += spp_batch) {
-      const uint32_t spp = std::min(spp_batch, o->sample_end - s0);
-      for (uint32_t p0 = 0; p0 < n_pixels_total; p0 += pix_chunk) {
-        R.pixel_base = p0;
-        R.n_pixels = std::min(pix_chunk, n_pixels_total - p0);
-        R.sample_base = s0;
-        R.spp_batch = spp;
-        CUDA_TRY(ctx, cudaMemsetAsync(counts, 0, 2 * sizeof(uint32_t), ctx->stream));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->work.p, 0, n_obj_slots * sizeof(uint32_t), ctx->stream));
-        k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, ctx->queue_a.as<uint32_t>(), counts + 1, N);
-        QueryArgs q;
-        memset(&q, 0, sizeof(q));
-        q.c.rays = R.st.rays;
-        q.c.queue = ctx->queue_a.as<uint32_t>();
-        q.c.n_items_dev = counts + 1;
-        q.c.n_rays = R.n_pixels * spp;
-        q.c.hits = R.st.hits;
-        q.c.t_min = 0.001; // the render's bounce 1: world.hit(ray, 0.001, f64::INFINITY) (main.rs:548)
-        q.c.t_max = INFINITY;
-        q.d_objects = ctx->scene.objects;
-        q.h_objects = ctx->h_objects.data();
-        q.n_objects = ctx->scene.n_objects; // all of them: there is no k_shade to intersect R.tail_begin..
-        q.ray_time = R.st.time;
-        q.seed = o->seed;
-        q.bounce = 1;
-        q.spp_batch = spp;
-        q.sample_base = s0;
-        q.pixel_base = p0;
-        q.work_counters = ctx->work.as<uint32_t>();
-        q.counters = ctx->counters.as<unsigned long long>();
-        q.near = o->order == YART_ORDER_NEAR;
-        q.count = (o->flags & YART_FLAG_COUNT_VISITS) != 0;
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[0], ctx->stream));
-        if ((rc = run_passes(ctx, q, &trace_launches)) != YART_OK) return rc;
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[1], ctx->stream));
-        k_aov_accumulate<<<stream_grid, 256, 0, ctx->stream>>>(R, d_plane[0], d_plane[1], d_plane[2]);
-        launches += 2;
-        CUDA_TRY(ctx, cudaGetLastError());
-        uint32_t n_rays = 0;
-        CUDA_TRY(ctx, cudaMemcpyAsync(&n_rays, counts + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-        float ms = 0.f;
-        CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[0], ctx->ev_pool[1]));
-        trace_ms += ms;
-        total_rays += n_rays;
-      }
-    }
+    rc = for_each_batch(ctx, o, spp_batch, pix_chunk, 2, n_obj_slots, R, [&]() -> int {
+      uint32_t* queue = ctx->queue_a.as<uint32_t>();
+      k_raygen<false><<<stream_grid, 256, 0, ctx->stream>>>(R, queue, counts + 1, N);
+      // the render's bounce 1 over all objects: there is no k_shade to intersect R.tail_begin..
+      const QueryArgs q = bounce_query(ctx, o, R, queue, counts + 1, 1, ctx->scene.n_objects, ctx->work.as<uint32_t>());
+      CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[0], ctx->stream));
+      if (int prc = run_passes(ctx, q, &t.trace_launches)) return prc;
+      CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[1], ctx->stream));
+      k_aov_accumulate<<<stream_grid, 256, 0, ctx->stream>>>(R, d_plane[0], d_plane[1], d_plane[2]);
+      t.launches += 2;
+      CUDA_TRY(ctx, cudaGetLastError());
+      uint32_t n_rays = 0;
+      CUDA_TRY(ctx, cudaMemcpyAsync(&n_rays, counts + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+      CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+      float ms = 0.f;
+      CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev_pool[0], ctx->ev_pool[1]));
+      t.trace_ms += ms;
+      t.rays += n_rays;
+      return YART_OK;
+    });
+    if (rc) return rc;
   }
   for (int k = 0; k < 3; ++k)
     if (user[k] && !dev) CUDA_TRY(ctx, cudaMemcpyAsync(user[k], d_plane[k], plane_bytes, cudaMemcpyDeviceToHost, ctx->stream));
-  unsigned long long visit[2] = {0, 0};
-  if ((o->flags & YART_FLAG_COUNT_VISITS) && o->sample_end > o->sample_begin)
-    CUDA_TRY(ctx, cudaMemcpyAsync(visit, ctx->counters.p, sizeof(visit), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
-  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  if (stats) {
-    float ms = 0.f;
-    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    stats->node_visits = visit[0];
-    stats->tri_tests = visit[1];
-    stats->rays = total_rays;
-    stats->paths = total_rays;
-    stats->kernel_launches = launches + trace_launches;
-    stats->trace_launches = (uint32_t)trace_launches;
-    stats->gpu_ms = ms;
-    stats->trace_ms = trace_ms;
-    stats->max_bounce = total_rays ? 1u : 0u;
-  }
-  return YART_OK;
+  t.paths = t.rays;
+  t.deepest = t.rays ? 1u : 0u;
+  return finish_render(ctx, o, t, stats);
 }
 
 int yart_render_aovs(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, const yart_aov_planes* planes,
@@ -2033,9 +1944,8 @@ int yart_measure_fetch_peak(yart_ctx* ctx, uint64_t table_bytes, uint32_t fetche
   float ms = 0.f;
   size_t threads = 0;
   if (e == cudaSuccess) {
-    static const int carve = tune_env("YART_TUNE_CARVEOUT_LEAN", 50);
     auto run = [&](auto kernel, int block, bool set_carve) {
-      if (set_carve) cudaFuncSetAttribute(reinterpret_cast<const void*>(kernel), cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+      if (set_carve) cudaFuncSetAttribute(reinterpret_cast<const void*>(kernel), cudaFuncAttributePreferredSharedMemoryCarveout, carveout(true));
       int per_sm = 1;
       cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reinterpret_cast<const void*>(kernel), block, 0);
       const int grid = std::max(per_sm, 1) * ctx->sm_count;
@@ -2055,8 +1965,6 @@ int yart_measure_fetch_peak(yart_ctx* ctx, uint64_t table_bytes, uint32_t fetche
     e = cudaStreamSynchronize(ctx->stream);
     if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
   }
-  table.release();
-  sink.release();
   if (e != cudaSuccess) {
     ctx->err = std::string("yart_measure_fetch_peak: ") + cudaGetErrorString(e);
     return YART_ERR_CUDA;
