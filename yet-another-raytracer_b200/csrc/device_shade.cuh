@@ -116,12 +116,20 @@ YART_DEV void prim_record(const DevScene& S, const yart_object& o, D3 ro, D3 rd,
     need_uv = pm.kind != YART_MAT_NONE && pm.kind != YART_MAT_DIELECTRIC && S.textures[pm.texture].kind == YART_TEX_IMAGE;
   }
   switch (o.kind) {
-    case YART_OBJ_SPHERE: { // sphere.rs:68-85
-      const D3 center = d3(o.p[0], o.p[1], o.p[2]);
-      const double radius = o.p[3];
+    case YART_OBJ_SPHERE: // sphere.rs:68-85
+    case YART_OBJ_MOVING_SPHERE: { // sphere.rs:175-197 (one copy of the shared steps: each `/` inlines a slow path)
+      const bool moving = o.kind == YART_OBJ_MOVING_SPHERE;
+      const D3 center = moving ? moving_center(o, time) : d3(o.p[0], o.p[1], o.p[2]);
+      const double radius = moving ? o.p[8] : o.p[3];
       rec.p = ro + t * rd;
-      D3 outward = vdiv(rec.p - center, fabs(radius));
-      if (radius < 0.0) {
+      D3 outward = vdiv(rec.p - center, moving ? radius : fabs(radius));
+      if (moving) {
+        if (dot(rd, outward) < 0.0) {
+          rec.normal = outward; rec.front_face = true;
+        } else {
+          rec.normal = -outward; rec.front_face = false;
+        }
+      } else if (radius < 0.0) {
         rec.normal = -outward; rec.front_face = dot(rd, outward) > 0.0;
       } else {
         rec.normal = outward; rec.front_face = dot(rd, outward) < 0.0;
@@ -130,26 +138,17 @@ YART_DEV void prim_record(const DevScene& S, const yart_object& o, D3 ro, D3 rd,
       if (need_uv) get_sphere_uv(outward, rec.u, rec.v);
       break;
     }
-    case YART_OBJ_MOVING_SPHERE: { // sphere.rs:175-197
-      const D3 center = moving_center(o, time);
-      rec.p = ro + t * rd;
-      D3 outward = vdiv(rec.p - center, o.p[8]);
-      if (dot(rd, outward) < 0.0) {
-        rec.normal = outward; rec.front_face = true;
-      } else {
-        rec.normal = -outward; rec.front_face = false;
-      }
-      rec.u = rec.v = 0.0;
-      if (need_uv) get_sphere_uv(outward, rec.u, rec.v);
-      break;
-    }
     case YART_OBJ_XY_RECT:
     case YART_OBJ_XZ_RECT:
-    case YART_OBJ_YZ_RECT: rect_record(rect_axis(o.kind), o.p[0], o.p[1], o.p[2], o.p[3], ro, rd, t, rec); break;
+    case YART_OBJ_YZ_RECT:
     case YART_OBJ_BOX: {
       int axis;
       double a0, a1, b0, b1, k;
-      box_side(o.p, (int)(prim & 7u), axis, a0, a1, b0, b1, k);
+      if (o.kind == YART_OBJ_BOX) {
+        box_side(o.p, (int)(prim & 7u), axis, a0, a1, b0, b1, k);
+      } else {
+        axis = rect_axis(o.kind); a0 = o.p[0]; a1 = o.p[1]; b0 = o.p[2]; b1 = o.p[3];
+      }
       rect_record(axis, a0, a1, b0, b1, ro, rd, t, rec);
       break;
     }
@@ -208,12 +207,9 @@ YART_DEV void world_record(const DevScene& S, const DevHit& h, D3 wo, D3 wd, dou
   }
   D3 ro = wo, rd = wd;
   to_object_space(o, ro, rd);
-  if (o.kind == YART_OBJ_GROUP) {
-    const DevGroup g = S.groups[o.index];
-    prim_record<ALL_UV>(S, g.members[h.prim >> 3], ro, rd, time, h.t, h.prim & 7u, h.bu, h.bv, rec);
-  } else {
-    prim_record<ALL_UV>(S, o, ro, rd, time, h.t, h.prim, h.bu, h.bv, rec);
-  }
+  const bool group = o.kind == YART_OBJ_GROUP; // one inlined prim_record for a group member and a plain object
+  const yart_object& po = group ? S.groups[o.index].members[h.prim >> 3] : o;
+  prim_record<ALL_UV>(S, po, ro, rd, time, h.t, group ? (h.prim & 7u) : h.prim, h.bu, h.bv, rec);
   if (o.wrap & YART_WRAP_FLIP_FACE) rec.front_face = !rec.front_face;
   if (o.wrap & YART_WRAP_ROTATE_Y) { // hittable.rs:232-246
     const double ct = o.cos_theta, st = o.sin_theta;
@@ -287,27 +283,24 @@ __device__ __noinline__ double perlin_turb(const yart_perlin& pn, uint32_t type,
   }
   return fabs(accum);
 }
-__device__ __noinline__ double texture_value(const DevScene& S, uint32_t tex, double wl, const HitRec& rec) {
-  const yart_texture& t = S.textures[tex];
+// Noise and image textures, out of line: they take the hit point / uv by value, so that no HitRec goes through
+// local memory on the way here.
+__device__ __noinline__ double texture_value_slow(const DevScene& S, const yart_texture& t, double wl, D3 p, double u,
+                                                  double v) {
   const double white[3] = {1.0, 1.0, 1.0};
   switch (t.kind) {
-    case YART_TEX_SOLID: return rgb_reflect(S, t.rgb_a, wl);
-    case YART_TEX_CHECKER: {
-      double sines = sin(10.0 * rec.p.x) * sin(10.0 * rec.p.y) * sin(10.0 * rec.p.z);
-      return sines < 0.0 ? rgb_reflect(S, t.rgb_a, wl) : rgb_reflect(S, t.rgb_b, wl);
-    }
     case YART_TEX_NOISE: {
       const yart_perlin& pn = S.perlins[t.perlin];
-      if (t.noise_type == YART_NOISE_NET) return rgb_reflect(S, white, wl) * perlin_turb(pn, t.noise_type, rec.p * t.scale, 7);
+      if (t.noise_type == YART_NOISE_NET) return rgb_reflect(S, white, wl) * perlin_turb(pn, t.noise_type, p * t.scale, 7);
       if (t.noise_type == YART_NOISE_MARBLE)
-        return rgb_reflect(S, white, wl) * 0.5 * (1.0 + sin(t.scale * rec.p.z + 10.0 * perlin_turb(pn, t.noise_type, rec.p, 7)));
-      return rgb_reflect(S, white, wl) * 0.5 * (1.0 + perlin_noise(pn, t.noise_type, rec.p * t.scale));
+        return rgb_reflect(S, white, wl) * 0.5 * (1.0 + sin(t.scale * p.z + 10.0 * perlin_turb(pn, t.noise_type, p, 7)));
+      return rgb_reflect(S, white, wl) * 0.5 * (1.0 + perlin_noise(pn, t.noise_type, p * t.scale));
     }
     case YART_TEX_IMAGE: {
       const DevImage im = S.images[t.image];
       if (im.rgb8 == nullptr) return 1.0;
-      double uu = rec.u < 0.0 ? 0.0 : (rec.u > 1.0 ? 1.0 : rec.u);
-      double vc = rec.v < 0.0 ? 0.0 : (rec.v > 1.0 ? 1.0 : rec.v);
+      double uu = u < 0.0 ? 0.0 : (u > 1.0 ? 1.0 : u);
+      double vc = v < 0.0 ? 0.0 : (v > 1.0 ? 1.0 : v);
       double vv = 1.0 - vc;
       uint32_t i = f64_as_u32(uu * (double)im.width);
       uint32_t j = f64_as_u32(vv * (double)im.height);
@@ -320,6 +313,16 @@ __device__ __noinline__ double texture_value(const DevScene& S, uint32_t tex, do
     }
     default: return 0.0;
   }
+}
+// Texture::value at hit point p, (u, v): solid and checker in line, the rest through texture_value_slow
+YART_DEV double texture_value(const DevScene& S, uint32_t tex, double wl, D3 p, double u, double v) {
+  const yart_texture& t = S.textures[tex];
+  if (t.kind == YART_TEX_SOLID) return rgb_reflect(S, t.rgb_a, wl);
+  if (t.kind == YART_TEX_CHECKER) {
+    double sines = sin(10.0 * p.x) * sin(10.0 * p.y) * sin(10.0 * p.z);
+    return sines < 0.0 ? rgb_reflect(S, t.rgb_a, wl) : rgb_reflect(S, t.rgb_b, wl);
+  }
+  return texture_value_slow(S, t, wl, p, u, v);
 }
 
 // The RGB a texture hands to rgb_reflect in texture_value (noise: its scalar times white; an image without texels:
@@ -402,7 +405,10 @@ YART_DEV double light_pdf_value(const yart_object& l, D3 origin, D3 direction) {
   }
   return 0.0;
 }
-YART_DEV D3 light_random(const yart_object& l, D3 origin, double r1, double r2) {
+// HAVE_CS: the caller gives cos / sin of the sphere case's phi = 2 pi r1 (shade_path forms them once for both halves of
+// the mixture pdf, whose lanes would otherwise run the two f64 sin / cos evaluations one after the other).
+template <bool HAVE_CS = false>
+YART_DEV D3 light_random(const yart_object& l, D3 origin, double r1, double r2, double cos_phi = 0.0, double sin_phi = 0.0) {
   if (l.wrap == 0 && l.kind == YART_OBJ_SPHERE) {
     const D3 center = d3(l.p[0], l.p[1], l.p[2]);
     const double radius = l.p[3];
@@ -410,9 +416,13 @@ YART_DEV D3 light_random(const yart_object& l, D3 origin, double r1, double r2) 
     double distance_squared = length_squared(direction);
     Onb uvw = onb_from_w(direction);
     double z = 1.0 + r2 * (sqrt(1.0 - radius * radius / distance_squared) - 1.0);
-    double phi = 2.0 * kPi * r1;
-    double x = cos(phi) * sqrt(1.0 - z * z);
-    double y = sin(phi) * sqrt(1.0 - z * z);
+    if (!HAVE_CS) {
+      const double phi = 2.0 * kPi * r1;
+      cos_phi = cos(phi);
+      sin_phi = sin(phi);
+    }
+    double x = cos_phi * sqrt(1.0 - z * z);
+    double y = sin_phi * sqrt(1.0 - z * z);
     return onb_local(uvw, d3(x, y, z));
   }
   if (l.wrap == 0 && l.kind == YART_OBJ_XZ_RECT) {
@@ -429,14 +439,17 @@ YART_DEV double lights_pdf_value(const DevScene& S, D3 origin, D3 direction) { /
 }
 // hittable.rs:113-122: `gen_range(0..len-1)` never picks the last light although pdf_value averages over all of
 // them (SURVEY Appendix A-2).  unbiased (YART_FLAG_UNBIASED_LIGHT_PICK): uniform over all n lights.
-YART_DEV D3 lights_random(const DevScene& S, D3 origin, double u_pick, double r1, double r2, bool unbiased) {
+YART_DEV D3 lights_random(const DevScene& S, D3 origin, double u_pick, double r1, double r2, bool unbiased, double cos_phi,
+                          double sin_phi) {
   const uint32_t n = S.n_lights;
   if (n == 0) return d3(1.0, 0.0, 0.0);
-  if (n == 1) return light_random(S.lights[0], origin, r1, r2);
-  const uint32_t m = unbiased ? n : n - 1;
-  uint32_t k = (uint32_t)(u_pick * (double)m);
-  if (k > m - 1) k = m - 1;
-  return light_random(S.lights[k], origin, r1, r2);
+  uint32_t k = 0;
+  if (n > 1) {
+    const uint32_t m = unbiased ? n : n - 1;
+    k = (uint32_t)(u_pick * (double)m);
+    if (k > m - 1) k = m - 1;
+  }
+  return light_random<true>(S.lights[k], origin, r1, r2, cos_phi, sin_phi); // (one inlined call site)
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -640,8 +653,11 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
     HitRec rec;
     world_record(S, h, wo, wd, time, rec);
     const yart_material& mat = S.materials[rec.material];
-    double emitted = 0.0;
-    if (mat.kind == YART_MAT_DIFFUSE_LIGHT) emitted = rec.front_face ? texture_value(S, mat.texture, wl, rec) : 0.0;
+    // the texture of every material that reads one (a DiffuseLight only where it emits), from one inlined call site
+    double tex = 0.0;
+    if (mat.kind != YART_MAT_NONE && mat.kind != YART_MAT_DIELECTRIC && (mat.kind != YART_MAT_DIFFUSE_LIGHT || rec.front_face))
+      tex = texture_value(S, mat.texture, wl, rec.p, rec.u, rec.v);
+    const double emitted = mat.kind == YART_MAT_DIFFUSE_LIGHT ? tex : 0.0;
     if (mat.kind == YART_MAT_NONE || mat.kind == YART_MAT_DIFFUSE_LIGHT) {
       terminal = emitted;
       if constexpr (NEE) {
@@ -651,12 +667,12 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
       D3 reflected = reflect(unit_vector(wd), rec.normal);
       next_d = reflected + mat.fuzz * random_in_unit_sphere(rng, bounce);
       next_o = rec.p;
-      thr = thr * texture_value(S, mat.texture, wl, rec);
+      thr = thr * tex;
       done = false;
     } else if (mat.kind == YART_MAT_ISOTROPIC) {
       next_d = random_in_unit_sphere(rng, bounce);
       next_o = rec.p;
-      thr = thr * texture_value(S, mat.texture, wl, rec);
+      thr = thr * tex;
       done = false;
     } else if (mat.kind == YART_MAT_DIELECTRIC) { // material.rs:213-301
       const double nidx = sellmeier_index(mat, wl);
@@ -666,12 +682,11 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
       if (ddn > 0.0) {
         outward = -rec.normal;
         ni_over_nt = nidx;
-        cosine = nidx * dot(wd, rec.normal) / length(wd);
       } else {
         outward = rec.normal;
         ni_over_nt = 1.0 / nidx;
-        cosine = -dot(wd, rec.normal) / length(wd);
       }
+      cosine = (ddn > 0.0 ? nidx * ddn : -ddn) / length(wd);
       D3 refracted;
       if (refract(wd, outward, ni_over_nt, refracted)) {
         double u0, u1;
@@ -684,23 +699,25 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
       thr = thr * 1.0;
       done = false;
     } else { // Lambertian through the mixture pdf (material.rs:44-61, main.rs:560-581)
-      const double atten = texture_value(S, mat.texture, wl, rec);
+      const double atten = tex;
       const Onb uvw = onb_from_w(rec.normal);
       double u_mix, u_pick, r1, r2;
       rng_draw(rng, bounce, YART_SLOT_MIX, u_mix, u_pick);
       rng_draw(rng, bounce, YART_SLOT_DIR, r1, r2);
       const bool have_lights = S.n_lights != 0;
+      const double phi = 2.0 * kPi * r1; // both halves of the mixture turn r1 into this angle
+      const double cos_phi = cos(phi), sin_phi = sin(phi);
       D3 dir;
       if (u_mix < 0.5 && have_lights) {
-        dir = lights_random(S, rec.p, u_pick, r1, r2, (R.flags & YART_FLAG_UNBIASED_LIGHT_PICK) != 0);
+        dir = lights_random(S, rec.p, u_pick, r1, r2, (R.flags & YART_FLAG_UNBIASED_LIGHT_PICK) != 0, cos_phi, sin_phi);
       } else { // random_cosine_direction (pdf.rs:15-25)
         const double z = sqrt(1.0 - r2);
-        const double phi = 2.0 * kPi * r1;
-        const double x = cos(phi) * sqrt(r2);
-        const double y = sin(phi) * sqrt(r2);
+        const double x = cos_phi * sqrt(r2);
+        const double y = sin_phi * sqrt(r2);
         dir = onb_local(uvw, d3(x, y, z));
       }
-      const double cosv = dot(unit_vector(dir), uvw.w);
+      const D3 udir = unit_vector(dir);
+      const double cosv = dot(udir, uvw.w);
       const double cos_pdf = cosv <= 0.0 ? 0.0 : cosv / kPi;
       const double p0 = have_lights ? lights_pdf_value(S, rec.p, dir) : cos_pdf;
       const double pdf_val = 0.5 * p0 + 0.5 * cos_pdf;
@@ -715,9 +732,10 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
           if (k > S.n_lights - 1) k = S.n_lights - 1;
           const D3 dl = light_random(S.lights[k], rec.p, s1, s2);
           const double p_l = lights_pdf_value(S, rec.p, dl);
-          const double cl = dot(unit_vector(dl), uvw.w);
+          const D3 udl = unit_vector(dl);
+          const double cl = dot(udl, uvw.w);
           const double p_m = 0.5 * p_l + 0.5 * (cl <= 0.0 ? 0.0 : cl / kPi);
-          const double csl = dot(rec.normal, unit_vector(dl));
+          const double csl = dot(rec.normal, udl);
           const double spdf_l = csl < 0.0 ? 0.0 : csl / kPi;
           if (isfinite(p_l) && p_l > 0.0 && spdf_l > 0.0) {
             store_ray(N.rays + id, rec.p, dl);
@@ -729,7 +747,7 @@ YART_DEV std::conditional_t<NEE, uint32_t, bool> shade_path(const RenderParams& 
       if (!isfinite(pdf_val) || pdf_val <= 0.0) {
         terminal = emitted;
       } else {
-        const double cs = dot(rec.normal, unit_vector(dir));
+        const double cs = dot(rec.normal, udir);
         const double spdf = cs < 0.0 ? 0.0 : cs / kPi;
         if constexpr (NEE) w_next = have_lights ? pdf_val * pdf_val / (pdf_val * pdf_val + p0 * p0) : 1.0;
         thr = thr * atten * spdf / pdf_val;
@@ -916,7 +934,7 @@ __global__ void __launch_bounds__(256) k_nee_resolve(const RenderParams R, uint3
     world_record(S, h, wo, wd, R.st.time[id], rec);
     const yart_material& mat = S.materials[rec.material];
     if (mat.kind != YART_MAT_DIFFUSE_LIGHT || !rec.front_face) continue;
-    N.sum[id] += N.pending[id] * texture_value(S, mat.texture, R.st.wavelength[id], rec);
+    N.sum[id] += N.pending[id] * texture_value(S, mat.texture, R.st.wavelength[id], rec.p, rec.u, rec.v);
   }
 }
 
