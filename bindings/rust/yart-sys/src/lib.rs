@@ -143,6 +143,10 @@ pub struct yart_render_opts {
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct yart_aov_planes { pub albedo: *mut f64, pub normal: *mut f64, pub depth: *mut f64 }
 
+/// The options of `yart_denoise`: 0 levels and sigmas <= 0 select the defaults.
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct yart_denoise_opts { pub levels: u32, pub flags: u32, pub sigma_color: f64, pub sigma_normal: f64, pub sigma_depth: f64 }
+
 #[repr(C)] #[derive(Clone, Copy)]
 pub struct yart_qbvh_info {
     pub n_nodes: u32, pub n_leaves: u32, pub n_tris: u32, pub height: u32, pub root: u32, pub max_stack: u32,
@@ -206,6 +210,9 @@ extern "C" {
                                      flags: u32, rgb: *mut f32) -> c_int;
     pub fn yart_render_aovs(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,
                             planes: *const yart_aov_planes, stats: *mut yart_stats) -> c_int;
+    pub fn yart_denoise(ctx: *mut yart_ctx, film_xyz: *const f64, spp: u32, planes: *const yart_aov_planes, width: u32,
+                        height: u32, opts: *const yart_denoise_opts, rgb: *mut f32, rgba8: *mut u8,
+                        stats: *mut yart_stats) -> c_int;
     pub fn yart_generate_camera_rays(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,
                                      rays_host: *mut yart_ray, wavelength_host: *mut f64, time_host: *mut f64) -> c_int;
     pub fn yart_dump_path_rays(ctx: *mut yart_ctx, camera: *const yart_camera, opts: *const yart_render_opts,

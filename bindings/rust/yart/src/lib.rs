@@ -3,7 +3,7 @@
 //!
 //! `GpuScene` plays the part of `world: Arc<HittableList>` (main.rs:434-446): `hit` has the shape of
 //! `Hittable::hit(&self, &Ray, t_min, t_max) -> Option<HitRecord>` (hittable.rs:24) for drop-in testing, `hit_many`
-//! is the batched form the GPU is for, `hit_records` / `hit_record` return the whole `HitRecord`, `render` replaces the tile loop of `render()` (main.rs:629-760), `render_aovs` gives a denoiser its inputs.
+//! is the batched form the GPU is for, `hit_records` / `hit_record` return the whole `HitRecord`, `render` replaces the tile loop of `render()` (main.rs:629-760), `render_aovs` gives a denoiser its inputs, `denoise` renders and denoises on the GPU.
 use std::ffi::{CStr, CString};
 use std::ptr;
 use yart_sys as sys;
@@ -207,6 +207,34 @@ impl GpuScene {
             if hits > 0.0 { out.depth[i] = (depth[i * 3] / hits) as f32; }
         }
         Ok(out)
+    }
+
+    /// `render(width, height, spp, ..)` denoised by the library's a-trous filter (`yart_denoise`, default options),
+    /// guided by the first-hit planes of samples `[0, aov_spp)`: linear RGB (`[h][w][3]` f32) and the RGBA8 image
+    /// through the same display rule as `render`.
+    pub fn denoise(&self, width: u32, height: u32, spp: u32, aov_spp: u32, max_depth: u32, seed: u64) -> Result<(Vec<f32>, Vec<u8>)> {
+        let mut cam: sys::yart_camera = unsafe { std::mem::zeroed() };
+        let rc = unsafe { sys::yart_preset_camera(self.preset, width, height, -1.0, -1.0, &mut cam) };
+        if rc != 0 { return Err(Self::global_err(rc)); }
+        let n = (width as usize) * (height as usize);
+        let mut opts = sys::yart_render_opts { width, height, sample_begin: 0, sample_end: spp, max_depth,
+                                               order: sys::YART_ORDER_NEAR, seed, ..Default::default() };
+        let mut film = vec![0f64; n * 3];
+        let (mut albedo, mut normal, mut depth) = (vec![0f64; n * 3], vec![0f64; n * 3], vec![0f64; n * 3]);
+        let (mut rgb, mut rgba) = (vec![0f32; n * 3], vec![0u8; n * 4]);
+        unsafe {
+            let rc = sys::yart_render(self.ctx, &cam, &opts, film.as_mut_ptr(), ptr::null_mut());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+            opts.sample_end = aov_spp;
+            let planes = sys::yart_aov_planes { albedo: albedo.as_mut_ptr(), normal: normal.as_mut_ptr(), depth: depth.as_mut_ptr() };
+            let rc = sys::yart_render_aovs(self.ctx, &cam, &opts, &planes, ptr::null_mut());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+            let dn = sys::yart_denoise_opts::default();
+            let rc = sys::yart_denoise(self.ctx, film.as_ptr(), spp, &planes, width, height, &dn, rgb.as_mut_ptr(),
+                                       rgba.as_mut_ptr(), ptr::null_mut());
+            if rc != 0 { return Err(self.ctx_err(rc)); }
+        }
+        Ok((rgb, rgba))
     }
 }
 

@@ -514,6 +514,43 @@ typedef struct yart_aov_planes {
 int yart_render_aovs(yart_ctx* ctx, const yart_camera* camera, const yart_render_opts* opts,
                      const yart_aov_planes* planes, yart_stats* stats /* may be NULL */);
 
+typedef struct yart_denoise_opts {
+  uint32_t levels;      /* a-trous levels L, 1..10; 0 = 5 */
+  uint32_t flags;       /* YART_FLAG_DEVICE_PTRS only */
+  double sigma_color;   /* <= 0: 8 */
+  double sigma_normal;  /* <= 0: 0.3 */
+  double sigma_depth;   /* <= 0: 0.05 */
+} yart_denoise_opts;
+
+/* A denoised image from a film and the planes of yart_render_aovs: the edge-avoiding a-trous wavelet filter of
+ * Dammertz, Sewtz, Hanika and Lensch (HPG 2010), guided by albedo, normal and distance, on the GPU.  Everything is f64
+ * in a fixed order without libm or FMA, so tests/denoise_ref.py (numpy) reproduces `rgb` bit for bit.  Per pixel p:
+ *   Prepare:  p is valid iff depth[p][2] > 0 (it has AOV samples); invalid pixels are never neighbours and output 0.
+ *     lin = the film as yart_film_finalize_linear computes it (f64, not rounded), a = albedo / depth[2],
+ *     n = normal / depth[2], hit = depth[1] > 0, z = depth[0] / depth[1] if hit, m = a + 1/128, c = lin / m
+ *     (demodulation, per channel).
+ *   Level i = 0 .. L-1, step s = 2^i: taps (dy, dx) in {-2..2}^2, row-major, at (y + dy*s, x + dx*s); taps outside the
+ *     image or at invalid pixels are skipped.  h = H[dy] * H[dx], H = {1/16, 1/4, 3/8, 1/4, 1/16}.  The centre tap has
+ *     weight h.  Another tap q is skipped if exactly one of p, q hits; else its weight is h * r(x) with
+ *       x = dc * kc + dn * kn (+ dz * dz * iz if both hit),
+ *       dc = ((c_q0-c_p0)^2 + (c_q1-c_p1)^2) + (c_q2-c_p2)^2, dn likewise for n, dz = z_q - z_p,
+ *       kc = 4^i / (sigma_color * sigma_color) (the colour term tightens by 4 per level), kn = 1 / (sigma_normal *
+ *       sigma_normal), iz = 1 / ((sigma_depth * sigma_depth * z_p) * z_p),
+ *       r(x) = (1 + x * 0.125)^-8 as t = 1 / (1 + x * 0.125); t = t * t; t = t * t; t = t * t (a stand-in for exp(-x)).
+ *     In tap order W += w, S += w * c_q; then c_p = S / W.
+ *   Finish: out = c * m (remodulation).  rgb: out rounded to f32; rgba8: yart_film_finalize's sRGB curve and clamp
+ *     applied to out, alpha 255.  Invalid pixels are 0 in both, alpha included.
+ * film_xyz: [height][width][3] f64 as yart_render fills it, with spp samples per pixel (>= 1).  planes: all three
+ * required, as yart_render_aovs fills them (any sample count; films and planes combined by yart_film_reduce are valid
+ * input, so a multi-GPU host denoises on the root).  The inputs are not modified.  opts: NULL = all defaults with host
+ * arrays.  With YART_FLAG_DEVICE_PTRS every array is a device array on ctx's GPU (f64 ones 8-byte aligned, rgb 4-byte
+ * aligned); any other flag bit is YART_ERR_INVALID, as are levels > 10, a non-finite sigma, width * height >= 2^32,
+ * spp 0 and both outputs NULL.  Scratch of 121 bytes a pixel stays on the context for the next call.
+ * stats (may be NULL): gpu_ms and kernel_launches (L + 2); the other fields are 0. */
+int yart_denoise(yart_ctx* ctx, const double* film_xyz, uint32_t spp, const yart_aov_planes* planes, uint32_t width,
+                 uint32_t height, const yart_denoise_opts* opts, float* rgb /* or NULL */, uint8_t* rgba8 /* or NULL */,
+                 yart_stats* stats /* may be NULL */);
+
 /* Camera rays exactly as the render loop generates them (main.rs:690-698, camera.rs:82-94):
  * one ray per (pixel, sample) in [sample_begin, sample_end), pixel-major.  For parity tests
  * and for dumping the ray distribution the renderer really sees. */

@@ -21,7 +21,9 @@ for scene, w, h, spp in (("david", 48, 32, 2), ("cornell-box-smoke", 32, 32, 2),
     ctx.render(cam, w, h, 0, spp, 50, 1, flags=y.FLAG_NEXT_EVENT)
     rgba = ctx.film_finalize(film, spp)
     ctx.film_finalize_linear(film, spp)  # k_film_finalize_linear
-    ctx.render_aovs(cam, w, h, 0, spp, 50, 1, batch_spp=1)  # k_aov_accumulate over every object (no tail fold)
+    planes, _ = ctx.render_aovs(cam, w, h, 0, spp, 50, 1, batch_spp=1)  # k_aov_accumulate over every object (no tail fold)
+    for levels in (1, 10):  # k_denoise_prepare / _atrous / _finish, steps past the image's edges
+        ctx.denoise(film, spp, planes, levels=levels, rgba=True)
     rays, _, times = ctx.camera_rays(cam, w, h, 0, 1)
     for order in (0, 1):
         ctx.closest_hit(rays, y.TARGET_WORLD, 0.001, float("inf"), order, count_visits=True)

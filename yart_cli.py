@@ -7,6 +7,7 @@
                        [--preview-every N] [--checkpoint FILE] [--resume]    (additions)
                        [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event]   (better sampling, off by default)
                        [--aovs [--aov-samples N]]                            (denoiser inputs)
+                       [--denoise]                                           (built-in denoiser)
 
 `--workers` is accepted for compatibility and ignored (the render runs on the GPU).  Option resolution
 follows resolve_render_options / resolve_dimensions (main.rs:166-209); the image is finalised exactly like
@@ -29,6 +30,10 @@ checkpoint's identity.
 distance of the samples that hit, 0 where none did) are the first-hit means of samples [0, --aov-samples) (default
 min(16, --samples)), the very camera samples the beauty pass started with (yart_render_aovs).  They are rendered once,
 after the beauty pass, on the first GPU, and are not part of a checkpoint.
+
+`--denoise` also writes <stem>.denoised.png and <stem>.denoised.pfm (linear RGB): the film denoised on the GPU by the
+library's own a-trous filter (yart_denoise), guided by the first-hit planes of samples [0, --aov-samples), rendered as
+for --aovs whether or not --aovs is given.  The main PNG is the same with or without it.
 """
 import argparse
 import importlib
@@ -83,6 +88,8 @@ def build_parser(scene_names):
                     help="also write <stem>.color/.albedo/.normal/.depth.pfm next to the PNG (denoiser inputs)")
     ap.add_argument("--aov-samples", type=positive_int, default=None, dest="aov_samples",
                     help="samples per pixel of the albedo / normal / depth images (default min(16, --samples))")
+    ap.add_argument("--denoise", action="store_true",
+                    help="also write <stem>.denoised.png / .denoised.pfm, denoised by yart_denoise")
     return ap
 
 
@@ -151,16 +158,27 @@ def aov_paths(output_path):
     return {k: "%s.%s.pfm" % (stem, k) for k in ("color", "albedo", "normal", "depth")}
 
 
+def denoised_paths(output_path):
+    stem = os.path.splitext(output_path)[0]
+    return {"png": stem + ".denoised.png", "pfm": stem + ".denoised.pfm"}
+
+
 def write_aovs(y, ctx, cam, o, args, order, flags, film, spp):
-    """The four denoiser inputs of --aovs; returns their paths."""
+    """The first-hit planes of samples [0, --aov-samples), then what --aovs and --denoise write from them."""
     n = args.aov_samples or min(16, spp)
     planes, _ = ctx.render_aovs(cam, o["width"], o["height"], 0, n, o["max_depth"], args.seed, order, flags=flags)
-    means = y.aov_means(planes)
-    paths = aov_paths(o["output_path"])
-    write_pfm(paths["color"], ctx.film_finalize_linear(film, spp))
-    for k in ("albedo", "normal", "depth"):
-        write_pfm(paths[k], means[k])
-    return paths
+    if args.aovs:
+        means = y.aov_means(planes)
+        paths = aov_paths(o["output_path"])
+        write_pfm(paths["color"], ctx.film_finalize_linear(film, spp))
+        for k in ("albedo", "normal", "depth"):
+            write_pfm(paths[k], means[k])
+    if args.denoise:
+        from PIL import Image
+        rgb, rgba = ctx.denoise(film, spp, planes, rgba=True)
+        paths = denoised_paths(o["output_path"])
+        write_pfm(paths["pfm"], rgb)
+        Image.fromarray(rgba, "RGBA").save(paths["png"])
 
 
 def main(argv=None):
@@ -222,7 +240,7 @@ def main(argv=None):
     if film is None:  # (resumed a finished render)
         raise SystemExit("nothing to do")
     write_png(ctx, film, total, o["output_path"])
-    if args.aovs:
+    if args.aovs or args.denoise:
         write_aovs(y, ctx, cam, o, args, order, flags, film, total)
     if multi is not None:
         multi.close()

@@ -112,6 +112,7 @@ def load_library():
         "yart_film_finalize": (i32, [vp, vp, u32, u32, u32, u32, vp]),
         "yart_film_finalize_linear": (i32, [vp, vp, u32, u32, u32, u32, vp]),
         "yart_render_aovs": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), P(abi.AovPlanes), P(abi.Stats)]),
+        "yart_denoise": (i32, [vp, vp, u32, P(abi.AovPlanes), u32, u32, P(abi.DenoiseOpts), vp, vp, P(abi.Stats)]),
         "yart_generate_camera_rays": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, vp, vp]),
         "yart_dump_path_rays": (i32, [vp, P(abi.Camera), P(abi.RenderOpts), vp, u64, P(u64)]),
         "yart_comm_unique_id": (i32, [vp]),
@@ -145,7 +146,7 @@ EXPORTED_SYMBOLS = [
     "yart_comm_destroy", "yart_comm_info", "yart_comm_last_error", "yart_film_reduce", "yart_film_create",
     "yart_film_clear", "yart_film_read", "yart_film_destroy", "yart_preset_note", "yart_closest_hit_f32",
     "yart_dump_path_rays", "yart_host_register", "yart_host_unregister", "yart_occluded", "yart_occluded_f32",
-    "yart_closest_hit_records", "yart_render_aovs", "yart_film_finalize_linear",
+    "yart_closest_hit_records", "yart_render_aovs", "yart_film_finalize_linear", "yart_denoise",
 ]
 
 
@@ -548,6 +549,32 @@ class Context:
         st = abi.Stats()
         o = self._opts(width, height, sample_begin, sample_end, max_depth, seed, order, batch_spp, FLAG_DEVICE_PTRS | flags)
         self._check(_lib.yart_render_aovs(self._h, C.byref(camera), C.byref(o), C.byref(ap), C.byref(st)))
+        return st
+
+    def denoise(self, film, spp, planes, levels=0, sigma_color=0.0, sigma_normal=0.0, sigma_depth=0.0, rgba=False):
+        """The film denoised by the a-trous filter of yart_denoise, guided by render_aovs' planes (a dict of the three
+        (H, W, 3) f64 sums).  Returns the (H, W, 3) f32 linear RGB image, and with rgba=True also the (H, W, 4) u8 image
+        through yart_film_finalize's display rule.  0 levels and sigmas <= 0 select the defaults."""
+        film = np.ascontiguousarray(film, dtype=np.float64)
+        h, w = film.shape[:2]
+        arrs = [np.ascontiguousarray(planes[k], dtype=np.float64) for k in AOV_PLANES]
+        for a in arrs:
+            assert a.shape == (h, w, 3), a.shape
+        rgb = np.empty((h, w, 3), dtype=np.float32)
+        out8 = np.empty((h, w, 4), dtype=np.uint8) if rgba else None
+        o = abi.DenoiseOpts(levels, 0, sigma_color, sigma_normal, sigma_depth)
+        self._check(_lib.yart_denoise(self._h, film.ctypes.data, spp, C.byref(abi.AovPlanes(*[a.ctypes.data for a in arrs])),
+                                      w, h, C.byref(o), rgb.ctypes.data, None if out8 is None else out8.ctypes.data, None))
+        return (rgb, out8) if rgba else rgb
+
+    def denoise_device(self, film_ptr, spp, albedo_ptr, normal_ptr, depth_ptr, width, height, rgb_ptr=None, rgba_ptr=None,
+                       levels=0, sigma_color=0.0, sigma_normal=0.0, sigma_depth=0.0):
+        """The same on device arrays (film and planes [h][w][3] f64, rgb [h][w][3] f32, rgba [h][w][4] u8; either output
+        may be None); returns the stats."""
+        st = abi.Stats()
+        o = abi.DenoiseOpts(levels, FLAG_DEVICE_PTRS, sigma_color, sigma_normal, sigma_depth)
+        self._check(_lib.yart_denoise(self._h, C.c_void_p(film_ptr), spp, C.byref(abi.AovPlanes(albedo_ptr, normal_ptr, depth_ptr)),
+                                      width, height, C.byref(o), C.c_void_p(rgb_ptr), C.c_void_p(rgba_ptr), C.byref(st)))
         return st
 
     def camera_rays(self, camera, width, height, sample_begin, sample_end, seed=1):

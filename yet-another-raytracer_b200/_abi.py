@@ -95,6 +95,11 @@ class AovPlanes(C.Structure):
     _fields_ = [("albedo", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p)]
 
 
+class DenoiseOpts(C.Structure):
+    _fields_ = [("levels", C.c_uint32), ("flags", C.c_uint32), ("sigma_color", C.c_double), ("sigma_normal", C.c_double),
+                ("sigma_depth", C.c_double)]
+
+
 class QbvhInfo(C.Structure):
     _fields_ = [("n_nodes", C.c_uint32), ("n_leaves", C.c_uint32), ("n_tris", C.c_uint32), ("height", C.c_uint32),
                 ("root", C.c_uint32), ("max_stack", C.c_uint32), ("_pad0", C.c_uint32), ("_pad1", C.c_uint32),

@@ -35,7 +35,8 @@ OBJ_DIR = PKG / "build"
 
 SOURCES = ["host_obj.cpp", "host_qbvh.cpp", "host_presets.cpp", "host_api.cpp", "yart_device.cu", "device_trace_lean.cu",
            "device_build.cu", "device_comm.cu", "device_occlude.cu"]
-HEADERS = ["host_common.h", "device_common.cuh", "device_trace.cuh", "device_shade.cuh", "device_build.h", "device_occlude.h"]
+HEADERS = ["host_common.h", "device_common.cuh", "device_trace.cuh", "device_shade.cuh", "device_denoise.cuh", "device_build.h",
+           "device_occlude.h"]
 INCLUDES = ["yart.h", "yart_rng.h", "yart_spectral_tables.h"]
 
 COMPILE_FLAGS = [

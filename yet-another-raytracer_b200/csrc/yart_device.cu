@@ -1,6 +1,6 @@
 // yart_device.cu -- the device half of the C ABI (include/yart.h): context, scene upload,
 // yart_closest_hit, yart_closest_hit_records, yart_occluded, yart_render, yart_render_aovs, yart_film_finalize(_linear),
-// yart_generate_camera_rays.
+// yart_denoise, yart_generate_camera_rays.
 //
 // There is no CPU fallback anywhere in this file: every entry point launches the sm_100a
 // kernels of device_trace.cuh / device_shade.cuh or fails with YART_ERR_CUDA.
@@ -17,6 +17,7 @@
 
 #include "../../include/yart_spectral_tables.h"
 #include "device_build.h"
+#include "device_denoise.cuh"
 #include "device_occlude.h"
 #include "device_shade.cuh"
 #include "host_common.h"
@@ -400,7 +401,10 @@ struct yart_ctx {
   DevBuf nee[5]; // YART_FLAG_NEXT_EVENT's per-path state, as kNeeBytes lists it
   DevBuf occluded; // staging of yart_occluded's flags for host arrays
   DevBuf ray_times; // staging of yart_closest_hit_records' ray times for host arrays
-  DevBuf aov[3];    // staging of yart_render_aovs' host planes
+  DevBuf aov[3];    // staging of yart_render_aovs' and yart_denoise's host planes
+  // yart_denoise's scratch (device_denoise.cuh): colour ping-pong, guides, remodulation factors, flags; and the
+  // staging of a host rgb output (a host rgba8 output stages in `rgba`)
+  DevBuf dn_color[2], dn_guide, dn_mod, dn_flags, dn_rgb;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::vector<cudaEvent_t> ev_pool;
   // host-buffer closest-hit queries: copy streams + events of the chunk pipeline (made on first use)
@@ -1894,6 +1898,101 @@ int yart_render_aovs(yart_ctx* ctx, const yart_camera* cam, const yart_render_op
   YART_ABI_GUARD_BEGIN
   return render_aovs_impl(ctx, cam, o, planes, stats);
   YART_ABI_GUARD_END(ctx, "yart_render_aovs")
+}
+
+// k_denoise_prepare, `levels` k_denoise_atrous ping-ponging ctx->dn_color, k_denoise_finish; host arrays are staged
+// through ctx->film, ctx->aov, ctx->dn_rgb and ctx->rgba.
+static int denoise_impl(yart_ctx* ctx, const double* film_xyz, uint32_t spp, const yart_aov_planes* planes, uint32_t width,
+                        uint32_t height, const yart_denoise_opts* opts, float* rgb, uint8_t* rgba8, yart_stats* stats) {
+  const yart_denoise_opts dflt = {0, 0, 0.0, 0.0, 0.0};
+  const yart_denoise_opts& op = opts ? *opts : dflt;
+  const double sig_in[3] = {op.sigma_color, op.sigma_normal, op.sigma_depth};
+  bool finite = true;
+  for (double s : sig_in) finite = finite && std::isfinite(s);
+  if (!film_xyz || !planes || !planes->albedo || !planes->normal || !planes->depth || (!rgb && !rgba8) || !width ||
+      !height || (uint64_t)width * height > 0xFFFFFFFFull || !spp || op.levels > 10 || (op.flags & ~YART_FLAG_DEVICE_PTRS) ||
+      !finite) {
+    ctx->err = "yart_denoise: bad argument";
+    return YART_ERR_INVALID;
+  }
+  const bool dev = (op.flags & YART_FLAG_DEVICE_PTRS) != 0;
+  const double* user[4] = {film_xyz, planes->albedo, planes->normal, planes->depth};
+  if (dev) {
+    bool aligned = (reinterpret_cast<uintptr_t>(rgb) & 3u) == 0;
+    for (const double* p : user) aligned = aligned && (reinterpret_cast<uintptr_t>(p) & 7u) == 0;
+    if (!aligned) {
+      ctx->err = "yart_denoise: device arrays must be aligned to their element size";
+      return YART_ERR_INVALID;
+    }
+  }
+  const uint32_t levels = op.levels ? op.levels : 5;
+  const double sc = op.sigma_color > 0.0 ? op.sigma_color : 8.0;
+  const double sn = op.sigma_normal > 0.0 ? op.sigma_normal : 0.3;
+  const double sz = op.sigma_depth > 0.0 ? op.sigma_depth : 0.05;
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (stats) memset(stats, 0, sizeof(*stats));
+  const uint32_t n = width * height;
+  const size_t film_bytes = (size_t)n * 3 * sizeof(double);
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  const double* d_in[4];
+  for (int k = 0; k < 4; ++k) {
+    d_in[k] = user[k];
+    if (dev) continue;
+    DevBuf& stage = k == 0 ? ctx->film : ctx->aov[k - 1];
+    CUDA_TRY(ctx, stage.reserve(film_bytes));
+    CUDA_TRY(ctx, cudaMemcpyAsync(stage.p, user[k], film_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    d_in[k] = stage.as<double>();
+  }
+  float* d_rgb = rgb;
+  uint8_t* d_rgba = rgba8;
+  if (!dev && rgb) {
+    CUDA_TRY(ctx, ctx->dn_rgb.reserve((size_t)n * 3 * sizeof(float)));
+    d_rgb = ctx->dn_rgb.as<float>();
+  }
+  if (!dev && rgba8) {
+    CUDA_TRY(ctx, ctx->rgba.reserve((size_t)n * 4));
+    d_rgba = ctx->rgba.as<uint8_t>();
+  }
+  for (DevBuf& b : ctx->dn_color) CUDA_TRY(ctx, b.reserve((size_t)n * 4 * sizeof(double)));
+  CUDA_TRY(ctx, ctx->dn_guide.reserve((size_t)n * 4 * sizeof(double)));
+  CUDA_TRY(ctx, ctx->dn_mod.reserve(film_bytes));
+  CUDA_TRY(ctx, ctx->dn_flags.reserve(n));
+  const uint8_t* flags = ctx->dn_flags.as<uint8_t>();
+  const int stream_grid = ctx->sm_count * 8;
+  k_denoise_prepare<<<stream_grid, 256, 0, ctx->stream>>>(d_in[0], spp, d_in[1], d_in[2], d_in[3], n,
+                                                          ctx->dn_flags.as<uint8_t>(), ctx->dn_color[0].as<double>(),
+                                                          ctx->dn_guide.as<double>(), ctx->dn_mod.as<double>());
+  CUDA_TRY(ctx, cudaGetLastError());
+  const dim3 block(kDenoiseTileX, kDenoiseTileY);
+  const dim3 grid((width + kDenoiseTileX - 1) / kDenoiseTileX, std::min<uint32_t>((height + kDenoiseTileY - 1) / kDenoiseTileY, 65535u));
+  for (uint32_t i = 0; i < levels; ++i) {
+    const double kc = std::ldexp(1.0, 2 * (int)i) / (sc * sc);
+    k_denoise_atrous<<<grid, block, 0, ctx->stream>>>(flags, ctx->dn_guide.as<double>(), ctx->dn_color[i & 1].as<double>(),
+                                                      ctx->dn_color[(i + 1) & 1].as<double>(), width, height, 1u << i, kc,
+                                                      1.0 / (sn * sn), sz * sz);
+    CUDA_TRY(ctx, cudaGetLastError());
+  }
+  k_denoise_finish<<<stream_grid, 256, 0, ctx->stream>>>(flags, ctx->dn_color[levels & 1].as<double>(),
+                                                         ctx->dn_mod.as<double>(), n, d_rgb, d_rgba);
+  CUDA_TRY(ctx, cudaGetLastError());
+  if (!dev && rgb) CUDA_TRY(ctx, cudaMemcpyAsync(rgb, d_rgb, (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  if (!dev && rgba8) CUDA_TRY(ctx, cudaMemcpyAsync(rgba8, d_rgba, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  if (!stats) return YART_OK;
+  float ms = 0.f;
+  CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+  stats->gpu_ms = ms;
+  stats->kernel_launches = levels + 2;
+  return YART_OK;
+}
+
+int yart_denoise(yart_ctx* ctx, const double* film_xyz, uint32_t spp, const yart_aov_planes* planes, uint32_t width,
+                 uint32_t height, const yart_denoise_opts* opts, float* rgb, uint8_t* rgba8, yart_stats* stats) {
+  if (!ctx) return YART_ERR_INVALID;
+  YART_ABI_GUARD_BEGIN
+  return denoise_impl(ctx, film_xyz, spp, planes, width, height, opts, rgb, rgba8, stats);
+  YART_ABI_GUARD_END(ctx, "yart_denoise")
 }
 
 int yart_generate_camera_rays(yart_ctx* ctx, const yart_camera* cam, const yart_render_opts* o, yart_ray* rays_host,

@@ -10,7 +10,8 @@
 // Additions: --seed S (the reference is OS-seeded), --device D, --gpus N (N GPUs of this box: one host thread per
 // context, yart_comm_init + yart_film_reduce = one in-place ncclReduce of the f64 film), --order near|reference,
 // --unbiased-light-pick / --russian-roulette / --depth-zero-black / --next-event (better sampling, OFF by default), --assets DIR,
-// --aovs [--aov-samples N] (denoiser inputs next to the PNG, as yart_cli.py writes them), --dry-run (print the
+// --aovs [--aov-samples N] (denoiser inputs next to the PNG, as yart_cli.py writes them), --denoise (<stem>.denoised.png
+// and .pfm from yart_denoise, guided by the same first-hit planes), --dry-run (print the
 // resolved options as one JSON line and exit: what the reference's unit tests check, main.rs:868-915), --list-scenes.  `--workers` is accepted and ignored.  There is no CPU mode.
 //
 // build (build.py does this): g++ -std=c++17 -O2 -Iinclude host/yart_main.cpp -o yart -L. -lyart_b200 -Wl,-rpath,'$ORIGIN' -pthread
@@ -122,7 +123,7 @@ struct Cli {
   int device = 0, gpus = 1;
   uint32_t flags = 0;
   bool dry_run = false, list_scenes = false;
-  bool aovs = false;
+  bool aovs = false, denoise = false;
   uint32_t aov_samples = 0; // 0 = min(16, samples)
 };
 
@@ -130,7 +131,7 @@ struct Cli {
   fprintf(stderr, "error: %s\n\nUsage: yart --scene <SCENE> [--output <OUTPUT>] [--width <WIDTH>] [--height <HEIGHT>] "
                   "[--samples <SAMPLES>] [--max-depth <MAX_DEPTH>] [--workers <WORKERS>] [--vfov <VFOV>] [--aperture <APERTURE>]\n"
                   "            [--seed S] [--device D] [--gpus N] [--order near|reference] [--assets DIR] [--dry-run] [--list-scenes]\n"
-                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event] [--aovs] [--aov-samples N]\n",
+                  "            [--unbiased-light-pick] [--russian-roulette] [--depth-zero-black] [--next-event] [--aovs] [--aov-samples N] [--denoise]\n",
           msg.c_str());
   exit(2);
 }
@@ -186,6 +187,7 @@ Cli parse(int argc, char** argv) {
     else if (a == "--depth-zero-black") c.flags |= YART_FLAG_DEPTH_ZERO_BLACK;
     else if (a == "--next-event") c.flags |= YART_FLAG_NEXT_EVENT;
     else if (a == "--aovs") c.aovs = true;
+    else if (a == "--denoise") c.denoise = true;
     else if (a == "--aov-samples") c.aov_samples = positive("--aov-samples", value());
     else if (a == "--dry-run") c.dry_run = true;
     else if (a == "--list-scenes") c.list_scenes = true;
@@ -316,11 +318,8 @@ int main(int argc, char** argv) {
     fprintf(stderr, "yart: cannot write %s\n", output.c_str());
     return 1;
   }
-  if (cli.aovs) { // denoiser inputs next to the PNG: linear colour + first-hit means of samples [0, aov_samples)
+  if (cli.aovs || cli.denoise) { // first-hit planes of samples [0, aov_samples) on the root, after the reduce
     const size_t np = (size_t)width * height;
-    std::vector<float> color(np * 3), albedo(np * 3), normal(np * 3), depth(np);
-    if (yart_film_finalize_linear(ctxs[0], film.data(), width, height, spp, 0, color.data()) != YART_OK)
-      return die("yart_film_finalize_linear", ctxs[0]);
     std::vector<double> pa(np * 3, 0.0), pn(np * 3, 0.0), pd(np * 3, 0.0);
     yart_aov_planes planes = {pa.data(), pn.data(), pd.data()};
     yart_render_opts o;
@@ -333,21 +332,36 @@ int main(int argc, char** argv) {
     o.flags = cli.flags;
     o.seed = cli.seed;
     if (yart_render_aovs(ctxs[0], &cam, &o, &planes, nullptr) != YART_OK) return die("yart_render_aovs", ctxs[0]);
-    for (size_t i = 0; i < np; ++i) { // the means of aov_means() in the Python package
-      const double n = pd[i * 3 + 2], hits = pd[i * 3 + 1];
-      for (int k = 0; k < 3; ++k) {
-        albedo[i * 3 + k] = n > 0 ? (float)(pa[i * 3 + k] / n) : 0.f;
-        normal[i * 3 + k] = n > 0 ? (float)(pn[i * 3 + k] / n) : 0.f;
-      }
-      depth[i] = hits > 0 ? (float)(pd[i * 3] / hits) : 0.f;
-    }
     const std::string stem = (std::filesystem::path(output).parent_path() / std::filesystem::path(output).stem()).string();
-    const struct { const char* name; const std::vector<float>& px; int ch; } files[] = {
-        {"color", color, 3}, {"albedo", albedo, 3}, {"normal", normal, 3}, {"depth", depth, 1}};
-    for (const auto& f : files) {
-      const std::string path = stem + "." + f.name + ".pfm";
-      if (!write_pfm(path, f.px, width, height, f.ch)) {
-        fprintf(stderr, "yart: cannot write %s\n", path.c_str());
+    if (cli.aovs) { // denoiser inputs next to the PNG: linear colour + first-hit means
+      std::vector<float> color(np * 3), albedo(np * 3), normal(np * 3), depth(np);
+      if (yart_film_finalize_linear(ctxs[0], film.data(), width, height, spp, 0, color.data()) != YART_OK)
+        return die("yart_film_finalize_linear", ctxs[0]);
+      for (size_t i = 0; i < np; ++i) { // the means of aov_means() in the Python package
+        const double n = pd[i * 3 + 2], hits = pd[i * 3 + 1];
+        for (int k = 0; k < 3; ++k) {
+          albedo[i * 3 + k] = n > 0 ? (float)(pa[i * 3 + k] / n) : 0.f;
+          normal[i * 3 + k] = n > 0 ? (float)(pn[i * 3 + k] / n) : 0.f;
+        }
+        depth[i] = hits > 0 ? (float)(pd[i * 3] / hits) : 0.f;
+      }
+      const struct { const char* name; const std::vector<float>& px; int ch; } files[] = {
+          {"color", color, 3}, {"albedo", albedo, 3}, {"normal", normal, 3}, {"depth", depth, 1}};
+      for (const auto& f : files) {
+        const std::string path = stem + "." + f.name + ".pfm";
+        if (!write_pfm(path, f.px, width, height, f.ch)) {
+          fprintf(stderr, "yart: cannot write %s\n", path.c_str());
+          return 1;
+        }
+      }
+    }
+    if (cli.denoise) { // the library's a-trous denoiser with its defaults: <stem>.denoised.png / .pfm
+      std::vector<float> rgb(np * 3);
+      std::vector<uint8_t> rgba_dn(np * 4);
+      if (yart_denoise(ctxs[0], film.data(), spp, &planes, width, height, nullptr, rgb.data(), rgba_dn.data(), nullptr) != YART_OK)
+        return die("yart_denoise", ctxs[0]);
+      if (!write_pfm(stem + ".denoised.pfm", rgb, width, height, 3) || !write_png(stem + ".denoised.png", rgba_dn.data(), width, height)) {
+        fprintf(stderr, "yart: cannot write %s.denoised.png / .pfm\n", stem.c_str());
         return 1;
       }
     }
